@@ -19,6 +19,8 @@ network outputs (SURVEY.md §8d), excluding the three network passes. Rank 0 pri
 cfg5 (configs[4]) is the mIoU evaluation sweep: 10 000 label maps sharded over the ranks, one int64
 confusion-matrix all-reduce per sweep; a "step" is one sweep (strong scaling).
 `--impl reference` times the CPU port alone on the full batch, same metric/config.
+`--dump-outputs DIR` writes what the last timed step returned as DIR/<name>.npy (see dump_outputs), so
+that two builds run with the same arguments (hence the same seeded inputs) can be compared output for output.
 """
 from __future__ import annotations
 
@@ -64,6 +66,30 @@ def config_dict(wl) -> dict:
 def eval_config_dict(ew) -> dict:
     return {"workload": ew.name, "maps": ew.maps, "classes": ew.C, "image": [ew.H, ew.W],
             "l2": "no flush: the resident maps cycled per sweep exceed the 126 MB L2"}
+
+
+DUMP_MAX_ELEMS = 1 << 19       # per array; 13 arrays of float64 at most stay under 64 MB
+DUMP_BUDGET = 64 << 20
+
+
+def dump_outputs(out_dir, arrays: dict) -> None:
+    """Write each tensor as <out_dir>/<name>.npy: float64 for 64-bit and int32 sources, float32 otherwise.
+    A tensor of more than DUMP_MAX_ELEMS elements is replaced by the flattened elements at DUMP_MAX_ELEMS
+    sorted indices drawn from a generator seeded with 0, so every run with the same shapes samples alike."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = torch.randint(t.numel(), (DUMP_MAX_ELEMS,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        wide = t.dtype in (torch.float64, torch.int64, torch.int32)
+        a = t.cpu().numpy().astype(np.float64 if wide else np.float32)
+        total += a.nbytes
+        if total > DUMP_BUDGET:
+            raise RuntimeError(f"--dump-outputs: more than {DUMP_BUDGET >> 20} MB at {name}")
+        np.save(d / f"{name}.npy", a)
 
 
 class ClockSampler:
@@ -323,12 +349,18 @@ def run_ours(args, wl, rank, world, local_rank):
     ev0.record()
     for k in range(args.steps):
         step.ema_events = ema_pairs[k]
-        one(warmup + k + 1)
+        out = one(warmup + k + 1)
     ev1.record()
     barrier()
     t_wall1 = time.time()
     clocks = sampler.stop(t_wall0, t_wall1)
     step.ema_events = None
+    if args.dump_outputs and rank == 0:
+        # before the EMA launches below move the teacher on: it is the step's in-place output
+        out = {k: v for k, v in out.items() if v is not None}
+        out["teacher"] = torch.cat([p.reshape(-1) for p in teacher])
+        dump_outputs(args.dump_outputs, out)
+        del out
     ms = ev0.elapsed_time(ev1)
     try:
         ema_overlapped_ms = statistics.mean(a.elapsed_time(b) for a, b in ema_pairs)
@@ -526,6 +558,8 @@ def run_eval_ours(args, ew, rank, world, local_rank):
     ev1.record()
     barrier()
     clocks = sampler.stop(t0, time.time())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"confusion": meter.conf})
     ms = ev0.elapsed_time(ev1)
     n_launch = launches[0]
     total = int(meter.conf.sum())
@@ -612,7 +646,13 @@ def main():
     ap.add_argument("--eval-resident", type=int, default=64, help="cfg5: distinct maps kept in HBM per GPU")
     ap.add_argument("--eval-e2e-maps", type=int, default=64, help="cfg5: maps per rank per e2e step")
     ap.add_argument("--ref-eval-maps", type=int, default=64, help="cfg5: maps per step of the CPU arms")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (rank 0; GPU arm only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs; it does not apply to --impl reference")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

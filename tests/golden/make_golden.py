@@ -1,9 +1,15 @@
 """Generate the committed golden fixtures from the REFERENCE code itself.
 
-Run in the build container (needs /root/reference): `python tests/golden/make_golden.py`.
+Needs a checkout of the reference named by PFST_REFERENCE: `python tests/golden/make_golden.py`.
 Every fixture stores the (small) inputs and the outputs the reference produced for
 them, so that tests can pin (a) the oracle and (b) the CUDA path against the
-reference on machines where the reference checkout does not exist (the GPU box).
+reference on machines where the reference checkout does not exist.
+
+reference_live.npz is the exception: `python tests/golden/make_golden.py reference_live` records
+the oracle's outputs on the inputs of the live comparisons in test_oracle_pins.py and
+test_host_logic.py, at a commit where each of those comparisons had passed bit for bit against the
+reference checkout. Those tests compare against it everywhere, and against the reference itself
+when PFST_REFERENCE is set.
 
   metrics.npz      rsiseg/core/evaluation/metrics.py  eval_metrics / intersect_and_union
   ema.npz          PFGST._init_ema_weights / _update_ema      (pfgst.py:105-127)
@@ -490,7 +496,126 @@ def gen_offline_labels():
     np.savez_compressed(OUT / "offline_labels.npz", **out)
 
 
+def strong_aug_digest(img):
+    import hashlib
+    return hashlib.sha256(np.ascontiguousarray(img).tobytes()).hexdigest()
+
+
+def live_eval_logits_inputs(seed, N, C, H, W):
+    g = torch.Generator().manual_seed(seed)
+    logits = teacher_logits(N, C, H, W, g)
+    logits[0, :, 0, 0] = 1.5            # exact tie -> first index
+    logits[0, 0, 0, 1] = float("nan")   # NaN -> softmax all NaN -> index 0
+    gt = torch.randint(0, C + 1, (N, H, W), generator=g).to(torch.uint8)
+    gt[:, :2] = 255
+    return logits, gt
+
+
+LIVE_EVAL_CASES = [(2, 6, 32, 32), (1, 19, 17, 23), (2, 2, 8, 12)]
+LIVE_THRESHOLD_CASES = [(2, 6, 32, 32, 0.5), (1, 33, 24, 24, 1.0), (2, 3, 17, 9, 0.3)]
+LIVE_FEAT_DIST_SHAPES = [(2, 16, 8, 8), (1, 512, 5, 7), (3, 4, 15, 15)]
+
+
+def gen_reference_live():
+    """What the live comparisons of test_oracle_pins.py / test_host_logic.py check the oracle
+    against, on their own inputs (see the module doc-string for where the values come from)."""
+    from oracle import class_thresholds as OT, metrics as om, mixing as omix, offline_labels as OLB
+    from oracle import pfgst_loss as OL, prototypes as OP, strong_aug as SA
+    from pfst_b200.synthetic import WORKLOADS, step_inputs
+    out = {}
+    # test_class_draw_reproduces_reference_get_class_masks
+    g = torch.Generator().manual_seed(0)
+    labels = torch.randint(0, 6, (3, 1, 16, 16), generator=g)
+    labels[0, 0, :2] = 255
+    np.random.seed(42)
+    out["class_draw_masks"] = torch.cat(omix.class_masks(labels)).numpy().astype(np.uint8)
+    # test_reference_golden_test_retargeted
+    o59 = om.eval_metrics(np.array([np.repeat(31, 59)]), np.array([np.arange(59)]), 59, 255, metrics='mIoU')
+    out["retargeted_IoU59"] = np.asarray(o59["IoU"])
+    # test_oracle_bitwise_equals_reference_live
+    inp = step_inputs(WORKLOADS["tiny"], seed=99)
+    np.random.seed(11)
+    masks = omix.class_masks(inp["gt"])
+    out["tiny_mix"] = torch.cat(masks).numpy().astype(np.uint8)
+    t = dict(logits_trg=inp['logits_trg'].clone().requires_grad_(True), logits_ema=None, gt_src=inp['gt'],
+             x_ema=inp['x_ema'], x_src=inp['x_src'].clone().requires_grad_(True), img_trg=None,
+             mix_masks=torch.cat(masks, 0))
+    res = OL.pfgst_loss(t, OL.LossCfg())
+    sum(res[k] for k in OL.LOSS_KEYS).backward()
+    out["tiny_losses"] = np.array([float(res[k].detach()) for k in OL.LOSS_KEYS], dtype=np.float32)
+    out["tiny_grad_x_src"] = t['x_src'].grad.numpy()
+    out["tiny_grad_logits"] = t['logits_trg'].grad.numpy()
+    # test_class_threshold_oracle_equals_reference_live
+    for seed, (B, C, H, W, ratio) in enumerate(LIVE_THRESHOLD_CASES):
+        logits = teacher_logits(B, C, H, W, torch.Generator().manual_seed(seed))
+        thr = OT.cal_threshold(logits, ratio, [0.1, 0.5, 0.9], np.random.RandomState(seed))
+        for k, v in thr.items():
+            out[f"threshold_{seed}_{k}"] = np.asarray(v, dtype=np.float64)
+    # test_masked_feat_dist_equals_reference_live
+    g = torch.Generator().manual_seed(21)
+    for i, (B, D, h, w) in enumerate(LIVE_FEAT_DIST_SHAPES):
+        f1 = torch.randn((B, D, h, w), generator=g).requires_grad_(True)
+        f2 = torch.randn((B, D, h, w), generator=g)
+        mask = torch.rand((B, 1, h, w), generator=g) > 0.4
+        for j, m in enumerate((None, mask)):
+            d = OP.masked_feat_dist(f1, f2, m)
+            d.backward()
+            out[f"feat_dist_{i}_{j}"], out[f"feat_dist_{i}_{j}_grad"] = d.detach().numpy(), f1.grad.numpy().copy()
+            f1.grad = None
+    # test_offline_labels_oracle_equals_reference_live
+    g = torch.Generator().manual_seed(11)
+    feats = [[torch.relu(torch.randn((10, 9, 14), generator=g))] for _ in range(2)]
+    lds = [OLB.cal_loc_dis(f, 3, [1, 3]) for f in feats]
+    for i, ld in enumerate(lds):
+        for k, v in ld.items():
+            out[f"offline_locdis_{i}_{k}"] = v.numpy()
+    for k, v in OLB.cal_sigmas(lds, [0], [1, 3], 0.7, 0.8, np.random.RandomState(5)).items():
+        out[f"offline_sigma_{k}"] = np.float64(v)
+    logits = (2 * torch.randn((5, 9, 7), generator=g)).numpy()
+    logits[1, 2, 3] = np.nan
+    thres = np.array([0.5, 1.0, 0.2, 0.0, 0.9], dtype=np.float32)
+    for rz in (False, True):
+        out[f"offline_loader_{int(rz)}"] = OLB.loader_pseudo_labels(logits, thres, rz)
+    # test_eval_logits_oracle_equals_reference_live
+    for seed, (N, C, H, W) in enumerate(LIVE_EVAL_CASES):
+        logits, gt = live_eval_logits_inputs(seed, N, C, H, W)
+        out[f"eval_{seed}_pred"] = om.seg_argmax(logits).numpy().astype(np.uint8)
+        out[f"eval_{seed}_areas"] = np.stack([np.stack([a.numpy() for a in t])
+                                              for t in om.pre_eval(logits, list(gt.numpy()), C, 255)])
+    # test_strong_aug_oracle_equals_reference_class_live: digests keep the 60 images small
+    rs = np.random.RandomState(5)
+    digests, after = [], []
+    for it in range(60):
+        H, W = [(64, 64), (33, 47), (120, 120), (16, 100)][it % 4]
+        img = rs.randint(0, 256, (H, W, 3)).astype(np.uint8)
+        np.random.seed(it)
+        ops_ = SA.draw_strong_aug(np.random, 20, (0.7, 1.3), (0.4, 1.6), 10)
+        after.append(np.random.random())
+        digests.append(strong_aug_digest(SA.apply_strong_aug(img.copy(), ops_)))
+    out["strong_aug_sha256"], out["strong_aug_after"] = np.array(digests), np.array(after)
+    # test_slide_inference_oracle_equals_reference_live (inputs: the fixture's plus 0.25)
+    for case in slide_cases():
+        name, B, C, H, W, mode, crop, stride, flip, direction, ori, seed = case
+        img = torch.randn((B, 3, H, W), generator=torch.Generator().manual_seed(900 + seed)) + 0.25
+        o, _ = om.inference(synthetic_encode_decode(C), img, slide_meta(flip, direction, ori, B), True, mode, crop,
+                            stride, C)
+        out[f"slide_{name}"] = o.numpy()
+    # test_aug_test_oracle_vs_golden_and_reference (inputs: the fixture's, scaled and shifted)
+    for case in aug_cases():
+        name, B, C, ori, mode, crop, stride, augs, seed = case
+        imgs, metas = aug_inputs(case)
+        pred, _ = om.aug_test(synthetic_encode_decode(C), [im * 0.5 + 0.1 for im in imgs], metas, True, mode, crop,
+                              stride, C)
+        out[f"aug_{name}_pred"] = np.stack(pred).astype(np.uint8)
+    np.savez_compressed(OUT / "reference_live.npz", **out)
+
+
 if __name__ == "__main__":
+    if len(sys.argv) > 1 and sys.argv[1] == "reference_live":
+        warnings.filterwarnings("ignore")
+        torch.set_num_threads(1)
+        gen_reference_live()
+        sys.exit(0)
     if len(sys.argv) > 1 and sys.argv[1] == "offline_labels":
         gen_offline_labels()
         sys.exit(0)

@@ -1,9 +1,9 @@
 """Load the reference's hot-path modules BY FILE PATH from a read-only checkout.
 
-Only usable where the reference checkout exists (the build container:
-/root/reference). Used by make_golden.py to produce the committed fixtures and by
-the `-m "not gpu"` pinning tests, which skip when the checkout is absent (it is
-absent on the GPU box). Nothing is copied: the files are executed where they lie
+Only usable where PFST_REFERENCE names a checkout of the reference. Used by
+make_golden.py to produce the committed fixtures and by the `-m "not gpu"` pinning
+tests, which then also compare the oracle with the reference live (without it they
+compare with the committed fixtures only). Nothing is copied: the files are executed where they lie
 with small import stubs for packages that are not installed here (mmcv,
 matplotlib, timm, the rsiseg package __init__ that asserts an mmcv version).
 SURVEY.md Appendix D is the recipe.
@@ -16,11 +16,11 @@ import sys
 import types
 from pathlib import Path
 
-REF_ROOT = Path(os.environ.get("PFST_REFERENCE", "/root/reference"))
+REF_ROOT = Path(os.environ["PFST_REFERENCE"]) if os.environ.get("PFST_REFERENCE") else None
 
 
 def available() -> bool:
-    return (REF_ROOT / "rsiseg" / "models" / "uda" / "pfgst.py").exists()
+    return REF_ROOT is not None and (REF_ROOT / "rsiseg" / "models" / "uda" / "pfgst.py").exists()
 
 
 def _load(name: str, rel: str):

@@ -56,6 +56,32 @@ def test_both_arms_describe_the_workload_with_the_same_config_dict():
     assert bench.eval_config_dict(EVAL_WORKLOADS["cfg5"])["maps"] == 10000
 
 
+def test_dump_outputs_writes_float_arrays_and_samples_large_ones_alike(tmp_path):
+    """--dump-outputs: every array lands as float32/float64 .npy; a large one is replaced by the same
+    seeded sample on every call, so two runs of two builds can be compared element for element."""
+    sys.path.insert(0, str(ROOT))
+    import numpy as np
+    import bench
+    big = torch.arange(bench.DUMP_MAX_ELEMS + 12345, dtype=torch.int64)
+    arrays = {"loss": torch.tensor([1.5, 2.5]), "label": torch.tensor([[0, 3], [255, 7]], dtype=torch.uint8),
+              "big": big}
+    for d in (tmp_path / "a", tmp_path / "b"):
+        bench.dump_outputs(d, arrays)
+    a = {p.stem: np.load(p) for p in (tmp_path / "a").glob("*.npy")}
+    assert sorted(a) == ["big", "label", "loss"]
+    assert a["loss"].dtype == np.float32 and a["label"].dtype == np.float32 and a["big"].dtype == np.float64
+    assert np.array_equal(a["label"], [[0, 3], [255, 7]])
+    assert a["big"].shape == (bench.DUMP_MAX_ELEMS,) and np.all(np.diff(a["big"]) >= 0)
+    assert np.array_equal(a["big"], np.load(tmp_path / "b" / "big.npy"))
+
+
+def test_steps_below_one_and_dumps_of_the_reference_arm_are_rejected():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        out = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--workload", "tiny", *extra],
+                             capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert out.returncode == 2 and "error" in out.stderr, extra
+
+
 def test_eval_sweep_reference_arm():
     out = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0",
                           "--workload", "tiny_eval"], capture_output=True, text=True, timeout=600, cwd=ROOT)
