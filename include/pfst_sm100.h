@@ -11,7 +11,9 @@
  *   - plain pointers and sizes only; all data pointers are DEVICE pointers on
  *     the current CUDA device unless the parameter comment says "host";
  *   - tensors are dense, row-major, in the reference's layouts (NCHW logits /
- *     features, (B,1,H,W) int64 label maps);
+ *     features, (B,1,H,W) int64 label maps); every entry point that takes label maps has a
+ *     `_lbl` sibling that takes them as void* plus an int32 label_dtype tag, PFST_DT_I64 or
+ *     PFST_DT_U8 (the dtype datasets store); one call's label maps share that dtype;
  *   - `stream` is a cudaStream_t passed as void*; work is enqueued
  *     asynchronously on it; nothing here synchronises the device, allocates
  *     device memory or throws;
@@ -127,6 +129,14 @@ int pfst_pseudo_label(const float* logits, int64_t B, int32_t C, int64_t HW,
                       float thr, const float* thr_per_class, int32_t mode,
                       int64_t reject_label, int64_t* label, float* conf,
                       float* weight_part, unsigned long long* count, void* stream);
+/* pfst_pseudo_label with the label map in label_dtype (PFST_DT_I64 or PFST_DT_U8; anything else
+ * returns PFST_ERR_UNSUPPORTED). Same rule, pfgst.py:259-266 / loading.py:474-487; with PFST_DT_U8 the
+ * labels are written as uint8, which needs C <= 255 and reject_label <= 255 (a negative value
+ * means no rejection, as above; otherwise PFST_ERR_UNSUPPORTED).                                                              */
+int pfst_pseudo_label_lbl(const float* logits, int64_t B, int32_t C, int64_t HW, float thr,
+                          const float* thr_per_class, int32_t mode, int64_t reject_label,
+                          void* label, int32_t label_dtype, float* conf, float* weight_part,
+                          unsigned long long* count, void* stream);
 
 /* Self-test of the kernel's hand-scheduled exp: *mismatches = number of x[i]
  * (x[i] <= 0) for which it differs bitwise from CUDA's expf. Must be 0.       */
@@ -150,6 +160,10 @@ int pfst_pseudo_weight_fill(float* weight, int64_t B, int64_t H, int64_t W,
  * set non-zero if any label lies outside [0,255]. Zeroed here.                  */
 int pfst_class_presence(const int64_t* gt, int64_t n, uint32_t* presence,
                         void* stream);
+/* pfst_class_presence for a gt of label_dtype (PFST_DT_I64 or PFST_DT_U8, else PFST_ERR_UNSUPPORTED):
+ * torch.unique of dacs_transforms.py:113. A uint8 map never sets word 8.                         */
+int pfst_class_presence_lbl(const void* gt, int32_t label_dtype, int64_t n, uint32_t* presence,
+                            void* stream);
 
 /* chosen: device uint32[B*8], per-image bitmask of the classes drawn by the
  * host RNG (np.random.choice, :115-117).
@@ -167,6 +181,14 @@ int pfst_class_mix(const int64_t* gt, const uint32_t* chosen, const float* img,
                    int64_t B, int32_t img_channels, int64_t H, int64_t W,
                    float* mixed_img, int64_t* mixed_lbl, float* mixed_weight,
                    int64_t* mix_mask, void* stream);
+/* pfst_class_mix (dacs_transforms.py:122-144, pfgst.py:287-300) with gt, pseudo_label, mixed_lbl and
+ * mix_mask all of label_dtype (PFST_DT_I64 or PFST_DT_U8, else PFST_ERR_UNSUPPORTED).            */
+int pfst_class_mix_lbl(const void* gt, const uint32_t* chosen, const float* img,
+                       const float* trg_img, const void* pseudo_label, const float* weight_in,
+                       const unsigned long long* count, int64_t ps_size, int32_t ignore_top,
+                       int32_t ignore_bottom, int64_t B, int32_t img_channels, int64_t H, int64_t W,
+                       float* mixed_img, void* mixed_lbl, float* mixed_weight, void* mix_mask,
+                       int32_t label_dtype, void* stream);
 
 /* one_mix for a caller-supplied mask (dacs_transforms.py:129-144), one image:
  * out[c,p] = mask[p]*a[c,p] + (1-mask[p])*b[c,p]; mask int64 {0,1} of HW entries;
@@ -219,6 +241,13 @@ int pfst_neigh_grad_proto(const float* x, const float* coef, int64_t B, int32_t 
                           int32_t lab_h, int32_t lab_w, const float* mu, const uint8_t* seen,
                           int32_t C, const float* dist, const double* acc,
                           const float* grad_loss, float* grad_x, void* stream);
+/* pfst_neigh_grad_proto with labels of label_dtype (PFST_DT_I64 or PFST_DT_U8, else
+ * PFST_ERR_UNSUPPORTED); pfgst_loss.py:181-201 backward + pfgst.py:168-177 backward.            */
+int pfst_neigh_grad_proto_lbl(const float* x, const float* coef, int64_t B, int32_t D, int32_t h,
+                              int32_t w, int32_t dilation, const void* labels, int32_t label_dtype,
+                              int32_t lab_h, int32_t lab_w, const float* mu, const uint8_t* seen,
+                              int32_t C, const float* dist, const double* acc,
+                              const float* grad_loss, float* grad_x, void* stream);
 
 /* Bytes of the `workspace` the two entry points below share (per-pixel maps written
  * by the forward's prep kernel and re-read by the backward). Host only.             */
@@ -301,6 +330,28 @@ int pfst_pfgst_loss_bwd_ex(const float* dots, int32_t ksplit, int64_t B, int32_t
                            const double* stats, const float* grad_losses, float* coef,
                            float* grad_logits, int32_t options, float sigma,
                            const float* logits_ema, const float* margin_host, void* stream);
+/* pfst_pfgst_loss_fwd_ex / _bwd_ex (pfgst_loss.py:44-234, nearest-sampled gt and mix of :62-67) with
+ * gt and mix of label_dtype (PFST_DT_I64 or PFST_DT_U8, else PFST_ERR_UNSUPPORTED), the last
+ * argument before the stream. Every option set goes through them.                                */
+int pfst_pfgst_loss_fwd_lbl(const float* dots, int32_t ksplit, int64_t B, int32_t fh,
+                            int32_t fw, int32_t up, const float* logits, int32_t C,
+                            int32_t lh, int32_t lw, float lscale_h, float lscale_w,
+                            const void* gt, const void* mix, int32_t gt_h,
+                            int32_t gt_w, int32_t dilation, int32_t top_k,
+                            const float* weights6_host, void* workspace, double* stats,
+                            float* losses, float* density, uint8_t* eroded, int32_t options,
+                            float sigma, const float* logits_ema, const float* margin_host,
+                            int32_t label_dtype, void* stream);
+int pfst_pfgst_loss_bwd_lbl(const float* dots, int32_t ksplit, int64_t B, int32_t fh,
+                            int32_t fw, int32_t up, const float* logits, int32_t C,
+                            int32_t lh, int32_t lw, float lscale_h, float lscale_w,
+                            const void* gt, const void* mix, int32_t gt_h,
+                            int32_t gt_w, int32_t dilation, int32_t top_k,
+                            const float* weights6_host, const void* workspace,
+                            const double* stats, const float* grad_losses, float* coef,
+                            float* grad_logits, int32_t options, float sigma,
+                            const float* logits_ema, const float* margin_host,
+                            int32_t label_dtype, void* stream);
 
 /* ---- P1-P3: class prototypes (north_star extension; no reference code) ----------
  * Anchor: PFGST.masked_feat_dist, rsiseg/models/uda/pfgst.py:168-177. Labels are
@@ -320,6 +371,11 @@ int pfst_proto_accum(const float* feats, int64_t B, int32_t D, int32_t h, int32_
                      const int64_t* labels, int32_t lab_h, int32_t lab_w,
                      const float* conf, float conf_thr, int32_t C, float* packed,
                      void* stream);
+/* pfst_proto_accum with labels of label_dtype (PFST_DT_I64 or PFST_DT_U8, else PFST_ERR_UNSUPPORTED);
+ * anchor pfgst.py:168-177, labels nearest-resampled as pfgst_loss.py:62.                         */
+int pfst_proto_accum_lbl(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
+                         const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w,
+                         const float* conf, float conf_thr, int32_t C, float* packed, void* stream);
 
 /* pfst_proto_accum split in two, so that the label sort is done ONCE per (image, tile) and
  * not by every streaming block:
@@ -335,6 +391,11 @@ int64_t pfst_proto_order_ws_bytes(int64_t B, int32_t h, int32_t w, int32_t C);
 int pfst_proto_order(const int64_t* labels, int64_t B, int32_t h, int32_t w, int32_t lab_h,
                      int32_t lab_w, const float* conf, float conf_thr, int32_t C, float* counts,
                      void* workspace, void* stream);
+/* pfst_proto_order with labels of label_dtype (PFST_DT_I64 or PFST_DT_U8, else PFST_ERR_UNSUPPORTED);
+ * the lists it writes do not depend on the label dtype (pfst_proto_accum_ordered is shared).     */
+int pfst_proto_order_lbl(const void* labels, int32_t label_dtype, int64_t B, int32_t h, int32_t w,
+                         int32_t lab_h, int32_t lab_w, const float* conf, float conf_thr, int32_t C,
+                         float* counts, void* workspace, void* stream);
 int pfst_proto_accum_ordered(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
                              int32_t C, const void* workspace, float* packed, void* stream);
 
@@ -422,6 +483,17 @@ int pfst_proto_dist_bwd(const float* feats, int64_t B, int32_t D, int32_t h, int
                         const float* mu, const uint8_t* seen, int32_t C,
                         const float* dist, const double* acc, const float* grad_loss,
                         float* grad_feats, int32_t accumulate, void* stream);
+/* pfst_proto_dist_fwd / _bwd (masked_feat_dist, pfgst.py:168-177, with f2 = mu[label]) with labels of
+ * label_dtype (PFST_DT_I64 or PFST_DT_U8, else PFST_ERR_UNSUPPORTED).                            */
+int pfst_proto_dist_fwd_lbl(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
+                            const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w,
+                            const float* mu, const uint8_t* seen, int32_t C, float* dist,
+                            double* acc, float* loss, void* stream);
+int pfst_proto_dist_bwd_lbl(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
+                            const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w,
+                            const float* mu, const uint8_t* seen, int32_t C,
+                            const float* dist, const double* acc, const float* grad_loss,
+                            float* grad_feats, int32_t accumulate, void* stream);
 
 /* out[b,c,n] = ||feats[b,:,n] - mu[c]||_2 for every class: (B,C,h,w).               */
 int pfst_proto_dist_all(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
@@ -441,6 +513,13 @@ int pfst_weighted_ce(const float* logits, const int64_t* labels, const float* we
                      const float* class_weight, int64_t B, int32_t C, int32_t lh, int32_t lw,
                      int32_t H, int32_t W, int64_t ignore_index, float loss_weight,
                      float* grad_logits, double* stats, float* out2, void* stream);
+/* pfst_weighted_ce (decode_head.py:249-283, cross_entropy_loss.py:12-65) with labels of label_dtype
+ * (PFST_DT_I64 or PFST_DT_U8, else PFST_ERR_UNSUPPORTED).                                         */
+int pfst_weighted_ce_lbl(const float* logits, const void* labels, int32_t label_dtype,
+                         const float* weight, const float* class_weight, int64_t B, int32_t C,
+                         int32_t lh, int32_t lw, int32_t H, int32_t W, int64_t ignore_index,
+                         float loss_weight, float* grad_logits, double* stats, float* out2,
+                         void* stream);
 
 /* ---- next row (SURVEY.md §8f rank 4): offline class-wise thresholds -------------------
  * Replaces PseudoLabelingHookV4._cal_threshold

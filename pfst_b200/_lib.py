@@ -38,11 +38,15 @@ SIGNATURES: dict[str, tuple] = {
     "pfst_ema_update_multi_dev": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i64, _i32, _vp, _i32, _vp]),
     "pfst_ema_update_flat": (C.c_int, [_vp, _vp, _i64, _f32, _f32, _i32, _vp]),
     "pfst_pseudo_label": (C.c_int, [_vp, _i64, _i32, _i64, _f32, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp]),
+    "pfst_pseudo_label_lbl": (C.c_int, [_vp, _i64, _i32, _i64, _f32, _vp, _i32, _i64, _vp, _i32, _vp, _vp, _vp, _vp]),
     "pfst_selftest_exp": (C.c_int, [_vp, _i64, _vp, _vp]),
     "pfst_pseudo_weight_fill": (C.c_int, [_vp, _i64, _i64, _i64, _vp, _i64, _i32, _i32, _vp]),
     "pfst_class_presence": (C.c_int, [_vp, _i64, _vp, _vp]),
+    "pfst_class_presence_lbl": (C.c_int, [_vp, _i32, _i64, _vp, _vp]),
     "pfst_class_mix": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _i32, _i64, _i32,
                                  _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
+    "pfst_class_mix_lbl": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _i32, _i64, _i32,
+                                     _i64, _i64, _vp, _vp, _vp, _vp, _i32, _vp]),
     "pfst_mask_mix": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i64, _i64, _vp]),
     "pfst_neigh_dots_splits": (_i32, [_i64, _i64, _i32, _i32, _i32]),
     "pfst_neigh_dots": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _i32, _vp, _vp]),
@@ -50,6 +54,8 @@ SIGNATURES: dict[str, tuple] = {
     "pfst_neigh_dots_slot": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp]),
     "pfst_neigh_grad_proto": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _i32, _vp, _i32, _i32, _vp, _vp, _i32,
                                         _vp, _vp, _vp, _vp, _vp]),
+    "pfst_neigh_grad_proto_lbl": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _vp,
+                                            _vp, _i32, _vp, _vp, _vp, _vp, _vp]),
     "pfst_pfgst_loss_ws_bytes": (_i64, [_i64, _i32, _i32, _i32, _i32]),
     "pfst_pfgst_loss_fwd": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _f32, _f32,
                                       _vp, _vp, _i32, _i32, _i32, _i32, C.POINTER(_f32), _vp, _vp, _vp, _vp, _vp, _vp]),
@@ -62,6 +68,12 @@ SIGNATURES: dict[str, tuple] = {
     "pfst_pfgst_loss_bwd_ex": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _f32, _f32,
                                          _vp, _vp, _i32, _i32, _i32, _i32, C.POINTER(_f32), _vp, _vp, _vp, _vp, _vp,
                                          _i32, _f32, _vp, C.POINTER(_f32), _vp]),
+    "pfst_pfgst_loss_fwd_lbl": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _f32, _f32,
+                                          _vp, _vp, _i32, _i32, _i32, _i32, C.POINTER(_f32), _vp, _vp, _vp, _vp, _vp,
+                                          _i32, _f32, _vp, C.POINTER(_f32), _i32, _vp]),
+    "pfst_pfgst_loss_bwd_lbl": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _f32, _f32,
+                                          _vp, _vp, _i32, _i32, _i32, _i32, C.POINTER(_f32), _vp, _vp, _vp, _vp, _vp,
+                                          _i32, _f32, _vp, C.POINTER(_f32), _i32, _vp]),
     "pfst_slide_add": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp]),
     "pfst_slide_finalize": (C.c_int, [_vp, _vp, _vp, _i64, _i32, _i32, _i32, _i32, _i32, _vp, _vp]),
     "pfst_softmax_accum": (C.c_int, [_vp, _vp, _i64, _i32, _i64, _i32, _vp]),
@@ -69,10 +81,14 @@ SIGNATURES: dict[str, tuple] = {
     "pfst_class_quantile_ws_bytes": (_i64, [_i64, _i32, _i32]),
     "pfst_class_quantile": (C.c_int, [_vp, _i64, _i32, _i64, _vp, _i64, _vp, _i32, _vp, _vp, _vp]),
     "pfst_weighted_ce": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i32, _i32, _i32, _i32, _i32, _i64, _f32, _vp, _vp, _vp, _vp]),
+    "pfst_weighted_ce_lbl": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _i64, _i32, _i32, _i32, _i32, _i32, _i64, _f32, _vp,
+                                       _vp, _vp, _vp]),
     "pfst_proto_accum_is_masked": (C.c_int, [_i32, _i32, _i32]),
     "pfst_proto_accum": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _vp, _f32, _i32, _vp, _vp]),
+    "pfst_proto_accum_lbl": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _vp, _f32, _i32, _vp, _vp]),
     "pfst_proto_order_ws_bytes": (_i64, [_i64, _i32, _i32, _i32]),
     "pfst_proto_order": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _i32, _vp, _f32, _i32, _vp, _vp, _vp]),
+    "pfst_proto_order_lbl": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _i32, _vp, _f32, _i32, _vp, _vp, _vp]),
     "pfst_proto_accum_ordered": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _i32, _vp, _vp, _vp]),
     "pfst_proto_finalize": (C.c_int, [_vp, _i32, _i32, _vp, _vp, _f32, _f32, _vp, _vp, _vp, _i32, _vp]),
     "pfst_proto_finalize_dev": (C.c_int, [_vp, _i32, _i32, _vp, _vp, _f64, _vp, _vp, _vp, _vp, _i32, _vp]),
@@ -94,6 +110,10 @@ SIGNATURES: dict[str, tuple] = {
     "pfst_pack_scalars": (C.c_int, [_vp, _vp, _i32, _vp, _vp]),
     "pfst_proto_dist_fwd": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _vp, _vp, _i32, _vp, _vp, _vp, _vp]),
     "pfst_proto_dist_bwd": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _i32, _vp]),
+    "pfst_proto_dist_fwd_lbl": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _vp, _vp, _i32, _vp, _vp,
+                                          _vp, _vp]),
+    "pfst_proto_dist_bwd_lbl": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _vp, _vp, _i32, _vp, _vp,
+                                          _vp, _vp, _i32, _vp]),
     "pfst_proto_dist_all": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _vp, _i32, _vp, _vp]),
     "pfst_confusion_accum": (C.c_int, [_vp, _i32, _vp, _i32, _i64, _i64, _i32, _i64, _i32, _vp, _vp,
                                        _i32, _vp]),

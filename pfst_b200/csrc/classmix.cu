@@ -20,8 +20,9 @@ namespace pfst {
 
 constexpr int kMixThreads = 256;
 
+template <class L>
 __global__ void __launch_bounds__(kMixThreads)
-class_presence_kernel(const int64_t* __restrict__ gt, int64_t n, uint32_t* __restrict__ presence) {
+class_presence_kernel(const L* __restrict__ gt, int64_t n, uint32_t* __restrict__ presence) {
   __shared__ uint8_t seen[256];
   __shared__ int bad;
   const int tid = threadIdx.x;
@@ -29,6 +30,36 @@ class_presence_kernel(const int64_t* __restrict__ gt, int64_t n, uint32_t* __res
   if (tid == 0) bad = 0;
   __syncthreads();
   const bool vec = aligned16(gt);
+  if constexpr (sizeof(L) == 1) {
+    // uint8: 16 labels per 16-byte load, every value is in range (word 8 stays 0)
+    const int64_t n16 = vec ? (n >> 4) : 0;
+    const int64_t stride = (int64_t)gridDim.x * kMixThreads;
+    for (int64_t i = (int64_t)blockIdx.x * kMixThreads + tid; i < n16; i += 4 * stride) {
+      int4 v[4];
+      bool ok[4];
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        ok[u] = i + u * stride < n16;
+        v[u] = ok[u] ? ldg_stream_i4(gt + 16 * (i + u * stride)) : make_int4(0, 0, 0, 0);
+      }
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        if (!ok[u]) continue;
+        const uint32_t words[4] = {(uint32_t)v[u].x, (uint32_t)v[u].y, (uint32_t)v[u].z, (uint32_t)v[u].w};
+#pragma unroll
+        for (int j = 0; j < 4; ++j)
+#pragma unroll
+          for (int k = 0; k < 4; ++k) seen[(words[j] >> (8 * k)) & 255u] = 1;
+      }
+    }
+    for (int64_t i = 16 * n16 + (int64_t)blockIdx.x * kMixThreads + tid; i < n;
+         i += (int64_t)gridDim.x * kMixThreads)
+      seen[gt[i]] = 1;
+    __syncthreads();
+    const unsigned word = __ballot_sync(0xffffffffu, seen[tid] != 0);
+    if ((tid & 31) == 0 && word) atomicOr(&presence[tid >> 5], word);
+    return;
+  }
   const int64_t n2 = vec ? (n >> 1) : 0;
   // four 16-byte loads in flight per thread (one per pass kept the kernel at a quarter of the copy rate)
   const int64_t stride = (int64_t)gridDim.x * kMixThreads;
@@ -38,7 +69,8 @@ class_presence_kernel(const int64_t* __restrict__ gt, int64_t n, uint32_t* __res
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
       ok[u] = i + u * stride < n2;
-      v[u] = ok[u] ? ldg_stream_l2(gt + 2 * (i + u * stride)) : make_longlong2(0, 0);
+      v[u] = ok[u] ? ldg_stream_l2(reinterpret_cast<const int64_t*>(gt) + 2 * (i + u * stride))
+                   : make_longlong2(0, 0);
     }
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
@@ -65,15 +97,18 @@ __device__ __forceinline__ float mix_f(float m, float a, float b) {
   return __fadd_rn(__fmul_rn(m, a), __fmul_rn(1.0f - m, b));
 }
 
-template <int VEC>
+// L = uint8: the 4-pixel unit reads gt and the pseudo label as one 32-bit word each and writes
+// the mixed label and the mask as one 32-bit word each.
+template <int VEC, class L>
 __global__ void __launch_bounds__(kMixThreads)
-class_mix_kernel(const int64_t* __restrict__ gt, const uint32_t* __restrict__ chosen,
+class_mix_kernel(const L* __restrict__ gt, const uint32_t* __restrict__ chosen,
                  const float* __restrict__ img, const float* __restrict__ trg,
-                 const int64_t* __restrict__ pl, const float* weight_in,
+                 const L* __restrict__ pl, const float* weight_in,
                  const unsigned long long* __restrict__ count, int64_t ps_size, int ignore_top,
                  int ignore_bottom, int64_t B, int channels, int64_t H, int64_t W,
-                 float* __restrict__ mixed_img, int64_t* __restrict__ mixed_lbl,
-                 float* mixed_weight, int64_t* __restrict__ mix_mask) {
+                 float* __restrict__ mixed_img, L* __restrict__ mixed_lbl,
+                 float* mixed_weight, L* __restrict__ mix_mask) {
+  constexpr bool kU8 = sizeof(L) == 1;
   // grid = (tiles of the image plane, images): 32-bit pixel index, no 64-bit divisions
   const int64_t HW = H * W;
   const unsigned per_img = (unsigned)(HW / VEC);
@@ -84,8 +119,13 @@ class_mix_kernel(const int64_t* __restrict__ gt, const uint32_t* __restrict__ ch
     const int64_t p = (int64_t)i * VEC;
     const int64_t o = b * HW + p;
     int64_t g[VEC];
-    if (VEC == 4) {
-      const longlong2 g0 = ldg_stream_l2(gt + o), g1 = ldg_stream_l2(gt + o + 2);
+    if (VEC == 4 && kU8) {
+      const uint32_t g4 = ldg_stream_u32(gt + o);
+#pragma unroll
+      for (int k = 0; k < VEC; ++k) g[k] = (g4 >> (8 * k)) & 255u;
+    } else if (VEC == 4) {
+      const longlong2 g0 = ldg_stream_l2(reinterpret_cast<const int64_t*>(gt) + o),
+                      g1 = ldg_stream_l2(reinterpret_cast<const int64_t*>(gt) + o + 2);
       g[0] = g0.x; g[1 % VEC] = g0.y; g[2 % VEC] = g1.x; g[3 % VEC] = g1.y;
     } else {
       g[0] = gt[o];
@@ -100,9 +140,13 @@ class_mix_kernel(const int64_t* __restrict__ gt, const uint32_t* __restrict__ ch
       m[k] = mb[k] ? 1.f : 0.f;
     }
     if (mix_mask) {
-      if (VEC == 4) {
-        stg_l2(mix_mask + o, make_longlong2(mb[0], mb[1 % VEC]));
-        stg_l2(mix_mask + o + 2, make_longlong2(mb[2 % VEC], mb[3 % VEC]));
+      if (VEC == 4 && kU8) {
+        *reinterpret_cast<uint32_t*>(mix_mask + o) = (uint32_t)mb[0] | ((uint32_t)mb[1 % VEC] << 8) |
+                                                     ((uint32_t)mb[2 % VEC] << 16) | ((uint32_t)mb[3 % VEC] << 24);
+      } else if (VEC == 4) {
+        int64_t* mm = reinterpret_cast<int64_t*>(mix_mask);
+        stg_l2(mm + o, make_longlong2(mb[0], mb[1 % VEC]));
+        stg_l2(mm + o + 2, make_longlong2(mb[2 % VEC], mb[3 % VEC]));
       } else {
         mix_mask[o] = mb[0];
       }
@@ -120,13 +164,22 @@ class_mix_kernel(const int64_t* __restrict__ gt, const uint32_t* __restrict__ ch
       }
     }
     if (mixed_lbl) {
-      if (VEC == 4) {
-        const longlong2 q0 = ldg_stream_l2(pl + o), q1 = ldg_stream_l2(pl + o + 2);
-        stg_l2(mixed_lbl + o, make_longlong2(mb[0] ? g[0] : q0.x, mb[1 % VEC] ? g[1 % VEC] : q0.y));
-        stg_l2(mixed_lbl + o + 2,
+      if (VEC == 4 && kU8) {
+        const uint32_t q4 = ldg_stream_u32(pl + o);
+        uint32_t r = 0;
+#pragma unroll
+        for (int k = 0; k < VEC; ++k)
+          r |= (mb[k] ? (uint32_t)g[k] : (q4 >> (8 * k)) & 255u) << (8 * k);
+        *reinterpret_cast<uint32_t*>(mixed_lbl + o) = r;
+      } else if (VEC == 4) {
+        const int64_t* pl8 = reinterpret_cast<const int64_t*>(pl);
+        int64_t* ml8 = reinterpret_cast<int64_t*>(mixed_lbl);
+        const longlong2 q0 = ldg_stream_l2(pl8 + o), q1 = ldg_stream_l2(pl8 + o + 2);
+        stg_l2(ml8 + o, make_longlong2(mb[0] ? g[0] : q0.x, mb[1 % VEC] ? g[1 % VEC] : q0.y));
+        stg_l2(ml8 + o + 2,
                make_longlong2(mb[2 % VEC] ? g[2 % VEC] : q1.x, mb[3 % VEC] ? g[3 % VEC] : q1.y));
       } else {
-        mixed_lbl[o] = mb[0] ? g[0] : pl[o];
+        mixed_lbl[o] = mb[0] ? (L)g[0] : pl[o];
       }
     }
     if (mixed_weight) {
@@ -213,18 +266,74 @@ int pfst_mask_mix(const int64_t* mask, const void* a, const void* b, void* out, 
   return PFST_OK;
 }
 
-int pfst_class_presence(const int64_t* gt, int64_t n, uint32_t* presence, void* stream) {
+}  // extern "C"
+
+namespace pfst {
+
+template <class L>
+static int class_presence(const L* gt, int64_t n, uint32_t* presence, void* stream) {
   if (!presence || n < 0 || (n > 0 && !gt)) return PFST_ERR_INVALID_ARG;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   PFST_CUDA_TRY(cudaMemsetAsync(presence, 0, 9 * sizeof(uint32_t), s), "pfst_class_presence/memset");
   if (n == 0) return PFST_OK;
-  int64_t g = (n / 2 + pfst::kMixThreads - 1) / pfst::kMixThreads;
-  const int64_t cap = (int64_t)pfst::kNumSMs * 8;
+  int64_t g = (n / (16 / sizeof(L)) + kMixThreads - 1) / kMixThreads;
+  const int64_t cap = (int64_t)kNumSMs * 8;
   if (g > cap) g = cap;
   if (g < 1) g = 1;
-  pfst::class_presence_kernel<<<(unsigned)g, pfst::kMixThreads, 0, s>>>(gt, n, presence);
+  class_presence_kernel<L><<<(unsigned)g, kMixThreads, 0, s>>>(gt, n, presence);
   PFST_CHECK_LAUNCH("pfst_class_presence");
   return PFST_OK;
+}
+
+template <class L>
+static int class_mix(const L* gt, const uint32_t* chosen, const float* img, const float* trg_img,
+                     const L* pseudo_label, const float* weight_in, const unsigned long long* count,
+                     int64_t ps_size, int32_t ignore_top, int32_t ignore_bottom, int64_t B,
+                     int32_t img_channels, int64_t H, int64_t W, float* mixed_img, L* mixed_lbl,
+                     float* mixed_weight, L* mix_mask, void* stream) {
+  if (!gt || !chosen || B < 0 || H < 0 || W < 0 || img_channels < 0) return PFST_ERR_INVALID_ARG;
+  if (mixed_img && (!img || !trg_img)) return PFST_ERR_INVALID_ARG;
+  if (mixed_lbl && !pseudo_label) return PFST_ERR_INVALID_ARG;
+  if (mixed_weight && !weight_in && (!count || ps_size <= 0)) return PFST_ERR_INVALID_ARG;
+  if (ignore_top < 0 || ignore_bottom < 0) return PFST_ERR_INVALID_ARG;
+  const int64_t HW = H * W;
+  if (B == 0 || HW == 0) return PFST_OK;
+  const bool vec4 = (HW % 4 == 0) && aligned_lbl4(gt) && (!mixed_img || (aligned16(img) && aligned16(trg_img) && aligned16(mixed_img))) &&
+                    (!mixed_lbl || (aligned_lbl4(pseudo_label) && aligned_lbl4(mixed_lbl))) &&
+                    (!mixed_weight || (aligned16(mixed_weight) && (!weight_in || aligned16(weight_in)))) &&
+                    (!mix_mask || aligned_lbl4(mix_mask));
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (HW > 0x7fffffffll) return PFST_ERR_UNSUPPORTED;
+  const int64_t items = vec4 ? HW / 4 : HW;
+  const dim3 g((unsigned)((items + kMixThreads - 1) / kMixThreads),
+               (unsigned)(B < 65535 ? B : 65535), 1);
+  if (vec4)
+    class_mix_kernel<4, L><<<g, kMixThreads, 0, s>>>(
+        gt, chosen, img, trg_img, pseudo_label, weight_in, count, ps_size, ignore_top, ignore_bottom,
+        B, img_channels, H, W, mixed_img, mixed_lbl, mixed_weight, mix_mask);
+  else
+    class_mix_kernel<1, L><<<g, kMixThreads, 0, s>>>(
+        gt, chosen, img, trg_img, pseudo_label, weight_in, count, ps_size, ignore_top, ignore_bottom,
+        B, img_channels, H, W, mixed_img, mixed_lbl, mixed_weight, mix_mask);
+  PFST_CHECK_LAUNCH("pfst_class_mix");
+  return PFST_OK;
+}
+
+}  // namespace pfst
+
+extern "C" {
+
+int pfst_class_presence(const int64_t* gt, int64_t n, uint32_t* presence, void* stream) {
+  return pfst::class_presence(gt, n, presence, stream);
+}
+
+int pfst_class_presence_lbl(const void* gt, int32_t label_dtype, int64_t n, uint32_t* presence,
+                            void* stream) {
+  if (label_dtype == PFST_DT_I64)
+    return pfst::class_presence(static_cast<const int64_t*>(gt), n, presence, stream);
+  if (label_dtype == PFST_DT_U8)
+    return pfst::class_presence(static_cast<const uint8_t*>(gt), n, presence, stream);
+  return PFST_ERR_UNSUPPORTED;
 }
 
 int pfst_class_mix(const int64_t* gt, const uint32_t* chosen, const float* img,
@@ -233,33 +342,28 @@ int pfst_class_mix(const int64_t* gt, const uint32_t* chosen, const float* img,
                    int32_t ignore_bottom, int64_t B, int32_t img_channels, int64_t H, int64_t W,
                    float* mixed_img, int64_t* mixed_lbl, float* mixed_weight, int64_t* mix_mask,
                    void* stream) {
-  if (!gt || !chosen || B < 0 || H < 0 || W < 0 || img_channels < 0) return PFST_ERR_INVALID_ARG;
-  if (mixed_img && (!img || !trg_img)) return PFST_ERR_INVALID_ARG;
-  if (mixed_lbl && !pseudo_label) return PFST_ERR_INVALID_ARG;
-  if (mixed_weight && !weight_in && (!count || ps_size <= 0)) return PFST_ERR_INVALID_ARG;
-  if (ignore_top < 0 || ignore_bottom < 0) return PFST_ERR_INVALID_ARG;
-  const int64_t HW = H * W;
-  if (B == 0 || HW == 0) return PFST_OK;
-  using pfst::aligned16;
-  const bool vec4 = (HW % 4 == 0) && aligned16(gt) && (!mixed_img || (aligned16(img) && aligned16(trg_img) && aligned16(mixed_img))) &&
-                    (!mixed_lbl || (aligned16(pseudo_label) && aligned16(mixed_lbl))) &&
-                    (!mixed_weight || (aligned16(mixed_weight) && (!weight_in || aligned16(weight_in)))) &&
-                    (!mix_mask || aligned16(mix_mask));
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  if (HW > 0x7fffffffll) return PFST_ERR_UNSUPPORTED;
-  const int64_t items = vec4 ? HW / 4 : HW;
-  const dim3 g((unsigned)((items + pfst::kMixThreads - 1) / pfst::kMixThreads),
-               (unsigned)(B < 65535 ? B : 65535), 1);
-  if (vec4)
-    pfst::class_mix_kernel<4><<<g, pfst::kMixThreads, 0, s>>>(
-        gt, chosen, img, trg_img, pseudo_label, weight_in, count, ps_size, ignore_top, ignore_bottom,
-        B, img_channels, H, W, mixed_img, mixed_lbl, mixed_weight, mix_mask);
-  else
-    pfst::class_mix_kernel<1><<<g, pfst::kMixThreads, 0, s>>>(
-        gt, chosen, img, trg_img, pseudo_label, weight_in, count, ps_size, ignore_top, ignore_bottom,
-        B, img_channels, H, W, mixed_img, mixed_lbl, mixed_weight, mix_mask);
-  PFST_CHECK_LAUNCH("pfst_class_mix");
-  return PFST_OK;
+  return pfst::class_mix(gt, chosen, img, trg_img, pseudo_label, weight_in, count, ps_size, ignore_top,
+                         ignore_bottom, B, img_channels, H, W, mixed_img, mixed_lbl, mixed_weight, mix_mask,
+                         stream);
+}
+
+int pfst_class_mix_lbl(const void* gt, const uint32_t* chosen, const float* img,
+                       const float* trg_img, const void* pseudo_label, const float* weight_in,
+                       const unsigned long long* count, int64_t ps_size, int32_t ignore_top,
+                       int32_t ignore_bottom, int64_t B, int32_t img_channels, int64_t H, int64_t W,
+                       float* mixed_img, void* mixed_lbl, float* mixed_weight, void* mix_mask,
+                       int32_t label_dtype, void* stream) {
+  if (label_dtype == PFST_DT_I64)
+    return pfst::class_mix(static_cast<const int64_t*>(gt), chosen, img, trg_img,
+                           static_cast<const int64_t*>(pseudo_label), weight_in, count, ps_size, ignore_top,
+                           ignore_bottom, B, img_channels, H, W, mixed_img, static_cast<int64_t*>(mixed_lbl),
+                           mixed_weight, static_cast<int64_t*>(mix_mask), stream);
+  if (label_dtype == PFST_DT_U8)
+    return pfst::class_mix(static_cast<const uint8_t*>(gt), chosen, img, trg_img,
+                           static_cast<const uint8_t*>(pseudo_label), weight_in, count, ps_size, ignore_top,
+                           ignore_bottom, B, img_channels, H, W, mixed_img, static_cast<uint8_t*>(mixed_lbl),
+                           mixed_weight, static_cast<uint8_t*>(mix_mask), stream);
+  return PFST_ERR_UNSUPPORTED;
 }
 
 }  // extern "C"

@@ -41,6 +41,21 @@ void set_last_cuda_error(cudaError_t e, const char* where);
 __host__ __device__ static inline bool aligned16(const void* p) {
   return (reinterpret_cast<uintptr_t>(p) & 15u) == 0;
 }
+__host__ __device__ static inline bool aligned4(const void* p) {
+  return (reinterpret_cast<uintptr_t>(p) & 3u) == 0;
+}
+
+// Label maps are int64 (the reference dtype) or uint8 (the dtype datasets store); the kernels that read
+// or write them are templated on the element type, and the entry points take a PFST_DT_* tag.
+template <class L> struct LabelDt;
+template <> struct LabelDt<int64_t> { static constexpr int value = PFST_DT_I64; };
+template <> struct LabelDt<uint8_t> { static constexpr int value = PFST_DT_U8; };
+// Bytes of 4 consecutive labels as one vector access (int64: two 16-byte halves, uint8: one 32-bit
+// word): the alignment the vectorised paths need.
+template <class L>
+__host__ __device__ static inline bool aligned_lbl4(const L* p) {
+  return sizeof(L) == 8 ? aligned16(p) : aligned4(p);
+}
 
 // ---- streaming 128-bit global accesses ------------------------------------
 // Inputs that are read exactly once bypass L1 (ld.global.nc.L1::no_allocate);
@@ -64,6 +79,11 @@ __device__ __forceinline__ longlong2 ldg_stream_l2(const int64_t* p) {
   asm volatile("ld.global.nc.L1::no_allocate.v2.s64 {%0,%1}, [%2];"
                : "=l"(r.x), "=l"(r.y)
                : "l"(p));
+  return r;
+}
+__device__ __forceinline__ uint32_t ldg_stream_u32(const void* p) {
+  uint32_t r;
+  asm volatile("ld.global.nc.L1::no_allocate.u32 %0, [%1];" : "=r"(r) : "l"(p));
   return r;
 }
 __device__ __forceinline__ void stg_f4(float* p, float4 v) {
@@ -95,7 +115,8 @@ __device__ __forceinline__ int pr_nearest(int dst, float scale, int in) {
 }
 
 // label of feature pixel p (0..h*w) of image b, 255 if outside [0,C) or masked out
-__device__ __forceinline__ uint8_t pr_label(const int64_t* __restrict__ labels, const float* __restrict__ conf,
+template <class L>
+__device__ __forceinline__ uint8_t pr_label(const L* __restrict__ labels, const float* __restrict__ conf,
                                             float conf_thr, int b, int p, int w, int lab_h, int lab_w,
                                             float sh, float sw, int C) {
   const int y = p / w, x = p - y * w;

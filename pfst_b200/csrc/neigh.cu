@@ -215,8 +215,9 @@ neigh_dots_tma_kernel(const __grid_constant__ NeighMaps maps, int n_tensors, int
 // PROTO: the prototype-distance gradient (P3 backward, proto.cu) is added in the same pass,
 //   grad[n,c] += g * (x[n,c] - mu[y_n,c]) / (dist_n * n_valid),
 // so x_src is read once and grad_x written once for both losses.
-struct ProtoBwd {
-  const int64_t* labels;   // (B, lab_h, lab_w)
+template <class L>
+struct ProtoBwdT {
+  const L* labels;         // (B, lab_h, lab_w), int64 or uint8
   int lab_h, lab_w;
   const float* mu;         // (C, D)
   const uint8_t* seen;     // (C) or null
@@ -226,11 +227,12 @@ struct ProtoBwd {
   const float* grad_loss;  // device scalar
   int mu_stride;           // shared-memory row stride of the staged prototypes
 };
+using ProtoBwd = ProtoBwdT<int64_t>;
 
-template <int DIL, bool PROTO>
+template <int DIL, bool PROTO, class L = int64_t>
 __global__ void __launch_bounds__(kNbThreads)
 neigh_grad_tma_kernel(const __grid_constant__ NeighMaps maps, const float* __restrict__ coef, int B, int D,
-                      int h, int w, int ksplit, float* __restrict__ grad, const ProtoBwd pb) {
+                      int h, int w, int ksplit, float* __restrict__ grad, const ProtoBwdT<L> pb) {
   using G = NbGeom<DIL>;
   constexpr int kStageFloats = kNbCH * G::BWD_ROWS * G::RS;
   extern __shared__ __align__(128) unsigned char nb_smem[];
@@ -512,10 +514,10 @@ neigh_dots_plane_kernel(const float* __restrict__ xa, const float* __restrict__ 
 }
 
 // grad[b,c,p] = sum_k coef[b,k,p] * x[b,c,p+delta_k]  (+ the prototype-distance term, as ProtoBwd above)
-template <bool PROTO>
+template <bool PROTO, class L = int64_t>
 __global__ void __launch_bounds__(kSpThreads)
 neigh_grad_plane_kernel(const float* __restrict__ x, const float* __restrict__ coef, int B, int D, int h, int w,
-                        int dil, int ksplit, float* __restrict__ grad, const ProtoBwd pb) {
+                        int dil, int ksplit, float* __restrict__ grad, const ProtoBwdT<L> pb) {
   extern __shared__ __align__(128) unsigned char sp_smem[];
   float* stage_buf = reinterpret_cast<float*>(sp_smem);
   __shared__ uint64_t full_bar[kSpStages], empty_bar[kSpStages];
@@ -632,16 +634,16 @@ static size_t nb_proto_smem(int C, int D, int ks, int* stride) {
   return (size_t)C * (nch + 1) * sizeof(float);
 }
 
-template <int DIL, bool PROTO>
+template <int DIL, bool PROTO, class L>
 static int launch_grad_tma(const float* x, const float* coef, int B, int D, int h, int w, int ks, float* grad,
-                           ProtoBwd pb, cudaStream_t s) {
+                           ProtoBwdT<L> pb, cudaStream_t s) {
   using G = NbGeom<DIL>;
   NeighMaps maps;
   if (!make_nchw_tensor_map(&maps.m[0], x, B, D, h, w, G::RS, G::BWD_ROWS, kNbCH)) return PFST_ERR_CUDA;
   maps.m[1] = maps.m[0];
   size_t smem = (size_t)kNbStages * kNbCH * G::BWD_ROWS * G::RS * sizeof(float);
   if (PROTO) smem += nb_proto_smem(pb.C, D, ks, &pb.mu_stride);
-  auto k = neigh_grad_tma_kernel<DIL, PROTO>;
+  auto k = neigh_grad_tma_kernel<DIL, PROTO, L>;
   PFST_CUDA_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "pfst_neigh_grad/attr");
   const int64_t tiles = (int64_t)((w + kNbTW - 1) / kNbTW) * ((h + kNbTH - 1) / kNbTH);
   const int64_t grid = (int64_t)B * tiles * ks;
@@ -650,13 +652,13 @@ static int launch_grad_tma(const float* x, const float* coef, int B, int D, int 
   return PFST_OK;
 }
 
-template <bool PROTO>
+template <bool PROTO, class L>
 static int dispatch_grad_tma(int dilation, const float* x, const float* coef, int B, int D, int h, int w, int ks,
-                             float* grad, const ProtoBwd& pb, cudaStream_t s) {
+                             float* grad, const ProtoBwdT<L>& pb, cudaStream_t s) {
   switch (dilation) {
-    case 1: return launch_grad_tma<1, PROTO>(x, coef, B, D, h, w, ks, grad, pb, s);
-    case 2: return launch_grad_tma<2, PROTO>(x, coef, B, D, h, w, ks, grad, pb, s);
-    default: return launch_grad_tma<4, PROTO>(x, coef, B, D, h, w, ks, grad, pb, s);
+    case 1: return launch_grad_tma<1, PROTO, L>(x, coef, B, D, h, w, ks, grad, pb, s);
+    case 2: return launch_grad_tma<2, PROTO, L>(x, coef, B, D, h, w, ks, grad, pb, s);
+    default: return launch_grad_tma<4, PROTO, L>(x, coef, B, D, h, w, ks, grad, pb, s);
   }
 }
 
@@ -681,15 +683,15 @@ static int sp_grad_splits(int64_t B, int D) {
   return ks;
 }
 
-template <bool PROTO>
+template <bool PROTO, class L>
 static int launch_grad_plane(const float* x, const float* coef, int64_t B, int D, int h, int w, int dilation,
-                             float* grad, ProtoBwd pb, int ks, cudaStream_t s) {
+                             float* grad, ProtoBwdT<L> pb, int ks, cudaStream_t s) {
   size_t smem = (size_t)kSpStages * kSpCH * h * w * sizeof(float);
   if (PROTO) {
     pb.mu_stride = D / ks + 1;
     smem += (size_t)pb.C * pb.mu_stride * sizeof(float);
   }
-  auto k = neigh_grad_plane_kernel<PROTO>;
+  auto k = neigh_grad_plane_kernel<PROTO, L>;
   PFST_CUDA_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "pfst_neigh_grad/attr");
   k<<<(unsigned)(B * ks), kSpThreads, smem, s>>>(x, coef, (int)B, D, h, w, dilation, ks, grad, pb);
   PFST_CHECK_LAUNCH("pfst_neigh_grad");
@@ -767,35 +769,65 @@ int pfst_neigh_grad(const float* x, const float* coef, int64_t B, int32_t D, int
   return pfst::launch_grad_generic(x, coef, B, D, h, w, dilation, grad_x, s);
 }
 
-int pfst_neigh_grad_proto(const float* x, const float* coef, int64_t B, int32_t D, int32_t h, int32_t w,
-                          int32_t dilation, const int64_t* labels, int32_t lab_h, int32_t lab_w,
-                          const float* mu, const uint8_t* seen, int32_t C, const float* dist,
-                          const double* acc, const float* grad_loss, float* grad_x, void* stream) {
+}  // extern "C"
+
+namespace pfst {
+
+template <class L>
+static int neigh_grad_proto(const float* x, const float* coef, int64_t B, int32_t D, int32_t h, int32_t w,
+                            int32_t dilation, const L* labels, int32_t lab_h, int32_t lab_w, const float* mu,
+                            const uint8_t* seen, int32_t C, const float* dist, const double* acc,
+                            const float* grad_loss, float* grad_x, void* stream) {
   if (!x || !coef || !grad_x || !labels || !mu || !dist || !acc || !grad_loss || B < 0 || D < 1 || h < 1 ||
       w < 1 || dilation < 1 || lab_h < 1 || lab_w < 1 || C < 1)
     return PFST_ERR_INVALID_ARG;
   if (B == 0) return PFST_OK;
   if (B > 65535) return PFST_ERR_UNSUPPORTED;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  if (pfst::nb_tma_ok(x, grad_x, w, dilation) && pfst::aligned16(coef)) {
-    const int ks = pfst::nb_splits(B, h, w, D);
+  if (nb_tma_ok(x, grad_x, w, dilation) && aligned16(coef)) {
+    const int ks = nb_splits(B, h, w, D);
     int stride = 0;
-    if (pfst::nb_proto_smem(C, D, ks, &stride) <= 64 * 1024) {
-      pfst::ProtoBwd pb{labels, lab_h, lab_w, mu, seen, C, dist, acc, grad_loss, stride};
-      return pfst::dispatch_grad_tma<true>(dilation, x, coef, (int)B, D, h, w, ks, grad_x, pb, s);
+    if (nb_proto_smem(C, D, ks, &stride) <= 64 * 1024) {
+      ProtoBwdT<L> pb{labels, lab_h, lab_w, mu, seen, C, dist, acc, grad_loss, stride};
+      return dispatch_grad_tma<true>(dilation, x, coef, (int)B, D, h, w, ks, grad_x, pb, s);
     }
   }
-  const int ksp = pfst::sp_grad_splits(B, D);
-  if (pfst::sp_ok(x, grad_x, D, h, w, ksp) &&
-      (size_t)pfst::kSpStages * pfst::kSpCH * h * w * 4 + (size_t)C * (D / ksp + 1) * 4 <= 200 * 1024) {
-    pfst::ProtoBwd pb{labels, lab_h, lab_w, mu, seen, C, dist, acc, grad_loss, 0};
-    return pfst::launch_grad_plane<true>(x, coef, B, D, h, w, dilation, grad_x, pb, ksp, s);
+  const int ksp = sp_grad_splits(B, D);
+  if (sp_ok(x, grad_x, D, h, w, ksp) &&
+      (size_t)kSpStages * kSpCH * h * w * 4 + (size_t)C * (D / ksp + 1) * 4 <= 200 * 1024) {
+    ProtoBwdT<L> pb{labels, lab_h, lab_w, mu, seen, C, dist, acc, grad_loss, 0};
+    return launch_grad_plane<true>(x, coef, B, D, h, w, dilation, grad_x, pb, ksp, s);
   }
   // shapes the fused kernels do not cover: two passes over grad_x
   const int rc = pfst_neigh_grad(x, coef, B, D, h, w, dilation, grad_x, stream);
   if (rc != PFST_OK) return rc;
-  return pfst_proto_dist_bwd(x, B, D, h, w, labels, lab_h, lab_w, mu, seen, C, dist, acc, grad_loss, grad_x, 1,
-                             stream);
+  return pfst_proto_dist_bwd_lbl(x, B, D, h, w, labels, LabelDt<L>::value, lab_h, lab_w, mu, seen, C, dist, acc,
+                                 grad_loss, grad_x, 1, stream);
+}
+
+}  // namespace pfst
+
+extern "C" {
+
+int pfst_neigh_grad_proto(const float* x, const float* coef, int64_t B, int32_t D, int32_t h, int32_t w,
+                          int32_t dilation, const int64_t* labels, int32_t lab_h, int32_t lab_w,
+                          const float* mu, const uint8_t* seen, int32_t C, const float* dist,
+                          const double* acc, const float* grad_loss, float* grad_x, void* stream) {
+  return pfst::neigh_grad_proto(x, coef, B, D, h, w, dilation, labels, lab_h, lab_w, mu, seen, C, dist, acc,
+                                grad_loss, grad_x, stream);
+}
+
+int pfst_neigh_grad_proto_lbl(const float* x, const float* coef, int64_t B, int32_t D, int32_t h, int32_t w,
+                              int32_t dilation, const void* labels, int32_t label_dtype, int32_t lab_h,
+                              int32_t lab_w, const float* mu, const uint8_t* seen, int32_t C, const float* dist,
+                              const double* acc, const float* grad_loss, float* grad_x, void* stream) {
+  if (label_dtype == PFST_DT_I64)
+    return pfst::neigh_grad_proto(x, coef, B, D, h, w, dilation, static_cast<const int64_t*>(labels), lab_h, lab_w,
+                                  mu, seen, C, dist, acc, grad_loss, grad_x, stream);
+  if (label_dtype == PFST_DT_U8)
+    return pfst::neigh_grad_proto(x, coef, B, D, h, w, dilation, static_cast<const uint8_t*>(labels), lab_h, lab_w,
+                                  mu, seen, C, dist, acc, grad_loss, grad_x, stream);
+  return PFST_ERR_UNSUPPORTED;
 }
 
 }  // extern "C"

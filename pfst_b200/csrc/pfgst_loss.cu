@@ -30,8 +30,8 @@ struct LossParams {
   const float* logits;        // (B, C, lh, lw) student logits on the mixed image
   int C, lh, lw;
   float lscale_h, lscale_w;   // torch nearest: src = min(floor(dst * scale), in - 1)
-  const int64_t* gt;          // (B,1,gt_h,gt_w) source labels
-  const int64_t* mix;         // (B,1,gt_h,gt_w) ClassMix masks
+  const void* gt;             // (B,1,gt_h,gt_w) source labels, int64 or uint8 (prep kernel's L)
+  const void* mix;            // (B,1,gt_h,gt_w) ClassMix masks, same dtype
   int gt_h, gt_w;
   float gscale_h, gscale_w;
   int gh, gw;                 // loss grid
@@ -74,7 +74,7 @@ __host__ __device__ inline size_t ws_floats(int B, int C, int fh, int fw, int up
 // the rest resample labels / masks and take the softmax (one thread per loss-grid pixel).
 constexpr int kPrepThreads = 128;
 
-template <int CMAX>
+template <int CMAX, class L>
 __global__ void __launch_bounds__(kPrepThreads)
 pfgst_loss_prep_kernel(const LossParams P, int blocks_a) {
   const int fplane = P.fh * P.fw, gplane = P.gh * P.gw;       // per-image planes: 32-bit offsets
@@ -108,8 +108,8 @@ pfgst_loss_prep_kernel(const LossParams P, int blocks_a) {
   const int y = r / P.gw, x = r - y * P.gw;
   const int sy = nearest_src(y, P.gscale_h, P.gt_h), sx = nearest_src(x, P.gscale_w, P.gt_w);
   const int64_t go = ((int64_t)b * P.gt_h + sy) * P.gt_w + sx;
-  const int64_t g = P.gt[go];
-  const int64_t mx = P.mix[go];
+  const int64_t g = static_cast<const L*>(P.gt)[go];
+  const int64_t mx = static_cast<const L*>(P.mix)[go];
   // softmax of the nearest-resampled logits (pfgst_loss.py:57, 145): every class plane of the pixel
   // is requested before the first value is used (one memory round trip instead of three per class)
   const int ly = nearest_src(y, P.lscale_h, P.lh), lx = nearest_src(x, P.lscale_w, P.lw);
@@ -691,8 +691,8 @@ pfgst_loss_unfold_grad_kernel(const LossParams P, float* __restrict__ grad_logit
 constexpr int kOptGauss = 1, kOptProbEma = 2, kOptUnfoldGrad = 4, kOptMargin = 8, kOptMargin2 = 16;
 
 static int fill_params(LossParams& P, const float* dots, int ksplit, int64_t B, int fh, int fw, int up,
-                       const float* logits, int C, int lh, int lw, float lsh, float lsw, const int64_t* gt,
-                       const int64_t* mix, int gt_h, int gt_w, int dil, int top_k, const float* w6, void* ws) {
+                       const float* logits, int C, int lh, int lw, float lsh, float lsw, const void* gt,
+                       const void* mix, int gt_h, int gt_w, int dil, int top_k, const float* w6, void* ws) {
   if (!dots || !logits || !gt || !mix || !w6 || !ws) return PFST_ERR_INVALID_ARG;
   if (B < 0 || B > 0x7fffffff || fh < 1 || fw < 1 || up < 1 || C < 1 || lh < 1 || lw < 1 || gt_h < 1 || gt_w < 1)
     return PFST_ERR_INVALID_ARG;
@@ -767,12 +767,14 @@ int64_t pfst_pfgst_loss_ws_bytes(int64_t B, int32_t C, int32_t fh, int32_t fw, i
   return pfst_pfgst_loss_ws_bytes_ex(B, C, fh, fw, up, 0);
 }
 
-int pfst_pfgst_loss_fwd_ex(const float* dots, int32_t ksplit, int64_t B, int32_t fh, int32_t fw, int32_t up,
-                           const float* logits, int32_t C, int32_t lh, int32_t lw, float lscale_h,
-                           float lscale_w, const int64_t* gt, const int64_t* mix, int32_t gt_h, int32_t gt_w,
-                           int32_t dilation, int32_t top_k, const float* weights6_host, void* workspace,
-                           double* stats, float* losses, float* density, uint8_t* eroded, int32_t options,
-                           float sigma, const float* logits_ema, const float* margin_host, void* stream) {
+int pfst_pfgst_loss_fwd_lbl(const float* dots, int32_t ksplit, int64_t B, int32_t fh, int32_t fw, int32_t up,
+                            const float* logits, int32_t C, int32_t lh, int32_t lw, float lscale_h,
+                            float lscale_w, const void* gt, const void* mix, int32_t gt_h, int32_t gt_w,
+                            int32_t dilation, int32_t top_k, const float* weights6_host, void* workspace,
+                            double* stats, float* losses, float* density, uint8_t* eroded, int32_t options,
+                            float sigma, const float* logits_ema, const float* margin_host, int32_t label_dtype,
+                            void* stream) {
+  if (label_dtype != PFST_DT_I64 && label_dtype != PFST_DT_U8) return PFST_ERR_UNSUPPORTED;
   pfst::LossParams P;
   int rc = pfst::fill_params(P, dots, ksplit, B, fh, fw, up, logits, C, lh, lw, lscale_h, lscale_w, gt,
                              mix, gt_h, gt_w, dilation, top_k, weights6_host, workspace);
@@ -789,8 +791,13 @@ int pfst_pfgst_loss_fwd_ex(const float* dots, int32_t ksplit, int64_t B, int32_t
     const int64_t blocks_a = (n_a + pfst::kPrepThreads - 1) / pfst::kPrepThreads;
     const int64_t blocks_b = (total + pfst::kPrepThreads - 1) / pfst::kPrepThreads;
     if (blocks_a + blocks_b > 0x7fffffffll) return PFST_ERR_UNSUPPORTED;
-    auto prep = C <= 8 ? pfst::pfgst_loss_prep_kernel<8>
-                       : (C <= 40 ? pfst::pfgst_loss_prep_kernel<40> : pfst::pfgst_loss_prep_kernel<pfst::kMaxC>);
+    void (*prep)(const pfst::LossParams, int);
+    if (label_dtype == PFST_DT_U8)
+      prep = C <= 8 ? pfst::pfgst_loss_prep_kernel<8, uint8_t>
+                    : (C <= 40 ? pfst::pfgst_loss_prep_kernel<40, uint8_t> : pfst::pfgst_loss_prep_kernel<pfst::kMaxC, uint8_t>);
+    else
+      prep = C <= 8 ? pfst::pfgst_loss_prep_kernel<8, int64_t>
+                    : (C <= 40 ? pfst::pfgst_loss_prep_kernel<40, int64_t> : pfst::pfgst_loss_prep_kernel<pfst::kMaxC, int64_t>);
     prep<<<(unsigned)(blocks_a + blocks_b), pfst::kPrepThreads, 0, s>>>(P, (int)blocks_a);
     PFST_CHECK_LAUNCH("pfst_pfgst_loss_fwd/prep");
   }
@@ -800,6 +807,17 @@ int pfst_pfgst_loss_fwd_ex(const float* dots, int32_t ksplit, int64_t B, int32_t
       P, stats, losses, density, eroded);
   PFST_CHECK_LAUNCH("pfst_pfgst_loss_fwd");
   return PFST_OK;
+}
+
+int pfst_pfgst_loss_fwd_ex(const float* dots, int32_t ksplit, int64_t B, int32_t fh, int32_t fw, int32_t up,
+                           const float* logits, int32_t C, int32_t lh, int32_t lw, float lscale_h,
+                           float lscale_w, const int64_t* gt, const int64_t* mix, int32_t gt_h, int32_t gt_w,
+                           int32_t dilation, int32_t top_k, const float* weights6_host, void* workspace,
+                           double* stats, float* losses, float* density, uint8_t* eroded, int32_t options,
+                           float sigma, const float* logits_ema, const float* margin_host, void* stream) {
+  return pfst_pfgst_loss_fwd_lbl(dots, ksplit, B, fh, fw, up, logits, C, lh, lw, lscale_h, lscale_w, gt, mix, gt_h,
+                                 gt_w, dilation, top_k, weights6_host, workspace, stats, losses, density, eroded,
+                                 options, sigma, logits_ema, margin_host, PFST_DT_I64, stream);
 }
 
 int pfst_pfgst_loss_fwd(const float* dots, int32_t ksplit, int64_t B, int32_t fh, int32_t fw, int32_t up,
@@ -812,13 +830,16 @@ int pfst_pfgst_loss_fwd(const float* dots, int32_t ksplit, int64_t B, int32_t fh
                                 0.f, nullptr, nullptr, stream);
 }
 
-int pfst_pfgst_loss_bwd_ex(const float* dots, int32_t ksplit, int64_t B, int32_t fh, int32_t fw, int32_t up,
-                           const float* logits, int32_t C, int32_t lh, int32_t lw, float lscale_h,
-                           float lscale_w, const int64_t* gt, const int64_t* mix, int32_t gt_h, int32_t gt_w,
-                           int32_t dilation, int32_t top_k, const float* weights6_host, const void* workspace,
-                           const double* stats, const float* grad_losses, float* coef, float* grad_logits,
-                           int32_t options, float sigma, const float* logits_ema, const float* margin_host,
-                           void* stream) {
+// The backward reads the per-pixel label classes the forward's prep kernel left in the workspace, never gt
+// or mix themselves: the label dtype is only validated here.
+int pfst_pfgst_loss_bwd_lbl(const float* dots, int32_t ksplit, int64_t B, int32_t fh, int32_t fw, int32_t up,
+                            const float* logits, int32_t C, int32_t lh, int32_t lw, float lscale_h,
+                            float lscale_w, const void* gt, const void* mix, int32_t gt_h, int32_t gt_w,
+                            int32_t dilation, int32_t top_k, const float* weights6_host, const void* workspace,
+                            const double* stats, const float* grad_losses, float* coef, float* grad_logits,
+                            int32_t options, float sigma, const float* logits_ema, const float* margin_host,
+                            int32_t label_dtype, void* stream) {
+  if (label_dtype != PFST_DT_I64 && label_dtype != PFST_DT_U8) return PFST_ERR_UNSUPPORTED;
   pfst::LossParams P;
   int rc = pfst::fill_params(P, dots, ksplit, B, fh, fw, up, logits, C, lh, lw, lscale_h, lscale_w, gt,
                              mix, gt_h, gt_w, dilation, top_k, weights6_host, const_cast<void*>(workspace));
@@ -859,6 +880,18 @@ int pfst_pfgst_loss_bwd_ex(const float* dots, int32_t ksplit, int64_t B, int32_t
     PFST_CHECK_LAUNCH("pfst_pfgst_loss_bwd/unfold_grad");
   }
   return PFST_OK;
+}
+
+int pfst_pfgst_loss_bwd_ex(const float* dots, int32_t ksplit, int64_t B, int32_t fh, int32_t fw, int32_t up,
+                           const float* logits, int32_t C, int32_t lh, int32_t lw, float lscale_h,
+                           float lscale_w, const int64_t* gt, const int64_t* mix, int32_t gt_h, int32_t gt_w,
+                           int32_t dilation, int32_t top_k, const float* weights6_host, const void* workspace,
+                           const double* stats, const float* grad_losses, float* coef, float* grad_logits,
+                           int32_t options, float sigma, const float* logits_ema, const float* margin_host,
+                           void* stream) {
+  return pfst_pfgst_loss_bwd_lbl(dots, ksplit, B, fh, fw, up, logits, C, lh, lw, lscale_h, lscale_w, gt, mix, gt_h,
+                                 gt_w, dilation, top_k, weights6_host, workspace, stats, grad_losses, coef,
+                                 grad_logits, options, sigma, logits_ema, margin_host, PFST_DT_I64, stream);
 }
 
 int pfst_pfgst_loss_bwd(const float* dots, int32_t ksplit, int64_t B, int32_t fh, int32_t fw, int32_t up,

@@ -69,10 +69,10 @@ __device__ __forceinline__ void pa_sync_consumers() {
 // the class-sorted lists to `ws` (and the pixel counts to `counts`). MODE 2: stream only — the
 // lists are copied from `ws`, so the ~18 us sort prologue is paid by 8 blocks once instead of by
 // every one of the 144 streaming blocks.
-template <int MODE>
+template <int MODE, class LabelT = int64_t>
 __global__ void __launch_bounds__(kPaThreads)
 proto_accum_kernel(const float* __restrict__ feats, int B, int D, int h, int w,
-                   const int64_t* __restrict__ labels, const float* __restrict__ conf, float conf_thr,
+                   const LabelT* __restrict__ labels, const float* __restrict__ conf, float conf_thr,
                    int lab_h, int lab_w, int C, int groups, int tile, int stages, int use_bulk,
                    float* __restrict__ packed, float* __restrict__ counts, unsigned char* __restrict__ ws) {
   extern __shared__ __align__(128) unsigned char pa_smem[];
@@ -138,7 +138,29 @@ proto_accum_kernel(const float* __restrict__ feats, int B, int D, int h, int w,
     for (int i = threadIdx.x; i < ng * C; i += kPaConsumers * 32) grp[i] = 0;
     // all label gathers of this warp's groups in flight at once (one memory latency, not 16)
     unsigned lv[kGroupsPerWarp];
-    {
+    if constexpr (sizeof(LabelT) == 1) {
+      // uint8: 32-bit offsets inside this image's map (the host keeps lab_h * lab_w below 2^31) and
+      // byte-sized label registers, so the gathers fit next to the sort without spilling
+      const LabelT* lb = labels + (int64_t)b * lab_h * lab_w;
+      const float* cb = conf ? conf + (int64_t)b * lab_h * lab_w : nullptr;
+      int off[kGroupsPerWarp];
+      unsigned raw[kGroupsPerWarp];
+  #pragma unroll
+      for (int u = 0; u < kGroupsPerWarp; ++u) {
+        const int p = p0 + (warp + u * kPaConsumers) * 32 + lane;
+        const int y = p / w, x = p - y * w;
+        off[u] = pr_nearest(y, sh, lab_h) * lab_w + pr_nearest(x, sw, lab_w);
+      }
+  #pragma unroll
+      for (int u = 0; u < kGroupsPerWarp; ++u)
+        raw[u] = (warp + u * kPaConsumers) * 32 + lane < np ? (unsigned)__ldg(lb + off[u]) : 255u;
+  #pragma unroll
+      for (int u = 0; u < kGroupsPerWarp; ++u) {
+        bool ok = raw[u] < (unsigned)C;
+        if (cb && ok) ok = __ldg(cb + off[u]) >= conf_thr;
+        lv[u] = ok ? raw[u] : 255u;
+      }
+    } else {
       int64_t off[kGroupsPerWarp], raw[kGroupsPerWarp];
   #pragma unroll
       for (int u = 0; u < kGroupsPerWarp; ++u) {           // addresses first ...
@@ -316,9 +338,9 @@ proto_accum_kernel(const float* __restrict__ feats, int B, int D, int h, int w,
 constexpr int kPmThreads = 256;
 constexpr int kPmTile = 4096;
 
-template <int NC, bool FULL>
+template <int NC, bool FULL, class L>
 __global__ void __launch_bounds__(kPmThreads, 2)
-proto_accum_masked_kernel(const float* __restrict__ feats, int D, int h, int w, const int64_t* __restrict__ labels,
+proto_accum_masked_kernel(const float* __restrict__ feats, int D, int h, int w, const L* __restrict__ labels,
                           const float* __restrict__ conf, float conf_thr, int lab_h, int lab_w, int groups,
                           float* __restrict__ packed, float* __restrict__ counts) {
   __shared__ __align__(16) uint8_t lab_s[kPmTile];
@@ -576,10 +598,10 @@ struct PdCtx {
 
 // BWD = false: dist[n] = ||f_n - mu_y||, block sums -> acc[0] (sum dist), acc[1] (n valid)
 // BWD = true : grad[n,d] = g * (f - mu_y) / (dist * n_valid)
-template <bool BWD>
+template <bool BWD, class L>
 __global__ void __launch_bounds__(kPrThreads)
 proto_dist_kernel(const float* __restrict__ feats, int B, int D, int h, int w,
-                  const int64_t* __restrict__ labels, int lab_h, int lab_w, const float* __restrict__ mu,
+                  const L* __restrict__ labels, int lab_h, int lab_w, const float* __restrict__ mu,
                   const uint8_t* __restrict__ seen, int C, float* __restrict__ dist, double* __restrict__ acc,
                   float* __restrict__ loss, const float* __restrict__ grad_loss, float* __restrict__ grad,
                   unsigned* __restrict__ done_counter, int accumulate) {
@@ -712,8 +734,9 @@ proto_dist_kernel(const float* __restrict__ feats, int B, int D, int h, int w,
 // of the SM). The eight channel partials of a pixel are summed in warp order: deterministic like the kernel above.
 constexpr int kPdsUnroll = 16;
 
+template <class L>
 __global__ void __launch_bounds__(kPrThreads)
-proto_dist_small_kernel(const float* __restrict__ feats, int D, int h, int w, const int64_t* __restrict__ labels,
+proto_dist_small_kernel(const float* __restrict__ feats, int D, int h, int w, const L* __restrict__ labels,
                         int lab_h, int lab_w, const float* __restrict__ mu, const uint8_t* __restrict__ seen, int C,
                         float* __restrict__ dist, double* __restrict__ acc, float* __restrict__ loss,
                         unsigned* __restrict__ done_counter) {
@@ -839,11 +862,11 @@ int pa_plan(PaPlan& P, const float* feats, int64_t B, int32_t D, int32_t h, int3
   return PFST_OK;
 }
 
-template <int MODE>
+template <int MODE, class L>
 int pa_launch(const PaPlan& P, const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
-              const int64_t* labels, int32_t lab_h, int32_t lab_w, const float* conf, float conf_thr, int32_t C,
+              const L* labels, int32_t lab_h, int32_t lab_w, const float* conf, float conf_thr, int32_t C,
               float* packed, float* counts, unsigned char* ws, cudaStream_t s, const char* what) {
-  auto k = pfst::proto_accum_kernel<MODE>;
+  auto k = pfst::proto_accum_kernel<MODE, L>;
   PFST_CUDA_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)P.L.total), what);
   const int64_t groups = MODE == 1 ? 1 : P.groups;
   k<<<(unsigned)(B * P.n_tiles * groups), pfst::kPaThreads, P.L.total, s>>>(
@@ -862,9 +885,14 @@ int pfst_proto_accum_is_masked(int32_t C, int32_t h, int32_t w) {
   return (!off && C >= 1 && C <= 8 && ((int64_t)h * w) % 4 == 0 && (int64_t)h * w > pfst::kPsMaxHw) ? 1 : 0;
 }
 
-int pfst_proto_accum(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
-                     const int64_t* labels, int32_t lab_h, int32_t lab_w, const float* conf,
-                     float conf_thr, int32_t C, float* packed, void* stream) {
+}  // extern "C"
+
+namespace {
+
+template <class L>
+int proto_accum(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w, const L* labels, int32_t lab_h,
+                int32_t lab_w, const float* conf, float conf_thr, int32_t C, float* packed, void* stream) {
+  if (sizeof(L) == 1 && (int64_t)lab_h * lab_w > 0x7fffffffll) return PFST_ERR_UNSUPPORTED;   // 32-bit gathers
   if (!feats || !labels || !packed || B < 0 || D < 1 || h < 1 || w < 1 || lab_h < 1 || lab_w < 1 || C < 1)
     return PFST_ERR_INVALID_ARG;
   if (C > pfst::kPrMaxC) return PFST_ERR_UNSUPPORTED;
@@ -879,10 +907,10 @@ int pfst_proto_accum(const float* feats, int64_t B, int32_t D, int32_t h, int32_
     if (groups < 1) groups = 1;
     const int64_t grid = B * n_tiles * groups;
     if (grid > 0x7fffffffll) return PFST_ERR_UNSUPPORTED;
-    void (*k)(const float*, int, int, int, const int64_t*, const float*, float, int, int, int, float*, float*);
+    void (*k)(const float*, int, int, int, const L*, const float*, float, int, int, int, float*, float*);
     // whole 128-float4 chunks in every tile: no bounds tests in the streaming loop
     const bool full = hw % 512 == 0;
-#define PFST_PM_PICK(N) (full ? pfst::proto_accum_masked_kernel<N, true> : pfst::proto_accum_masked_kernel<N, false>)
+#define PFST_PM_PICK(N) (full ? pfst::proto_accum_masked_kernel<N, true, L> : pfst::proto_accum_masked_kernel<N, false, L>)
     switch (C) {
       case 1: k = PFST_PM_PICK(1); break;
       case 2: k = PFST_PM_PICK(2); break;
@@ -906,6 +934,28 @@ int pfst_proto_accum(const float* feats, int64_t B, int32_t D, int32_t h, int32_
                       packed + (int64_t)C * D, nullptr, static_cast<cudaStream_t>(stream), "pfst_proto_accum");
 }
 
+}  // namespace
+
+extern "C" {
+
+int pfst_proto_accum(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
+                     const int64_t* labels, int32_t lab_h, int32_t lab_w, const float* conf,
+                     float conf_thr, int32_t C, float* packed, void* stream) {
+  return proto_accum(feats, B, D, h, w, labels, lab_h, lab_w, conf, conf_thr, C, packed, stream);
+}
+
+int pfst_proto_accum_lbl(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
+                         const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w,
+                         const float* conf, float conf_thr, int32_t C, float* packed, void* stream) {
+  if (label_dtype == PFST_DT_I64)
+    return proto_accum(feats, B, D, h, w, static_cast<const int64_t*>(labels), lab_h, lab_w, conf, conf_thr, C,
+                       packed, stream);
+  if (label_dtype == PFST_DT_U8)
+    return proto_accum(feats, B, D, h, w, static_cast<const uint8_t*>(labels), lab_h, lab_w, conf, conf_thr, C,
+                       packed, stream);
+  return PFST_ERR_UNSUPPORTED;
+}
+
 int64_t pfst_proto_order_ws_bytes(int64_t B, int32_t h, int32_t w, int32_t C) {
   if (B < 1 || h < 1 || w < 1 || C < 1 || C > pfst::kPrMaxC) return 0;
   PaPlan P;
@@ -913,9 +963,14 @@ int64_t pfst_proto_order_ws_bytes(int64_t B, int32_t h, int32_t w, int32_t C) {
   return (int64_t)(B * P.n_tiles * P.list_bytes);
 }
 
-int pfst_proto_order(const int64_t* labels, int64_t B, int32_t h, int32_t w, int32_t lab_h, int32_t lab_w,
-                     const float* conf, float conf_thr, int32_t C, float* counts, void* workspace,
-                     void* stream) {
+}  // extern "C"
+
+namespace {
+
+template <class L>
+int proto_order(const L* labels, int64_t B, int32_t h, int32_t w, int32_t lab_h, int32_t lab_w,
+                const float* conf, float conf_thr, int32_t C, float* counts, void* workspace, void* stream) {
+  if (sizeof(L) == 1 && (int64_t)lab_h * lab_w > 0x7fffffffll) return PFST_ERR_UNSUPPORTED;   // 32-bit gathers
   if (!labels || !workspace || B < 0 || h < 1 || w < 1 || lab_h < 1 || lab_w < 1 || C < 1)
     return PFST_ERR_INVALID_ARG;
   if (C > pfst::kPrMaxC || !pfst::aligned16(workspace)) return PFST_ERR_UNSUPPORTED;
@@ -925,6 +980,28 @@ int pfst_proto_order(const int64_t* labels, int64_t B, int32_t h, int32_t w, int
   if (rc != PFST_OK) return rc;
   return pa_launch<1>(P, nullptr, B, 1, h, w, labels, lab_h, lab_w, conf, conf_thr, C, nullptr, counts,
                       static_cast<unsigned char*>(workspace), static_cast<cudaStream_t>(stream), "pfst_proto_order");
+}
+
+}  // namespace
+
+extern "C" {
+
+int pfst_proto_order(const int64_t* labels, int64_t B, int32_t h, int32_t w, int32_t lab_h, int32_t lab_w,
+                     const float* conf, float conf_thr, int32_t C, float* counts, void* workspace,
+                     void* stream) {
+  return proto_order(labels, B, h, w, lab_h, lab_w, conf, conf_thr, C, counts, workspace, stream);
+}
+
+int pfst_proto_order_lbl(const void* labels, int32_t label_dtype, int64_t B, int32_t h, int32_t w, int32_t lab_h,
+                         int32_t lab_w, const float* conf, float conf_thr, int32_t C, float* counts,
+                         void* workspace, void* stream) {
+  if (label_dtype == PFST_DT_I64)
+    return proto_order(static_cast<const int64_t*>(labels), B, h, w, lab_h, lab_w, conf, conf_thr, C, counts,
+                       workspace, stream);
+  if (label_dtype == PFST_DT_U8)
+    return proto_order(static_cast<const uint8_t*>(labels), B, h, w, lab_h, lab_w, conf, conf_thr, C, counts,
+                       workspace, stream);
+  return PFST_ERR_UNSUPPORTED;
 }
 
 int pfst_proto_accum_ordered(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w, int32_t C,
@@ -950,7 +1027,7 @@ int pfst_proto_accum_ordered(const float* feats, int64_t B, int32_t D, int32_t h
   }
   const int rc = pa_plan(P, feats, B, D, h, w, C, true);
   if (rc != PFST_OK) return rc;
-  return pa_launch<2>(P, feats, B, D, h, w, nullptr, 1, 1, nullptr, 0.f, C, packed, nullptr,
+  return pa_launch<2>(P, feats, B, D, h, w, (const int64_t*)nullptr, 1, 1, nullptr, 0.f, C, packed, nullptr,
                       static_cast<unsigned char*>(const_cast<void*>(workspace)), static_cast<cudaStream_t>(stream),
                       "pfst_proto_accum_ordered");
 }
@@ -976,8 +1053,11 @@ int pfst_proto_finalize_dev(float* packed, int32_t C, int32_t D, const float* mu
   return PFST_OK;
 }
 
+}  // extern "C"
+
+template <class L>
 static int proto_dist_common(bool bwd, const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
-                             const int64_t* labels, int32_t lab_h, int32_t lab_w, const float* mu,
+                             const L* labels, int32_t lab_h, int32_t lab_w, const float* mu,
                              const uint8_t* seen, int32_t C, float* dist, double* acc, float* loss,
                              const float* grad_loss, float* grad, int accumulate, cudaStream_t s) {
   if (!feats || !labels || !mu || !dist || !acc || B < 0 || D < 1 || h < 1 || w < 1 || C < 1)
@@ -995,19 +1075,19 @@ static int proto_dist_common(bool bwd, const float* feats, int64_t B, int32_t D,
     if (hw % 4 != 0 && !no_small) {
       const int64_t grid_s = B * ((hw + 31) / 32);
       if (grid_s > 0x7fffffffll) return PFST_ERR_UNSUPPORTED;
-      pfst::proto_dist_small_kernel<<<(unsigned)grid_s, pfst::kPrThreads, 0, s>>>(
+      pfst::proto_dist_small_kernel<L><<<(unsigned)grid_s, pfst::kPrThreads, 0, s>>>(
           feats, D, h, w, labels, lab_h, lab_w, mu, seen, C, dist, acc, loss, reinterpret_cast<unsigned*>(acc + 3));
       PFST_CHECK_LAUNCH("pfst_proto_dist_fwd/small");
       return PFST_OK;
     }
-    auto k = pfst::proto_dist_kernel<false>;
+    auto k = pfst::proto_dist_kernel<false, L>;
     PFST_CUDA_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "pfst_proto_dist_fwd/attr");
     k<<<(unsigned)grid, pfst::kPrThreads, smem, s>>>(feats, (int)B, D, h, w, labels, lab_h, lab_w, mu, seen, C, dist,
                                                      acc, loss, nullptr, nullptr,
                                                      reinterpret_cast<unsigned*>(acc + 3), 0);
   } else {
     if (!grad_loss || !grad) return PFST_ERR_INVALID_ARG;
-    auto k = pfst::proto_dist_kernel<true>;
+    auto k = pfst::proto_dist_kernel<true, L>;
     PFST_CUDA_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "pfst_proto_dist_bwd/attr");
     k<<<(unsigned)grid, pfst::kPrThreads, smem, s>>>(feats, (int)B, D, h, w, labels, lab_h, lab_w, mu, seen, C, dist,
                                                      acc, nullptr, grad_loss, grad, nullptr, accumulate);
@@ -1015,6 +1095,8 @@ static int proto_dist_common(bool bwd, const float* feats, int64_t B, int32_t D,
   PFST_CHECK_LAUNCH(bwd ? "pfst_proto_dist_bwd" : "pfst_proto_dist_fwd");
   return PFST_OK;
 }
+
+extern "C" {
 
 int pfst_proto_dist_fwd(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
                         const int64_t* labels, int32_t lab_h, int32_t lab_w, const float* mu,
@@ -1030,6 +1112,32 @@ int pfst_proto_dist_bwd(const float* feats, int64_t B, int32_t D, int32_t h, int
   return proto_dist_common(true, feats, B, D, h, w, labels, lab_h, lab_w, mu, seen, C, const_cast<float*>(dist),
                            const_cast<double*>(acc), nullptr, grad_loss, grad_feats, accumulate,
                            static_cast<cudaStream_t>(stream));
+}
+
+int pfst_proto_dist_fwd_lbl(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
+                            const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w, const float* mu,
+                            const uint8_t* seen, int32_t C, float* dist, double* acc, float* loss, void* stream) {
+  if (label_dtype == PFST_DT_I64)
+    return pfst_proto_dist_fwd(feats, B, D, h, w, static_cast<const int64_t*>(labels), lab_h, lab_w, mu, seen, C,
+                               dist, acc, loss, stream);
+  if (label_dtype == PFST_DT_U8)
+    return proto_dist_common(false, feats, B, D, h, w, static_cast<const uint8_t*>(labels), lab_h, lab_w, mu, seen,
+                             C, dist, acc, loss, nullptr, nullptr, 0, static_cast<cudaStream_t>(stream));
+  return PFST_ERR_UNSUPPORTED;
+}
+
+int pfst_proto_dist_bwd_lbl(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
+                            const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w, const float* mu,
+                            const uint8_t* seen, int32_t C, const float* dist, const double* acc,
+                            const float* grad_loss, float* grad_feats, int32_t accumulate, void* stream) {
+  if (label_dtype == PFST_DT_I64)
+    return pfst_proto_dist_bwd(feats, B, D, h, w, static_cast<const int64_t*>(labels), lab_h, lab_w, mu, seen, C,
+                               dist, acc, grad_loss, grad_feats, accumulate, stream);
+  if (label_dtype == PFST_DT_U8)
+    return proto_dist_common(true, feats, B, D, h, w, static_cast<const uint8_t*>(labels), lab_h, lab_w, mu, seen,
+                             C, const_cast<float*>(dist), const_cast<double*>(acc), nullptr, grad_loss, grad_feats,
+                             accumulate, static_cast<cudaStream_t>(stream));
+  return PFST_ERR_UNSUPPORTED;
 }
 
 int pfst_proto_dist_all(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w, const float* mu,

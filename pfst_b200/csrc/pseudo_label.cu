@@ -129,11 +129,12 @@ __device__ __forceinline__ void pl_load(float (&x)[VEC][CMAX], const float* __re
     }
 }
 
-template <int VEC, int CMAX, int MODE, bool EXACT>
+// L = uint8: one 32-bit store per 4 labels (the host guarantees C <= 255 and reject_label <= 255).
+template <int VEC, int CMAX, int MODE, bool EXACT, class L>
 __global__ void __launch_bounds__(kPlThreads)
 pseudo_label_kernel(const float* __restrict__ logits, int64_t B, int C, int64_t HW, float thr,
                     const float* __restrict__ thr_per_class, int64_t reject_label,
-                    int64_t* __restrict__ label, float* __restrict__ conf,
+                    L* __restrict__ label, float* __restrict__ conf,
                     float* __restrict__ weight_part, unsigned long long* __restrict__ count) {
   __shared__ float thr_s[CMAX];
   const float* thr_pc = nullptr;
@@ -172,15 +173,21 @@ pseudo_label_kernel(const float* __restrict__ logits, int64_t B, int C, int64_t 
     for (int k = 0; k < VEC; ++k)
       lab[k] = (reject_label >= 0 && !o[k].confident) ? reject_label : (int64_t)o[k].label;
     if (VEC == 4) {
-      stg_l2(label + out, make_longlong2(lab[0], lab[1 % VEC]));
-      stg_l2(label + out + 2, make_longlong2(lab[2 % VEC], lab[3 % VEC]));
+      if constexpr (sizeof(L) == 1) {
+        *reinterpret_cast<uint32_t*>(label + out) =
+            ((uint32_t)lab[0] & 255u) | (((uint32_t)lab[1 % VEC] & 255u) << 8) |
+            (((uint32_t)lab[2 % VEC] & 255u) << 16) | ((uint32_t)lab[3 % VEC] << 24);
+      } else {
+        stg_l2(label + out, make_longlong2(lab[0], lab[1 % VEC]));
+        stg_l2(label + out + 2, make_longlong2(lab[2 % VEC], lab[3 % VEC]));
+      }
       stg_f4(conf + out, make_float4(o[0].conf, o[1 % VEC].conf, o[2 % VEC].conf, o[3 % VEC].conf));
       if (weight_part)
         stg_f4(weight_part + out,
                make_float4(o[0].confident ? 1.f : 0.f, o[1 % VEC].confident ? 1.f : 0.f,
                            o[2 % VEC].confident ? 1.f : 0.f, o[3 % VEC].confident ? 1.f : 0.f));
     } else {
-      label[out] = lab[0];
+      label[out] = (L)lab[0];
       conf[out] = o[0].conf;
       if (weight_part) weight_part[out] = o[0].confident ? 1.f : 0.f;
     }
@@ -196,11 +203,11 @@ pseudo_label_kernel(const float* __restrict__ logits, int64_t B, int C, int64_t 
 
 // Any C: one pixel per thread, two passes over the pixel's logits (the second
 // pass is served from L1/L2).
-template <int MODE>
+template <int MODE, class L>
 __global__ void __launch_bounds__(kPlThreads)
 pseudo_label_generic_kernel(const float* __restrict__ logits, int64_t B, int C, int64_t HW,
                             float thr, const float* __restrict__ thr_per_class,
-                            int64_t reject_label, int64_t* __restrict__ label,
+                            int64_t reject_label, L* __restrict__ label,
                             float* __restrict__ conf, float* __restrict__ weight_part,
                             unsigned long long* __restrict__ count) {
   const int64_t total = B * HW;
@@ -244,7 +251,7 @@ pseudo_label_generic_kernel(const float* __restrict__ logits, int64_t B, int C, 
       confident = ent < t;
     }
     local += confident ? 1u : 0u;
-    label[i] = (reject_label >= 0 && !confident) ? reject_label : (int64_t)lab;
+    label[i] = (L)((reject_label >= 0 && !confident) ? reject_label : (int64_t)lab);
     conf[i] = cf;
     if (weight_part) weight_part[i] = confident ? 1.f : 0.f;
   }
@@ -279,11 +286,11 @@ __global__ void exp_selftest_kernel(const float* __restrict__ x, int64_t n,
   if ((threadIdx.x & 31) == 0 && bad) atomicAdd(mismatches, (unsigned long long)bad);
 }
 
-template <int MODE>
+template <int MODE, class L>
 static int launch_pl(const float* logits, int64_t B, int C, int64_t HW, float thr,
-                     const float* thr_pc, int64_t reject, int64_t* label, float* conf,
+                     const float* thr_pc, int64_t reject, L* label, float* conf,
                      float* wpart, unsigned long long* count, cudaStream_t s) {
-  const bool vec4 = (HW % 4 == 0) && aligned16(logits) && aligned16(label) && aligned16(conf) &&
+  const bool vec4 = (HW % 4 == 0) && aligned16(logits) && aligned_lbl4(label) && aligned16(conf) &&
                     (!wpart || aligned16(wpart));
   if (HW > 0x7fffffffll || B * (HW / 4 + 1) > 0x7fffffffll * 2) return PFST_ERR_UNSUPPORTED;
   auto grid_flat = [](int64_t items) {
@@ -293,7 +300,7 @@ static int launch_pl(const float* logits, int64_t B, int C, int64_t HW, float th
   };
 #define PFST_PL_LAUNCH(VEC_, CMAX_, EXACT_)                                                      \
   do {                                                                                           \
-    auto k = pseudo_label_kernel<VEC_, CMAX_, MODE, EXACT_>;                                     \
+    auto k = pseudo_label_kernel<VEC_, CMAX_, MODE, EXACT_, L>;                                     \
     int occ = 0;                                                                                 \
     PFST_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k, kPlThreads, 0),         \
                   "pfst_pseudo_label/occupancy");                                                \
@@ -305,16 +312,19 @@ static int launch_pl(const float* logits, int64_t B, int C, int64_t HW, float th
                                                        label, conf, wpart, count);              \
   } while (0)
   if (C <= 8 && vec4 && MODE == 0) {
-    // exact-C instantiations of the hot configuration (no per-class predicates)
-    switch (C) {
-      case 2: PFST_PL_LAUNCH(4, 2, true); break;
-      case 3: PFST_PL_LAUNCH(4, 3, true); break;
-      case 4: PFST_PL_LAUNCH(4, 4, true); break;
-      case 5: PFST_PL_LAUNCH(4, 5, true); break;
-      case 6: PFST_PL_LAUNCH(4, 6, true); break;
-      case 7: PFST_PL_LAUNCH(4, 7, true); break;
-      case 8: PFST_PL_LAUNCH(4, 8, true); break;
-      default: PFST_PL_LAUNCH(4, 8, false); break;
+    // exact-C instantiations of the hot configuration (no per-class predicates); the uint8 build
+    // does not instantiate the MODE 1 copies this branch never reaches
+    if constexpr (MODE == 0 || sizeof(L) == 8) {
+      switch (C) {
+        case 2: PFST_PL_LAUNCH(4, 2, true); break;
+        case 3: PFST_PL_LAUNCH(4, 3, true); break;
+        case 4: PFST_PL_LAUNCH(4, 4, true); break;
+        case 5: PFST_PL_LAUNCH(4, 5, true); break;
+        case 6: PFST_PL_LAUNCH(4, 6, true); break;
+        case 7: PFST_PL_LAUNCH(4, 7, true); break;
+        case 8: PFST_PL_LAUNCH(4, 8, true); break;
+        default: PFST_PL_LAUNCH(4, 8, false); break;
+      }
     }
   } else if (C <= 8 && vec4) {
     PFST_PL_LAUNCH(4, 8, false);
@@ -327,7 +337,7 @@ static int launch_pl(const float* logits, int64_t B, int C, int64_t HW, float th
   } else if (C <= 40) {
     PFST_PL_LAUNCH(1, 40, false);
   } else {
-    pseudo_label_generic_kernel<MODE><<<grid_flat(B * HW), kPlThreads, 0, s>>>(
+    pseudo_label_generic_kernel<MODE, L><<<grid_flat(B * HW), kPlThreads, 0, s>>>(
         logits, B, C, HW, thr, thr_pc, reject, label, conf, wpart, count);
   }
 #undef PFST_PL_LAUNCH
@@ -339,21 +349,51 @@ static int launch_pl(const float* logits, int64_t B, int C, int64_t HW, float th
 
 extern "C" {
 
-int pfst_pseudo_label(const float* logits, int64_t B, int32_t C, int64_t HW, float thr,
-                      const float* thr_per_class, int32_t mode, int64_t reject_label,
-                      int64_t* label, float* conf, float* weight_part,
-                      unsigned long long* count, void* stream) {
+}  // extern "C"
+
+namespace pfst {
+
+template <class L>
+static int pseudo_label(const float* logits, int64_t B, int32_t C, int64_t HW, float thr,
+                        const float* thr_per_class, int32_t mode, int64_t reject_label, L* label,
+                        float* conf, float* weight_part, unsigned long long* count, void* stream) {
   if (!logits || !label || !conf || !count) return PFST_ERR_INVALID_ARG;
   if (B < 0 || HW < 0 || C < 1) return PFST_ERR_INVALID_ARG;
   if (mode != 0 && mode != 1) return PFST_ERR_INVALID_ARG;
+  if (sizeof(L) == 1 && (C > 255 || reject_label > 255)) return PFST_ERR_UNSUPPORTED;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   PFST_CUDA_TRY(cudaMemsetAsync(count, 0, sizeof(unsigned long long), s), "pfst_pseudo_label/memset");
   if (B == 0 || HW == 0) return PFST_OK;
   if (mode == 0)
-    return pfst::launch_pl<0>(logits, B, C, HW, thr, thr_per_class, reject_label, label, conf,
-                              weight_part, count, s);
-  return pfst::launch_pl<1>(logits, B, C, HW, thr, thr_per_class, reject_label, label, conf,
-                            weight_part, count, s);
+    return launch_pl<0>(logits, B, C, HW, thr, thr_per_class, reject_label, label, conf,
+                        weight_part, count, s);
+  return launch_pl<1>(logits, B, C, HW, thr, thr_per_class, reject_label, label, conf,
+                      weight_part, count, s);
+}
+
+}  // namespace pfst
+
+extern "C" {
+
+int pfst_pseudo_label(const float* logits, int64_t B, int32_t C, int64_t HW, float thr,
+                      const float* thr_per_class, int32_t mode, int64_t reject_label,
+                      int64_t* label, float* conf, float* weight_part,
+                      unsigned long long* count, void* stream) {
+  return pfst::pseudo_label(logits, B, C, HW, thr, thr_per_class, mode, reject_label, label, conf,
+                            weight_part, count, stream);
+}
+
+int pfst_pseudo_label_lbl(const float* logits, int64_t B, int32_t C, int64_t HW, float thr,
+                          const float* thr_per_class, int32_t mode, int64_t reject_label,
+                          void* label, int32_t label_dtype, float* conf, float* weight_part,
+                          unsigned long long* count, void* stream) {
+  if (label_dtype == PFST_DT_I64)
+    return pfst::pseudo_label(logits, B, C, HW, thr, thr_per_class, mode, reject_label,
+                              static_cast<int64_t*>(label), conf, weight_part, count, stream);
+  if (label_dtype == PFST_DT_U8)
+    return pfst::pseudo_label(logits, B, C, HW, thr, thr_per_class, mode, reject_label,
+                              static_cast<uint8_t*>(label), conf, weight_part, count, stream);
+  return PFST_ERR_UNSUPPORTED;
 }
 
 int pfst_selftest_exp(const float* x, int64_t n, unsigned long long* mismatches, void* stream) {

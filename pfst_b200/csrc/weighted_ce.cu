@@ -32,7 +32,7 @@ constexpr int kCeRegC = 8;                       // up to this many classes the 
 
 struct CeParams {
   const float* logits;       // (B, C, lh, lw)
-  const int64_t* labels;     // (B, H, W)
+  const void* labels;        // (B, H, W), int64 or uint8 (the kernels' L)
   const float* weight;       // (B, H, W) or null
   const float* class_weight; // (C) or null
   int B, C, lh, lw, H, W, s; // H = s * lh, W = s * lw
@@ -58,7 +58,7 @@ __device__ __forceinline__ void ce_src(int dst, float scale, int in, int& i0, in
 // corners, so their per-class gradients are summed in a private shared-memory accumulator
 // ([class][corner][thread]: conflict-free, no atomics) and only four shared atomics per class and
 // thread fold them into the block's low-res tile; the tile goes to global memory once.
-template <bool REGC, bool PRIV>
+template <bool REGC, bool PRIV, class L>
 __global__ void __launch_bounds__(kCeThreads)
 weighted_ce_kernel(const CeParams P) {
   extern __shared__ __align__(16) float ce_smem[];
@@ -104,7 +104,7 @@ weighted_ce_kernel(const CeParams P) {
         if (x0 != x0c) continue;
         const int dx = x1 - x0;
         const int64_t pix = ((int64_t)b * P.H + y) * P.W + x;
-        const int64_t lab = P.labels[pix];
+        const int64_t lab = static_cast<const L*>(P.labels)[pix];
         const float t00 = hy0l * wx0l, t01 = hy0l * wx1l, t10 = hy1l * wx0l, t11 = hy1l * wx1l;
         auto up = [&](int c) {
           const float* z = z_s + c * (kCeHalo * kCeHalo) + i00;
@@ -249,7 +249,9 @@ __device__ __forceinline__ float ex2_approx(float x) {
   return y;
 }
 
-template <int CMAX, bool EXACT, bool FAST, bool GRAD, int TY>
+// L = uint8: a cell row of 4 labels starts 2 pixels into a 4-pixel group (xb = 4 kx + 2), so it is
+// read as two 16-bit halves, as the int64 kernel reads two 16-byte halves (2-byte aligned rows).
+template <int CMAX, bool EXACT, bool FAST, bool GRAD, int TY, class L>
 __global__ void __launch_bounds__(kCeTile * TY, 512 / (kCeTile * TY))
 weighted_ce_s4_kernel(const CeParams P) {
   extern __shared__ __align__(16) float ce_smem[];
@@ -267,7 +269,7 @@ weighted_ce_s4_kernel(const CeParams P) {
   const int ky = ly0 + cy, kx = lx0 + cx;
   const bool active = ky < P.lh && kx < P.lw;
   const int xb = 4 * kx + 2, yb = 4 * ky + 2;
-  const int64_t* labp = P.labels + (int64_t)b * P.H * P.W;
+  const L* labp = static_cast<const L*>(P.labels) + (int64_t)b * P.H * P.W;
   const float* wp = P.weight ? P.weight + (int64_t)b * P.H * P.W : nullptr;
 
   // the cell's sixteen pixels first (all loads in flight before anything waits): labels as bytes
@@ -278,6 +280,7 @@ weighted_ce_s4_kernel(const CeParams P) {
     return (l == P.ignore_index || l < 0 || l >= C) ? 255u : (unsigned)l;
   };
   longlong2 lraw[4][2];
+  uint16_t lraw8[4][2];
   float2 wraw[4][2];
   {
     const bool right = xb + 3 < P.W;                  // false only in the last cell column (2 pixels)
@@ -286,8 +289,13 @@ weighted_ce_s4_kernel(const CeParams P) {
       const int y = yb + i;
       const int64_t o = (int64_t)y * P.W + xb;
       const bool rowok = active && y < P.H;
-      lraw[i][0] = rowok ? *reinterpret_cast<const longlong2*>(labp + o) : make_longlong2(-1, -1);
-      lraw[i][1] = rowok && right ? *reinterpret_cast<const longlong2*>(labp + o + 2) : make_longlong2(-1, -1);
+      if constexpr (sizeof(L) == 1) {
+        lraw8[i][0] = rowok ? *reinterpret_cast<const uint16_t*>(labp + o) : (uint16_t)0xffffu;
+        lraw8[i][1] = rowok && right ? *reinterpret_cast<const uint16_t*>(labp + o + 2) : (uint16_t)0xffffu;
+      } else {
+        lraw[i][0] = rowok ? *reinterpret_cast<const longlong2*>(labp + o) : make_longlong2(-1, -1);
+        lraw[i][1] = rowok && right ? *reinterpret_cast<const longlong2*>(labp + o + 2) : make_longlong2(-1, -1);
+      }
       if (wp) {
         wraw[i][0] = rowok ? *reinterpret_cast<const float2*>(wp + o) : make_float2(0.f, 0.f);
         wraw[i][1] = rowok && right ? *reinterpret_cast<const float2*>(wp + o + 2) : make_float2(0.f, 0.f);
@@ -319,8 +327,12 @@ weighted_ce_s4_kernel(const CeParams P) {
   }
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
-    lab4[i] = lab_byte(lraw[i][0].x) | (lab_byte(lraw[i][0].y) << 8) | (lab_byte(lraw[i][1].x) << 16) |
-              (lab_byte(lraw[i][1].y) << 24);
+    if constexpr (sizeof(L) == 1)
+      lab4[i] = lab_byte(lraw8[i][0] & 255u) | (lab_byte(lraw8[i][0] >> 8) << 8) |
+                (lab_byte(lraw8[i][1] & 255u) << 16) | (lab_byte(lraw8[i][1] >> 8) << 24);
+    else
+      lab4[i] = lab_byte(lraw[i][0].x) | (lab_byte(lraw[i][0].y) << 8) | (lab_byte(lraw[i][1].x) << 16) |
+                (lab_byte(lraw[i][1].y) << 24);
     wv[i][0] = wraw[i][0].x; wv[i][1] = wraw[i][0].y; wv[i][2] = wraw[i][1].x; wv[i][3] = wraw[i][1].y;
   }
   __syncthreads();
@@ -501,13 +513,10 @@ weighted_ce_s4_kernel(const CeParams P) {
   }
 }
 
-}  // namespace pfst
-
-extern "C" {
-
-int pfst_weighted_ce(const float* logits, const int64_t* labels, const float* weight, const float* class_weight,
-                     int64_t B, int32_t C, int32_t lh, int32_t lw, int32_t H, int32_t W, int64_t ignore_index,
-                     float loss_weight, float* grad_logits, double* stats, float* out2, void* stream) {
+template <class L>
+static int weighted_ce(const float* logits, const L* labels, const float* weight, const float* class_weight,
+                       int64_t B, int32_t C, int32_t lh, int32_t lw, int32_t H, int32_t W, int64_t ignore_index,
+                       float loss_weight, float* grad_logits, double* stats, float* out2, void* stream) {
   if (!logits || !labels || !stats || !out2 || B < 0 || C < 1 || lh < 1 || lw < 1 || H < 1 || W < 1)
     return PFST_ERR_INVALID_ARG;
   if (C > pfst::kCeMaxC || B > 65535) return PFST_ERR_UNSUPPORTED;
@@ -528,14 +537,15 @@ int pfst_weighted_ce(const float* logits, const int64_t* labels, const float* we
   static const bool force_v1 = getenv("PFST_CE_V1") != nullptr;
   static const bool fast = getenv("PFST_CE_EXACT") == nullptr;
   static const int ty = getenv("PFST_CE_TY") ? atoi(getenv("PFST_CE_TY")) : 8;
-  if (!force_v1 && C <= 8 && H == 4 * lh && W == 4 * lw) {
+  const bool rows_ok = sizeof(L) == 8 || (reinterpret_cast<uintptr_t>(labels) & 1u) == 0;
+  if (!force_v1 && C <= 8 && H == 4 * lh && W == 4 * lw && rows_ok) {
     const int TY = ty == 16 ? 16 : 8;
     const dim3 grid4((unsigned)((lw + pfst::kCeTile - 1) / pfst::kCeTile), (unsigned)((lh + TY - 1) / TY), (unsigned)B);
     if (grid4.y > 65535) return PFST_ERR_UNSUPPORTED;
     const size_t smem4 = ((size_t)C * pfst::kCeHalo * (TY + 1) + (size_t)C * 4 * pfst::kCeTile * TY) * sizeof(float);
     void (*k4)(const pfst::CeParams);
     const bool gr = grad_logits != nullptr;
-#define PFST_CE_PICK2(CM, EX, F, G) (TY == 16 ? pfst::weighted_ce_s4_kernel<CM, EX, F, G, 16> : pfst::weighted_ce_s4_kernel<CM, EX, F, G, 8>)
+#define PFST_CE_PICK2(CM, EX, F, G) (TY == 16 ? pfst::weighted_ce_s4_kernel<CM, EX, F, G, 16, L> : pfst::weighted_ce_s4_kernel<CM, EX, F, G, 8, L>)
 #define PFST_CE_PICK(CM, EX)                                                       \
   (fast ? (gr ? PFST_CE_PICK2(CM, EX, true, true) : PFST_CE_PICK2(CM, EX, true, false)) \
         : (gr ? PFST_CE_PICK2(CM, EX, false, true) : PFST_CE_PICK2(CM, EX, false, false)))
@@ -557,12 +567,36 @@ int pfst_weighted_ce(const float* logits, const int64_t* labels, const float* we
   const bool use_priv = tile + priv <= 100 * 1024;          // keeps two blocks per SM
   const size_t smem = tile + (use_priv ? priv : 0);
   if (smem > 200 * 1024) return PFST_ERR_UNSUPPORTED;
-  auto k = C <= pfst::kCeRegC ? pfst::weighted_ce_kernel<true, true>
-                              : (use_priv ? pfst::weighted_ce_kernel<false, true> : pfst::weighted_ce_kernel<false, false>);
+  auto k = C <= pfst::kCeRegC ? pfst::weighted_ce_kernel<true, true, L>
+                              : (use_priv ? pfst::weighted_ce_kernel<false, true, L> : pfst::weighted_ce_kernel<false, false, L>);
   PFST_CUDA_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "pfst_weighted_ce/attr");
   k<<<grid, pfst::kCeThreads, smem, s>>>(P);
   PFST_CHECK_LAUNCH("pfst_weighted_ce");
   return PFST_OK;
+}
+
+}  // namespace pfst
+
+extern "C" {
+
+int pfst_weighted_ce(const float* logits, const int64_t* labels, const float* weight, const float* class_weight,
+                     int64_t B, int32_t C, int32_t lh, int32_t lw, int32_t H, int32_t W, int64_t ignore_index,
+                     float loss_weight, float* grad_logits, double* stats, float* out2, void* stream) {
+  return pfst::weighted_ce(logits, labels, weight, class_weight, B, C, lh, lw, H, W, ignore_index, loss_weight,
+                           grad_logits, stats, out2, stream);
+}
+
+int pfst_weighted_ce_lbl(const float* logits, const void* labels, int32_t label_dtype, const float* weight,
+                         const float* class_weight, int64_t B, int32_t C, int32_t lh, int32_t lw, int32_t H,
+                         int32_t W, int64_t ignore_index, float loss_weight, float* grad_logits, double* stats,
+                         float* out2, void* stream) {
+  if (label_dtype == PFST_DT_I64)
+    return pfst::weighted_ce(logits, static_cast<const int64_t*>(labels), weight, class_weight, B, C, lh, lw, H, W,
+                             ignore_index, loss_weight, grad_logits, stats, out2, stream);
+  if (label_dtype == PFST_DT_U8)
+    return pfst::weighted_ce(logits, static_cast<const uint8_t*>(labels), weight, class_weight, B, C, lh, lw, H, W,
+                             ignore_index, loss_weight, grad_logits, stats, out2, stream);
+  return PFST_ERR_UNSUPPORTED;
 }
 
 }  // extern "C"

@@ -136,19 +136,23 @@ class PluginEngine:
         return self.bank
 
     def teacher_outputs(self, ema_logits: torch.Tensor, x_ema: Optional[torch.Tensor], thr: float,
-                        thr_vec: Optional[torch.Tensor], want_part: bool, geo: Optional[ops.LossGeometry]):
-        """-> (pseudo_label int64 (B,H,W), pseudo_prob fp32, count int64[1], part-weight|None).
-        x_ema: the (B,D,h,w) teacher features (None: no loss / prototypes on features)."""
+                        thr_vec: Optional[torch.Tensor], want_part: bool, geo: Optional[ops.LossGeometry],
+                        label_dtype: torch.dtype = torch.int64):
+        """-> (pseudo_label (B,H,W) of label_dtype (int64 or uint8, the dtype of the batch's gt), pseudo_prob
+        fp32, count int64[1], part-weight|None). x_ema: the (B,D,h,w) teacher features (None: no loss /
+        prototypes on features)."""
+        if label_dtype not in ops.LABEL_DTYPES:
+            raise TypeError(f"label maps must be torch.int64 or torch.uint8, got {label_dtype}")
         B, Cc, H, W = ema_logits.shape
         ops._dev(ema_logits, "ema_logits", torch.float32)
         use_x = x_ema is not None and (self.loss_cfg is not None or self.proto_cfg is not None)
         if use_x:
             ops._dev(x_ema, "x_ema", torch.float32)
-        skey = ("a", tuple(ema_logits.shape), None if not use_x else tuple(x_ema.shape), want_part)
+        skey = ("a", tuple(ema_logits.shape), None if not use_x else tuple(x_ema.shape), want_part, label_dtype)
         b = self._bufs.get(skey)
         if b is None:
             e = lambda shape, dt: torch.empty(shape, dtype=dt, device=self.device)  # noqa: E731
-            b = dict(label=e((B, H, W), torch.int64), conf=e((B, H, W), torch.float32), count=e((1,), torch.int64),
+            b = dict(label=e((B, H, W), label_dtype), conf=e((B, H, W), torch.float32), count=e((1,), torch.int64),
                      wpart=e((B, H, W), torch.float32) if want_part else None, dots=None, ks=0)
             if use_x and self.loss_cfg is not None:
                 Bf, D, h, w = x_ema.shape
@@ -167,9 +171,9 @@ class PluginEngine:
                 with torch.cuda.stream(self._side):
                     ops.neigh_dots_slot(x_ema, geo.dilation // geo.up, 0, b["dots"])
                     self._ev[3].record(self._side)
-            _lib.call("pfst_pseudo_label", ema_logits.data_ptr(), B, Cc, H * W, float(thr),
+            _lib.call("pfst_pseudo_label_lbl", ema_logits.data_ptr(), B, Cc, H * W, float(thr),
                       None if thr_vec is None else thr_vec.data_ptr(), 0, -1, b["label"].data_ptr(),
-                      b["conf"].data_ptr(), None if b["wpart"] is None else b["wpart"].data_ptr(),
+                      ops._TORCH2DT[label_dtype], b["conf"].data_ptr(), None if b["wpart"] is None else b["wpart"].data_ptr(),
                       b["count"].data_ptr(), main.cuda_stream)
             masked = bank is not None and bank.masked(x_ema.shape[2], x_ema.shape[3], x_ema)
             if dots_here and not masked:
@@ -212,14 +216,15 @@ class PluginEngine:
         a = self._a
         if a is None or a["dots"] is None:
             raise PfstError("aux_forward without teacher_outputs(x_ema) in this iteration")
-        for name, t, dt in (("logits_trg", logits_trg, torch.float32), ("x_src", x_src, torch.float32),
-                            ("gt", gt, torch.int64), ("mix_masks", mix_masks, torch.int64)):
+        for name, t, dt in (("logits_trg", logits_trg, torch.float32), ("x_src", x_src, torch.float32)):
             ops._dev(t, name, dt)
+        ldt = ops._labels(gt, "gt")                  # int64 or uint8; mix_masks shares gt's dtype
+        ops._labels(mix_masks, "mix_masks", like=gt)
         Bf, D, h, w = x_src.shape
         if a["dots"].shape[2:] != (Bf, 5, h, w):
             raise PfstError("PFGSTLoss: x_ema / x_src shape mismatch")
         bank = self.bank if self.proto_cfg is not None else None
-        skey = ("b", tuple(logits_trg.shape), tuple(x_src.shape), tuple(gt.shape), want_vis)
+        skey = ("b", tuple(logits_trg.shape), tuple(x_src.shape), tuple(gt.shape), want_vis, gt.dtype)
         b = self._bufs.get(skey)
         if b is None:
             e = lambda shape, dt: torch.empty(shape, dtype=dt, device=self.device)  # noqa: E731
@@ -249,22 +254,22 @@ class PluginEngine:
                 ops.neigh_dots_slot(x_src, geo.dilation // geo.up, 1, dots)
                 self._ev[5].record(self._side)
                 if bank is not None:
-                    _lib.call("pfst_proto_dist_fwd", x_src.data_ptr(), Bf, D, h, w, gt.data_ptr(), H, W,
+                    _lib.call("pfst_proto_dist_fwd_lbl", x_src.data_ptr(), Bf, D, h, w, gt.data_ptr(), ldt, H, W,
                               bank.mu.data_ptr(), bank.seen.data_ptr(), self.C, b["dist"].data_ptr(),
                               b["acc"].data_ptr(), b["ploss"].data_ptr(), self._side.cuda_stream)
                     _lib.call("pfst_pack_scalars", pp, pw, 1, b["ploss_w"].data_ptr(), self._side.cuda_stream)
                     self._ev[6].record(self._side)
             main.wait_event(self._ev[5])
-            _lib.call("pfst_pfgst_loss_fwd", *common, b["losses"].data_ptr(),
+            _lib.call("pfst_pfgst_loss_fwd_lbl", *common, b["losses"].data_ptr(),
                       None if b["density"] is None else b["density"].data_ptr(),
-                      None if b["eroded"] is None else b["eroded"].data_ptr(), main.cuda_stream)
+                      None if b["eroded"] is None else b["eroded"].data_ptr(), *ops.SHIPPED_LOSS_ARGS, ldt, main.cuda_stream)
             if bank is not None:
                 main.wait_event(self._ev[6])
 
         key = skey + (logits_trg.data_ptr(), x_src.data_ptr(), gt.data_ptr(), mix_masks.data_ptr(), dots.data_ptr(),
                       bank is not None)
         return dict(key=key, launch=launch, common=common, w6=w6, b=b, geo=geo, bank=bank, keep=(pw, pp),
-                    shapes=(Bf, D, h, w, H, W))
+                    shapes=(Bf, D, h, w, H, W), ldt=ldt)
 
     def aux_run(self, plan: dict) -> None:
         self._gb.run(plan["key"], plan["launch"])
@@ -298,15 +303,15 @@ class PluginEngine:
         Bf, D, h, w, H, W = f["shapes"]
         coef = torch.empty((Bf, 9, h, w), dtype=torch.float32, device=self.device)
         glog = torch.empty_like(logits_trg) if need_logits else None
-        _lib.call("pfst_pfgst_loss_bwd", *f["common"], self._gout.data_ptr(), coef.data_ptr(),
-                  None if glog is None else glog.data_ptr(), s)
+        _lib.call("pfst_pfgst_loss_bwd_lbl", *f["common"], self._gout.data_ptr(), coef.data_ptr(),
+                  None if glog is None else glog.data_ptr(), *ops.SHIPPED_LOSS_ARGS, f["ldt"], s)
         gx = None
         if need_x:
             gx = torch.empty_like(x_src)
             d = geo.dilation // geo.up
             if bank is not None:
-                _lib.call("pfst_neigh_grad_proto", x_src.data_ptr(), coef.data_ptr(), Bf, D, h, w, d, gt.data_ptr(),
-                          H, W, bank.mu.data_ptr(), bank.seen.data_ptr(), self.C, b["dist"].data_ptr(),
+                _lib.call("pfst_neigh_grad_proto_lbl", x_src.data_ptr(), coef.data_ptr(), Bf, D, h, w, d,
+                          gt.data_ptr(), f["ldt"], H, W, bank.mu.data_ptr(), bank.seen.data_ptr(), self.C, b["dist"].data_ptr(),
                           b["acc"].data_ptr(), self._gout.data_ptr() + 24, gx.data_ptr(), s)
             else:
                 _lib.call("pfst_neigh_grad", x_src.data_ptr(), coef.data_ptr(), Bf, D, h, w, d, gx.data_ptr(), s)

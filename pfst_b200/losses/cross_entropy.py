@@ -33,8 +33,8 @@ class _UpsampleCE(torch.autograd.Function):
         grad = torch.empty_like(seg_logit) if need_grad else None
         stats = torch.empty(4, dtype=torch.float64, device=dev)
         out2 = torch.empty(2, dtype=torch.float32, device=dev)
-        _lib.call("pfst_weighted_ce", ops._dev(seg_logit, "seg_logit", torch.float32),
-                  ops._dev(labels, "seg_label", torch.int64), ops._opt(seg_weight, "seg_weight", torch.float32),
+        _lib.call("pfst_weighted_ce_lbl", ops._dev(seg_logit, "seg_logit", torch.float32),
+                  labels.data_ptr(), ops._labels(labels, "seg_label"), ops._opt(seg_weight, "seg_weight", torch.float32),
                   ops._opt(class_weight, "class_weight", torch.float32), B, C, lh, lw, H, W, int(ignore_index),
                   float(loss_weight), None if grad is None else grad.data_ptr(), stats.data_ptr(), out2.data_ptr(),
                   ops._stream())
@@ -52,7 +52,7 @@ class _UpsampleCE(torch.autograd.Function):
 def upsample_cross_entropy(seg_logit: torch.Tensor, seg_label: torch.Tensor, seg_weight: Optional[torch.Tensor] = None,
                            class_weight: Optional[torch.Tensor] = None, ignore_index: int = 255,
                            loss_weight: float = 1.0):
-    """-> (loss 0-dim, acc_seg (1,)). seg_logit (B,C,lh,lw) fp32; seg_label (B,1,H,W) or (B,H,W) int64;
+    """-> (loss 0-dim, acc_seg (1,)). seg_logit (B,C,lh,lw) fp32; seg_label (B,1,H,W) or (B,H,W) int64 or uint8;
     seg_weight (B,H,W) fp32 or None; class_weight (C,) fp32 or None."""
     if seg_label.dim() == 4:
         seg_label = seg_label[:, 0]

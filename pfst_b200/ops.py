@@ -33,6 +33,20 @@ def _opt(t: Optional[torch.Tensor], name: str, dtype=None) -> Optional[int]:
     return None if t is None else _dev(t, name, dtype)
 
 
+LABEL_DTYPES = (torch.int64, torch.uint8)
+
+
+def _labels(t: torch.Tensor, name: str, like: Optional[torch.Tensor] = None) -> int:
+    """Checks a label map (int64, the reference dtype, or uint8, the dtype datasets store) and returns
+    its PFST_DT_* tag. `like`: another label map of the same call, whose dtype it must share."""
+    if isinstance(t, torch.Tensor) and t.dtype not in LABEL_DTYPES:
+        raise TypeError(f"{name}: label maps must be torch.int64 or torch.uint8, got {t.dtype}")
+    if like is not None and isinstance(t, torch.Tensor) and t.dtype != like.dtype:
+        raise TypeError(f"{name}: every label map of one call has one dtype ({like.dtype}), got {t.dtype}")
+    _dev(t, name)
+    return _TORCH2DT[t.dtype]
+
+
 def _stream() -> int:
     # raw cudaStream_t of torch's current stream (also the capturing stream inside torch.cuda.graph);
     # the public torch.cuda.current_stream() builds a Stream object per call (~2 us each, ~10 per step)
@@ -133,13 +147,20 @@ def ema_update_flat(ema: torch.Tensor, param: torch.Tensor, a32: float, b32: flo
 
 # ---------------------------------------------------------- S1/S2: pseudo labels
 def pseudo_label(logits: torch.Tensor, thr: float = 0.0, thr_per_class: Optional[torch.Tensor] = None,
-                 mode: int = 0, reject_label: int = -1, want_part_weight: bool = False):
-    """-> (label int64 (B,H,W), conf fp32 (B,H,W), count int64[1] on device, weight_part|None)."""
+                 mode: int = 0, reject_label: int = -1, want_part_weight: bool = False,
+                 label_dtype: torch.dtype = torch.int64):
+    """-> (label (B,H,W) of label_dtype (int64 or uint8), conf fp32 (B,H,W), count int64[1] on device,
+    weight_part|None). uint8 labels need C <= 255 and reject_label <= 255 (negative: no rejection)."""
     if logits.dim() != 4:
         raise ValueError("logits must be (B,C,H,W)")
     B, Cc, H, W = logits.shape
     _dev(logits, "logits", torch.float32)
-    label = torch.empty((B, H, W), dtype=torch.int64, device=logits.device)
+    if label_dtype not in LABEL_DTYPES:
+        raise TypeError(f"label_dtype must be torch.int64 or torch.uint8, got {label_dtype}")
+    if label_dtype == torch.uint8 and (Cc > 255 or int(reject_label) > 255):
+        raise ValueError(f"uint8 pseudo labels need C <= 255 (got {Cc}) and reject_label <= 255 "
+                         f"(got {reject_label}; a negative value means no rejection)")
+    label = torch.empty((B, H, W), dtype=label_dtype, device=logits.device)
     conf = torch.empty((B, H, W), dtype=torch.float32, device=logits.device)
     count = torch.empty(1, dtype=torch.int64, device=logits.device)  # written as uint64
     wpart = torch.empty((B, H, W), dtype=torch.float32, device=logits.device) if want_part_weight else None
@@ -147,9 +168,9 @@ def pseudo_label(logits: torch.Tensor, thr: float = 0.0, thr_per_class: Optional
         if thr_per_class.numel() != Cc:
             raise ValueError("thr_per_class must have C entries")
         _dev(thr_per_class, "thr_per_class", torch.float32)
-    _lib.call("pfst_pseudo_label", logits.data_ptr(), B, Cc, H * W, float(thr),
+    _lib.call("pfst_pseudo_label_lbl", logits.data_ptr(), B, Cc, H * W, float(thr),
               None if thr_per_class is None else thr_per_class.data_ptr(), mode, int(reject_label),
-              label.data_ptr(), conf.data_ptr(), None if wpart is None else wpart.data_ptr(),
+              label.data_ptr(), _TORCH2DT[label_dtype], conf.data_ptr(), None if wpart is None else wpart.data_ptr(),
               count.data_ptr(), _stream())
     return label, conf, count, wpart
 
@@ -165,11 +186,12 @@ def pseudo_weight_fill(shape, count: torch.Tensor, ps_size: int, ignore_top: int
 
 # ------------------------------------------------------------- M1/M2: ClassMix
 def class_presence(gt: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """-> int32[9] on device: 256 presence bits + out-of-range flag."""
-    _dev(gt, "gt", torch.int64)
+    """gt: int64 or uint8. -> int32[9] on device: 256 presence bits + out-of-range flag."""
+    dt = _labels(gt, "gt")
     if out is None:
         out = torch.empty(9, dtype=torch.int32, device=gt.device)
-    _lib.call("pfst_class_presence", gt.data_ptr(), gt.numel(), _dev(out, "presence", torch.int32), _stream())
+    _lib.call("pfst_class_presence_lbl", gt.data_ptr(), dt, gt.numel(), _dev(out, "presence", torch.int32),
+              _stream())
     return out
 
 
@@ -178,9 +200,10 @@ def class_mix(gt: torch.Tensor, chosen: torch.Tensor, img: Optional[torch.Tensor
               weight_in: Optional[torch.Tensor] = None, count: Optional[torch.Tensor] = None,
               ps_size: int = 0, ignore_top: int = 0, ignore_bottom: int = 0,
               want_weight: bool = True, want_mask: bool = True, weight_out: Optional[torch.Tensor] = None):
-    """Fused ClassMix. gt (B,1,H,W) int64; chosen int32 (B,8) bitmasks.
+    """Fused ClassMix. gt (B,1,H,W) int64 or uint8; chosen int32 (B,8) bitmasks. The pseudo label, the
+    mixed label and the mask share gt's dtype.
     -> (mixed_img|None, mixed_lbl|None, mixed_weight|None, mix_mask|None)"""
-    _dev(gt, "gt", torch.int64)
+    dt = _labels(gt, "gt")
     B, H, W = gt.shape[0], gt.shape[-2], gt.shape[-1]
     if gt.numel() != B * H * W:
         raise ValueError("gt must be (B,1,H,W) or (B,H,W)")
@@ -198,10 +221,10 @@ def class_mix(gt: torch.Tensor, chosen: torch.Tensor, img: Optional[torch.Tensor
         channels = img.shape[1]
         mixed_img = torch.empty_like(img)
     if pseudo_lbl is not None:
-        _dev(pseudo_lbl, "pseudo_label", torch.int64)
+        _labels(pseudo_lbl, "pseudo_label", like=gt)
         if pseudo_lbl.numel() != B * H * W:
             raise ValueError("pseudo_label shape mismatch")
-        mixed_lbl = torch.empty((B, 1, H, W), dtype=torch.int64, device=dev)
+        mixed_lbl = torch.empty((B, 1, H, W), dtype=gt.dtype, device=dev)
     if want_weight:
         if weight_in is not None:
             _dev(weight_in, "weight_in", torch.float32)
@@ -210,11 +233,11 @@ def class_mix(gt: torch.Tensor, chosen: torch.Tensor, img: Optional[torch.Tensor
         mixed_w = weight_out if weight_out is not None else torch.empty((B, H, W), dtype=torch.float32, device=dev)
         _dev(mixed_w, "weight_out", torch.float32)
     if want_mask:
-        mask = torch.empty((B, 1, H, W), dtype=torch.int64, device=dev)
+        mask = torch.empty((B, 1, H, W), dtype=gt.dtype, device=dev)
     p = lambda t: None if t is None else t.data_ptr()
-    _lib.call("pfst_class_mix", gt.data_ptr(), chosen.data_ptr(), p(img), p(trg_img), p(pseudo_lbl),
+    _lib.call("pfst_class_mix_lbl", gt.data_ptr(), chosen.data_ptr(), p(img), p(trg_img), p(pseudo_lbl),
               p(weight_in) if want_weight else None, p(count), int(ps_size), int(ignore_top),
-              int(ignore_bottom), B, channels, H, W, p(mixed_img), p(mixed_lbl), p(mixed_w), p(mask),
+              int(ignore_bottom), B, channels, H, W, p(mixed_img), p(mixed_lbl), p(mixed_w), p(mask), dt,
               _stream())
     return mixed_img, mixed_lbl, mixed_w, mask
 
@@ -431,7 +454,7 @@ def neigh_dots_slot(x: torch.Tensor, dilation: int, slot: int, dots: Optional[to
 
 def neigh_grad(x: torch.Tensor, coef: torch.Tensor, dilation: int, out: Optional[torch.Tensor] = None,
                proto: Optional[dict] = None) -> torch.Tensor:
-    """grad_x of the neighbourhood-cosine losses; with `proto` (labels (B,H,W) int64, mu, seen,
+    """grad_x of the neighbourhood-cosine losses; with `proto` (labels (B,H,W) int64 or uint8, mu, seen,
     dist, acc, grad_loss — the saved state of pfst_proto_dist_fwd) the prototype-distance
     gradient is added in the same pass over x."""
     _dev(x, "x", torch.float32)
@@ -446,8 +469,9 @@ def neigh_grad(x: torch.Tensor, coef: torch.Tensor, dilation: int, out: Optional
                   _stream())
     else:
         lab, mu, seen = proto["labels"], proto["mu"], proto.get("seen")
-        _lib.call("pfst_neigh_grad_proto", x.data_ptr(), coef.data_ptr(), B, D, h, w, int(dilation),
-                  _dev(lab, "labels", torch.int64), lab.shape[-2], lab.shape[-1], _dev(mu, "mu", torch.float32),
+        dt = _labels(lab, "labels")
+        _lib.call("pfst_neigh_grad_proto_lbl", x.data_ptr(), coef.data_ptr(), B, D, h, w, int(dilation),
+                  lab.data_ptr(), dt, lab.shape[-2], lab.shape[-1], _dev(mu, "mu", torch.float32),
                   _opt(seen, "seen", torch.uint8), mu.shape[0], _dev(proto["dist"], "dist", torch.float32),
                   _dev(proto["acc"], "acc", torch.float64), _dev(proto["grad_loss"], "grad_loss", torch.float32),
                   grad.data_ptr(), _stream())
@@ -486,6 +510,9 @@ def _w6(weights6):
 
 
 LOSS_SIM_GAUSSIAN, LOSS_CROSS_PROB_EMA, LOSS_UNFOLD_GRAD, LOSS_SRC_MARGIN, LOSS_SRC_MARGIN2 = 1, 2, 4, 8, 16   # PFST_LOSS_*
+# the (options, sigma, logits_ema, margin) arguments of pfst_pfgst_loss_{fwd,bwd}_lbl for the shipped
+# configuration: options 0, so sigma, logits_ema and margin are not read
+SHIPPED_LOSS_ARGS = (0, 0.0, None, None)
 
 
 def _loss_options(options: int, logits_ema, geo: LossGeometry):
@@ -508,12 +535,13 @@ def _margin(margin):
 
 def pfgst_loss_fwd(dots, ks, geo: LossGeometry, logits, gt, mix, top_k, weights6, want_vis=True,
                    options: int = 0, sigma: float = 30.0, logits_ema=None, margin=None):
-    """-> (losses float32[6], (stats float64[16], workspace), density|None, eroded|None)."""
+    """gt / mix: int64 or uint8, one dtype.
+    -> (losses float32[6], (stats float64[16], workspace), density|None, eroded|None)."""
     dev = logits.device
     _dev(dots, "dots", torch.float32)
     _dev(logits, "logits", torch.float32)
-    _dev(gt, "gt", torch.int64)
-    _dev(mix, "mix", torch.int64)
+    dt = _labels(gt, "gt")
+    _labels(mix, "mix", like=gt)
     q_ptr = _loss_options(options, logits_ema, geo)
     stats = torch.empty(16, dtype=torch.float64, device=dev)
     ws_bytes = int(_lib.load().pfst_pfgst_loss_ws_bytes_ex(geo.B, geo.C, geo.fh, geo.fw, geo.up, int(options)))
@@ -521,11 +549,11 @@ def pfgst_loss_fwd(dots, ks, geo: LossGeometry, logits, gt, mix, top_k, weights6
     losses = torch.empty(6, dtype=torch.float32, device=dev)
     density = torch.empty((geo.B, 1, geo.gh, geo.gw), dtype=torch.float32, device=dev) if want_vis else None
     eroded = torch.empty((geo.B, 1, geo.gh, geo.gw), dtype=torch.uint8, device=dev) if want_vis else None
-    _lib.call("pfst_pfgst_loss_fwd_ex", dots.data_ptr(), ks, geo.B, geo.fh, geo.fw, geo.up, logits.data_ptr(),
+    _lib.call("pfst_pfgst_loss_fwd_lbl", dots.data_ptr(), ks, geo.B, geo.fh, geo.fw, geo.up, logits.data_ptr(),
               geo.C, geo.lh, geo.lw, geo.lscale, geo.lscale, gt.data_ptr(), mix.data_ptr(), geo.gt_h, geo.gt_w,
               geo.dilation, int(top_k), _w6(weights6), ws.data_ptr(), stats.data_ptr(), losses.data_ptr(),
               None if density is None else density.data_ptr(), None if eroded is None else eroded.data_ptr(),
-              int(options), float(sigma), q_ptr, _margin(margin), _stream())
+              int(options), float(sigma), q_ptr, _margin(margin), dt, _stream())
     return losses, (stats, ws), density, eroded
 
 
@@ -534,13 +562,15 @@ def pfgst_loss_bwd(dots, ks, geo: LossGeometry, logits, gt, mix, top_k, weights6
     """-> (coef (B,9,fh,fw), grad_logits|None)."""
     dev = logits.device
     _dev(grad_losses, "grad_losses", torch.float32)
+    dt = _labels(gt, "gt")
+    _labels(mix, "mix", like=gt)
     q_ptr = _loss_options(options, logits_ema, geo)
     stats, ws = stats
     coef = torch.empty((geo.B, 9, geo.fh, geo.fw), dtype=torch.float32, device=dev)
     glog = torch.empty_like(logits) if want_logits_grad else None
-    _lib.call("pfst_pfgst_loss_bwd_ex", dots.data_ptr(), ks, geo.B, geo.fh, geo.fw, geo.up, logits.data_ptr(),
+    _lib.call("pfst_pfgst_loss_bwd_lbl", dots.data_ptr(), ks, geo.B, geo.fh, geo.fw, geo.up, logits.data_ptr(),
               geo.C, geo.lh, geo.lw, geo.lscale, geo.lscale, gt.data_ptr(), mix.data_ptr(), geo.gt_h, geo.gt_w,
               geo.dilation, int(top_k), _w6(weights6), ws.data_ptr(), stats.data_ptr(), grad_losses.data_ptr(),
               coef.data_ptr(), None if glog is None else glog.data_ptr(), int(options), float(sigma), q_ptr,
-              _margin(margin), _stream())
+              _margin(margin), dt, _stream())
     return coef, glog

@@ -20,6 +20,7 @@ from ._lib import PfstError
 
 
 def _lab3(labels: torch.Tensor) -> torch.Tensor:
+    """(B,1,H,W) or (B,H,W) label map, int64 or uint8 -> contiguous (B,H,W) of the same dtype."""
     if labels.dim() == 4:
         labels = labels[:, 0]
     return labels.contiguous()
@@ -142,7 +143,7 @@ class PrototypeBank:
                 raise PfstError(f"prototype accumulation does not support B={B}, h={h}, w={w}, C={self.C}")
             self._order_ws = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
             self._order_key = key
-        _lib.call("pfst_proto_order", ops._dev(labels, "labels", torch.int64), B, h, w, labels.shape[-2],
+        _lib.call("pfst_proto_order_lbl", labels.data_ptr(), ops._labels(labels, "labels"), B, h, w, labels.shape[-2],
                   labels.shape[-1], ops._opt(conf, "conf", torch.float32), float(conf_thr), self.C,
                   self.packed.data_ptr() + 4 * self.C * self.D, self._order_ws.data_ptr(), ops._stream())
 
@@ -162,8 +163,8 @@ class PrototypeBank:
         B, D, h, w = feats.shape
         if D != self.D:
             raise ValueError("feature dim mismatch")
-        _lib.call("pfst_proto_accum", ops._dev(feats, "feats", torch.float32), B, D, h, w,
-                  ops._dev(labels, "labels", torch.int64), labels.shape[-2], labels.shape[-1],
+        _lib.call("pfst_proto_accum_lbl", ops._dev(feats, "feats", torch.float32), B, D, h, w,
+                  labels.data_ptr(), ops._labels(labels, "labels"), labels.shape[-2], labels.shape[-1],
                   ops._opt(conf, "conf", torch.float32), float(conf_thr), self.C, self.packed.data_ptr(),
                   ops._stream())
 
@@ -223,8 +224,8 @@ class _ProtoDistFn(torch.autograd.Function):
         dist = torch.empty((B, h, w), dtype=torch.float32, device=dev)
         acc = torch.empty(4, dtype=torch.float64, device=dev)
         loss = torch.empty(1, dtype=torch.float32, device=dev)
-        _lib.call("pfst_proto_dist_fwd", ops._dev(feats, "feats", torch.float32), B, D, h, w,
-                  ops._dev(labels, "labels", torch.int64), labels.shape[-2], labels.shape[-1],
+        _lib.call("pfst_proto_dist_fwd_lbl", ops._dev(feats, "feats", torch.float32), B, D, h, w,
+                  labels.data_ptr(), ops._labels(labels, "labels"), labels.shape[-2], labels.shape[-1],
                   ops._dev(mu, "mu", torch.float32), ops._opt(seen, "seen", torch.uint8), C, dist.data_ptr(),
                   acc.data_ptr(), loss.data_ptr(), ops._stream())
         ctx.save_for_backward(feats, labels, mu, seen, dist, acc)
@@ -236,7 +237,8 @@ class _ProtoDistFn(torch.autograd.Function):
         B, D, h, w = feats.shape
         grad = torch.empty_like(feats)
         g = grad_out.reshape(1).contiguous().float()
-        _lib.call("pfst_proto_dist_bwd", feats.data_ptr(), B, D, h, w, labels.data_ptr(), labels.shape[-2],
+        _lib.call("pfst_proto_dist_bwd_lbl", feats.data_ptr(), B, D, h, w, labels.data_ptr(),
+                  ops._labels(labels, "labels"), labels.shape[-2],
                   labels.shape[-1], mu.data_ptr(), None if seen is None else seen.data_ptr(), mu.shape[0],
                   dist.data_ptr(), acc.data_ptr(), g.data_ptr(), grad.data_ptr(), 0, ops._stream())
         return grad, None, None, None

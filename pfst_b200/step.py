@@ -54,12 +54,15 @@ W6_DEFAULT = (0.1, 0.1, 0.1, 0.1, 0.1, 0.1)   # src_pos, src_neg, src_pos_std, s
 class _Buffers:
     """Every output / workspace of one step for a fixed set of input shapes."""
 
-    def __init__(self, dev, B, C, H, W, img_shape, logits_shape, feat_shape, geo: ops.LossGeometry):
+    def __init__(self, dev, B, C, H, W, img_shape, logits_shape, feat_shape, geo: ops.LossGeometry,
+                 label_dtype=torch.int64):
         f32, i64 = torch.float32, torch.int64
         e = lambda shape, dt: torch.empty(shape, dtype=dt, device=dev)  # noqa: E731
-        self.label, self.conf, self.count = e((B, H, W), i64), e((B, H, W), f32), e((1,), i64)
-        self.mixed_img, self.mixed_lbl = e(img_shape, f32), e((B, 1, H, W), i64)
-        self.weight, self.mix_mask = e((B, H, W), f32), e((B, 1, H, W), i64)
+        # the label maps follow gt's dtype (int64 or uint8)
+        self.ldt = ops._TORCH2DT[label_dtype]
+        self.label, self.conf, self.count = e((B, H, W), label_dtype), e((B, H, W), f32), e((1,), i64)
+        self.mixed_img, self.mixed_lbl = e(img_shape, f32), e((B, 1, H, W), label_dtype)
+        self.weight, self.mix_mask = e((B, H, W), f32), e((B, 1, H, W), label_dtype)
         Bf, D, h, w = feat_shape
         self.ks = ops.neigh_dots_splits(Bf, D, h, w)
         self.dots = e((self.ks, 2, Bf, 5, h, w), f32)
@@ -140,8 +143,8 @@ class SelfTrainingStep:
         with torch.cuda.stream(self._side):                       # branch 2: L2 on x_ema
             ops.neigh_dots_slot(x_ema, geo.dilation // geo.up, 0, b.dots)
             join.record(self._side)
-        _lib.call("pfst_pseudo_label", ema_logits.data_ptr(), B, C, H * W, float(self.thr), None, 0, -1,
-                  b.label.data_ptr(), b.conf.data_ptr(), None, b.count.data_ptr(), ops._stream())
+        _lib.call("pfst_pseudo_label_lbl", ema_logits.data_ptr(), B, C, H * W, float(self.thr), None, 0, -1,
+                  b.label.data_ptr(), b.ldt, b.conf.data_ptr(), None, b.count.data_ptr(), ops._stream())
         if self.bank.masked(x_ema.shape[2], x_ema.shape[3], x_ema):
             self.bank.accumulate(x_ema, b.label)                  # one masked launch next to dots(x_ema)
             main.wait_event(join)
@@ -162,7 +165,7 @@ class SelfTrainingStep:
         fork, dots_done, join = self._ev[2], self._ev[3], self._ev[4]
 
         def dist_fwd():
-            _lib.call("pfst_proto_dist_fwd", x_src.data_ptr(), Bf, D, h, w, gt.data_ptr(), H, W,
+            _lib.call("pfst_proto_dist_fwd_lbl", x_src.data_ptr(), Bf, D, h, w, gt.data_ptr(), b.ldt, H, W,
                       bank.mu.data_ptr(), bank.seen.data_ptr(), self.C, b.dist.data_ptr(), b.acc.data_ptr(),
                       b.ploss.data_ptr(), ops._stream())
 
@@ -177,26 +180,26 @@ class SelfTrainingStep:
                         self._side.wait_event(mu_ready)
                     dist_fwd()
                     join.record(self._side)
-            _lib.call("pfst_class_mix", gt.data_ptr(), chosen.data_ptr(), img.data_ptr(), trg_img.data_ptr(),
+            _lib.call("pfst_class_mix_lbl", gt.data_ptr(), chosen.data_ptr(), img.data_ptr(), trg_img.data_ptr(),
                       b.label.data_ptr(), None, b.count.data_ptr(), b.label.numel(), 0, 0, B, img.shape[1], H, W,
                       b.mixed_img.data_ptr(), b.mixed_lbl.data_ptr(), b.weight.data_ptr(), b.mix_mask.data_ptr(),
-                      s)
+                      b.ldt, s)
             main.wait_event(dots_done)
             w6 = ops._w6(self.w6)
             common = (b.dots.data_ptr(), b.ks, geo.B, geo.fh, geo.fw, geo.up, logits_trg.data_ptr(), geo.C,
                       geo.lh, geo.lw, geo.lscale, geo.lscale, gt.data_ptr(), b.mix_mask.data_ptr(), geo.gt_h,
                       geo.gt_w, geo.dilation, int(self.top_k), w6, b.ws.data_ptr(), b.stats.data_ptr())
-            _lib.call("pfst_pfgst_loss_fwd", *common, b.losses.data_ptr(), None, None, s)
+            _lib.call("pfst_pfgst_loss_fwd_lbl", *common, b.losses.data_ptr(), None, None, *ops.SHIPPED_LOSS_ARGS, b.ldt, s)
             # backward of (sum of the six losses + proto_weight * proto loss)
-            _lib.call("pfst_pfgst_loss_bwd", *common, self.gout.data_ptr(), b.coef.data_ptr(),
-                      b.grad_logits.data_ptr(), s)
+            _lib.call("pfst_pfgst_loss_bwd_lbl", *common, self.gout.data_ptr(), b.coef.data_ptr(),
+                      b.grad_logits.data_ptr(), *ops.SHIPPED_LOSS_ARGS, b.ldt, s)
             if part == "all":
                 main.wait_event(join)
         if part == "b2":
             dist_fwd()
         if part in ("all", "b2"):
-            _lib.call("pfst_neigh_grad_proto", x_src.data_ptr(), b.coef.data_ptr(), Bf, D, h, w,
-                      geo.dilation // geo.up, gt.data_ptr(), H, W, bank.mu.data_ptr(), bank.seen.data_ptr(),
+            _lib.call("pfst_neigh_grad_proto_lbl", x_src.data_ptr(), b.coef.data_ptr(), Bf, D, h, w,
+                      geo.dilation // geo.up, gt.data_ptr(), b.ldt, H, W, bank.mu.data_ptr(), bank.seen.data_ptr(),
                       self.C, b.dist.data_ptr(), b.acc.data_ptr(), self.gproto.data_ptr(), b.grad_x.data_ptr(), s)
 
     def _multi_rank(self) -> bool:
@@ -247,8 +250,8 @@ class SelfTrainingStep:
         with torch.cuda.stream(self._side):
             ops.neigh_dots_slot(x_ema, geo.dilation // geo.up, 0, b.dots)
             dots_ema.record(self._side)
-        _lib.call("pfst_pseudo_label", ema_logits.data_ptr(), B, C, H * W, float(self.thr), None, 0, -1,
-                  b.label.data_ptr(), b.conf.data_ptr(), None, b.count.data_ptr(), s)
+        _lib.call("pfst_pseudo_label_lbl", ema_logits.data_ptr(), B, C, H * W, float(self.thr), None, 0, -1,
+                  b.label.data_ptr(), b.ldt, b.conf.data_ptr(), None, b.count.data_ptr(), s)
         pl_done.record(main)
         unsafe = os.environ.get("PFST_DAG_UNSAFE") == "1"           # reproduces DESIGN.md 3.2 (tools/dots_replay_check.py)
         masked = bank.masked(h, w, x_ema)      # few classes: no sort kernel -> nothing to keep away from the TMA kernels
@@ -274,34 +277,36 @@ class SelfTrainingStep:
                 dist.all_reduce(bank.packed, op=dist.ReduceOp.SUM, group=bank.group)
             bank.finalize_captured(self._comm.cuda_stream, local_only=not reduce)
             self._comm.wait_event(dots_src)
-            _lib.call("pfst_proto_dist_fwd", x_src.data_ptr(), Bf, D, h, w, gt.data_ptr(), H, W,
+            _lib.call("pfst_proto_dist_fwd_lbl", x_src.data_ptr(), Bf, D, h, w, gt.data_ptr(), b.ldt, H, W,
                       bank.mu.data_ptr(), bank.seen.data_ptr(), self.C, b.dist.data_ptr(), b.acc.data_ptr(),
                       b.ploss.data_ptr(), self._comm.cuda_stream)
             proto_done.record(self._comm)
-        _lib.call("pfst_class_mix", gt.data_ptr(), chosen.data_ptr(), img.data_ptr(), trg_img.data_ptr(),
+        _lib.call("pfst_class_mix_lbl", gt.data_ptr(), chosen.data_ptr(), img.data_ptr(), trg_img.data_ptr(),
                   b.label.data_ptr(), None, b.count.data_ptr(), b.label.numel(), 0, 0, B, img.shape[1], H, W,
-                  b.mixed_img.data_ptr(), b.mixed_lbl.data_ptr(), b.weight.data_ptr(), b.mix_mask.data_ptr(), s)
+                  b.mixed_img.data_ptr(), b.mixed_lbl.data_ptr(), b.weight.data_ptr(), b.mix_mask.data_ptr(),
+                  b.ldt, s)
         main.wait_event(dots_src)
         w6 = ops._w6(self.w6)
         common = (b.dots.data_ptr(), b.ks, geo.B, geo.fh, geo.fw, geo.up, logits_trg.data_ptr(), geo.C,
                   geo.lh, geo.lw, geo.lscale, geo.lscale, gt.data_ptr(), b.mix_mask.data_ptr(), geo.gt_h,
                   geo.gt_w, geo.dilation, int(self.top_k), w6, b.ws.data_ptr(), b.stats.data_ptr())
-        _lib.call("pfst_pfgst_loss_fwd", *common, b.losses.data_ptr(), None, None, s)
+        _lib.call("pfst_pfgst_loss_fwd_lbl", *common, b.losses.data_ptr(), None, None, *ops.SHIPPED_LOSS_ARGS, b.ldt, s)
         if self.split_bwd:
             # the x_src gradient pass only needs the coefficient maps: grad_logits on the idle side stream
             stats_done, logits_done = self._ev[9], self._ev[0]
             stats_done.record(main)
             self._side.wait_event(stats_done)
-            _lib.call("pfst_pfgst_loss_bwd", *common, self.gout.data_ptr(), None, b.grad_logits.data_ptr(),
-                      self._side.cuda_stream)
+            _lib.call("pfst_pfgst_loss_bwd_lbl", *common, self.gout.data_ptr(), None, b.grad_logits.data_ptr(),
+                      *ops.SHIPPED_LOSS_ARGS, b.ldt, self._side.cuda_stream)
             logits_done.record(self._side)
-            _lib.call("pfst_pfgst_loss_bwd", *common, self.gout.data_ptr(), b.coef.data_ptr(), None, s)
+            _lib.call("pfst_pfgst_loss_bwd_lbl", *common, self.gout.data_ptr(), b.coef.data_ptr(), None,
+                      *ops.SHIPPED_LOSS_ARGS, b.ldt, s)
         else:
-            _lib.call("pfst_pfgst_loss_bwd", *common, self.gout.data_ptr(), b.coef.data_ptr(),
-                      b.grad_logits.data_ptr(), s)
+            _lib.call("pfst_pfgst_loss_bwd_lbl", *common, self.gout.data_ptr(), b.coef.data_ptr(),
+                      b.grad_logits.data_ptr(), *ops.SHIPPED_LOSS_ARGS, b.ldt, s)
         main.wait_event(proto_done)
-        _lib.call("pfst_neigh_grad_proto", x_src.data_ptr(), b.coef.data_ptr(), Bf, D, h, w,
-                  geo.dilation // geo.up, gt.data_ptr(), H, W, bank.mu.data_ptr(), bank.seen.data_ptr(),
+        _lib.call("pfst_neigh_grad_proto_lbl", x_src.data_ptr(), b.coef.data_ptr(), Bf, D, h, w,
+                  geo.dilation // geo.up, gt.data_ptr(), b.ldt, H, W, bank.mu.data_ptr(), bank.seen.data_ptr(),
                   self.C, b.dist.data_ptr(), b.acc.data_ptr(), self.gproto.data_ptr(), b.grad_x.data_ptr(), s)
         if self.split_bwd:
             main.wait_event(logits_done)
@@ -412,17 +417,20 @@ class SelfTrainingStep:
 
     # ----------------------------------------------------------------------- run
     def run(self, it: int, img, trg_img, gt, ema_logits, logits_trg, x_src, x_ema, rng=np.random):
+        """gt: int64 or uint8; the pseudo labels, ClassMix labels and masks returned have its dtype."""
         B, H, W = gt.shape[0], gt.shape[-2], gt.shape[-1]
+        ops._labels(gt, "gt")
         for name, t, dt in (("img", img, torch.float32), ("target_img", trg_img, torch.float32),
-                            ("gt", gt, torch.int64), ("ema_logits", ema_logits, torch.float32),
+                            ("ema_logits", ema_logits, torch.float32),
                             ("logits_trg", logits_trg, torch.float32), ("x_src", x_src, torch.float32),
                             ("x_ema", x_ema, torch.float32)):
             ops._dev(t, name, dt)
-        skey = (tuple(img.shape), tuple(ema_logits.shape), tuple(logits_trg.shape), tuple(x_src.shape))
+        skey = (tuple(img.shape), tuple(ema_logits.shape), tuple(logits_trg.shape), tuple(x_src.shape), gt.dtype)
         ent = self._bufs.get(skey)
         if ent is None:
             geo = ops.LossGeometry(logits_trg.shape, x_src.shape, gt.shape, self.downscale, self.dilation)
-            ent = (_Buffers(self.device, B, self.C, H, W, img.shape, logits_trg.shape, x_src.shape, geo), geo)
+            ent = (_Buffers(self.device, B, self.C, H, W, img.shape, logits_trg.shape, x_src.shape, geo, gt.dtype),
+                   geo)
             self._bufs[skey] = ent
         b, geo = ent
         main = torch.cuda.current_stream()
@@ -476,19 +484,22 @@ class SelfTrainingStep:
                     grad_x_src=b.grad_x, grad_logits_trg=b.grad_logits, mu=mu)
 
 
-def algorithmic_bytes(B: int, C: int, H: int, W: int, D: int, h: int, w: int, n_params: int) -> dict:
+def algorithmic_bytes(B: int, C: int, H: int, W: int, D: int, h: int, w: int, n_params: int,
+                      label_bytes: int = 8) -> dict:
     """Algorithmic HBM bytes per step and per kernel family — exactly SURVEY.md §8(d)'s figures
     (cfg2: 1.3115 GB): K_ema 12 B/param; K_pl (4C+12) B/px; K_mask+K_mix 84 B/px (presence read 8
     + mix reads 44 + writes 32); K_sim fwd two feature tensors; K_loss bwd read x_src + write grad;
     K_proto one feature read + the labels; K_dist fwd+bwd 3 feature-sized passes. The small loss
-    maps (dots, coefficient maps, ~3.7 MB at cfg2) are not counted."""
-    P, p = B * H * W, B * h * w
+    maps (dots, coefficient maps, ~3.7 MB at cfg2) are not counted. label_bytes = bytes of one
+    label-map element (8: int64, 1: uint8): the pseudo-label write, the presence read of gt, the two
+    label reads and the two label-map writes of the mix, and the label gather of K_proto."""
+    P, p, lb = B * H * W, B * h * w, int(label_bytes)
     return {
         "ema": 12 * n_params,
-        "pseudo_label": (4 * C + 12) * P,
-        "class_presence_and_mix": 84 * P,
+        "pseudo_label": (4 * C + 4 + lb) * P,
+        "class_presence_and_mix": (44 + 5 * lb) * P,
         "neigh_dots": 2 * 4 * D * p,
-        "proto_accum": 4 * D * p + 8 * p,
+        "proto_accum": 4 * D * p + lb * p,
         "neigh_grad": 2 * 4 * D * p,
         "proto_dist_fwd_bwd": 3 * 4 * D * p,
     }

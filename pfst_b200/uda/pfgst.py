@@ -246,7 +246,10 @@ class PFGST(UDADecorator):
 
     def forward_train(self, img, img_metas, gt_semantic_seg, target_img, target_img_metas,
                       target_img_strong_aug):
-        """pfgst.py:179-356."""
+        """pfgst.py:179-356. gt_semantic_seg: int64 or uint8; the iteration's pseudo labels, ClassMix labels
+        and masks follow its dtype (the student's forward_train receives source and mixed labels in it)."""
+        if gt_semantic_seg.dtype not in ops.LABEL_DTYPES:     # before any launch or RNG draw
+            raise TypeError(f"gt_semantic_seg: label maps must be torch.int64 or torch.uint8, got {gt_semantic_seg.dtype}")
         log_vars = {}
         vis_states = {}
         batch_size = img.shape[0]
@@ -324,7 +327,7 @@ class PFGST(UDADecorator):
         x_ema = ema_feats.detach().contiguous() if (fused or self.proto_cfg is not None) else None
         pseudo_label, pseudo_prob, count, weight_part = eng.teacher_outputs(
             ema_logits.detach().contiguous(), x_ema, thr, thr_vec,
-            self.thre_type == 'part', geo)
+            self.thre_type == 'part', geo, label_dtype=gt_semantic_seg.dtype)
         ps_size = pseudo_label.numel()
 
         # ⑥⑦ ClassMix (pfgst.py:281-300): host draw, then ONE fused launch

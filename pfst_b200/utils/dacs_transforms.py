@@ -131,6 +131,8 @@ class ClassMixPlan:
         self._batch = 0
 
     def start(self, gt: torch.Tensor, stream: Optional[torch.cuda.Stream] = None) -> None:
+        """gt: int64 or uint8 label maps of the batch."""
+        dt = ops._labels(gt, "gt")              # before any state changes: a refused gt leaves the FIFO aligned
         if self._started - self._chosen_count >= self.SLOTS:
             raise PfstError("ClassMixPlan: more start() calls in flight than staging slots")
         slot = self._started % self.SLOTS
@@ -141,7 +143,7 @@ class ClassMixPlan:
         self._batches[slot] = batch
         if stream is None:
             stream = torch.cuda.current_stream()
-        _lib.call("pfst_class_presence", ops._dev(gt, "gt", torch.int64), gt.numel(), self._presence.data_ptr(),
+        _lib.call("pfst_class_presence_lbl", gt.data_ptr(), dt, gt.numel(), self._presence.data_ptr(),
                   stream.cuda_stream)
         _lib.call("pfst_copy_async", self._presence_host.data_ptr() + 36 * slot, self._presence.data_ptr(), 36,
                   stream.cuda_stream)
