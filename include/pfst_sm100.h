@@ -41,6 +41,12 @@ extern "C" {
 #define PFST_DT_U8 0
 #define PFST_DT_I32 1
 #define PFST_DT_I64 2
+/* dtype tags for the teacher-output entry points (`_ft` siblings): the EMA teacher's logits and
+ * features may be fp32, fp16 or bf16. Converting fp16 / bf16 to fp32 is exact, so every output
+ * equals the fp32 entry point's output on the upcast tensor. */
+#define PFST_DT_F32 16
+#define PFST_DT_F16 17
+#define PFST_DT_BF16 18
 
 /* ---- library ------------------------------------------------------------ */
 const char* pfst_version(void);
@@ -137,6 +143,14 @@ int pfst_pseudo_label_lbl(const float* logits, int64_t B, int32_t C, int64_t HW,
                           const float* thr_per_class, int32_t mode, int64_t reject_label,
                           void* label, int32_t label_dtype, float* conf, float* weight_part,
                           unsigned long long* count, void* stream);
+/* pfst_pseudo_label_lbl with the logits in logit_dtype (PFST_DT_F32, PFST_DT_F16 or PFST_DT_BF16; anything
+ * else returns PFST_ERR_UNSUPPORTED): the teacher pass run under autocast, pfgst.py:259-266 (torch.softmax
+ * is on autocast's fp32 list, so the reference upcasts first). Every value is converted to fp32 once, on
+ * load; labels, conf, weight_part and count are bit-identical to pfst_pseudo_label_lbl on the upcast logits. */
+int pfst_pseudo_label_ft(const void* logits, int32_t logit_dtype, int64_t B, int32_t C, int64_t HW, float thr,
+                         const float* thr_per_class, int32_t mode, int64_t reject_label, void* label,
+                         int32_t label_dtype, float* conf, float* weight_part, unsigned long long* count,
+                         void* stream);
 
 /* Self-test of the kernel's hand-scheduled exp: *mismatches = number of x[i]
  * (x[i] <= 0) for which it differs bitwise from CUDA's expf. Must be 0.       */
@@ -231,6 +245,13 @@ int pfst_neigh_grad(const float* x, const float* coef, int64_t B, int32_t D, int
 int pfst_neigh_dots_slot(const float* x, int64_t B, int32_t D, int32_t h, int32_t w,
                          int32_t dilation, int32_t slot, int32_t n_slots, float* dots,
                          void* stream);
+/* pfst_neigh_dots_slot for x of x_dtype (PFST_DT_F32, PFST_DT_F16 or PFST_DT_BF16, else
+ * PFST_ERR_UNSUPPORTED): the EMA features of a teacher run under autocast, get_sim_feat
+ * pfgst_loss.py:181-201 (cosine_similarity is on autocast's fp32 list). The dot maps are bit-identical to
+ * pfst_neigh_dots_slot on the upcast tensor: the same channel splits, the same per-warp channel order and
+ * the same merge order, on every path (TMA, small-plane bulk copy, generic).                        */
+int pfst_neigh_dots_slot_ft(const void* x, int32_t x_dtype, int64_t B, int32_t D, int32_t h, int32_t w,
+                            int32_t dilation, int32_t slot, int32_t n_slots, float* dots, void* stream);
 
 /* pfst_neigh_grad and pfst_proto_dist_bwd (below) in one pass over x: grad_x =
  * neighbourhood-cosine gradient + grad_loss * (x - mu[label]) / (dist * n_valid).
@@ -376,6 +397,12 @@ int pfst_proto_accum(const float* feats, int64_t B, int32_t D, int32_t h, int32_
 int pfst_proto_accum_lbl(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
                          const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w,
                          const float* conf, float conf_thr, int32_t C, float* packed, void* stream);
+/* pfst_proto_accum_lbl with feats of feat_dtype (PFST_DT_F32, PFST_DT_F16 or PFST_DT_BF16, else
+ * PFST_ERR_UNSUPPORTED): the EMA features of a teacher run under autocast; anchor pfgst.py:168-177.
+ * Every value is converted to fp32 on load; the sums are float atomics as on the fp32 path.     */
+int pfst_proto_accum_ft(const void* feats, int32_t feat_dtype, int64_t B, int32_t D, int32_t h, int32_t w,
+                        const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w,
+                        const float* conf, float conf_thr, int32_t C, float* packed, void* stream);
 
 /* pfst_proto_accum split in two, so that the label sort is done ONCE per (image, tile) and
  * not by every streaming block:
@@ -398,6 +425,10 @@ int pfst_proto_order_lbl(const void* labels, int32_t label_dtype, int64_t B, int
                          float* counts, void* workspace, void* stream);
 int pfst_proto_accum_ordered(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
                              int32_t C, const void* workspace, float* packed, void* stream);
+/* pfst_proto_accum_ordered with feats of feat_dtype (PFST_DT_F32, PFST_DT_F16 or PFST_DT_BF16, else
+ * PFST_ERR_UNSUPPORTED); anchor pfgst.py:168-177. The workspace of pfst_proto_order is shared.  */
+int pfst_proto_accum_ordered_ft(const void* feats, int32_t feat_dtype, int64_t B, int32_t D, int32_t h,
+                                int32_t w, int32_t C, const void* workspace, float* packed, void* stream);
 
 /* mu_out[c] = packed sums / max(count,1) for classes with pixels; classes already
  * seen (seen_prev[c] != 0) are EMA-updated fl(fl(a32*mu_prev)+fl(b32*mean)) (the E2

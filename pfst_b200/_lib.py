@@ -16,6 +16,7 @@ LIB_PATH = Path(os.environ.get("PFST_LIB") or (Path(__file__).resolve().parent /
 
 PFST_OK = 0
 DT_U8, DT_I32, DT_I64 = 0, 1, 2
+DT_F32, DT_F16, DT_BF16 = 16, 17, 18
 
 
 class PfstError(RuntimeError):
@@ -39,6 +40,8 @@ SIGNATURES: dict[str, tuple] = {
     "pfst_ema_update_flat": (C.c_int, [_vp, _vp, _i64, _f32, _f32, _i32, _vp]),
     "pfst_pseudo_label": (C.c_int, [_vp, _i64, _i32, _i64, _f32, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp]),
     "pfst_pseudo_label_lbl": (C.c_int, [_vp, _i64, _i32, _i64, _f32, _vp, _i32, _i64, _vp, _i32, _vp, _vp, _vp, _vp]),
+    "pfst_pseudo_label_ft": (C.c_int, [_vp, _i32, _i64, _i32, _i64, _f32, _vp, _i32, _i64, _vp, _i32, _vp, _vp, _vp,
+                                       _vp]),
     "pfst_selftest_exp": (C.c_int, [_vp, _i64, _vp, _vp]),
     "pfst_pseudo_weight_fill": (C.c_int, [_vp, _i64, _i64, _i64, _vp, _i64, _i32, _i32, _vp]),
     "pfst_class_presence": (C.c_int, [_vp, _i64, _vp, _vp]),
@@ -52,6 +55,7 @@ SIGNATURES: dict[str, tuple] = {
     "pfst_neigh_dots": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _i32, _vp, _vp]),
     "pfst_neigh_grad": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _i32, _vp, _vp]),
     "pfst_neigh_dots_slot": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp]),
+    "pfst_neigh_dots_slot_ft": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp]),
     "pfst_neigh_grad_proto": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _i32, _vp, _i32, _i32, _vp, _vp, _i32,
                                         _vp, _vp, _vp, _vp, _vp]),
     "pfst_neigh_grad_proto_lbl": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _vp,
@@ -86,10 +90,13 @@ SIGNATURES: dict[str, tuple] = {
     "pfst_proto_accum_is_masked": (C.c_int, [_i32, _i32, _i32]),
     "pfst_proto_accum": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _vp, _f32, _i32, _vp, _vp]),
     "pfst_proto_accum_lbl": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _vp, _f32, _i32, _vp, _vp]),
+    "pfst_proto_accum_ft": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _vp, _f32, _i32, _vp,
+                                      _vp]),
     "pfst_proto_order_ws_bytes": (_i64, [_i64, _i32, _i32, _i32]),
     "pfst_proto_order": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _i32, _vp, _f32, _i32, _vp, _vp, _vp]),
     "pfst_proto_order_lbl": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _i32, _vp, _f32, _i32, _vp, _vp, _vp]),
     "pfst_proto_accum_ordered": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _i32, _vp, _vp, _vp]),
+    "pfst_proto_accum_ordered_ft": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _i32, _vp, _vp, _vp]),
     "pfst_proto_finalize": (C.c_int, [_vp, _i32, _i32, _vp, _vp, _f32, _f32, _vp, _vp, _vp, _i32, _vp]),
     "pfst_proto_finalize_dev": (C.c_int, [_vp, _i32, _i32, _vp, _vp, _f64, _vp, _vp, _vp, _vp, _i32, _vp]),
     "pfst_feat_dist_fwd": (C.c_int, [_vp, _vp, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp, _vp]),

@@ -2,6 +2,8 @@
 // Everything in this library is written for B200 (sm_100a) only: no other
 // -gencode is ever passed and there is no CPU fallback.
 #pragma once
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -57,6 +59,34 @@ __host__ __device__ static inline bool aligned_lbl4(const L* p) {
   return sizeof(L) == 8 ? aligned16(p) : aligned4(p);
 }
 
+// Teacher outputs (the pseudo-label logits and the EMA features) are fp32, fp16 or bf16; the kernels that
+// read them are templated on the element type and convert every value to fp32 once, on load (exact), so
+// the arithmetic after the load is the fp32 code. The entry points take a PFST_DT_F* tag.
+template <class T> struct FloatDt;
+template <> struct FloatDt<float> { static constexpr int value = PFST_DT_F32; };
+template <> struct FloatDt<__half> { static constexpr int value = PFST_DT_F16; };
+template <> struct FloatDt<__nv_bfloat16> { static constexpr int value = PFST_DT_BF16; };
+
+__device__ __forceinline__ float to_f32(float v) { return v; }
+__device__ __forceinline__ float to_f32(__half v) { return __half2float(v); }
+__device__ __forceinline__ float to_f32(__nv_bfloat16 v) { return __bfloat162float(v); }
+template <class T> __device__ __forceinline__ float ldgf(const T* p) { return to_f32(__ldg(p)); }
+// the low / high 16-bit element of a 32-bit word as fp32
+template <class T> __device__ __forceinline__ float lo_f32(uint32_t w);
+template <class T> __device__ __forceinline__ float hi_f32(uint32_t w);
+template <> __device__ __forceinline__ float lo_f32<__nv_bfloat16>(uint32_t w) { return __uint_as_float(w << 16); }
+template <> __device__ __forceinline__ float hi_f32<__nv_bfloat16>(uint32_t w) { return __uint_as_float(w & 0xffff0000u); }
+template <> __device__ __forceinline__ float lo_f32<__half>(uint32_t w) {
+  return __half2float(__ushort_as_half((unsigned short)(w & 0xffffu)));
+}
+template <> __device__ __forceinline__ float hi_f32<__half>(uint32_t w) {
+  return __half2float(__ushort_as_half((unsigned short)(w >> 16)));
+}
+// four consecutive 16-bit elements (one 64-bit word) as fp32
+template <class T> __device__ __forceinline__ float4 unpack4(uint2 v) {
+  return make_float4(lo_f32<T>(v.x), hi_f32<T>(v.x), lo_f32<T>(v.y), hi_f32<T>(v.y));
+}
+
 // ---- streaming 128-bit global accesses ------------------------------------
 // Inputs that are read exactly once bypass L1 (ld.global.nc.L1::no_allocate);
 // outputs that are not re-read by the same kernel use plain vector stores.
@@ -85,6 +115,16 @@ __device__ __forceinline__ uint32_t ldg_stream_u32(const void* p) {
   uint32_t r;
   asm volatile("ld.global.nc.L1::no_allocate.u32 %0, [%1];" : "=r"(r) : "l"(p));
   return r;
+}
+// four consecutive elements as fp32: one 128-bit (fp32) or 64-bit (fp16 / bf16) streaming load
+__device__ __forceinline__ float4 ldg_stream_4(const float* p) { return ldg_stream_f4(p); }
+// (not volatile: a read-only load the compiler may schedule; with `volatile` ptxas spilled the C = 4 pseudo-label
+// instantiation)
+template <class T>
+__device__ __forceinline__ float4 ldg_stream_4(const T* p) {
+  uint2 r;
+  asm("ld.global.nc.L1::no_allocate.v2.u32 {%0,%1}, [%2];" : "=r"(r.x), "=r"(r.y) : "l"(p));
+  return unpack4<T>(r);
 }
 __device__ __forceinline__ void stg_f4(float* p, float4 v) {
   *reinterpret_cast<float4*>(p) = v;

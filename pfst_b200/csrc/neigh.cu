@@ -40,11 +40,13 @@ constexpr int kNbThreads = kNbConsumers + 32;
 // TMA requires the box to start on a 16-byte boundary in the innermost dimension
 // (x_start % 4 == 0 for fp32), so the left halo is always kNbHL = 4 columns wide
 // (>= every supported dilation) and the box is 32 + 4 + 4 = 40 columns.
+// For 16-bit elements 16 bytes are 8 columns: the halo is 8 columns wide and the box 48 columns.
 constexpr int kNbHL = 4;
-template <int DIL>
+template <int DIL, int HL_ = kNbHL>
 struct NbGeom {
-  static_assert(DIL <= kNbHL, "dilation larger than the aligned halo");
-  static constexpr int RS = kNbTW + 2 * kNbHL;                // smem row stride = box width (40)
+  static_assert(DIL <= HL_, "dilation larger than the aligned halo");
+  static constexpr int HL = HL_;
+  static constexpr int RS = kNbTW + 2 * HL;                   // smem row stride = box width (40; 48 for 16-bit)
   static constexpr int FWD_ROWS = kNbTH + DIL;               // rows y0 .. y0+TH-1+d
   static constexpr int BWD_ROWS = kNbTH + 2 * DIL;           // rows y0-d .. y0+TH-1+d
 };
@@ -86,12 +88,12 @@ __device__ __forceinline__ void nb_init_barriers(uint64_t* full_bar, uint64_t* e
   __syncthreads();
 }
 
-template <int ROWS, int RS>
-__device__ __forceinline__ void nb_produce(const CUtensorMap* map, float* stage_buf, uint64_t* full_bar,
+template <int ROWS, int RS, class T = float>
+__device__ __forceinline__ void nb_produce(const CUtensorMap* map, T* stage_buf, uint64_t* full_bar,
                                            uint64_t* empty_bar, const NbTile& tl, int x_start,
                                            int y_start) {
   constexpr int kStageFloats = kNbCH * ROWS * RS;
-  constexpr uint32_t kStageBytes = kStageFloats * sizeof(float);
+  constexpr uint32_t kStageBytes = kStageFloats * sizeof(T);
   tma_prefetch_desc(map);
   int it = 0;
   for (int c = tl.c_begin; c < tl.c_end; ++c, ++it) {
@@ -104,15 +106,28 @@ __device__ __forceinline__ void nb_produce(const CUtensorMap* map, float* stage_
   }
 }
 
+// four consecutive shared-memory elements as fp32: one 128-bit (fp32) or 64-bit (fp16 / bf16) load
+__device__ __forceinline__ float4 lds4(const float* p) { return *reinterpret_cast<const float4*>(p); }
+template <class T>
+__device__ __forceinline__ float4 lds4(const T* p) { return unpack4<T>(*reinterpret_cast<const uint2*>(p)); }
+
 // ---------------------------------------------------------------- forward (TMA)
-template <int DIL>
+// T = fp16 / bf16 (the EMA features of a teacher run under autocast): the same tile, channel-to-warp
+// assignment and merge order; the box has the 8-column (16-byte) halo, each strip row is three 64-bit shared
+// loads, converted to fp32 on load, so the dot maps equal the fp32 kernel's on the upcast tensor bit for bit.
+template <int DIL, class T>
+using NbGeomFor = NbGeom<DIL, sizeof(T) == 4 ? kNbHL : 2 * kNbHL>;
+
+template <int DIL, class T = float>
 __global__ void __launch_bounds__(kNbThreads)
 neigh_dots_tma_kernel(const __grid_constant__ NeighMaps maps, int n_tensors, int B, int D, int h, int w,
                       int ksplit, int slot0, int n_slots, float* __restrict__ dots) {
-  using G = NbGeom<DIL>;
+  using G = NbGeomFor<DIL, T>;
   constexpr int kStageFloats = kNbCH * G::FWD_ROWS * G::RS;
+  // the merge below reuses the stage ring: [3 warps][80 values][32 lanes] fp32
+  static_assert(kNbStages * kStageFloats * sizeof(T) >= 4 * 80 * 32 * sizeof(float), "merge buffer");
   extern __shared__ __align__(128) unsigned char nb_smem[];
-  float* stage_buf = reinterpret_cast<float*>(nb_smem);
+  T* stage_buf = reinterpret_cast<T*>(nb_smem);
   __shared__ uint64_t full_bar[kNbStages], empty_bar[kNbStages];
   const NbTile tl = nb_decode(n_tensors, B, h, w, D, ksplit);
   nb_init_barriers(full_bar, empty_bar);
@@ -120,7 +135,7 @@ neigh_dots_tma_kernel(const __grid_constant__ NeighMaps maps, int n_tensors, int
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (warp == kNbConsumers / 32) {
     if (lane == 0)
-      nb_produce<G::FWD_ROWS, G::RS>(&maps.m[tl.t], stage_buf, full_bar, empty_bar, tl, tl.x0 - kNbHL, tl.y0);
+      nb_produce<G::FWD_ROWS, G::RS, T>(&maps.m[tl.t], stage_buf, full_bar, empty_bar, tl, tl.x0 - G::HL, tl.y0);
     return;
   }
   // Each lane owns a CHAIN of four 1x4 pixel strips, rows r0 + k*DIL (k = 0..3): the row read
@@ -142,16 +157,16 @@ neigh_dots_tma_kernel(const __grid_constant__ NeighMaps maps, int n_tensors, int
   for (int c = tl.c_begin; c < tl.c_end; ++c, ++it) {
     const int s = it % kNbStages;
     mbar_wait(&full_bar[s], (uint32_t)(it / kNbStages) & 1u);
-    const float* buf = stage_buf + (size_t)s * kStageFloats + r0 * G::RS + lx;
+    const T* buf = stage_buf + (size_t)s * kStageFloats + r0 * G::RS + lx + (G::HL - kNbHL);
 #pragma unroll
     for (int cc = 0; cc < kNbCH / (kNbConsumers / 32); ++cc) {
       const int ch = warp + cc * (kNbConsumers / 32);
       // smem column of image column x is (x - x0 + 4); this strip's pixels sit at lx+4+i
-      const float* row = buf + ch * G::FWD_ROWS * G::RS;
+      const T* row = buf + ch * G::FWD_ROWS * G::RS;
       float P[12], Q[12];                                  // P[j] = col lx+j of the current row
 #pragma unroll
       for (int v = 1; v < 3; ++v) {
-        const float4 f = *reinterpret_cast<const float4*>(row + 4 * v);
+        const float4 f = lds4(row + 4 * v);
         P[4 * v] = f.x; P[4 * v + 1] = f.y; P[4 * v + 2] = f.z; P[4 * v + 3] = f.w;
       }
 #pragma unroll
@@ -159,7 +174,7 @@ neigh_dots_tma_kernel(const __grid_constant__ NeighMaps maps, int n_tensors, int
         row += DIL * G::RS;
 #pragma unroll
         for (int v = 0; v < 3; ++v) {
-          const float4 f = *reinterpret_cast<const float4*>(row + 4 * v);
+          const float4 f = lds4(row + 4 * v);
           Q[4 * v] = f.x; Q[4 * v + 1] = f.y; Q[4 * v + 2] = f.z; Q[4 * v + 3] = f.w;
         }
 #pragma unroll
@@ -181,7 +196,7 @@ neigh_dots_tma_kernel(const __grid_constant__ NeighMaps maps, int n_tensors, int
   // The four warps hold partial sums over disjoint channels: merge through shared memory
   // (the stage ring is idle now) in a fixed order, then one warp-row-coalesced store per map.
   asm volatile("bar.sync 1, %0;" ::"n"(kNbConsumers) : "memory");
-  float* red = stage_buf;                                   // [4 warps][5*16 values][32 lanes]
+  float* red = reinterpret_cast<float*>(nb_smem);          // [4 warps][5*16 values][32 lanes]
   if (warp > 0) {
 #pragma unroll
     for (int m = 0; m < 5; ++m)
@@ -356,8 +371,14 @@ neigh_grad_tma_kernel(const __grid_constant__ NeighMaps maps, const float* __res
 }
 
 // ------------------------------------------------- generic (any shape) kernels
+// TMA_ORDER (fp16 / bf16 tensors the TMA kernel cannot describe while their fp32 upcast would take it):
+// the sums are formed in the TMA kernel's order — split over 8-channel chunks, per consumer warp
+// g = 0..3 the channels 8k+g and 8k+g+4 in chunk order, then ((g0 + g1) + g2) + g3 — so the dot maps
+// still equal the fp32 path's bit for bit. Taps the TMA kernel reads as zero fill (outside the image,
+// channels past D) add exact zeros there and are skipped here.
+template <class T = float, bool TMA_ORDER = false>
 __global__ void __launch_bounds__(128)
-neigh_dots_generic_kernel(const float* __restrict__ xa, const float* __restrict__ xb, int n_tensors, int B,
+neigh_dots_generic_kernel(const T* __restrict__ xa, const T* __restrict__ xb, int n_tensors, int B,
                           int D, int h, int w, int dil, int ksplit, int slot0, int n_slots,
                           float* __restrict__ dots) {
   const int64_t plane = (int64_t)h * w;
@@ -368,18 +389,44 @@ neigh_dots_generic_kernel(const float* __restrict__ xa, const float* __restrict_
   if (p >= plane) return;
   const int y = p / w, x = p - y * w;
   const int c_begin = (int)((int64_t)split * D / ksplit), c_end = (int)((int64_t)(split + 1) * D / ksplit);
-  const float* src = (t == 0 ? xa : xb) + ((int64_t)b * D) * plane + p;
+  const T* src = (t == 0 ? xa : xb) + ((int64_t)b * D) * plane + p;
   const bool in1 = x + dil < w, inr = y + dil < h;
   const bool in2 = inr && x - dil >= 0, in4 = inr && x + dil < w;
   float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f, a4 = 0.f;
-  for (int c = c_begin; c < c_end; ++c) {
-    const float* q = src + (int64_t)c * plane;
-    const float v = __ldg(q);
-    a0 = fmaf(v, v, a0);
-    if (in1) a1 = fmaf(v, __ldg(q + dil), a1);
-    if (in2) a2 = fmaf(v, __ldg(q + (int64_t)dil * w - dil), a2);
-    if (inr) a3 = fmaf(v, __ldg(q + (int64_t)dil * w), a3);
-    if (in4) a4 = fmaf(v, __ldg(q + (int64_t)dil * w + dil), a4);
+  if constexpr (TMA_ORDER) {
+    const int chunks = (D + kNbCH - 1) / kNbCH;
+    const int k_begin = (int)((int64_t)split * chunks / ksplit), k_end = (int)((int64_t)(split + 1) * chunks / ksplit);
+    for (int g = 0; g < kNbConsumers / 32; ++g) {
+      float b0 = 0.f, b1 = 0.f, b2 = 0.f, b3 = 0.f, b4 = 0.f;
+      for (int k = k_begin; k < k_end; ++k)
+#pragma unroll
+        for (int cc = 0; cc < kNbCH / (kNbConsumers / 32); ++cc) {
+          const int c = k * kNbCH + g + cc * (kNbConsumers / 32);
+          if (c >= D) continue;
+          const T* q = src + (int64_t)c * plane;
+          const float v = ldgf(q);
+          b0 = fmaf(v, v, b0);
+          if (in1) b1 = fmaf(v, ldgf(q + dil), b1);
+          if (in2) b2 = fmaf(v, ldgf(q + (int64_t)dil * w - dil), b2);
+          if (inr) b3 = fmaf(v, ldgf(q + (int64_t)dil * w), b3);
+          if (in4) b4 = fmaf(v, ldgf(q + (int64_t)dil * w + dil), b4);
+        }
+      if (g == 0) {
+        a0 = b0; a1 = b1; a2 = b2; a3 = b3; a4 = b4;
+      } else {
+        a0 += b0; a1 += b1; a2 += b2; a3 += b3; a4 += b4;
+      }
+    }
+  } else {
+    for (int c = c_begin; c < c_end; ++c) {
+      const T* q = src + (int64_t)c * plane;
+      const float v = ldgf(q);
+      a0 = fmaf(v, v, a0);
+      if (in1) a1 = fmaf(v, ldgf(q + dil), a1);
+      if (in2) a2 = fmaf(v, ldgf(q + (int64_t)dil * w - dil), a2);
+      if (inr) a3 = fmaf(v, ldgf(q + (int64_t)dil * w), a3);
+      if (in4) a4 = fmaf(v, ldgf(q + (int64_t)dil * w + dil), a4);
+    }
   }
   float* out = dots + ((((int64_t)split * n_slots + slot0 + t) * B + b) * 5) * plane + p;
   out[0] = a0; out[plane] = a1; out[2 * plane] = a2; out[3 * plane] = a3; out[4 * plane] = a4;
@@ -438,30 +485,33 @@ __device__ __forceinline__ void sp_init(uint64_t* full_bar, uint64_t* empty_bar)
   __syncthreads();
 }
 
-__device__ __forceinline__ void sp_produce(const float* src, int hw, int c_begin, int c_end, float* stage_buf,
+template <class T = float>
+__device__ __forceinline__ void sp_produce(const T* src, int hw, int c_begin, int c_end, T* stage_buf,
                                            uint64_t* full_bar, uint64_t* empty_bar) {
   int it = 0;
   for (int c = c_begin; c < c_end; c += kSpCH, ++it) {
     const int s = it % kSpStages, n = min(kSpCH, c_end - c);
     if (it >= kSpStages) mbar_wait(&empty_bar[s], ((uint32_t)(it / kSpStages) & 1u) ^ 1u);
-    const uint32_t bytes = (uint32_t)n * hw * sizeof(float);
+    const uint32_t bytes = (uint32_t)n * hw * sizeof(T);
     mbar_arrive_expect_tx(&full_bar[s], bytes);
     bulk_load_1d(stage_buf + (size_t)s * kSpCH * hw, src + (int64_t)c * hw, bytes, &full_bar[s]);
   }
 }
 
+// T = fp16 / bf16: half the bytes per stage, every value converted to fp32 as it is read from shared memory
+template <class T = float>
 __global__ void __launch_bounds__(kSpThreads)
-neigh_dots_plane_kernel(const float* __restrict__ xa, const float* __restrict__ xb, int B, int D, int h, int w,
+neigh_dots_plane_kernel(const T* __restrict__ xa, const T* __restrict__ xb, int B, int D, int h, int w,
                         int dil, int ksplit, int slot0, int n_slots, float* __restrict__ dots) {
   extern __shared__ __align__(128) unsigned char sp_smem[];
-  float* stage_buf = reinterpret_cast<float*>(sp_smem);
+  T* stage_buf = reinterpret_cast<T*>(sp_smem);
   __shared__ uint64_t full_bar[kSpStages], empty_bar[kSpStages];
   const int hw = h * w;
   int z = blockIdx.x;
   const int split = z % ksplit; z /= ksplit;
   const int b = z % B, t = z / B;
   const int c_begin = (int)((int64_t)split * D / ksplit), c_end = (int)((int64_t)(split + 1) * D / ksplit);
-  const float* src = (t == 0 ? xa : xb) + (int64_t)b * D * hw;
+  const T* src = (t == 0 ? xa : xb) + (int64_t)b * D * hw;
   sp_init(full_bar, empty_bar);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (warp == kSpConsumers / 32) {
@@ -488,18 +538,18 @@ neigh_dots_plane_kernel(const float* __restrict__ xa, const float* __restrict__ 
   for (int c = c_begin; c < c_end; c += kSpCH, ++it) {
     const int s = it % kSpStages, n = min(kSpCH, c_end - c);
     mbar_wait(&full_bar[s], (uint32_t)(it / kSpStages) & 1u);
-    const float* buf = stage_buf + (size_t)s * kSpCH * hw;
+    const T* buf = stage_buf + (size_t)s * kSpCH * hw;
 #pragma unroll
     for (int q = 0; q < kSpPix; ++q) {
       if (!live[q]) continue;
-      const float* pq = buf + threadIdx.x + q * kSpConsumers;
+      const T* pq = buf + threadIdx.x + q * kSpConsumers;
       for (int ch = 0; ch < n; ++ch) {
-        const float* r = pq + ch * hw;
-        const float v = r[0];
+        const T* r = pq + ch * hw;
+        const float v = to_f32(r[0]);
         acc[q][0] = fmaf(v, v, acc[q][0]);
 #pragma unroll
         for (int k = 0; k < 4; ++k)
-          if (ok[q][k]) acc[q][k + 1] = fmaf(v, r[off[q][k]], acc[q][k + 1]);
+          if (ok[q][k]) acc[q][k + 1] = fmaf(v, to_f32(r[off[q][k]]), acc[q][k + 1]);
       }
     }
     __syncwarp();
@@ -589,14 +639,15 @@ neigh_grad_plane_kernel(const float* __restrict__ x, const float* __restrict__ c
 }
 
 // planes the bulk-copy kernels cover: small, 16-byte aligned channel chunks for every split
-static bool sp_ok(const void* p0, const void* p1, int D, int h, int w, int ks) {
+// (esz = bytes per element: a chunk of n channels is n * hw * esz bytes, hw may be odd)
+static bool sp_ok(const void* p0, const void* p1, int D, int h, int w, int ks, int esz = 4) {
   const int hw = h * w;
-  return hw <= kSpMaxHW && aligned16(p0) && (!p1 || aligned16(p1)) && D % (4 * ks) == 0;
+  return hw <= kSpMaxHW && aligned16(p0) && (!p1 || aligned16(p1)) && D % ((16 / esz) * ks) == 0;
 }
 
-static bool nb_tma_ok(const void* p0, const void* p1, int w, int dil) {
-  return (w % 4 == 0) && aligned16(p0) && (!p1 || aligned16(p1)) && (dil == 1 || dil == 2 || dil == 4) &&
-         get_encode_tiled() != nullptr;
+static bool nb_tma_ok(const void* p0, const void* p1, int w, int dil, int esz = 4) {
+  return ((int64_t)w * esz % 16 == 0) && aligned16(p0) && (!p1 || aligned16(p1)) &&
+         (dil == 1 || dil == 2 || dil == 4) && get_encode_tiled() != nullptr;
 }
 
 static int nb_splits(int64_t units, int h, int w, int D) {
@@ -609,15 +660,23 @@ static int nb_splits(int64_t units, int h, int w, int D) {
   return ks;
 }
 
-template <int DIL>
-static int launch_dots_tma(const float* xa, const float* xb, int T, int B, int D, int h, int w, int ks,
+template <class E> struct TmaDt;
+template <> struct TmaDt<float> { static constexpr CUtensorMapDataType value = CU_TENSOR_MAP_DATA_TYPE_FLOAT32; };
+template <> struct TmaDt<__half> { static constexpr CUtensorMapDataType value = CU_TENSOR_MAP_DATA_TYPE_FLOAT16; };
+template <> struct TmaDt<__nv_bfloat16> { static constexpr CUtensorMapDataType value = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16; };
+
+template <int DIL, class E = float>
+static int launch_dots_tma(const E* xa, const E* xb, int T, int B, int D, int h, int w, int ks,
                            int slot0, int n_slots, float* dots, cudaStream_t s) {
-  using G = NbGeom<DIL>;
+  using G = NbGeomFor<DIL, E>;
   NeighMaps maps;
-  if (!make_nchw_tensor_map(&maps.m[0], xa, B, D, h, w, G::RS, G::FWD_ROWS, kNbCH)) return PFST_ERR_CUDA;
-  if (!make_nchw_tensor_map(&maps.m[1], xb ? xb : xa, B, D, h, w, G::RS, G::FWD_ROWS, kNbCH)) return PFST_ERR_CUDA;
-  const size_t smem = (size_t)kNbStages * kNbCH * G::FWD_ROWS * G::RS * sizeof(float);
-  auto k = neigh_dots_tma_kernel<DIL>;
+  if (!make_nchw_tensor_map(&maps.m[0], xa, B, D, h, w, G::RS, G::FWD_ROWS, kNbCH, TmaDt<E>::value, sizeof(E)))
+    return PFST_ERR_CUDA;
+  if (!make_nchw_tensor_map(&maps.m[1], xb ? xb : xa, B, D, h, w, G::RS, G::FWD_ROWS, kNbCH, TmaDt<E>::value,
+                            sizeof(E)))
+    return PFST_ERR_CUDA;
+  const size_t smem = (size_t)kNbStages * kNbCH * G::FWD_ROWS * G::RS * sizeof(E);
+  auto k = neigh_dots_tma_kernel<DIL, E>;
   PFST_CUDA_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "pfst_neigh_dots/attr");
   const int64_t tiles = (int64_t)((w + kNbTW - 1) / kNbTW) * ((h + kNbTH - 1) / kNbTH);
   const int64_t grid = (int64_t)T * B * tiles * ks;
@@ -707,22 +766,33 @@ int32_t pfst_neigh_dots_splits(int64_t n_tensors, int64_t B, int32_t D, int32_t 
   return pfst::nb_splits(n_tensors * B, h, w, D);
 }
 
-static int neigh_dots_impl(const float* x_a, const float* x_b, int64_t B, int32_t D, int32_t h, int32_t w,
+}  // extern "C"
+
+namespace pfst {
+
+// E = fp16 / bf16: every path produces the dot maps the fp32 path produces on the upcast tensor. The
+// upcast is a fresh, aligned fp32 tensor, so the path the fp32 entry point would take is decided on the
+// shape alone; where the 16-bit tensor cannot take that path itself (a width whose rows are not whole
+// 16-byte units, an unaligned view) the generic kernel reproduces its summation order.
+template <class E>
+static int neigh_dots_impl(const E* x_a, const E* x_b, int64_t B, int32_t D, int32_t h, int32_t w,
                            int32_t dilation, int slot0, int n_slots, float* dots, cudaStream_t s) {
   const int T = x_b ? 2 : 1;
-  const int ks = pfst::nb_splits((int64_t)T * B, h, w, D);
-  if (pfst::nb_tma_ok(x_a, x_b, w, dilation)) {
+  const int ks = nb_splits((int64_t)T * B, h, w, D);
+  constexpr int esz = (int)sizeof(E);
+  if (pfst::nb_tma_ok(x_a, x_b, w, dilation, esz)) {
     switch (dilation) {
       case 1: return pfst::launch_dots_tma<1>(x_a, x_b, T, (int)B, D, h, w, ks, slot0, n_slots, dots, s);
       case 2: return pfst::launch_dots_tma<2>(x_a, x_b, T, (int)B, D, h, w, ks, slot0, n_slots, dots, s);
       default: return pfst::launch_dots_tma<4>(x_a, x_b, T, (int)B, D, h, w, ks, slot0, n_slots, dots, s);
     }
   }
-  if (pfst::sp_ok(x_a, x_b, D, h, w, ks) && (int64_t)T * B * ks <= 0x7fffffffll) {
-    const size_t smem = (size_t)pfst::kSpStages * pfst::kSpCH * h * w * sizeof(float);
-    PFST_CUDA_TRY(cudaFuncSetAttribute(pfst::neigh_dots_plane_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+  const bool fp32_tma = esz != 4 && nb_tma_ok(nullptr, nullptr, w, dilation);   // the upcast's path
+  if (!fp32_tma && pfst::sp_ok(x_a, x_b, D, h, w, ks, esz) && (int64_t)T * B * ks <= 0x7fffffffll) {
+    const size_t smem = (size_t)pfst::kSpStages * pfst::kSpCH * h * w * sizeof(E);
+    PFST_CUDA_TRY(cudaFuncSetAttribute(pfst::neigh_dots_plane_kernel<E>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)smem), "pfst_neigh_dots/attr");
-    pfst::neigh_dots_plane_kernel<<<(unsigned)(T * B * ks), pfst::kSpThreads, smem, s>>>(
+    pfst::neigh_dots_plane_kernel<E><<<(unsigned)(T * B * ks), pfst::kSpThreads, smem, s>>>(
         x_a, x_b, (int)B, D, h, w, dilation, ks, slot0, n_slots, dots);
     PFST_CHECK_LAUNCH("pfst_neigh_dots");
     return PFST_OK;
@@ -730,18 +800,30 @@ static int neigh_dots_impl(const float* x_a, const float* x_b, int64_t B, int32_
   const int64_t plane = (int64_t)h * w;
   const dim3 grid((unsigned)((plane + 127) / 128), (unsigned)(T * B * ks), 1);
   if (grid.y > 65535) return PFST_ERR_UNSUPPORTED;
-  pfst::neigh_dots_generic_kernel<<<grid, 128, 0, s>>>(x_a, x_b, T, (int)B, D, h, w, dilation, ks, slot0, n_slots,
-                                                       dots);
+  if constexpr (esz != 4) {
+    if (fp32_tma) {
+      neigh_dots_generic_kernel<E, true><<<grid, 128, 0, s>>>(x_a, x_b, T, (int)B, D, h, w, dilation, ks, slot0,
+                                                              n_slots, dots);
+      PFST_CHECK_LAUNCH("pfst_neigh_dots");
+      return PFST_OK;
+    }
+  }
+  pfst::neigh_dots_generic_kernel<E, false><<<grid, 128, 0, s>>>(x_a, x_b, T, (int)B, D, h, w, dilation, ks, slot0,
+                                                                    n_slots, dots);
   PFST_CHECK_LAUNCH("pfst_neigh_dots");
   return PFST_OK;
 }
+
+}  // namespace pfst
+
+extern "C" {
 
 int pfst_neigh_dots(const float* x_a, const float* x_b, int64_t B, int32_t D, int32_t h, int32_t w,
                     int32_t dilation, float* dots, void* stream) {
   if (!x_a || !dots || B < 0 || D < 1 || h < 1 || w < 1 || dilation < 1) return PFST_ERR_INVALID_ARG;
   if (B == 0) return PFST_OK;
   if (B > 0x7fffffffll / 4) return PFST_ERR_UNSUPPORTED;
-  return neigh_dots_impl(x_a, x_b, B, D, h, w, dilation, 0, x_b ? 2 : 1, dots, static_cast<cudaStream_t>(stream));
+  return pfst::neigh_dots_impl(x_a, x_b, B, D, h, w, dilation, 0, x_b ? 2 : 1, dots, static_cast<cudaStream_t>(stream));
 }
 
 int pfst_neigh_dots_slot(const float* x, int64_t B, int32_t D, int32_t h, int32_t w, int32_t dilation,
@@ -750,7 +832,25 @@ int pfst_neigh_dots_slot(const float* x, int64_t B, int32_t D, int32_t h, int32_
     return PFST_ERR_INVALID_ARG;
   if (B == 0) return PFST_OK;
   if (B > 0x7fffffffll / 4) return PFST_ERR_UNSUPPORTED;
-  return neigh_dots_impl(x, nullptr, B, D, h, w, dilation, slot, n_slots, dots, static_cast<cudaStream_t>(stream));
+  return pfst::neigh_dots_impl(x, (const float*)nullptr, B, D, h, w, dilation, slot, n_slots, dots,
+                         static_cast<cudaStream_t>(stream));
+}
+
+int pfst_neigh_dots_slot_ft(const void* x, int32_t x_dtype, int64_t B, int32_t D, int32_t h, int32_t w,
+                            int32_t dilation, int32_t slot, int32_t n_slots, float* dots, void* stream) {
+  if (x_dtype == PFST_DT_F32)
+    return pfst_neigh_dots_slot(static_cast<const float*>(x), B, D, h, w, dilation, slot, n_slots, dots, stream);
+  if (x_dtype != PFST_DT_F16 && x_dtype != PFST_DT_BF16) return PFST_ERR_UNSUPPORTED;
+  if (!x || !dots || B < 0 || D < 1 || h < 1 || w < 1 || dilation < 1 || n_slots < 1 || slot < 0 || slot >= n_slots)
+    return PFST_ERR_INVALID_ARG;
+  if (B == 0) return PFST_OK;
+  if (B > 0x7fffffffll / 4) return PFST_ERR_UNSUPPORTED;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (x_dtype == PFST_DT_F16)
+    return pfst::neigh_dots_impl(static_cast<const __half*>(x), (const __half*)nullptr, B, D, h, w, dilation, slot,
+                           n_slots, dots, s);
+  return pfst::neigh_dots_impl(static_cast<const __nv_bfloat16*>(x), (const __nv_bfloat16*)nullptr, B, D, h, w, dilation,
+                         slot, n_slots, dots, s);
 }
 
 int pfst_neigh_grad(const float* x, const float* coef, int64_t B, int32_t D, int32_t h, int32_t w,

@@ -69,9 +69,13 @@ __device__ __forceinline__ void pa_sync_consumers() {
 // the class-sorted lists to `ws` (and the pixel counts to `counts`). MODE 2: stream only — the
 // lists are copied from `ws`, so the ~18 us sort prologue is paid by 8 blocks once instead of by
 // every one of the 144 streaming blocks.
-template <int MODE, class LabelT = int64_t>
-__global__ void __launch_bounds__(kPaThreads)
-proto_accum_kernel(const float* __restrict__ feats, int B, int D, int h, int w,
+// T = fp16 / bf16 feature planes: the same layout (a plane slot holds the 16-bit plane), half the bytes per
+// bulk copy; every value is converted to fp32 as the gather reads it.
+// (16-bit copies: a minimum of one resident block per SM; without it ptxas spilled the int64 MODE 0 copy. For
+// fp32 the minimum is 0, i.e. none, which leaves those kernels as they were.)
+template <int MODE, class LabelT = int64_t, class T = float>
+__global__ void __launch_bounds__(kPaThreads, sizeof(T) == 4 ? 0 : 1)
+proto_accum_kernel(const T* __restrict__ feats, int B, int D, int h, int w,
                    const LabelT* __restrict__ labels, const float* __restrict__ conf, float conf_thr,
                    int lab_h, int lab_w, int C, int groups, int tile, int stages, int use_bulk,
                    float* __restrict__ packed, float* __restrict__ counts, unsigned char* __restrict__ ws) {
@@ -79,7 +83,9 @@ proto_accum_kernel(const float* __restrict__ feats, int B, int D, int h, int w,
   __shared__ uint64_t full_bar[kPaMaxStages], empty_bar[kPaMaxStages];
   __shared__ int issued;          // number of planes the producer has issued so far
   const PaLayout L = pa_layout(tile, stages, C);
-  float* planes = reinterpret_cast<float*>(pa_smem);
+  T* planes = reinterpret_cast<T*>(pa_smem);
+  // a plane slot is plane_stride floats whatever T is: every slot starts on a 16-byte boundary (bulk copies)
+  const int pstride = L.plane_stride * (int)(sizeof(float) / sizeof(T));
   uint16_t* order = reinterpret_cast<uint16_t*>(pa_smem + L.off_order);
   uint16_t* grp = reinterpret_cast<uint16_t*>(pa_smem + L.off_grp);
   uint8_t* rowcls = pa_smem + L.off_rows;
@@ -96,7 +102,7 @@ proto_accum_kernel(const float* __restrict__ feats, int B, int D, int h, int w,
   const int ch0 = (int)((int64_t)grp_id * D / groups), ch1 = (int)((int64_t)(grp_id + 1) * D / groups);
   const int n_items = ch1 - ch0;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const float* base = feats + ((int64_t)b * D + ch0) * hw + p0;
+  const T* base = feats + ((int64_t)b * D + ch0) * hw + p0;
 
   const size_t list_bytes = L.total - L.off_order;           // order | grp | rowcls | seg, tot
   unsigned char* ws_tile = ws ? ws + ((size_t)b * n_tiles + tile_id) * list_bytes : nullptr;
@@ -108,17 +114,17 @@ proto_accum_kernel(const float* __restrict__ feats, int B, int D, int h, int w,
     mbar_fence_init();
     issued = 0;
   }
-  for (int s = threadIdx.x; s < stages; s += kPaThreads) planes[(size_t)s * L.plane_stride + np] = 0.f;  // zero slot
+  for (int s = threadIdx.x; s < stages; s += kPaThreads) planes[(size_t)s * pstride + np] = T(0.f);  // zero slot
   __syncthreads();
 
   if (warp == kPaConsumers) {          // ---- producer: stream the channel planes
     if (MODE != 1 && lane == 0 && use_bulk) {
-      const uint32_t bytes = (uint32_t)np * sizeof(float);
+      const uint32_t bytes = (uint32_t)np * sizeof(T);
       for (int i = 0; i < n_items; ++i) {
         const int s = i % stages;
         if (i >= stages) mbar_wait(&empty_bar[s], (uint32_t)((i / stages) & 1) ^ 1u);
         mbar_arrive_expect_tx(&full_bar[s], bytes);
-        bulk_load_1d(planes + (size_t)s * L.plane_stride, base + (int64_t)i * hw, bytes, &full_bar[s]);
+        bulk_load_1d(planes + (size_t)s * pstride, base + (int64_t)i * hw, bytes, &full_bar[s]);
         *reinterpret_cast<volatile int*>(&issued) = i + 1;
       }
     }
@@ -265,7 +271,7 @@ proto_accum_kernel(const float* __restrict__ feats, int B, int D, int h, int w,
   // ---- consumers: one channel plane per warp per turn ------------------------------------
   for (int i = warp; i < n_items; i += kPaConsumers) {
     const int s = use_bulk ? i % stages : warp;
-    float* pl = planes + (size_t)s * L.plane_stride;
+    T* pl = planes + (size_t)s * pstride;
     if (use_bulk) {
       // A stage is consumed by a different warp on every revolution of the ring, and a parity
       // wait is only meaningful within one phase of the barrier: this warp may get here before
@@ -275,9 +281,9 @@ proto_accum_kernel(const float* __restrict__ feats, int B, int D, int h, int w,
       while (*reinterpret_cast<volatile int*>(&issued) <= i) {}
       mbar_wait(&full_bar[s], (uint32_t)((i / stages) & 1));
     } else {                             // planes a bulk copy cannot describe: the warp stages its own
-      const float* src = base + (int64_t)i * hw;
+      const T* src = base + (int64_t)i * hw;
       for (int e0 = lane; e0 < np; e0 += 32 * kPaUnroll) {
-        float v[kPaUnroll];
+        T v[kPaUnroll];
 #pragma unroll
         for (int u = 0; u < kPaUnroll; ++u)
           if (e0 + u * 32 < np) v[u] = __ldg(src + e0 + u * 32);
@@ -298,7 +304,7 @@ proto_accum_kernel(const float* __restrict__ feats, int B, int D, int h, int w,
       const uint16_t* op = order + r8 * 256 + lane;
       float v[8];
 #pragma unroll
-      for (int u = 0; u < 8; ++u) v[u] = pl[op[32 * u]];
+      for (int u = 0; u < 8; ++u) v[u] = to_f32(pl[op[32 * u]]);
       const unsigned same = cur * 0x01010101u;
       if (cls.x == same && cls.y == same) {
         run += ((v[0] + v[1]) + (v[2] + v[3])) + ((v[4] + v[5]) + (v[6] + v[7]));
@@ -338,9 +344,10 @@ proto_accum_kernel(const float* __restrict__ feats, int B, int D, int h, int w,
 constexpr int kPmThreads = 256;
 constexpr int kPmTile = 4096;
 
-template <int NC, bool FULL, class L>
+// T = fp16 / bf16: a "float4" unit of the loop below is four pixels of one 64-bit load, converted on load.
+template <int NC, bool FULL, class L, class T = float>
 __global__ void __launch_bounds__(kPmThreads, 2)
-proto_accum_masked_kernel(const float* __restrict__ feats, int D, int h, int w, const L* __restrict__ labels,
+proto_accum_masked_kernel(const T* __restrict__ feats, int D, int h, int w, const L* __restrict__ labels,
                           const float* __restrict__ conf, float conf_thr, int lab_h, int lab_w, int groups,
                           float* __restrict__ packed, float* __restrict__ counts) {
   __shared__ __align__(16) uint8_t lab_s[kPmTile];
@@ -363,18 +370,29 @@ proto_accum_masked_kernel(const float* __restrict__ feats, int D, int h, int w, 
   const int n_planes = ch1 - ch0 > warp ? (ch1 - ch0 - warp + 7) / 8 : 0;
   const int n_pairs = (n_planes + 1) / 2;
   const int total = n_pairs * cpp;
-  const float* base = feats + ((int64_t)b * D) * hw + p0;
+  const T* base = feats + ((int64_t)b * D) * hw + p0;
   struct Buf { float4 a[4], b[4]; };
   auto issue = [&](int pair_i, int chunk_i, Buf& q) {
     const int ch = ch0 + warp + 16 * pair_i;
     const bool has_b = ch + 8 < ch1;
-    const float4* pa = reinterpret_cast<const float4*>(base + (int64_t)ch * hw) + lane + 128 * chunk_i;
-    const float4* pb = reinterpret_cast<const float4*>(base + (int64_t)(ch + (has_b ? 8 : 0)) * hw) + lane + 128 * chunk_i;
+    if constexpr (sizeof(T) == 4) {
+      const float4* pa = reinterpret_cast<const float4*>(base + (int64_t)ch * hw) + lane + 128 * chunk_i;
+      const float4* pb = reinterpret_cast<const float4*>(base + (int64_t)(ch + (has_b ? 8 : 0)) * hw) + lane + 128 * chunk_i;
 #pragma unroll
-    for (int u = 0; u < 4; ++u) {
-      const bool ok = FULL || lane + 128 * chunk_i + 32 * u < nvec;
-      q.a[u] = ok ? __ldcs(pa + 32 * u) : make_float4(0.f, 0.f, 0.f, 0.f);
-      q.b[u] = (ok && has_b) ? __ldcs(pb + 32 * u) : make_float4(0.f, 0.f, 0.f, 0.f);
+      for (int u = 0; u < 4; ++u) {
+        const bool ok = FULL || lane + 128 * chunk_i + 32 * u < nvec;
+        q.a[u] = ok ? __ldcs(pa + 32 * u) : make_float4(0.f, 0.f, 0.f, 0.f);
+        q.b[u] = (ok && has_b) ? __ldcs(pb + 32 * u) : make_float4(0.f, 0.f, 0.f, 0.f);
+      }
+    } else {
+      const uint2* pa = reinterpret_cast<const uint2*>(base + (int64_t)ch * hw) + lane + 128 * chunk_i;
+      const uint2* pb = reinterpret_cast<const uint2*>(base + (int64_t)(ch + (has_b ? 8 : 0)) * hw) + lane + 128 * chunk_i;
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        const bool ok = FULL || lane + 128 * chunk_i + 32 * u < nvec;
+        q.a[u] = ok ? unpack4<T>(__ldcs(pa + 32 * u)) : make_float4(0.f, 0.f, 0.f, 0.f);
+        q.b[u] = (ok && has_b) ? unpack4<T>(__ldcs(pb + 32 * u)) : make_float4(0.f, 0.f, 0.f, 0.f);
+      }
     }
   };
   Buf va, vb;
@@ -475,8 +493,9 @@ __host__ __device__ inline size_t ps_smem_bytes(int hw, int C) {
   return ((size_t)kPsCh * stride + (size_t)(kPsThreads / 32) * C * kPsCh) * sizeof(float) + (size_t)((hw + 15) / 16) * 16;
 }
 
+template <class T = float>
 __global__ void __launch_bounds__(kPsThreads)
-proto_accum_small_kernel(const float* __restrict__ feats, int D, int hw, int C, const unsigned char* __restrict__ ws,
+proto_accum_small_kernel(const T* __restrict__ feats, int D, int hw, int C, const unsigned char* __restrict__ ws,
                          size_t list_bytes, size_t off_rows, size_t off_seg, float* __restrict__ packed) {
   extern __shared__ __align__(16) unsigned char ps_smem[];
   const int stride = hw | 1;
@@ -488,10 +507,10 @@ proto_accum_small_kernel(const float* __restrict__ feats, int D, int hw, int C, 
   const int nch = min(kPsCh, D - c0);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   // stage the chunk: nch planes of hw floats, contiguous in global memory
-  const float* src = feats + ((int64_t)b * D + c0) * hw;
+  const T* src = feats + ((int64_t)b * D + c0) * hw;
   for (int e = threadIdx.x; e < nch * hw; e += kPsThreads) {
     const int ch = e / hw, px = e - ch * hw;
-    F[ch * stride + px] = __ldg(src + e);
+    F[ch * stride + px] = ldgf(src + e);
   }
   for (int i = threadIdx.x; i < (kPsThreads / 32) * C * kPsCh; i += kPsThreads) acc[i] = 0.f;
   for (int i = threadIdx.x; i < hw; i += kPsThreads) lab[i] = 255;
@@ -835,12 +854,13 @@ struct PaPlan {
 };
 
 // Launch geometry shared by the three accumulate entry points (stream = with plane stages).
-int pa_plan(PaPlan& P, const float* feats, int64_t B, int32_t D, int32_t h, int32_t w, int32_t C, bool stream) {
+int pa_plan(PaPlan& P, const void* feats, int64_t B, int32_t D, int32_t h, int32_t w, int32_t C, bool stream,
+            int esz = 4) {
   const int64_t hw = (int64_t)h * w;
   P.tile = (int)(hw < pfst::kPaTile ? hw : pfst::kPaTile);
   P.n_tiles = (int)((hw + P.tile - 1) / P.tile);
   // bulk async copies need 16-byte aligned planes whose tiles are multiples of 16 bytes
-  P.use_bulk = (hw % 4 == 0) && (!feats || pfst::aligned16(feats)) ? 1 : 0;
+  P.use_bulk = (hw % (16 / esz) == 0) && (!feats || pfst::aligned16(feats)) ? 1 : 0;
   if (getenv("PFST_ACCUM_NO_BULK")) P.use_bulk = 0;   // debugging aid
   P.stages = 0;
   if (stream) {   // stages: as many as fit next to the sort buffers, at least one per consumer warp + 1
@@ -862,11 +882,11 @@ int pa_plan(PaPlan& P, const float* feats, int64_t B, int32_t D, int32_t h, int3
   return PFST_OK;
 }
 
-template <int MODE, class L>
-int pa_launch(const PaPlan& P, const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
+template <int MODE, class L, class T = float>
+int pa_launch(const PaPlan& P, const T* feats, int64_t B, int32_t D, int32_t h, int32_t w,
               const L* labels, int32_t lab_h, int32_t lab_w, const float* conf, float conf_thr, int32_t C,
               float* packed, float* counts, unsigned char* ws, cudaStream_t s, const char* what) {
-  auto k = pfst::proto_accum_kernel<MODE, L>;
+  auto k = pfst::proto_accum_kernel<MODE, L, T>;
   PFST_CUDA_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)P.L.total), what);
   const int64_t groups = MODE == 1 ? 1 : P.groups;
   k<<<(unsigned)(B * P.n_tiles * groups), pfst::kPaThreads, P.L.total, s>>>(
@@ -889,8 +909,8 @@ int pfst_proto_accum_is_masked(int32_t C, int32_t h, int32_t w) {
 
 namespace {
 
-template <class L>
-int proto_accum(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w, const L* labels, int32_t lab_h,
+template <class L, class T = float>
+int proto_accum(const T* feats, int64_t B, int32_t D, int32_t h, int32_t w, const L* labels, int32_t lab_h,
                 int32_t lab_w, const float* conf, float conf_thr, int32_t C, float* packed, void* stream) {
   if (sizeof(L) == 1 && (int64_t)lab_h * lab_w > 0x7fffffffll) return PFST_ERR_UNSUPPORTED;   // 32-bit gathers
   if (!feats || !labels || !packed || B < 0 || D < 1 || h < 1 || w < 1 || lab_h < 1 || lab_w < 1 || C < 1)
@@ -907,10 +927,10 @@ int proto_accum(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w, 
     if (groups < 1) groups = 1;
     const int64_t grid = B * n_tiles * groups;
     if (grid > 0x7fffffffll) return PFST_ERR_UNSUPPORTED;
-    void (*k)(const float*, int, int, int, const L*, const float*, float, int, int, int, float*, float*);
+    void (*k)(const T*, int, int, int, const L*, const float*, float, int, int, int, float*, float*);
     // whole 128-float4 chunks in every tile: no bounds tests in the streaming loop
     const bool full = hw % 512 == 0;
-#define PFST_PM_PICK(N) (full ? pfst::proto_accum_masked_kernel<N, true, L> : pfst::proto_accum_masked_kernel<N, false, L>)
+#define PFST_PM_PICK(N) (full ? pfst::proto_accum_masked_kernel<N, true, L, T> : pfst::proto_accum_masked_kernel<N, false, L, T>)
     switch (C) {
       case 1: k = PFST_PM_PICK(1); break;
       case 2: k = PFST_PM_PICK(2); break;
@@ -928,7 +948,7 @@ int proto_accum(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w, 
     return PFST_OK;
   }
   PaPlan P;
-  const int rc = pa_plan(P, feats, B, D, h, w, C, true);
+  const int rc = pa_plan(P, feats, B, D, h, w, C, true, (int)sizeof(T));
   if (rc != PFST_OK) return rc;
   return pa_launch<0>(P, feats, B, D, h, w, labels, lab_h, lab_w, conf, conf_thr, C, packed,
                       packed + (int64_t)C * D, nullptr, static_cast<cudaStream_t>(stream), "pfst_proto_accum");
@@ -956,6 +976,46 @@ int pfst_proto_accum_lbl(const float* feats, int64_t B, int32_t D, int32_t h, in
   return PFST_ERR_UNSUPPORTED;
 }
 
+}  // extern "C"
+
+namespace {
+
+template <class T>
+int proto_accum_ft(const void* feats, int64_t B, int32_t D, int32_t h, int32_t w, const void* labels,
+                   int32_t label_dtype, int32_t lab_h, int32_t lab_w, const float* conf, float conf_thr, int32_t C,
+                   float* packed, void* stream) {
+  const T* f = static_cast<const T*>(feats);
+  if (label_dtype == PFST_DT_I64)
+    return proto_accum(f, B, D, h, w, static_cast<const int64_t*>(labels), lab_h, lab_w, conf, conf_thr, C, packed,
+                       stream);
+  if (label_dtype == PFST_DT_U8)
+    return proto_accum(f, B, D, h, w, static_cast<const uint8_t*>(labels), lab_h, lab_w, conf, conf_thr, C, packed,
+                       stream);
+  return PFST_ERR_UNSUPPORTED;
+}
+
+}  // namespace
+
+extern "C" {
+
+int pfst_proto_accum_ft(const void* feats, int32_t feat_dtype, int64_t B, int32_t D, int32_t h, int32_t w,
+                        const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w,
+                        const float* conf, float conf_thr, int32_t C, float* packed, void* stream) {
+  switch (feat_dtype) {
+    case PFST_DT_F32:
+      return proto_accum_ft<float>(feats, B, D, h, w, labels, label_dtype, lab_h, lab_w, conf, conf_thr, C, packed,
+                                   stream);
+    case PFST_DT_F16:
+      return proto_accum_ft<__half>(feats, B, D, h, w, labels, label_dtype, lab_h, lab_w, conf, conf_thr, C, packed,
+                                    stream);
+    case PFST_DT_BF16:
+      return proto_accum_ft<__nv_bfloat16>(feats, B, D, h, w, labels, label_dtype, lab_h, lab_w, conf, conf_thr, C,
+                                           packed, stream);
+    default:
+      return PFST_ERR_UNSUPPORTED;
+  }
+}
+
 int64_t pfst_proto_order_ws_bytes(int64_t B, int32_t h, int32_t w, int32_t C) {
   if (B < 1 || h < 1 || w < 1 || C < 1 || C > pfst::kPrMaxC) return 0;
   PaPlan P;
@@ -978,7 +1038,7 @@ int proto_order(const L* labels, int64_t B, int32_t h, int32_t w, int32_t lab_h,
   PaPlan P;
   const int rc = pa_plan(P, nullptr, B, 1, h, w, C, false);
   if (rc != PFST_OK) return rc;
-  return pa_launch<1>(P, nullptr, B, 1, h, w, labels, lab_h, lab_w, conf, conf_thr, C, nullptr, counts,
+  return pa_launch<1>(P, (const float*)nullptr, B, 1, h, w, labels, lab_h, lab_w, conf, conf_thr, C, nullptr, counts,
                       static_cast<unsigned char*>(workspace), static_cast<cudaStream_t>(stream), "pfst_proto_order");
 }
 
@@ -1004,8 +1064,13 @@ int pfst_proto_order_lbl(const void* labels, int32_t label_dtype, int64_t B, int
   return PFST_ERR_UNSUPPORTED;
 }
 
-int pfst_proto_accum_ordered(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w, int32_t C,
-                             const void* workspace, float* packed, void* stream) {
+}  // extern "C"
+
+namespace {
+
+template <class T>
+int proto_accum_ordered(const T* feats, int64_t B, int32_t D, int32_t h, int32_t w, int32_t C,
+                        const void* workspace, float* packed, void* stream) {
   if (!feats || !workspace || !packed || B < 0 || D < 1 || h < 1 || w < 1 || C < 1) return PFST_ERR_INVALID_ARG;
   if (C > pfst::kPrMaxC || !pfst::aligned16(workspace)) return PFST_ERR_UNSUPPORTED;
   if (B == 0) return PFST_OK;
@@ -1015,21 +1080,44 @@ int pfst_proto_accum_ordered(const float* feats, int64_t B, int32_t D, int32_t h
     // small planes: one block per (image, 32-channel chunk), lists from the MODE 1 launch
     if (pa_plan(P, nullptr, B, 1, h, w, C, false) != PFST_OK) return PFST_ERR_UNSUPPORTED;
     const size_t smem = pfst::ps_smem_bytes(hw, C);
-    PFST_CUDA_TRY(cudaFuncSetAttribute(pfst::proto_accum_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    PFST_CUDA_TRY(cudaFuncSetAttribute(pfst::proto_accum_small_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)smem), "pfst_proto_accum_ordered/attr");
     const int64_t grid = B * ((D + pfst::kPsCh - 1) / pfst::kPsCh);
     if (grid > 0x7fffffffll) return PFST_ERR_UNSUPPORTED;
-    pfst::proto_accum_small_kernel<<<(unsigned)grid, pfst::kPsThreads, smem, static_cast<cudaStream_t>(stream)>>>(
+    pfst::proto_accum_small_kernel<T><<<(unsigned)grid, pfst::kPsThreads, smem, static_cast<cudaStream_t>(stream)>>>(
         feats, D, hw, C, static_cast<const unsigned char*>(workspace), P.list_bytes, P.L.off_rows - P.L.off_order,
         P.L.off_seg - P.L.off_order, packed);
     PFST_CHECK_LAUNCH("pfst_proto_accum_ordered/small");
     return PFST_OK;
   }
-  const int rc = pa_plan(P, feats, B, D, h, w, C, true);
+  const int rc = pa_plan(P, feats, B, D, h, w, C, true, (int)sizeof(T));
   if (rc != PFST_OK) return rc;
   return pa_launch<2>(P, feats, B, D, h, w, (const int64_t*)nullptr, 1, 1, nullptr, 0.f, C, packed, nullptr,
                       static_cast<unsigned char*>(const_cast<void*>(workspace)), static_cast<cudaStream_t>(stream),
                       "pfst_proto_accum_ordered");
+}
+
+}  // namespace
+
+extern "C" {
+
+int pfst_proto_accum_ordered(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w, int32_t C,
+                             const void* workspace, float* packed, void* stream) {
+  return proto_accum_ordered(feats, B, D, h, w, C, workspace, packed, stream);
+}
+
+int pfst_proto_accum_ordered_ft(const void* feats, int32_t feat_dtype, int64_t B, int32_t D, int32_t h, int32_t w,
+                                int32_t C, const void* workspace, float* packed, void* stream) {
+  switch (feat_dtype) {
+    case PFST_DT_F32:
+      return proto_accum_ordered(static_cast<const float*>(feats), B, D, h, w, C, workspace, packed, stream);
+    case PFST_DT_F16:
+      return proto_accum_ordered(static_cast<const __half*>(feats), B, D, h, w, C, workspace, packed, stream);
+    case PFST_DT_BF16:
+      return proto_accum_ordered(static_cast<const __nv_bfloat16*>(feats), B, D, h, w, C, workspace, packed, stream);
+    default:
+      return PFST_ERR_UNSUPPORTED;
+  }
 }
 
 int pfst_proto_finalize(float* packed, int32_t C, int32_t D, const float* mu_prev,

@@ -46,13 +46,24 @@ __device__ __noinline__ int pl_tie_label(const float* __restrict__ px, int64_t H
   }
   return label;
 }
+// the same for 16-bit logits (the float overload above is the one fp32 calls resolve to)
+template <class T>
+__device__ __noinline__ int pl_tie_label(const T* __restrict__ px, int64_t HW, float m, float s, int am,
+                                         float conf) {
+  int label = am;
+  for (int c = am - 1; c >= 0; --c) {
+    const float d = to_f32(px[(int64_t)c * HW]) - m;
+    if (d > -3.0e-4f && exp_exact(d) / s == conf) label = c;
+  }
+  return label;
+}
 
 // x[0..C) are the pixel's logits, held in registers (CMAX is a compile-time
 // bound so the array never spills to local memory; EXACT means C == CMAX).
-template <int CMAX, int MODE, bool EXACT>
+template <int CMAX, int MODE, bool EXACT, class T>
 __device__ __forceinline__ PlOut pl_pixel(const float (&x)[CMAX], int C, float thr,
                                           const float* __restrict__ thr_pc,
-                                          const float* __restrict__ px, int64_t HW) {
+                                          const T* __restrict__ px, int64_t HW) {
   float m = x[0];
   int am = 0;
 #pragma unroll
@@ -113,26 +124,27 @@ __device__ __forceinline__ void pl_block_count(unsigned local, unsigned long lon
 // Persistent grid (one resident wave) with a two-stage software pipeline: the
 // loads of a thread's NEXT item are issued before the ~100 instructions/pixel of
 // exp/divide work on the current one, so HBM never idles behind the math.
-template <int VEC, int CMAX, bool EXACT>
-__device__ __forceinline__ void pl_load(float (&x)[VEC][CMAX], const float* __restrict__ src, int C,
+// T = fp16 / bf16: four pixels are one 64-bit load, converted to fp32 here (once per value).
+template <int VEC, int CMAX, bool EXACT, class T>
+__device__ __forceinline__ void pl_load(float (&x)[VEC][CMAX], const T* __restrict__ src, int C,
                                         int64_t HW) {
 #pragma unroll
   for (int c = 0; c < CMAX; ++c)
     if (EXACT || c < C) {
       if (VEC == 4) {
-        const float4 v = ldg_stream_f4(src);
+        const float4 v = ldg_stream_4(src);
         x[0][c] = v.x; x[1 % VEC][c] = v.y; x[2 % VEC][c] = v.z; x[3 % VEC][c] = v.w;
       } else {
-        x[0][c] = __ldg(src);
+        x[0][c] = ldgf(src);
       }
       src += HW;
     }
 }
 
 // L = uint8: one 32-bit store per 4 labels (the host guarantees C <= 255 and reject_label <= 255).
-template <int VEC, int CMAX, int MODE, bool EXACT, class L>
+template <int VEC, int CMAX, int MODE, bool EXACT, class L, class T = float>
 __global__ void __launch_bounds__(kPlThreads)
-pseudo_label_kernel(const float* __restrict__ logits, int64_t B, int C, int64_t HW, float thr,
+pseudo_label_kernel(const T* __restrict__ logits, int64_t B, int C, int64_t HW, float thr,
                     const float* __restrict__ thr_per_class, int64_t reject_label,
                     L* __restrict__ label, float* __restrict__ conf,
                     float* __restrict__ weight_part, unsigned long long* __restrict__ count) {
@@ -153,17 +165,17 @@ pseudo_label_kernel(const float* __restrict__ logits, int64_t B, int C, int64_t 
   int64_t b = i / per_img;
   i -= (unsigned)b * per_img;
   float cur[VEC][CMAX], nxt[VEC][CMAX];
-  if (b < B) pl_load<VEC, CMAX, EXACT>(cur, logits + b * CHW + (int64_t)i * VEC, C, HW);
+  if (b < B) pl_load<VEC, CMAX, EXACT, T>(cur, logits + b * CHW + (int64_t)i * VEC, C, HW);
   while (b < B) {
     unsigned in = i + stride;
     int64_t bn = b;
     while (in >= per_img) { in -= per_img; ++bn; }
-    if (bn < B) pl_load<VEC, CMAX, EXACT>(nxt, logits + bn * CHW + (int64_t)in * VEC, C, HW);
+    if (bn < B) pl_load<VEC, CMAX, EXACT, T>(nxt, logits + bn * CHW + (int64_t)in * VEC, C, HW);
 
     PlOut o[VEC];
 #pragma unroll
     for (int k = 0; k < VEC; ++k) {
-      o[k] = pl_pixel<CMAX, MODE, EXACT>(cur[k], C, thr, thr_pc,
+      o[k] = pl_pixel<CMAX, MODE, EXACT, T>(cur[k], C, thr, thr_pc,
                                            logits + b * CHW + (int64_t)i * VEC + k, HW);
       local += o[k].confident ? 1u : 0u;
     }
@@ -203,9 +215,9 @@ pseudo_label_kernel(const float* __restrict__ logits, int64_t B, int C, int64_t 
 
 // Any C: one pixel per thread, two passes over the pixel's logits (the second
 // pass is served from L1/L2).
-template <int MODE, class L>
+template <int MODE, class L, class T = float>
 __global__ void __launch_bounds__(kPlThreads)
-pseudo_label_generic_kernel(const float* __restrict__ logits, int64_t B, int C, int64_t HW,
+pseudo_label_generic_kernel(const T* __restrict__ logits, int64_t B, int C, int64_t HW,
                             float thr, const float* __restrict__ thr_per_class,
                             int64_t reject_label, L* __restrict__ label,
                             float* __restrict__ conf, float* __restrict__ weight_part,
@@ -216,16 +228,16 @@ pseudo_label_generic_kernel(const float* __restrict__ logits, int64_t B, int C, 
        i += (int64_t)gridDim.x * kPlThreads) {
     const int64_t b = i / HW;
     const int64_t p = i - b * HW;
-    const float* src = logits + (b * C) * HW + p;
-    float m = src[0];
+    const T* src = logits + (b * C) * HW + p;
+    float m = to_f32(src[0]);
     int am = 0;
     for (int c = 1; c < C; ++c) {
-      const float v = src[(int64_t)c * HW];
+      const float v = to_f32(src[(int64_t)c * HW]);
       if (v > m) { m = v; am = c; }
     }
     float s = 0.f;
     for (int c = 0; c < C; ++c) {
-      const ExpParts e = exp_split(src[(int64_t)c * HW] - m);
+      const ExpParts e = exp_split(to_f32(src[(int64_t)c * HW]) - m);
       s = __fmaf_rn(e.scale, e.mant, s);
     }
     const float cf = 1.0f / s;
@@ -234,7 +246,7 @@ pseudo_label_generic_kernel(const float* __restrict__ logits, int64_t B, int C, 
       lab = 0;
     } else {
       for (int c = am - 1; c >= 0; --c) {
-        const float d = src[(int64_t)c * HW] - m;
+        const float d = to_f32(src[(int64_t)c * HW]) - m;
         if (d > -3.0e-4f && exp_exact(d) / s == cf) lab = c;
       }
     }
@@ -245,7 +257,7 @@ pseudo_label_generic_kernel(const float* __restrict__ logits, int64_t B, int C, 
     } else {
       float ent = 0.f;
       for (int c = 0; c < C; ++c) {
-        const float pc = exp_exact(src[(int64_t)c * HW] - m) / s;
+        const float pc = exp_exact(to_f32(src[(int64_t)c * HW]) - m) / s;
         ent -= pc * logf(pc + 1e-8f);
       }
       confident = ent < t;
@@ -286,11 +298,12 @@ __global__ void exp_selftest_kernel(const float* __restrict__ x, int64_t n,
   if ((threadIdx.x & 31) == 0 && bad) atomicAdd(mismatches, (unsigned long long)bad);
 }
 
-template <int MODE, class L>
-static int launch_pl(const float* logits, int64_t B, int C, int64_t HW, float thr,
+template <int MODE, class L, class T>
+static int launch_pl(const T* logits, int64_t B, int C, int64_t HW, float thr,
                      const float* thr_pc, int64_t reject, L* label, float* conf,
                      float* wpart, unsigned long long* count, cudaStream_t s) {
-  const bool vec4 = (HW % 4 == 0) && aligned16(logits) && aligned_lbl4(label) && aligned16(conf) &&
+  // four pixels per load: 16 bytes of fp32, 8 bytes of fp16 / bf16
+  const bool vec4 = (HW % 4 == 0) && (reinterpret_cast<uintptr_t>(logits) % (4 * sizeof(T)) == 0) && aligned_lbl4(label) && aligned16(conf) &&
                     (!wpart || aligned16(wpart));
   if (HW > 0x7fffffffll || B * (HW / 4 + 1) > 0x7fffffffll * 2) return PFST_ERR_UNSUPPORTED;
   auto grid_flat = [](int64_t items) {
@@ -300,7 +313,7 @@ static int launch_pl(const float* logits, int64_t B, int C, int64_t HW, float th
   };
 #define PFST_PL_LAUNCH(VEC_, CMAX_, EXACT_)                                                      \
   do {                                                                                           \
-    auto k = pseudo_label_kernel<VEC_, CMAX_, MODE, EXACT_, L>;                                     \
+    auto k = pseudo_label_kernel<VEC_, CMAX_, MODE, EXACT_, L, T>;                                     \
     int occ = 0;                                                                                 \
     PFST_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k, kPlThreads, 0),         \
                   "pfst_pseudo_label/occupancy");                                                \
@@ -312,9 +325,9 @@ static int launch_pl(const float* logits, int64_t B, int C, int64_t HW, float th
                                                        label, conf, wpart, count);              \
   } while (0)
   if (C <= 8 && vec4 && MODE == 0) {
-    // exact-C instantiations of the hot configuration (no per-class predicates); the uint8 build
-    // does not instantiate the MODE 1 copies this branch never reaches
-    if constexpr (MODE == 0 || sizeof(L) == 8) {
+    // exact-C instantiations of the hot configuration (no per-class predicates); the uint8 and 16-bit
+    // builds do not instantiate the MODE 1 copies this branch never reaches
+    if constexpr (MODE == 0 || (sizeof(L) == 8 && sizeof(T) == 4)) {
       switch (C) {
         case 2: PFST_PL_LAUNCH(4, 2, true); break;
         case 3: PFST_PL_LAUNCH(4, 3, true); break;
@@ -337,7 +350,7 @@ static int launch_pl(const float* logits, int64_t B, int C, int64_t HW, float th
   } else if (C <= 40) {
     PFST_PL_LAUNCH(1, 40, false);
   } else {
-    pseudo_label_generic_kernel<MODE, L><<<grid_flat(B * HW), kPlThreads, 0, s>>>(
+    pseudo_label_generic_kernel<MODE, L, T><<<grid_flat(B * HW), kPlThreads, 0, s>>>(
         logits, B, C, HW, thr, thr_pc, reject, label, conf, wpart, count);
   }
 #undef PFST_PL_LAUNCH
@@ -353,8 +366,8 @@ extern "C" {
 
 namespace pfst {
 
-template <class L>
-static int pseudo_label(const float* logits, int64_t B, int32_t C, int64_t HW, float thr,
+template <class L, class T = float>
+static int pseudo_label(const T* logits, int64_t B, int32_t C, int64_t HW, float thr,
                         const float* thr_per_class, int32_t mode, int64_t reject_label, L* label,
                         float* conf, float* weight_part, unsigned long long* count, void* stream) {
   if (!logits || !label || !conf || !count) return PFST_ERR_INVALID_ARG;
@@ -394,6 +407,48 @@ int pfst_pseudo_label_lbl(const float* logits, int64_t B, int32_t C, int64_t HW,
     return pfst::pseudo_label(logits, B, C, HW, thr, thr_per_class, mode, reject_label,
                               static_cast<uint8_t*>(label), conf, weight_part, count, stream);
   return PFST_ERR_UNSUPPORTED;
+}
+
+}  // extern "C"
+
+namespace pfst {
+
+template <class T>
+static int pseudo_label_ft(const void* logits, int64_t B, int32_t C, int64_t HW, float thr,
+                           const float* thr_per_class, int32_t mode, int64_t reject_label, void* label,
+                           int32_t label_dtype, float* conf, float* weight_part, unsigned long long* count,
+                           void* stream) {
+  const T* x = static_cast<const T*>(logits);
+  if (label_dtype == PFST_DT_I64)
+    return pseudo_label(x, B, C, HW, thr, thr_per_class, mode, reject_label, static_cast<int64_t*>(label), conf,
+                        weight_part, count, stream);
+  if (label_dtype == PFST_DT_U8)
+    return pseudo_label(x, B, C, HW, thr, thr_per_class, mode, reject_label, static_cast<uint8_t*>(label), conf,
+                        weight_part, count, stream);
+  return PFST_ERR_UNSUPPORTED;
+}
+
+}  // namespace pfst
+
+extern "C" {
+
+int pfst_pseudo_label_ft(const void* logits, int32_t logit_dtype, int64_t B, int32_t C, int64_t HW, float thr,
+                         const float* thr_per_class, int32_t mode, int64_t reject_label, void* label,
+                         int32_t label_dtype, float* conf, float* weight_part, unsigned long long* count,
+                         void* stream) {
+  switch (logit_dtype) {
+    case PFST_DT_F32:
+      return pfst::pseudo_label_ft<float>(logits, B, C, HW, thr, thr_per_class, mode, reject_label, label,
+                                          label_dtype, conf, weight_part, count, stream);
+    case PFST_DT_F16:
+      return pfst::pseudo_label_ft<__half>(logits, B, C, HW, thr, thr_per_class, mode, reject_label, label,
+                                           label_dtype, conf, weight_part, count, stream);
+    case PFST_DT_BF16:
+      return pfst::pseudo_label_ft<__nv_bfloat16>(logits, B, C, HW, thr, thr_per_class, mode, reject_label, label,
+                                                  label_dtype, conf, weight_part, count, stream);
+    default:
+      return PFST_ERR_UNSUPPORTED;
+  }
 }
 
 int pfst_selftest_exp(const float* x, int64_t n, unsigned long long* mismatches, void* stream) {

@@ -26,20 +26,22 @@ static inline EncodeTiledFn get_encode_tiled() {
   return fn;
 }
 
-// fp32 NCHW tensor (B, D, H, W) viewed as a rank-4 TMA tensor (W, H, D, B); box =
-// (box_w, box_h, box_c, 1); out-of-bounds elements (negative or past-the-end
+// NCHW tensor (B, D, H, W) of `dtype` (esz bytes per element) viewed as a rank-4 TMA tensor
+// (W, H, D, B); box = (box_w, box_h, box_c, 1); out-of-bounds elements (negative or past-the-end
 // coordinates = the unfold's zero padding) are filled with zeros by the hardware.
-// Requires W % 4 == 0 (global strides must be multiples of 16 bytes).
-static inline bool make_nchw_tensor_map(CUtensorMap* map, const float* base, int64_t B, int64_t D,
+// Requires W * esz % 16 == 0 (global strides must be multiples of 16 bytes).
+static inline bool make_nchw_tensor_map(CUtensorMap* map, const void* base, int64_t B, int64_t D,
                                         int64_t H, int64_t W, uint32_t box_w, uint32_t box_h,
-                                        uint32_t box_c) {
+                                        uint32_t box_c,
+                                        CUtensorMapDataType dtype = CU_TENSOR_MAP_DATA_TYPE_FLOAT32,
+                                        int64_t esz = 4) {
   EncodeTiledFn enc = get_encode_tiled();
   if (!enc) return false;
   cuuint64_t dims[4] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)D, (cuuint64_t)B};
-  cuuint64_t strides[3] = {(cuuint64_t)W * 4, (cuuint64_t)W * H * 4, (cuuint64_t)W * H * D * 4};
+  cuuint64_t strides[3] = {(cuuint64_t)(W * esz), (cuuint64_t)(W * H * esz), (cuuint64_t)(W * H * D * esz)};
   cuuint32_t box[4] = {box_w, box_h, box_c, 1};
   cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(base), dims, strides,
+  CUresult r = enc(map, dtype, 4, const_cast<void*>(base), dims, strides,
                    box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
                    CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   return r == CUDA_SUCCESS;

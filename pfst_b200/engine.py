@@ -144,11 +144,12 @@ class PluginEngine:
         if label_dtype not in ops.LABEL_DTYPES:
             raise TypeError(f"label maps must be torch.int64 or torch.uint8, got {label_dtype}")
         B, Cc, H, W = ema_logits.shape
-        ops._dev(ema_logits, "ema_logits", torch.float32)
+        ldt = ops._teacher(ema_logits, "ema_logits")      # fp32, fp16 or bf16: the teacher pass's own dtype
         use_x = x_ema is not None and (self.loss_cfg is not None or self.proto_cfg is not None)
         if use_x:
-            ops._dev(x_ema, "x_ema", torch.float32)
-        skey = ("a", tuple(ema_logits.shape), None if not use_x else tuple(x_ema.shape), want_part, label_dtype)
+            ops._teacher(x_ema, "x_ema")
+        skey = ("a", tuple(ema_logits.shape), None if not use_x else tuple(x_ema.shape), want_part, label_dtype,
+                ema_logits.dtype, None if not use_x else x_ema.dtype)
         b = self._bufs.get(skey)
         if b is None:
             e = lambda shape, dt: torch.empty(shape, dtype=dt, device=self.device)  # noqa: E731
@@ -171,7 +172,7 @@ class PluginEngine:
                 with torch.cuda.stream(self._side):
                     ops.neigh_dots_slot(x_ema, geo.dilation // geo.up, 0, b["dots"])
                     self._ev[3].record(self._side)
-            _lib.call("pfst_pseudo_label_lbl", ema_logits.data_ptr(), B, Cc, H * W, float(thr),
+            _lib.call("pfst_pseudo_label_ft", ema_logits.data_ptr(), ldt, B, Cc, H * W, float(thr),
                       None if thr_vec is None else thr_vec.data_ptr(), 0, -1, b["label"].data_ptr(),
                       ops._TORCH2DT[label_dtype], b["conf"].data_ptr(), None if b["wpart"] is None else b["wpart"].data_ptr(),
                       b["count"].data_ptr(), main.cuda_stream)

@@ -37,6 +37,11 @@ class _PFGSTLossFn(torch.autograd.Function):
         geo = ops.LossGeometry(logits_trg.shape, x_src.shape, gt_src.shape, cfg["downscale"], cfg["dilation"])
         if x_ema.shape != x_src.shape:
             raise PfstError("PFGSTLoss: x_ema / x_src shape mismatch")
+        for name, t in (("logits_trg", logits_trg), ("x_src", x_src), ("logits_ema", logits_ema)):
+            if t is not None and t.dtype != torch.float32:
+                raise TypeError(f"PFGSTLoss: {name} must be torch.float32, got {t.dtype} (only the teacher's "
+                                "x_ema may be fp16 / bf16: the student's tensors carry gradients, and the loss's "
+                                "second soft-max of logits_ema is fp32 only)")
         dots, ks = ops.neigh_dots(x_ema, x_src, geo.dilation // geo.up)
         opts, sigma = cfg.get("options", 0), cfg.get("sigma", 30.0)
         if logits_ema is not None:

@@ -47,6 +47,30 @@ def _labels(t: torch.Tensor, name: str, like: Optional[torch.Tensor] = None) -> 
     return _TORCH2DT[t.dtype]
 
 
+# The EMA teacher's outputs (pseudo-label logits, features) may come from a pass run under autocast; the
+# kernels that read them take fp32, fp16 or bf16 (converted to fp32 on load, exactly). Everything that
+# carries a gradient (the student's logits and features) stays fp32.
+TEACHER_DTYPES = (torch.float32, torch.float16, torch.bfloat16)
+_FLOAT2DT = {torch.float32: _lib.DT_F32, torch.float16: _lib.DT_F16, torch.bfloat16: _lib.DT_BF16}
+
+
+def float_dtype_tag(dtype: torch.dtype, name: str = "tensor") -> int:
+    """PFST_DT_F32 / F16 / BF16 tag of a teacher-output dtype; TypeError for any other dtype."""
+    tag = _FLOAT2DT.get(dtype)
+    if tag is None:
+        raise TypeError(f"{name}: teacher outputs must be torch.float32, torch.float16 or torch.bfloat16, "
+                        f"got {dtype}")
+    return tag
+
+
+def _teacher(t: torch.Tensor, name: str) -> int:
+    """Checks a teacher-output tensor and returns its float dtype tag."""
+    if isinstance(t, torch.Tensor):
+        float_dtype_tag(t.dtype, name)
+    _dev(t, name)
+    return _FLOAT2DT[t.dtype]
+
+
 def _stream() -> int:
     # raw cudaStream_t of torch's current stream (also the capturing stream inside torch.cuda.graph);
     # the public torch.cuda.current_stream() builds a Stream object per call (~2 us each, ~10 per step)
@@ -150,11 +174,12 @@ def pseudo_label(logits: torch.Tensor, thr: float = 0.0, thr_per_class: Optional
                  mode: int = 0, reject_label: int = -1, want_part_weight: bool = False,
                  label_dtype: torch.dtype = torch.int64):
     """-> (label (B,H,W) of label_dtype (int64 or uint8), conf fp32 (B,H,W), count int64[1] on device,
-    weight_part|None). uint8 labels need C <= 255 and reject_label <= 255 (negative: no rejection)."""
+    weight_part|None). logits: fp32, fp16 or bf16 (the outputs equal those of the fp32 logits upcast).
+    uint8 labels need C <= 255 and reject_label <= 255 (negative: no rejection)."""
     if logits.dim() != 4:
         raise ValueError("logits must be (B,C,H,W)")
     B, Cc, H, W = logits.shape
-    _dev(logits, "logits", torch.float32)
+    fdt = _teacher(logits, "logits")
     if label_dtype not in LABEL_DTYPES:
         raise TypeError(f"label_dtype must be torch.int64 or torch.uint8, got {label_dtype}")
     if label_dtype == torch.uint8 and (Cc > 255 or int(reject_label) > 255):
@@ -168,7 +193,7 @@ def pseudo_label(logits: torch.Tensor, thr: float = 0.0, thr_per_class: Optional
         if thr_per_class.numel() != Cc:
             raise ValueError("thr_per_class must have C entries")
         _dev(thr_per_class, "thr_per_class", torch.float32)
-    _lib.call("pfst_pseudo_label_lbl", logits.data_ptr(), B, Cc, H * W, float(thr),
+    _lib.call("pfst_pseudo_label_ft", logits.data_ptr(), fdt, B, Cc, H * W, float(thr),
               None if thr_per_class is None else thr_per_class.data_ptr(), mode, int(reject_label),
               label.data_ptr(), _TORCH2DT[label_dtype], conf.data_ptr(), None if wpart is None else wpart.data_ptr(),
               count.data_ptr(), _stream())
@@ -416,15 +441,20 @@ def gaussian_blur(data: torch.Tensor, sigmas: Sequence[float], kernel_size: Opti
 
 # ------------------------------------------------------------ L1-L6: PFGST loss
 def neigh_dots(x_a: torch.Tensor, x_b: Optional[torch.Tensor], dilation: int):
-    """-> (dots float32 (splits, T, B, 5, h, w), splits)."""
-    _dev(x_a, "x_a", torch.float32)
+    """-> (dots float32 (splits, T, B, 5, h, w), splits). x_a / x_b: fp32, fp16 or bf16. Two fp32 tensors
+    are one launch; otherwise each tensor is its own slot launch into the same buffer."""
+    ta = _teacher(x_a, "x_a")
     B, D, h, w = x_a.shape
     T = 1
     if x_b is not None:
-        _dev(x_b, "x_b", torch.float32)
+        tb = _teacher(x_b, "x_b")
         if x_b.shape != x_a.shape:
             raise ValueError("x_a / x_b shape mismatch")
         T = 2
+        if ta != _lib.DT_F32 or tb != _lib.DT_F32:
+            dots, ks = neigh_dots_slot(x_a, dilation, 0)
+            neigh_dots_slot(x_b, dilation, 1, dots)
+            return dots, ks
     ks = int(_lib.load().pfst_neigh_dots_splits(T, B, D, h, w))
     dots = torch.empty((ks, T, B, 5, h, w), dtype=torch.float32, device=x_a.device)
     _lib.call("pfst_neigh_dots", x_a.data_ptr(), None if x_b is None else x_b.data_ptr(), B, D, h, w,
@@ -439,15 +469,15 @@ def neigh_dots_splits(B: int, D: int, h: int, w: int, n_tensors: int = 1) -> int
 def neigh_dots_slot(x: torch.Tensor, dilation: int, slot: int, dots: Optional[torch.Tensor] = None,
                     n_slots: int = 2):
     """One feature tensor into slot `slot` of a (splits, n_slots, B, 5, h, w) dots buffer
-    (slot 0 = x_ema, slot 1 = x_src for the loss). -> (dots, splits)."""
-    _dev(x, "x", torch.float32)
+    (slot 0 = x_ema, slot 1 = x_src for the loss). x: fp32, fp16 or bf16. -> (dots, splits)."""
+    fdt = _teacher(x, "x")
     B, D, h, w = x.shape
     ks = neigh_dots_splits(B, D, h, w)
     if dots is None:
         dots = torch.empty((ks, n_slots, B, 5, h, w), dtype=torch.float32, device=x.device)
     elif dots.numel() != ks * n_slots * B * 5 * h * w:
         raise ValueError("dots buffer has the wrong size")
-    _lib.call("pfst_neigh_dots_slot", x.data_ptr(), B, D, h, w, int(dilation), int(slot), int(n_slots),
+    _lib.call("pfst_neigh_dots_slot_ft", x.data_ptr(), fdt, B, D, h, w, int(dilation), int(slot), int(n_slots),
               _dev(dots, "dots", torch.float32), _stream())
     return dots, ks
 

@@ -104,9 +104,10 @@ class PrototypeBank:
     # P1
     def accumulate(self, feats: torch.Tensor, labels: torch.Tensor, conf: Optional[torch.Tensor] = None,
                    conf_thr: float = 0.0) -> None:
-        """packed += [class sums | class counts] of `feats` over `labels`. Few classes (`masked`): one
+        """packed += [class sums | class counts] of `feats` (fp32, fp16 or bf16) over `labels`. Few classes (`masked`): one
         launch. Otherwise two: the label sort (once per image tile) and the streaming segment-reduce
         (`order` / `accumulate_ordered` can also be issued separately)."""
+        ops._teacher(feats, "feats")        # before the label sort is launched
         B, D, h, w = feats.shape
         if self.masked(h, w, feats):        # few classes: one masked-accumulation launch, no sort
             self.accumulate_single_launch(feats, labels, conf, conf_thr)
@@ -153,7 +154,7 @@ class PrototypeBank:
             raise ValueError("feature dim mismatch")
         if self._order_key != (B, h, w):
             raise PfstError("accumulate_ordered: call order() for this batch geometry first")
-        _lib.call("pfst_proto_accum_ordered", ops._dev(feats, "feats", torch.float32), B, D, h, w, self.C,
+        _lib.call("pfst_proto_accum_ordered_ft", feats.data_ptr(), ops._teacher(feats, "feats"), B, D, h, w, self.C,
                   self._order_ws.data_ptr(), self.packed.data_ptr(), ops._stream())
 
     def accumulate_single_launch(self, feats: torch.Tensor, labels: torch.Tensor,
@@ -163,7 +164,7 @@ class PrototypeBank:
         B, D, h, w = feats.shape
         if D != self.D:
             raise ValueError("feature dim mismatch")
-        _lib.call("pfst_proto_accum_lbl", ops._dev(feats, "feats", torch.float32), B, D, h, w,
+        _lib.call("pfst_proto_accum_ft", feats.data_ptr(), ops._teacher(feats, "feats"), B, D, h, w,
                   labels.data_ptr(), ops._labels(labels, "labels"), labels.shape[-2], labels.shape[-1],
                   ops._opt(conf, "conf", torch.float32), float(conf_thr), self.C, self.packed.data_ptr(),
                   ops._stream())

@@ -143,8 +143,9 @@ class SelfTrainingStep:
         with torch.cuda.stream(self._side):                       # branch 2: L2 on x_ema
             ops.neigh_dots_slot(x_ema, geo.dilation // geo.up, 0, b.dots)
             join.record(self._side)
-        _lib.call("pfst_pseudo_label_lbl", ema_logits.data_ptr(), B, C, H * W, float(self.thr), None, 0, -1,
-                  b.label.data_ptr(), b.ldt, b.conf.data_ptr(), None, b.count.data_ptr(), ops._stream())
+        _lib.call("pfst_pseudo_label_ft", ema_logits.data_ptr(), ops._FLOAT2DT[ema_logits.dtype], B, C, H * W,
+                  float(self.thr), None, 0, -1, b.label.data_ptr(), b.ldt, b.conf.data_ptr(), None, b.count.data_ptr(),
+                  ops._stream())
         if self.bank.masked(x_ema.shape[2], x_ema.shape[3], x_ema):
             self.bank.accumulate(x_ema, b.label)                  # one masked launch next to dots(x_ema)
             main.wait_event(join)
@@ -250,8 +251,9 @@ class SelfTrainingStep:
         with torch.cuda.stream(self._side):
             ops.neigh_dots_slot(x_ema, geo.dilation // geo.up, 0, b.dots)
             dots_ema.record(self._side)
-        _lib.call("pfst_pseudo_label_lbl", ema_logits.data_ptr(), B, C, H * W, float(self.thr), None, 0, -1,
-                  b.label.data_ptr(), b.ldt, b.conf.data_ptr(), None, b.count.data_ptr(), s)
+        _lib.call("pfst_pseudo_label_ft", ema_logits.data_ptr(), ops._FLOAT2DT[ema_logits.dtype], B, C, H * W,
+                  float(self.thr), None, 0, -1, b.label.data_ptr(), b.ldt, b.conf.data_ptr(), None, b.count.data_ptr(),
+                  s)
         pl_done.record(main)
         unsafe = os.environ.get("PFST_DAG_UNSAFE") == "1"           # reproduces DESIGN.md 3.2 (tools/dots_replay_check.py)
         masked = bank.masked(h, w, x_ema)      # few classes: no sort kernel -> nothing to keep away from the TMA kernels
@@ -417,15 +419,18 @@ class SelfTrainingStep:
 
     # ----------------------------------------------------------------------- run
     def run(self, it: int, img, trg_img, gt, ema_logits, logits_trg, x_src, x_ema, rng=np.random):
-        """gt: int64 or uint8; the pseudo labels, ClassMix labels and masks returned have its dtype."""
+        """gt: int64 or uint8; the pseudo labels, ClassMix labels and masks returned have its dtype.
+        ema_logits / x_ema: the teacher's outputs in fp32, fp16 or bf16, each in the dtype the teacher pass
+        produced (a pass under torch.autocast); every other tensor is fp32."""
         B, H, W = gt.shape[0], gt.shape[-2], gt.shape[-1]
         ops._labels(gt, "gt")
         for name, t, dt in (("img", img, torch.float32), ("target_img", trg_img, torch.float32),
-                            ("ema_logits", ema_logits, torch.float32),
-                            ("logits_trg", logits_trg, torch.float32), ("x_src", x_src, torch.float32),
-                            ("x_ema", x_ema, torch.float32)):
+                            ("logits_trg", logits_trg, torch.float32), ("x_src", x_src, torch.float32)):
             ops._dev(t, name, dt)
-        skey = (tuple(img.shape), tuple(ema_logits.shape), tuple(logits_trg.shape), tuple(x_src.shape), gt.dtype)
+        ops._teacher(ema_logits, "ema_logits")
+        ops._teacher(x_ema, "x_ema")
+        skey = (tuple(img.shape), tuple(ema_logits.shape), tuple(logits_trg.shape), tuple(x_src.shape), gt.dtype,
+                ema_logits.dtype, x_ema.dtype)
         ent = self._bufs.get(skey)
         if ent is None:
             geo = ops.LossGeometry(logits_trg.shape, x_src.shape, gt.shape, self.downscale, self.dilation)
@@ -485,21 +490,23 @@ class SelfTrainingStep:
 
 
 def algorithmic_bytes(B: int, C: int, H: int, W: int, D: int, h: int, w: int, n_params: int,
-                      label_bytes: int = 8) -> dict:
+                      label_bytes: int = 8, teacher_bytes: int = 4) -> dict:
     """Algorithmic HBM bytes per step and per kernel family — exactly SURVEY.md §8(d)'s figures
     (cfg2: 1.3115 GB): K_ema 12 B/param; K_pl (4C+12) B/px; K_mask+K_mix 84 B/px (presence read 8
     + mix reads 44 + writes 32); K_sim fwd two feature tensors; K_loss bwd read x_src + write grad;
     K_proto one feature read + the labels; K_dist fwd+bwd 3 feature-sized passes. The small loss
     maps (dots, coefficient maps, ~3.7 MB at cfg2) are not counted. label_bytes = bytes of one
     label-map element (8: int64, 1: uint8): the pseudo-label write, the presence read of gt, the two
-    label reads and the two label-map writes of the mix, and the label gather of K_proto."""
-    P, p, lb = B * H * W, B * h * w, int(label_bytes)
+    label reads and the two label-map writes of the mix, and the label gather of K_proto. teacher_bytes =
+    bytes of one element of the teacher's outputs (4: fp32, 2: fp16 / bf16): the ema_logits read of K_pl,
+    the x_ema half of K_sim fwd and the feature read of K_proto."""
+    P, p, lb, tb = B * H * W, B * h * w, int(label_bytes), int(teacher_bytes)
     return {
         "ema": 12 * n_params,
-        "pseudo_label": (4 * C + 4 + lb) * P,
+        "pseudo_label": (tb * C + 4 + lb) * P,
         "class_presence_and_mix": (44 + 5 * lb) * P,
-        "neigh_dots": 2 * 4 * D * p,
-        "proto_accum": 4 * D * p + lb * p,
+        "neigh_dots": (tb + 4) * D * p,
+        "proto_accum": tb * D * p + lb * p,
         "neigh_grad": 2 * 4 * D * p,
         "proto_dist_fwd_bwd": 3 * 4 * D * p,
     }
