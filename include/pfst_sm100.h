@@ -11,9 +11,11 @@
  *   - plain pointers and sizes only; all data pointers are DEVICE pointers on
  *     the current CUDA device unless the parameter comment says "host";
  *   - tensors are dense, row-major, in the reference's layouts (NCHW logits /
- *     features, (B,1,H,W) int64 label maps); every entry point that takes label maps has a
- *     `_lbl` sibling that takes them as void* plus an int32 label_dtype tag, PFST_DT_I64 or
- *     PFST_DT_U8 (the dtype datasets store); one call's label maps share that dtype;
+ *     features, (B,1,H,W) label maps); every entry point that takes label maps takes them as
+ *     void* plus an int32 label_dtype tag, PFST_DT_I64 (the reference dtype) or PFST_DT_U8 (the
+ *     dtype datasets store); one call's label maps share that dtype. The entry points that read
+ *     the EMA teacher's outputs take them as void* plus a float tag, PFST_DT_F32, PFST_DT_F16 or
+ *     PFST_DT_BF16. Any other tag returns PFST_ERR_UNSUPPORTED before any other argument check;
  *   - `stream` is a cudaStream_t passed as void*; work is enqueued
  *     asynchronously on it; nothing here synchronises the device, allocates
  *     device memory or throws;
@@ -41,9 +43,9 @@ extern "C" {
 #define PFST_DT_U8 0
 #define PFST_DT_I32 1
 #define PFST_DT_I64 2
-/* dtype tags for the teacher-output entry points (`_ft` siblings): the EMA teacher's logits and
- * features may be fp32, fp16 or bf16. Converting fp16 / bf16 to fp32 is exact, so every output
- * equals the fp32 entry point's output on the upcast tensor. */
+/* dtype tags for the teacher outputs: the EMA teacher's logits and features may be fp32, fp16 or
+ * bf16 (a teacher pass run under autocast). Converting fp16 / bf16 to fp32 is exact, so every
+ * output equals the fp32 output on the upcast tensor. */
 #define PFST_DT_F32 16
 #define PFST_DT_F16 17
 #define PFST_DT_BF16 18
@@ -87,25 +89,18 @@ int pfst_ema_coeffs(int64_t iter, double alpha, float* a32_host, float* b32_host
  * ema_ptrs/param_ptrs/numel: device arrays of n_tensors entries.
  * chunk_tensor/chunk_begin: device arrays of n_chunks entries; chunk i covers
  * elements [chunk_begin[i], min(chunk_begin[i]+chunk_elems, numel[t])) of
- * tensor t = chunk_tensor[i]. chunk_elems must be a multiple of 1024.          */
+ * tensor t = chunk_tensor[i]. chunk_elems must be a multiple of 1024.
+ * blocks_per_sm > 0 launches a bounded, persistent grid of 148 * blocks_per_sm blocks that
+ * stride over the chunk table (0 = one block per chunk). A small grid leaves registers and
+ * issue slots for kernels of other streams: the EMA update is independent of the rest of the
+ * step and overlaps its latency-bound kernels.                                  */
 int pfst_ema_update_multi(float* const* ema_ptrs, const float* const* param_ptrs,
                           const int64_t* numel, const int32_t* chunk_tensor,
                           const int64_t* chunk_begin, int64_t n_chunks,
                           int32_t chunk_elems, float a32, float b32, int32_t mode,
-                          void* stream);
+                          int32_t blocks_per_sm, void* stream);
 
-/* Same arithmetic over one flat buffer (e.g. a flattened parameter bucket).   */
-/* pfst_ema_update_multi with a bounded, persistent grid: blocks_per_sm > 0 launches
- * 148 * blocks_per_sm blocks that stride over the chunk table (0 = one block per chunk).
- * A small grid leaves registers and issue slots for kernels of other streams: the EMA
- * update is independent of the rest of the step and overlaps its latency-bound kernels. */
-int pfst_ema_update_multi_ex(float* const* ema_ptrs, const float* const* param_ptrs,
-                             const int64_t* numel, const int32_t* chunk_tensor,
-                             const int64_t* chunk_begin, int64_t n_chunks,
-                             int32_t chunk_elems, float a32, float b32, int32_t mode,
-                             int32_t blocks_per_sm, void* stream);
-
-/* pfst_ema_update_multi_ex (mode 0) with the two coefficients read from DEVICE memory
+/* pfst_ema_update_multi's mode 0 arithmetic with the two coefficients read from DEVICE memory
  * (coefs_dev = float[2] {a32, b32}, e.g. uploaded from pinned memory before a graph launch):
  * no per-step host argument, so the launch can sit at any point of a captured CUDA graph. */
 int pfst_ema_update_multi_dev(float* const* ema_ptrs, const float* const* param_ptrs,
@@ -114,13 +109,17 @@ int pfst_ema_update_multi_dev(float* const* ema_ptrs, const float* const* param_
                               int32_t chunk_elems, const float* coefs_dev,
                               int32_t blocks_per_sm, void* stream);
 
+/* Same arithmetic over one flat buffer (e.g. a flattened parameter bucket).   */
 int pfst_ema_update_flat(float* ema, const float* param, int64_t n, float a32,
                          float b32, int32_t mode, void* stream);
 
 /* ---- S1/S2: pseudo-label generation ----------------------------------------
  * Replaces pfgst.py:259-262 (softmax -> max -> ge(thr)) and the count used for
- * the pseudo-weight at pfgst.py:264-266. One pass over NCHW fp32 logits.
- *   label[b,p] = argmax_c softmax(logits[b,:,p])  (first index on ties, int64)
+ * the pseudo-weight at pfgst.py:264-266. One pass over NCHW logits of logit_dtype
+ * (PFST_DT_F32, PFST_DT_F16 or PFST_DT_BF16: the teacher pass may run under autocast;
+ * torch.softmax is on autocast's fp32 list, so the reference upcasts first). Every value
+ * is converted to fp32 once, on load: the outputs equal the fp32 outputs on the upcast logits.
+ *   label[b,p] = argmax_c softmax(logits[b,:,p])  (first index on ties, label_dtype)
  *   conf[b,p]  = max_c softmax(...)               (fp32, = 1/sum exp(x-max))
  *   confident  = mode 0: conf >= thr[label]  (reference online rule; thr is one
  *                        scalar broadcast, or a per-class vector)
@@ -130,27 +129,14 @@ int pfst_ema_update_flat(float* ema, const float* param, int64_t n, float a32,
  *   weight_part (nullable) = confident ? 1.f : 0.f   (thre_type='part', :267-268)
  *   If reject_label >= 0, label is replaced by reject_label where not confident
  *   (loading.py:484 writes 255).
- * thr_per_class: device pointer to C floats, or NULL to use the scalar `thr`. */
-int pfst_pseudo_label(const float* logits, int64_t B, int32_t C, int64_t HW,
-                      float thr, const float* thr_per_class, int32_t mode,
-                      int64_t reject_label, int64_t* label, float* conf,
-                      float* weight_part, unsigned long long* count, void* stream);
-/* pfst_pseudo_label with the label map in label_dtype (PFST_DT_I64 or PFST_DT_U8; anything else
- * returns PFST_ERR_UNSUPPORTED). Same rule, pfgst.py:259-266 / loading.py:474-487; with PFST_DT_U8 the
- * labels are written as uint8, which needs C <= 255 and reject_label <= 255 (a negative value
- * means no rejection, as above; otherwise PFST_ERR_UNSUPPORTED).                                                              */
-int pfst_pseudo_label_lbl(const float* logits, int64_t B, int32_t C, int64_t HW, float thr,
-                          const float* thr_per_class, int32_t mode, int64_t reject_label,
-                          void* label, int32_t label_dtype, float* conf, float* weight_part,
-                          unsigned long long* count, void* stream);
-/* pfst_pseudo_label_lbl with the logits in logit_dtype (PFST_DT_F32, PFST_DT_F16 or PFST_DT_BF16; anything
- * else returns PFST_ERR_UNSUPPORTED): the teacher pass run under autocast, pfgst.py:259-266 (torch.softmax
- * is on autocast's fp32 list, so the reference upcasts first). Every value is converted to fp32 once, on
- * load; labels, conf, weight_part and count are bit-identical to pfst_pseudo_label_lbl on the upcast logits. */
-int pfst_pseudo_label_ft(const void* logits, int32_t logit_dtype, int64_t B, int32_t C, int64_t HW, float thr,
-                         const float* thr_per_class, int32_t mode, int64_t reject_label, void* label,
-                         int32_t label_dtype, float* conf, float* weight_part, unsigned long long* count,
-                         void* stream);
+ * thr_per_class: device pointer to C floats, or NULL to use the scalar `thr`.
+ * label: PFST_DT_I64 or PFST_DT_U8; uint8 labels need C <= 255 and reject_label <= 255
+ * (otherwise PFST_ERR_UNSUPPORTED). An unknown logit_dtype or label_dtype returns
+ * PFST_ERR_UNSUPPORTED.                                                         */
+int pfst_pseudo_label(const void* logits, int32_t logit_dtype, int64_t B, int32_t C, int64_t HW,
+                      float thr, const float* thr_per_class, int32_t mode, int64_t reject_label,
+                      void* label, int32_t label_dtype, float* conf, float* weight_part,
+                      unsigned long long* count, void* stream);
 
 /* Self-test of the kernel's hand-scheduled exp: *mismatches = number of x[i]
  * (x[i] <= 0) for which it differs bitwise from CUDA's expf. Must be 0.       */
@@ -171,38 +157,28 @@ int pfst_pseudo_weight_fill(float* weight, int64_t B, int64_t H, int64_t W,
 
 /* presence: device uint32[9]; words 0..7 = bitmask of label values 0..255 that
  * occur anywhere in gt[0..n) (torch.unique of the whole batch, :113); word 8 is
- * set non-zero if any label lies outside [0,255]. Zeroed here.                  */
-int pfst_class_presence(const int64_t* gt, int64_t n, uint32_t* presence,
+ * set non-zero if any label lies outside [0,255] (never for a uint8 map). Zeroed here.
+ * gt: label_dtype PFST_DT_I64 or PFST_DT_U8, else PFST_ERR_UNSUPPORTED.         */
+int pfst_class_presence(const void* gt, int32_t label_dtype, int64_t n, uint32_t* presence,
                         void* stream);
-/* pfst_class_presence for a gt of label_dtype (PFST_DT_I64 or PFST_DT_U8, else PFST_ERR_UNSUPPORTED):
- * torch.unique of dacs_transforms.py:113. A uint8 map never sets word 8.                         */
-int pfst_class_presence_lbl(const void* gt, int32_t label_dtype, int64_t n, uint32_t* presence,
-                            void* stream);
 
 /* chosen: device uint32[B*8], per-image bitmask of the classes drawn by the
  * host RNG (np.random.choice, :115-117).
- *   mask        = chosen[b] has bit gt[b,p]                      -> mix_mask int64
+ *   mask        = chosen[b] has bit gt[b,p]                      -> mix_mask
  *   mixed_img   = mask*img + (1-mask)*trg_img  (fp32 arithmetic as one_mix)
- *   mixed_lbl   = mask ? gt : pseudo_label                       (int64)
+ *   mixed_lbl   = mask ? gt : pseudo_label
  *   mixed_weight= mask*1 + (1-mask)*w, w = weight_in[b,p] if weight_in != NULL,
  *                 else the thre_type='all' ratio (float)(count/ps_size) with the
  *                 ignore_top/bottom rows zeroed (pfgst.py:264-277, 295-298).
+ * gt, pseudo_label, mixed_lbl and mix_mask are all of label_dtype (PFST_DT_I64 or
+ * PFST_DT_U8, else PFST_ERR_UNSUPPORTED).
  * Any output pointer may be NULL to skip it. weight_in may alias mixed_weight.  */
-int pfst_class_mix(const int64_t* gt, const uint32_t* chosen, const float* img,
-                   const float* trg_img, const int64_t* pseudo_label,
-                   const float* weight_in, const unsigned long long* count,
-                   int64_t ps_size, int32_t ignore_top, int32_t ignore_bottom,
-                   int64_t B, int32_t img_channels, int64_t H, int64_t W,
-                   float* mixed_img, int64_t* mixed_lbl, float* mixed_weight,
-                   int64_t* mix_mask, void* stream);
-/* pfst_class_mix (dacs_transforms.py:122-144, pfgst.py:287-300) with gt, pseudo_label, mixed_lbl and
- * mix_mask all of label_dtype (PFST_DT_I64 or PFST_DT_U8, else PFST_ERR_UNSUPPORTED).            */
-int pfst_class_mix_lbl(const void* gt, const uint32_t* chosen, const float* img,
-                       const float* trg_img, const void* pseudo_label, const float* weight_in,
-                       const unsigned long long* count, int64_t ps_size, int32_t ignore_top,
-                       int32_t ignore_bottom, int64_t B, int32_t img_channels, int64_t H, int64_t W,
-                       float* mixed_img, void* mixed_lbl, float* mixed_weight, void* mix_mask,
-                       int32_t label_dtype, void* stream);
+int pfst_class_mix(const void* gt, const uint32_t* chosen, const float* img,
+                   const float* trg_img, const void* pseudo_label, const float* weight_in,
+                   const unsigned long long* count, int64_t ps_size, int32_t ignore_top,
+                   int32_t ignore_bottom, int64_t B, int32_t img_channels, int64_t H, int64_t W,
+                   float* mixed_img, void* mixed_lbl, float* mixed_weight, void* mix_mask,
+                   int32_t label_dtype, void* stream);
 
 /* one_mix for a caller-supplied mask (dacs_transforms.py:129-144), one image:
  * out[c,p] = mask[p]*a[c,p] + (1-mask[p])*b[c,p]; mask int64 {0,1} of HW entries;
@@ -241,77 +217,30 @@ int pfst_neigh_grad(const float* x, const float* coef, int64_t B, int32_t D, int
  * buffer of pfst_neigh_dots_splits(1,B,D,h,w) channel splits (the loss reads slot 0 =
  * x_ema, slot 1 = x_src), so the two feature tensors can be processed at different
  * points of the step (x_ema next to the prototype accumulation, x_src next to the
- * prototype distance: the second kernel of each pair then hits the 126 MB L2).       */
-int pfst_neigh_dots_slot(const float* x, int64_t B, int32_t D, int32_t h, int32_t w,
-                         int32_t dilation, int32_t slot, int32_t n_slots, float* dots,
-                         void* stream);
-/* pfst_neigh_dots_slot for x of x_dtype (PFST_DT_F32, PFST_DT_F16 or PFST_DT_BF16, else
- * PFST_ERR_UNSUPPORTED): the EMA features of a teacher run under autocast, get_sim_feat
- * pfgst_loss.py:181-201 (cosine_similarity is on autocast's fp32 list). The dot maps are bit-identical to
- * pfst_neigh_dots_slot on the upcast tensor: the same channel splits, the same per-warp channel order and
- * the same merge order, on every path (TMA, small-plane bulk copy, generic).                        */
-int pfst_neigh_dots_slot_ft(const void* x, int32_t x_dtype, int64_t B, int32_t D, int32_t h, int32_t w,
-                            int32_t dilation, int32_t slot, int32_t n_slots, float* dots, void* stream);
+ * prototype distance: the second kernel of each pair then hits the 126 MB L2).
+ * x: x_dtype PFST_DT_F32, PFST_DT_F16 or PFST_DT_BF16 (the EMA features of a teacher run
+ * under autocast; get_sim_feat pfgst_loss.py:181-201, cosine_similarity is on autocast's
+ * fp32 list), else PFST_ERR_UNSUPPORTED. A 16-bit x gives the dot maps of its fp32 upcast
+ * bit for bit: the same channel splits, the same per-warp channel order and the same merge
+ * order, on every path (TMA, small-plane bulk copy, generic).                          */
+int pfst_neigh_dots_slot(const void* x, int32_t x_dtype, int64_t B, int32_t D, int32_t h, int32_t w,
+                         int32_t dilation, int32_t slot, int32_t n_slots, float* dots, void* stream);
 
 /* pfst_neigh_grad and pfst_proto_dist_bwd (below) in one pass over x: grad_x =
- * neighbourhood-cosine gradient + grad_loss * (x - mu[label]) / (dist * n_valid).
+ * neighbourhood-cosine gradient + grad_loss * (x - mu[label]) / (dist * n_valid)
+ * (pfgst_loss.py:181-201 backward + pfgst.py:168-177 backward).
  * x is read once and grad_x written once for both losses (8*D B/pixel instead of
- * 20*D). Same argument meaning as the two entry points it fuses.                     */
+ * 20*D). Same argument meaning as the two entry points it fuses; labels of label_dtype
+ * (PFST_DT_I64 or PFST_DT_U8, else PFST_ERR_UNSUPPORTED).                              */
 int pfst_neigh_grad_proto(const float* x, const float* coef, int64_t B, int32_t D, int32_t h,
-                          int32_t w, int32_t dilation, const int64_t* labels,
+                          int32_t w, int32_t dilation, const void* labels, int32_t label_dtype,
                           int32_t lab_h, int32_t lab_w, const float* mu, const uint8_t* seen,
                           int32_t C, const float* dist, const double* acc,
                           const float* grad_loss, float* grad_x, void* stream);
-/* pfst_neigh_grad_proto with labels of label_dtype (PFST_DT_I64 or PFST_DT_U8, else
- * PFST_ERR_UNSUPPORTED); pfgst_loss.py:181-201 backward + pfgst.py:168-177 backward.            */
-int pfst_neigh_grad_proto_lbl(const float* x, const float* coef, int64_t B, int32_t D, int32_t h,
-                              int32_t w, int32_t dilation, const void* labels, int32_t label_dtype,
-                              int32_t lab_h, int32_t lab_w, const float* mu, const uint8_t* seen,
-                              int32_t C, const float* dist, const double* acc,
-                              const float* grad_loss, float* grad_x, void* stream);
 
-/* Bytes of the `workspace` the two entry points below share (per-pixel maps written
- * by the forward's prep kernel and re-read by the backward). Host only.             */
-int64_t pfst_pfgst_loss_ws_bytes(int64_t B, int32_t C, int32_t fh, int32_t fw, int32_t up);
-
-/* dots: output of pfst_neigh_dots(x_ema, x_src) on the (fh,fw) feature grid with
- * dilation `dilation/up`; the loss grid is (fh*up, fw*up) (features nearest-
- * upsampled by the integer factor `up`, pfgst_loss.py:58-59).
- * logits: (B,C,lh,lw), sampled at src = min(floor(dst*lscale), in-1) (nearest
- * down-scaling by `downscale`, :57; lscale = 1/downscale).
- * gt, mix: (B,1,gt_h,gt_w) int64 source labels / ClassMix masks, nearest-sampled
- * to the loss grid (:62-67). weights6 (host): src_pos, src_neg, src_pos_std,
- * src_neg_std, sim_pos, sim_neg (:110-135).
- * workspace: device buffer of pfst_pfgst_loss_ws_bytes() bytes, 16-byte aligned, kept
- * (with stats) for the backward. stats: device double[16] (first nine written here).
- * losses: device float[6] = loss_src_pos_mean, loss_src_neg_mean, loss_src_pos_std,
- * loss_src_neg_std, loss_sim_pos, loss_sim_neg. density (nullable): (B,fh*up,fw*up)
- * = 1 - mean_k cos_ema ('vis|density_sim_feat', :136); eroded (nullable): uint8 of
- * the eroded target mask (:69-71).                                                 */
-int pfst_pfgst_loss_fwd(const float* dots, int32_t ksplit, int64_t B, int32_t fh,
-                        int32_t fw, int32_t up, const float* logits, int32_t C,
-                        int32_t lh, int32_t lw, float lscale_h, float lscale_w,
-                        const int64_t* gt, const int64_t* mix, int32_t gt_h,
-                        int32_t gt_w, int32_t dilation, int32_t top_k,
-                        const float* weights6_host, void* workspace, double* stats,
-                        float* losses, float* density, uint8_t* eroded, void* stream);
-
-/* grad_losses: device float[6], upstream gradient of each loss. coef (nullable): (B,9,fh,fw)
- * for pfst_neigh_grad(x_src, dilation/up). grad_logits (nullable): (B,C,lh,lw),
- * zero-filled here, gradient of the two loss_sim terms. At least one of the two outputs;
- * two launches (coef only / grad_logits only) let the coefficient maps — the only part the
- * x_src gradient pass waits for — leave the critical path early.                    */
-int pfst_pfgst_loss_bwd(const float* dots, int32_t ksplit, int64_t B, int32_t fh,
-                        int32_t fw, int32_t up, const float* logits, int32_t C,
-                        int32_t lh, int32_t lw, float lscale_h, float lscale_w,
-                        const int64_t* gt, const int64_t* mix, int32_t gt_h,
-                        int32_t gt_w, int32_t dilation, int32_t top_k,
-                        const float* weights6_host, const void* workspace,
-                        const double* stats, const float* grad_losses, float* coef,
-                        float* grad_logits, void* stream);
-
-/* The same two entry points with the PFGSTLoss options outside the shipped configuration
- * (pfgst_loss.py:16-18). `options` is a bit set:
+/* PFGSTLoss.forward and its backward (pfgst_loss.py:44-234). `options` is a bit set of the
+ * PFGSTLoss options outside the shipped configuration (pfgst_loss.py:16-18); 0 = the shipped
+ * configuration:
  *   PFST_LOSS_SIM_GAUSSIAN   sim_type='gaussian' (:189-191): exp(-|x_n - x_m|^2 / sigma^2), formed from the
  *                            same five dot maps as the cosine (|x_n|^2 + |x_m|^2 - 2 x_n.x_m); the zero
  *                            padding of the unfold is the zero vector (similarity exp(-|x_n|^2 / sigma^2));
@@ -324,55 +253,60 @@ int pfst_pfgst_loss_bwd(const float* dots, int32_t ksplit, int64_t B, int32_t fh
  *                            relu(S - margin[1]) over negative pairs (margin2: squared); margin_host = HOST
  *                            float[2], |margin| <= 1. losses[0], losses[1] = loss_src_pos, loss_src_neg;
  *                            losses[2], losses[3] = 0.
- * top_k = 0 stands for the reference's top_k=None (:218-220): every tap enters both consistency terms.
- * 0 = the shipped configuration. The workspace is pfst_pfgst_loss_ws_bytes_ex(..., options) bytes.          */
+ * top_k = 0 stands for the reference's top_k=None (:218-220): every tap enters both consistency terms.   */
 #define PFST_LOSS_SIM_GAUSSIAN 1
 #define PFST_LOSS_CROSS_PROB_EMA 2
 #define PFST_LOSS_UNFOLD_GRAD 4
 #define PFST_LOSS_SRC_MARGIN 8
 #define PFST_LOSS_SRC_MARGIN2 16
-int64_t pfst_pfgst_loss_ws_bytes_ex(int64_t B, int32_t C, int32_t fh, int32_t fw, int32_t up,
-                                    int32_t options);
-int pfst_pfgst_loss_fwd_ex(const float* dots, int32_t ksplit, int64_t B, int32_t fh,
-                           int32_t fw, int32_t up, const float* logits, int32_t C,
-                           int32_t lh, int32_t lw, float lscale_h, float lscale_w,
-                           const int64_t* gt, const int64_t* mix, int32_t gt_h,
-                           int32_t gt_w, int32_t dilation, int32_t top_k,
-                           const float* weights6_host, void* workspace, double* stats,
-                           float* losses, float* density, uint8_t* eroded, int32_t options,
-                           float sigma, const float* logits_ema, const float* margin_host,
-                           void* stream);
-int pfst_pfgst_loss_bwd_ex(const float* dots, int32_t ksplit, int64_t B, int32_t fh,
-                           int32_t fw, int32_t up, const float* logits, int32_t C,
-                           int32_t lh, int32_t lw, float lscale_h, float lscale_w,
-                           const int64_t* gt, const int64_t* mix, int32_t gt_h,
-                           int32_t gt_w, int32_t dilation, int32_t top_k,
-                           const float* weights6_host, const void* workspace,
-                           const double* stats, const float* grad_losses, float* coef,
-                           float* grad_logits, int32_t options, float sigma,
-                           const float* logits_ema, const float* margin_host, void* stream);
-/* pfst_pfgst_loss_fwd_ex / _bwd_ex (pfgst_loss.py:44-234, nearest-sampled gt and mix of :62-67) with
- * gt and mix of label_dtype (PFST_DT_I64 or PFST_DT_U8, else PFST_ERR_UNSUPPORTED), the last
- * argument before the stream. Every option set goes through them.                                */
-int pfst_pfgst_loss_fwd_lbl(const float* dots, int32_t ksplit, int64_t B, int32_t fh,
-                            int32_t fw, int32_t up, const float* logits, int32_t C,
-                            int32_t lh, int32_t lw, float lscale_h, float lscale_w,
-                            const void* gt, const void* mix, int32_t gt_h,
-                            int32_t gt_w, int32_t dilation, int32_t top_k,
-                            const float* weights6_host, void* workspace, double* stats,
-                            float* losses, float* density, uint8_t* eroded, int32_t options,
-                            float sigma, const float* logits_ema, const float* margin_host,
-                            int32_t label_dtype, void* stream);
-int pfst_pfgst_loss_bwd_lbl(const float* dots, int32_t ksplit, int64_t B, int32_t fh,
-                            int32_t fw, int32_t up, const float* logits, int32_t C,
-                            int32_t lh, int32_t lw, float lscale_h, float lscale_w,
-                            const void* gt, const void* mix, int32_t gt_h,
-                            int32_t gt_w, int32_t dilation, int32_t top_k,
-                            const float* weights6_host, const void* workspace,
-                            const double* stats, const float* grad_losses, float* coef,
-                            float* grad_logits, int32_t options, float sigma,
-                            const float* logits_ema, const float* margin_host,
-                            int32_t label_dtype, void* stream);
+
+/* Bytes of the `workspace` pfst_pfgst_loss_fwd / _bwd share for these `options` (per-pixel
+ * maps written by the forward's prep kernel and re-read by the backward). Host only.   */
+int64_t pfst_pfgst_loss_ws_bytes(int64_t B, int32_t C, int32_t fh, int32_t fw, int32_t up,
+                                 int32_t options);
+
+/* dots: output of pfst_neigh_dots(x_ema, x_src) on the (fh,fw) feature grid with
+ * dilation `dilation/up`; the loss grid is (fh*up, fw*up) (features nearest-
+ * upsampled by the integer factor `up`, pfgst_loss.py:58-59).
+ * logits: (B,C,lh,lw), sampled at src = min(floor(dst*lscale), in-1) (nearest
+ * down-scaling by `downscale`, :57; lscale = 1/downscale).
+ * gt, mix: (B,1,gt_h,gt_w) source labels / ClassMix masks of label_dtype (PFST_DT_I64 or
+ * PFST_DT_U8, else PFST_ERR_UNSUPPORTED), nearest-sampled to the loss grid (:62-67).
+ * weights6 (host): src_pos, src_neg, src_pos_std, src_neg_std, sim_pos, sim_neg (:110-135).
+ * workspace: device buffer of pfst_pfgst_loss_ws_bytes(..., options) bytes, 16-byte aligned,
+ * kept (with stats) for the backward. stats: device double[16] (first nine written here).
+ * losses: device float[6] = loss_src_pos_mean, loss_src_neg_mean, loss_src_pos_std,
+ * loss_src_neg_std, loss_sim_pos, loss_sim_neg. density (nullable): (B,fh*up,fw*up)
+ * = 1 - mean_k cos_ema ('vis|density_sim_feat', :136); eroded (nullable): uint8 of
+ * the eroded target mask (:69-71). options / sigma / logits_ema / margin_host: above
+ * (0, 0, NULL, NULL for the shipped configuration).                                 */
+int pfst_pfgst_loss_fwd(const float* dots, int32_t ksplit, int64_t B, int32_t fh,
+                        int32_t fw, int32_t up, const float* logits, int32_t C,
+                        int32_t lh, int32_t lw, float lscale_h, float lscale_w,
+                        const void* gt, const void* mix, int32_t gt_h,
+                        int32_t gt_w, int32_t dilation, int32_t top_k,
+                        const float* weights6_host, void* workspace, double* stats,
+                        float* losses, float* density, uint8_t* eroded, int32_t options,
+                        float sigma, const float* logits_ema, const float* margin_host,
+                        int32_t label_dtype, void* stream);
+
+/* The arguments the forward took, plus: grad_losses: device float[6], upstream gradient of
+ * each loss. coef (nullable): (B,9,fh,fw) for pfst_neigh_grad(x_src, dilation/up).
+ * grad_logits (nullable): (B,C,lh,lw), zero-filled here, gradient of the two loss_sim
+ * terms. At least one of the two outputs; two launches (coef only / grad_logits only) let
+ * the coefficient maps — the only part the x_src gradient pass waits for — leave the
+ * critical path early. gt and mix are not read (the forward left their classes in the
+ * workspace); label_dtype is still validated.                                        */
+int pfst_pfgst_loss_bwd(const float* dots, int32_t ksplit, int64_t B, int32_t fh,
+                        int32_t fw, int32_t up, const float* logits, int32_t C,
+                        int32_t lh, int32_t lw, float lscale_h, float lscale_w,
+                        const void* gt, const void* mix, int32_t gt_h,
+                        int32_t gt_w, int32_t dilation, int32_t top_k,
+                        const float* weights6_host, const void* workspace,
+                        const double* stats, const float* grad_losses, float* coef,
+                        float* grad_logits, int32_t options, float sigma,
+                        const float* logits_ema, const float* margin_host,
+                        int32_t label_dtype, void* stream);
 
 /* ---- P1-P3: class prototypes (north_star extension; no reference code) ----------
  * Anchor: PFGST.masked_feat_dist, rsiseg/models/uda/pfgst.py:168-177. Labels are
@@ -386,70 +320,50 @@ int pfst_proto_accum_is_masked(int32_t C, int32_t h, int32_t w);
 /* packed: float[C*D + C], ACCUMULATED INTO (caller zeroes it; it is the NCCL
  * all-reduce buffer): packed[c*D+d] += sum of feats[b,d,n] over pixels n with
  * label c (0 <= label < C, and conf >= conf_thr when conf != NULL);
- * packed[C*D+c] += number of such pixels. labels: (B,lab_h,lab_w) int64,
- * conf: (B,lab_h,lab_w) fp32 or NULL.                                              */
-int pfst_proto_accum(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
-                     const int64_t* labels, int32_t lab_h, int32_t lab_w,
-                     const float* conf, float conf_thr, int32_t C, float* packed,
-                     void* stream);
-/* pfst_proto_accum with labels of label_dtype (PFST_DT_I64 or PFST_DT_U8, else PFST_ERR_UNSUPPORTED);
- * anchor pfgst.py:168-177, labels nearest-resampled as pfgst_loss.py:62.                         */
-int pfst_proto_accum_lbl(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
-                         const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w,
-                         const float* conf, float conf_thr, int32_t C, float* packed, void* stream);
-/* pfst_proto_accum_lbl with feats of feat_dtype (PFST_DT_F32, PFST_DT_F16 or PFST_DT_BF16, else
- * PFST_ERR_UNSUPPORTED): the EMA features of a teacher run under autocast; anchor pfgst.py:168-177.
- * Every value is converted to fp32 on load; the sums are float atomics as on the fp32 path.     */
-int pfst_proto_accum_ft(const void* feats, int32_t feat_dtype, int64_t B, int32_t D, int32_t h, int32_t w,
-                        const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w,
-                        const float* conf, float conf_thr, int32_t C, float* packed, void* stream);
+ * packed[C*D+c] += number of such pixels. labels: (B,lab_h,lab_w) of label_dtype
+ * (PFST_DT_I64 or PFST_DT_U8), conf: (B,lab_h,lab_w) fp32 or NULL. feats: feat_dtype
+ * PFST_DT_F32, PFST_DT_F16 or PFST_DT_BF16 (the EMA features of a teacher run under
+ * autocast), every value converted to fp32 on load; the sums are float atomics.
+ * An unknown feat_dtype or label_dtype returns PFST_ERR_UNSUPPORTED.                */
+int pfst_proto_accum(const void* feats, int32_t feat_dtype, int64_t B, int32_t D, int32_t h, int32_t w,
+                     const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w,
+                     const float* conf, float conf_thr, int32_t C, float* packed, void* stream);
 
 /* pfst_proto_accum split in two, so that the label sort is done ONCE per (image, tile) and
  * not by every streaming block:
  *   pfst_proto_order          builds, per 4096-pixel tile of every image, the list of pixel
- *                             offsets sorted by class (labels nearest-resampled to (h,w), confidence
- *                             mask applied) into `workspace` (pfst_proto_order_ws_bytes() bytes,
- *                             16-byte aligned) and adds the per-class pixel counts to counts[C]
- *                             (nullable; pass packed + C*D);
- *   pfst_proto_accum_ordered  streams the feature planes against those lists:
+ *                             offsets sorted by class (labels of label_dtype, PFST_DT_I64 or
+ *                             PFST_DT_U8, nearest-resampled to (h,w), confidence mask applied)
+ *                             into `workspace` (pfst_proto_order_ws_bytes() bytes, 16-byte
+ *                             aligned) and adds the per-class pixel counts to counts[C]
+ *                             (nullable; pass packed + C*D). The lists do not depend on the
+ *                             label dtype;
+ *   pfst_proto_accum_ordered  streams the feature planes (feat_dtype PFST_DT_F32, PFST_DT_F16
+ *                             or PFST_DT_BF16) against those lists:
  *                             packed[c*D+d] += sum of feats over the pixels of class c.
- * Together they equal pfst_proto_accum.                                                 */
+ * Together they equal pfst_proto_accum. An unknown tag returns PFST_ERR_UNSUPPORTED.   */
 int64_t pfst_proto_order_ws_bytes(int64_t B, int32_t h, int32_t w, int32_t C);
-int pfst_proto_order(const int64_t* labels, int64_t B, int32_t h, int32_t w, int32_t lab_h,
-                     int32_t lab_w, const float* conf, float conf_thr, int32_t C, float* counts,
-                     void* workspace, void* stream);
-/* pfst_proto_order with labels of label_dtype (PFST_DT_I64 or PFST_DT_U8, else PFST_ERR_UNSUPPORTED);
- * the lists it writes do not depend on the label dtype (pfst_proto_accum_ordered is shared).     */
-int pfst_proto_order_lbl(const void* labels, int32_t label_dtype, int64_t B, int32_t h, int32_t w,
-                         int32_t lab_h, int32_t lab_w, const float* conf, float conf_thr, int32_t C,
-                         float* counts, void* workspace, void* stream);
-int pfst_proto_accum_ordered(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
-                             int32_t C, const void* workspace, float* packed, void* stream);
-/* pfst_proto_accum_ordered with feats of feat_dtype (PFST_DT_F32, PFST_DT_F16 or PFST_DT_BF16, else
- * PFST_ERR_UNSUPPORTED); anchor pfgst.py:168-177. The workspace of pfst_proto_order is shared.  */
-int pfst_proto_accum_ordered_ft(const void* feats, int32_t feat_dtype, int64_t B, int32_t D, int32_t h,
-                                int32_t w, int32_t C, const void* workspace, float* packed, void* stream);
+int pfst_proto_order(const void* labels, int32_t label_dtype, int64_t B, int32_t h, int32_t w,
+                     int32_t lab_h, int32_t lab_w, const float* conf, float conf_thr, int32_t C,
+                     float* counts, void* workspace, void* stream);
+int pfst_proto_accum_ordered(const void* feats, int32_t feat_dtype, int64_t B, int32_t D, int32_t h,
+                             int32_t w, int32_t C, const void* workspace, float* packed, void* stream);
 
 /* mu_out[c] = packed sums / max(count,1) for classes with pixels; classes already
  * seen (seen_prev[c] != 0) are EMA-updated fl(fl(a32*mu_prev)+fl(b32*mean)) (the E2
  * rule); classes without pixels keep mu_prev. mu_prev / seen_prev may be NULL
  * (first call) and may alias mu_out / seen_out (in-place bank update). cnt_out
  * int64[C], seen_out uint8[C] may be NULL. reset_packed != 0 zeroes `packed` after it
- * has been consumed (ready for the next step's accumulation; no separate memset).   */
-int pfst_proto_finalize(float* packed, int32_t C, int32_t D, const float* mu_prev,
-                        const uint8_t* seen_prev, float a32, float b32, float* mu_out,
-                        int64_t* cnt_out, uint8_t* seen_out, int32_t reset_packed,
-                        void* stream);
-
-/* pfst_proto_finalize with the bank iteration kept ON THE DEVICE: iter_state = int64[2]
- * {iteration (0 on the first call), internal block counter (0)}. The kernel derives
- * a = min(1 - 1/(iter+1), alpha), b = 1 - a in fp64 exactly as pfst_ema_coeffs does (iter 0:
+ * has been consumed (ready for the next step's accumulation; no separate memset).
+ * The bank iteration is kept ON THE DEVICE: iter_state = int64[2] {iteration (0 on the
+ * first call), internal block counter (0)}. The kernel derives a = min(1 - 1/(iter+1), alpha),
+ * b = 1 - a in fp64 exactly as pfst_ema_coeffs does (a32 = (float)a, b32 = (float)b; iter 0:
  * plain mean) and advances the iteration itself, so the launch carries no per-step host
  * argument and can be captured in a CUDA graph.                                        */
-int pfst_proto_finalize_dev(float* packed, int32_t C, int32_t D, const float* mu_prev,
-                            const uint8_t* seen_prev, double alpha, int64_t* iter_state,
-                            float* mu_out, int64_t* cnt_out, uint8_t* seen_out,
-                            int32_t reset_packed, void* stream);
+int pfst_proto_finalize(float* packed, int32_t C, int32_t D, const float* mu_prev,
+                        const uint8_t* seen_prev, double alpha, int64_t* iter_state,
+                        float* mu_out, int64_t* cnt_out, uint8_t* seen_out,
+                        int32_t reset_packed, void* stream);
 
 /* ---- G1: PFGST.masked_feat_dist (rsiseg/models/uda/pfgst.py:168-177) -----------------------
  * loss = mean over the selected pixels of ||f1[:,n] - f2[:,n]||_2; selected = mask[n] != 0
@@ -473,7 +387,7 @@ int pfst_feat_dist_bwd(const float* f1, const float* f2, const uint8_t* mask, in
  * u64) that all peers map through a CUDA IPC handle; pfst_proto_finalize_peer pushes this
  * rank's packed [sums|counts] into every board, waits for the peers' step tokens and sums the
  * inbox in rank order (bit-identical prototypes on every rank), then finalises like
- * pfst_proto_finalize_dev (which it equals for nranks = 1).
+ * pfst_proto_finalize (which it equals for nranks = 1).
  *
  * Set-up entry points (called once; these DO allocate / synchronise):
  *   pfst_peer_board_bytes  size of a board; also returns the inbox stride (floats) and the
@@ -498,33 +412,25 @@ int pfst_proto_finalize_peer(float* packed, int32_t C, int32_t D, const float* m
                              const uint64_t* boards, int32_t rank, int32_t nranks,
                              int64_t* status, int64_t timeout_ns, void* stream);
 
-/* loss = mean over valid pixels of ||feats[:,n] - mu[label_n]||_2 (masked_feat_dist
- * with f2 = mu[label]); valid = label in [0,C) and seen[label] (seen may be NULL).
+/* loss = mean over valid pixels of ||feats[:,n] - mu[label_n]||_2 (masked_feat_dist,
+ * pfgst.py:168-177, with f2 = mu[label]); valid = label in [0,C) and seen[label] (seen may
+ * be NULL). labels: (B,lab_h,lab_w) of label_dtype (PFST_DT_I64 or PFST_DT_U8, else
+ * PFST_ERR_UNSUPPORTED), nearest-resampled to (h,w).
  * dist: (B,h,w) per-pixel distances (0 where invalid), kept for the backward.
  * acc: device double[4] workspace (zeroed here; acc[1] = number of valid pixels).  */
 int pfst_proto_dist_fwd(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
-                        const int64_t* labels, int32_t lab_h, int32_t lab_w,
+                        const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w,
                         const float* mu, const uint8_t* seen, int32_t C, float* dist,
                         double* acc, float* loss, void* stream);
 
 /* grad_feats[b,d,n] (+)= grad_loss * (f - mu[label]) / (dist * n_valid), 0 where
- * invalid; accumulate != 0 adds into grad_feats (e.g. on top of pfst_neigh_grad).   */
+ * invalid; accumulate != 0 adds into grad_feats (e.g. on top of pfst_neigh_grad).
+ * labels and label_dtype as in pfst_proto_dist_fwd.                                 */
 int pfst_proto_dist_bwd(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
-                        const int64_t* labels, int32_t lab_h, int32_t lab_w,
+                        const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w,
                         const float* mu, const uint8_t* seen, int32_t C,
                         const float* dist, const double* acc, const float* grad_loss,
                         float* grad_feats, int32_t accumulate, void* stream);
-/* pfst_proto_dist_fwd / _bwd (masked_feat_dist, pfgst.py:168-177, with f2 = mu[label]) with labels of
- * label_dtype (PFST_DT_I64 or PFST_DT_U8, else PFST_ERR_UNSUPPORTED).                            */
-int pfst_proto_dist_fwd_lbl(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
-                            const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w,
-                            const float* mu, const uint8_t* seen, int32_t C, float* dist,
-                            double* acc, float* loss, void* stream);
-int pfst_proto_dist_bwd_lbl(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
-                            const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w,
-                            const float* mu, const uint8_t* seen, int32_t C,
-                            const float* dist, const double* acc, const float* grad_loss,
-                            float* grad_feats, int32_t accumulate, void* stream);
 
 /* out[b,c,n] = ||feats[b,:,n] - mu[c]||_2 for every class: (B,C,h,w).               */
 int pfst_proto_dist_all(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
@@ -539,18 +445,13 @@ int pfst_proto_dist_all(const float* feats, int64_t B, int32_t D, int32_t h, int
  *   out2[1] = top-1 accuracy in percent over the non-ignored pixels
  *   grad_logits (nullable, (B,C,lh,lw), zeroed here) = d out2[0] / d logits
  * in ONE pass: the up-sampled logits are never materialised. Integer up-sampling factors
- * only (H = s*lh, W = s*lw). stats: device double[4] workspace (zeroed here).             */
-int pfst_weighted_ce(const float* logits, const int64_t* labels, const float* weight,
-                     const float* class_weight, int64_t B, int32_t C, int32_t lh, int32_t lw,
-                     int32_t H, int32_t W, int64_t ignore_index, float loss_weight,
-                     float* grad_logits, double* stats, float* out2, void* stream);
-/* pfst_weighted_ce (decode_head.py:249-283, cross_entropy_loss.py:12-65) with labels of label_dtype
- * (PFST_DT_I64 or PFST_DT_U8, else PFST_ERR_UNSUPPORTED).                                         */
-int pfst_weighted_ce_lbl(const float* logits, const void* labels, int32_t label_dtype,
-                         const float* weight, const float* class_weight, int64_t B, int32_t C,
-                         int32_t lh, int32_t lw, int32_t H, int32_t W, int64_t ignore_index,
-                         float loss_weight, float* grad_logits, double* stats, float* out2,
-                         void* stream);
+ * only (H = s*lh, W = s*lw). stats: device double[4] workspace (zeroed here).
+ * labels: (B,H,W) of label_dtype (PFST_DT_I64 or PFST_DT_U8, else PFST_ERR_UNSUPPORTED).  */
+int pfst_weighted_ce(const float* logits, const void* labels, int32_t label_dtype,
+                     const float* weight, const float* class_weight, int64_t B, int32_t C,
+                     int32_t lh, int32_t lw, int32_t H, int32_t W, int64_t ignore_index,
+                     float loss_weight, float* grad_logits, double* stats, float* out2,
+                     void* stream);
 
 /* ---- next row (SURVEY.md §8f rank 4): offline class-wise thresholds -------------------
  * Replaces PseudoLabelingHookV4._cal_threshold

@@ -34,71 +34,45 @@ SIGNATURES: dict[str, tuple] = {
     "pfst_copy_async": (C.c_int, [_vp, _vp, _i64, _vp]),
     "pfst_classmix_draw": (C.c_int, [_vp, _i64, _vp, _i32, _i32, _vp, _vp, _vp]),   # host-only (no device work)
     "pfst_ema_coeffs": (C.c_int, [_i64, _f64, C.POINTER(_f32), C.POINTER(_f32)]),
-    "pfst_ema_update_multi": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i64, _i32, _f32, _f32, _i32, _vp]),
-    "pfst_ema_update_multi_ex": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i64, _i32, _f32, _f32, _i32, _i32, _vp]),
+    "pfst_ema_update_multi": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i64, _i32, _f32, _f32, _i32, _i32, _vp]),
     "pfst_ema_update_multi_dev": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i64, _i32, _vp, _i32, _vp]),
     "pfst_ema_update_flat": (C.c_int, [_vp, _vp, _i64, _f32, _f32, _i32, _vp]),
-    "pfst_pseudo_label": (C.c_int, [_vp, _i64, _i32, _i64, _f32, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp]),
-    "pfst_pseudo_label_lbl": (C.c_int, [_vp, _i64, _i32, _i64, _f32, _vp, _i32, _i64, _vp, _i32, _vp, _vp, _vp, _vp]),
-    "pfst_pseudo_label_ft": (C.c_int, [_vp, _i32, _i64, _i32, _i64, _f32, _vp, _i32, _i64, _vp, _i32, _vp, _vp, _vp,
-                                       _vp]),
+    "pfst_pseudo_label": (C.c_int, [_vp, _i32, _i64, _i32, _i64, _f32, _vp, _i32, _i64, _vp, _i32, _vp, _vp, _vp,
+                                    _vp]),
     "pfst_selftest_exp": (C.c_int, [_vp, _i64, _vp, _vp]),
     "pfst_pseudo_weight_fill": (C.c_int, [_vp, _i64, _i64, _i64, _vp, _i64, _i32, _i32, _vp]),
-    "pfst_class_presence": (C.c_int, [_vp, _i64, _vp, _vp]),
-    "pfst_class_presence_lbl": (C.c_int, [_vp, _i32, _i64, _vp, _vp]),
+    "pfst_class_presence": (C.c_int, [_vp, _i32, _i64, _vp, _vp]),
     "pfst_class_mix": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _i32, _i64, _i32,
-                                 _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
-    "pfst_class_mix_lbl": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _i32, _i64, _i32,
-                                     _i64, _i64, _vp, _vp, _vp, _vp, _i32, _vp]),
+                                 _i64, _i64, _vp, _vp, _vp, _vp, _i32, _vp]),
     "pfst_mask_mix": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i64, _i64, _vp]),
     "pfst_neigh_dots_splits": (_i32, [_i64, _i64, _i32, _i32, _i32]),
     "pfst_neigh_dots": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _i32, _vp, _vp]),
     "pfst_neigh_grad": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _i32, _vp, _vp]),
-    "pfst_neigh_dots_slot": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp]),
-    "pfst_neigh_dots_slot_ft": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp]),
-    "pfst_neigh_grad_proto": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _i32, _vp, _i32, _i32, _vp, _vp, _i32,
-                                        _vp, _vp, _vp, _vp, _vp]),
-    "pfst_neigh_grad_proto_lbl": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _vp,
-                                            _vp, _i32, _vp, _vp, _vp, _vp, _vp]),
-    "pfst_pfgst_loss_ws_bytes": (_i64, [_i64, _i32, _i32, _i32, _i32]),
+    "pfst_neigh_dots_slot": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _i32, _i32, _i32, _vp, _vp]),
+    "pfst_neigh_grad_proto": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _vp, _vp,
+                                        _i32, _vp, _vp, _vp, _vp, _vp]),
+    "pfst_pfgst_loss_ws_bytes": (_i64, [_i64, _i32, _i32, _i32, _i32, _i32]),
     "pfst_pfgst_loss_fwd": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _f32, _f32,
-                                      _vp, _vp, _i32, _i32, _i32, _i32, C.POINTER(_f32), _vp, _vp, _vp, _vp, _vp, _vp]),
+                                      _vp, _vp, _i32, _i32, _i32, _i32, C.POINTER(_f32), _vp, _vp, _vp, _vp, _vp,
+                                      _i32, _f32, _vp, C.POINTER(_f32), _i32, _vp]),
     "pfst_pfgst_loss_bwd": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _f32, _f32,
-                                      _vp, _vp, _i32, _i32, _i32, _i32, C.POINTER(_f32), _vp, _vp, _vp, _vp, _vp, _vp]),
-    "pfst_pfgst_loss_ws_bytes_ex": (_i64, [_i64, _i32, _i32, _i32, _i32, _i32]),
-    "pfst_pfgst_loss_fwd_ex": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _f32, _f32,
-                                         _vp, _vp, _i32, _i32, _i32, _i32, C.POINTER(_f32), _vp, _vp, _vp, _vp, _vp,
-                                         _i32, _f32, _vp, C.POINTER(_f32), _vp]),
-    "pfst_pfgst_loss_bwd_ex": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _f32, _f32,
-                                         _vp, _vp, _i32, _i32, _i32, _i32, C.POINTER(_f32), _vp, _vp, _vp, _vp, _vp,
-                                         _i32, _f32, _vp, C.POINTER(_f32), _vp]),
-    "pfst_pfgst_loss_fwd_lbl": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _f32, _f32,
-                                          _vp, _vp, _i32, _i32, _i32, _i32, C.POINTER(_f32), _vp, _vp, _vp, _vp, _vp,
-                                          _i32, _f32, _vp, C.POINTER(_f32), _i32, _vp]),
-    "pfst_pfgst_loss_bwd_lbl": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _f32, _f32,
-                                          _vp, _vp, _i32, _i32, _i32, _i32, C.POINTER(_f32), _vp, _vp, _vp, _vp, _vp,
-                                          _i32, _f32, _vp, C.POINTER(_f32), _i32, _vp]),
+                                      _vp, _vp, _i32, _i32, _i32, _i32, C.POINTER(_f32), _vp, _vp, _vp, _vp, _vp,
+                                      _i32, _f32, _vp, C.POINTER(_f32), _i32, _vp]),
     "pfst_slide_add": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _i32, _i32, _i32, _i32, _vp]),
     "pfst_slide_finalize": (C.c_int, [_vp, _vp, _vp, _i64, _i32, _i32, _i32, _i32, _i32, _vp, _vp]),
     "pfst_softmax_accum": (C.c_int, [_vp, _vp, _i64, _i32, _i64, _i32, _vp]),
     "pfst_div_argmax": (C.c_int, [_vp, _i64, _i32, _i64, _f32, _vp, _vp]),
     "pfst_class_quantile_ws_bytes": (_i64, [_i64, _i32, _i32]),
     "pfst_class_quantile": (C.c_int, [_vp, _i64, _i32, _i64, _vp, _i64, _vp, _i32, _vp, _vp, _vp]),
-    "pfst_weighted_ce": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i32, _i32, _i32, _i32, _i32, _i64, _f32, _vp, _vp, _vp, _vp]),
-    "pfst_weighted_ce_lbl": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _i64, _i32, _i32, _i32, _i32, _i32, _i64, _f32, _vp,
-                                       _vp, _vp, _vp]),
+    "pfst_weighted_ce": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _i64, _i32, _i32, _i32, _i32, _i32, _i64, _f32, _vp,
+                                   _vp, _vp, _vp]),
     "pfst_proto_accum_is_masked": (C.c_int, [_i32, _i32, _i32]),
-    "pfst_proto_accum": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _vp, _f32, _i32, _vp, _vp]),
-    "pfst_proto_accum_lbl": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _vp, _f32, _i32, _vp, _vp]),
-    "pfst_proto_accum_ft": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _vp, _f32, _i32, _vp,
-                                      _vp]),
+    "pfst_proto_accum": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _vp, _f32, _i32, _vp,
+                                   _vp]),
     "pfst_proto_order_ws_bytes": (_i64, [_i64, _i32, _i32, _i32]),
-    "pfst_proto_order": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _i32, _vp, _f32, _i32, _vp, _vp, _vp]),
-    "pfst_proto_order_lbl": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _i32, _vp, _f32, _i32, _vp, _vp, _vp]),
-    "pfst_proto_accum_ordered": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _i32, _vp, _vp, _vp]),
-    "pfst_proto_accum_ordered_ft": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _i32, _vp, _vp, _vp]),
-    "pfst_proto_finalize": (C.c_int, [_vp, _i32, _i32, _vp, _vp, _f32, _f32, _vp, _vp, _vp, _i32, _vp]),
-    "pfst_proto_finalize_dev": (C.c_int, [_vp, _i32, _i32, _vp, _vp, _f64, _vp, _vp, _vp, _vp, _i32, _vp]),
+    "pfst_proto_order": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _i32, _vp, _f32, _i32, _vp, _vp, _vp]),
+    "pfst_proto_accum_ordered": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _i32, _vp, _vp, _vp]),
+    "pfst_proto_finalize": (C.c_int, [_vp, _i32, _i32, _vp, _vp, _f64, _vp, _vp, _vp, _vp, _i32, _vp]),
     "pfst_feat_dist_fwd": (C.c_int, [_vp, _vp, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp, _vp]),
     "pfst_feat_dist_bwd": (C.c_int, [_vp, _vp, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "pfst_peer_board_bytes": (_i64, [_i32, _i32, _i32, C.POINTER(_i64), C.POINTER(_i64)]),
@@ -115,12 +89,10 @@ SIGNATURES: dict[str, tuple] = {
     "pfst_gather_scalars": (C.c_int, [_vp, _vp, _i32, C.c_uint32, _f32, _vp, _vp, _vp]),
     "pfst_gather_segments": (C.c_int, [_vp, _vp, _vp, _i32, _f32, _vp, _vp, _vp]),
     "pfst_pack_scalars": (C.c_int, [_vp, _vp, _i32, _vp, _vp]),
-    "pfst_proto_dist_fwd": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _vp, _vp, _i32, _vp, _vp, _vp, _vp]),
-    "pfst_proto_dist_bwd": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _i32, _vp]),
-    "pfst_proto_dist_fwd_lbl": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _vp, _vp, _i32, _vp, _vp,
-                                          _vp, _vp]),
-    "pfst_proto_dist_bwd_lbl": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _vp, _vp, _i32, _vp, _vp,
-                                          _vp, _vp, _i32, _vp]),
+    "pfst_proto_dist_fwd": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _vp, _vp, _i32, _vp, _vp,
+                                      _vp, _vp]),
+    "pfst_proto_dist_bwd": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _vp, _vp, _i32, _vp, _vp,
+                                      _vp, _vp, _i32, _vp]),
     "pfst_proto_dist_all": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _vp, _i32, _vp, _vp]),
     "pfst_confusion_accum": (C.c_int, [_vp, _i32, _vp, _i32, _i64, _i64, _i32, _i64, _i32, _vp, _vp,
                                        _i32, _vp]),

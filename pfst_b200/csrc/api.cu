@@ -17,7 +17,7 @@ void set_last_cuda_error(cudaError_t e, const char* where) {
 
 extern "C" {
 
-const char* pfst_version(void) { return "pfst_sm100 0.1.0 (sm_100a)"; }
+const char* pfst_version(void) { return "pfst_sm100 0.2.0 (sm_100a)"; }
 
 const char* pfst_error_string(int code) {
   switch (code) {

@@ -323,47 +323,25 @@ static int class_mix(const L* gt, const uint32_t* chosen, const float* img, cons
 
 extern "C" {
 
-int pfst_class_presence(const int64_t* gt, int64_t n, uint32_t* presence, void* stream) {
-  return pfst::class_presence(gt, n, presence, stream);
+int pfst_class_presence(const void* gt, int32_t label_dtype, int64_t n, uint32_t* presence, void* stream) {
+  return pfst::with_label_dt(label_dtype, [&](auto l) {
+    using L = decltype(l);
+    return pfst::class_presence(static_cast<const L*>(gt), n, presence, stream);
+  });
 }
 
-int pfst_class_presence_lbl(const void* gt, int32_t label_dtype, int64_t n, uint32_t* presence,
-                            void* stream) {
-  if (label_dtype == PFST_DT_I64)
-    return pfst::class_presence(static_cast<const int64_t*>(gt), n, presence, stream);
-  if (label_dtype == PFST_DT_U8)
-    return pfst::class_presence(static_cast<const uint8_t*>(gt), n, presence, stream);
-  return PFST_ERR_UNSUPPORTED;
-}
-
-int pfst_class_mix(const int64_t* gt, const uint32_t* chosen, const float* img,
-                   const float* trg_img, const int64_t* pseudo_label, const float* weight_in,
+int pfst_class_mix(const void* gt, const uint32_t* chosen, const float* img,
+                   const float* trg_img, const void* pseudo_label, const float* weight_in,
                    const unsigned long long* count, int64_t ps_size, int32_t ignore_top,
                    int32_t ignore_bottom, int64_t B, int32_t img_channels, int64_t H, int64_t W,
-                   float* mixed_img, int64_t* mixed_lbl, float* mixed_weight, int64_t* mix_mask,
-                   void* stream) {
-  return pfst::class_mix(gt, chosen, img, trg_img, pseudo_label, weight_in, count, ps_size, ignore_top,
-                         ignore_bottom, B, img_channels, H, W, mixed_img, mixed_lbl, mixed_weight, mix_mask,
-                         stream);
-}
-
-int pfst_class_mix_lbl(const void* gt, const uint32_t* chosen, const float* img,
-                       const float* trg_img, const void* pseudo_label, const float* weight_in,
-                       const unsigned long long* count, int64_t ps_size, int32_t ignore_top,
-                       int32_t ignore_bottom, int64_t B, int32_t img_channels, int64_t H, int64_t W,
-                       float* mixed_img, void* mixed_lbl, float* mixed_weight, void* mix_mask,
-                       int32_t label_dtype, void* stream) {
-  if (label_dtype == PFST_DT_I64)
-    return pfst::class_mix(static_cast<const int64_t*>(gt), chosen, img, trg_img,
-                           static_cast<const int64_t*>(pseudo_label), weight_in, count, ps_size, ignore_top,
-                           ignore_bottom, B, img_channels, H, W, mixed_img, static_cast<int64_t*>(mixed_lbl),
-                           mixed_weight, static_cast<int64_t*>(mix_mask), stream);
-  if (label_dtype == PFST_DT_U8)
-    return pfst::class_mix(static_cast<const uint8_t*>(gt), chosen, img, trg_img,
-                           static_cast<const uint8_t*>(pseudo_label), weight_in, count, ps_size, ignore_top,
-                           ignore_bottom, B, img_channels, H, W, mixed_img, static_cast<uint8_t*>(mixed_lbl),
-                           mixed_weight, static_cast<uint8_t*>(mix_mask), stream);
-  return PFST_ERR_UNSUPPORTED;
+                   float* mixed_img, void* mixed_lbl, float* mixed_weight, void* mix_mask,
+                   int32_t label_dtype, void* stream) {
+  return pfst::with_label_dt(label_dtype, [&](auto l) {
+    using L = decltype(l);
+    return pfst::class_mix(static_cast<const L*>(gt), chosen, img, trg_img, static_cast<const L*>(pseudo_label),
+                           weight_in, count, ps_size, ignore_top, ignore_bottom, B, img_channels, H, W, mixed_img,
+                           static_cast<L*>(mixed_lbl), mixed_weight, static_cast<L*>(mix_mask), stream);
+  });
 }
 
 }  // extern "C"

@@ -87,6 +87,24 @@ template <class T> __device__ __forceinline__ float4 unpack4(uint2 v) {
   return make_float4(lo_f32<T>(v.x), hi_f32<T>(v.x), lo_f32<T>(v.y), hi_f32<T>(v.y));
 }
 
+// ---- dtype-tag dispatch of the entry points (host) -------------------------
+// f(L{}) with L = int64_t or uint8_t for a PFST_DT_I64 / PFST_DT_U8 label tag; f(T{}) with T = float,
+// __half or __nv_bfloat16 for a PFST_DT_F32 / F16 / BF16 float tag. Any other tag is
+// PFST_ERR_UNSUPPORTED, returned before f runs (so before any argument check inside f).
+template <class F>
+static inline int with_label_dt(int32_t tag, F&& f) {
+  if (tag == PFST_DT_I64) return f(int64_t{});
+  if (tag == PFST_DT_U8) return f(uint8_t{});
+  return PFST_ERR_UNSUPPORTED;
+}
+template <class F>
+static inline int with_float_dt(int32_t tag, F&& f) {
+  if (tag == PFST_DT_F32) return f(float{});
+  if (tag == PFST_DT_F16) return f(__half{});
+  if (tag == PFST_DT_BF16) return f(__nv_bfloat16{});
+  return PFST_ERR_UNSUPPORTED;
+}
+
 // ---- streaming 128-bit global accesses ------------------------------------
 // Inputs that are read exactly once bypass L1 (ld.global.nc.L1::no_allocate);
 // outputs that are not re-read by the same kernel use plain vector stores.

@@ -112,15 +112,7 @@ int pfst_ema_coeffs(int64_t iter, double alpha, float* a32_host, float* b32_host
 int pfst_ema_update_multi(float* const* ema_ptrs, const float* const* param_ptrs,
                           const int64_t* numel, const int32_t* chunk_tensor,
                           const int64_t* chunk_begin, int64_t n_chunks, int32_t chunk_elems,
-                          float a32, float b32, int32_t mode, void* stream) {
-  return pfst_ema_update_multi_ex(ema_ptrs, param_ptrs, numel, chunk_tensor, chunk_begin, n_chunks, chunk_elems,
-                                  a32, b32, mode, 0, stream);
-}
-
-int pfst_ema_update_multi_ex(float* const* ema_ptrs, const float* const* param_ptrs,
-                             const int64_t* numel, const int32_t* chunk_tensor,
-                             const int64_t* chunk_begin, int64_t n_chunks, int32_t chunk_elems,
-                             float a32, float b32, int32_t mode, int32_t blocks_per_sm, void* stream) {
+                          float a32, float b32, int32_t mode, int32_t blocks_per_sm, void* stream) {
   if (n_chunks == 0) return PFST_OK;
   if (!ema_ptrs || !param_ptrs || !numel || !chunk_tensor || !chunk_begin || n_chunks < 0)
     return PFST_ERR_INVALID_ARG;

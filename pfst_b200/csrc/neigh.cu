@@ -826,31 +826,18 @@ int pfst_neigh_dots(const float* x_a, const float* x_b, int64_t B, int32_t D, in
   return pfst::neigh_dots_impl(x_a, x_b, B, D, h, w, dilation, 0, x_b ? 2 : 1, dots, static_cast<cudaStream_t>(stream));
 }
 
-int pfst_neigh_dots_slot(const float* x, int64_t B, int32_t D, int32_t h, int32_t w, int32_t dilation,
-                         int32_t slot, int32_t n_slots, float* dots, void* stream) {
-  if (!x || !dots || B < 0 || D < 1 || h < 1 || w < 1 || dilation < 1 || n_slots < 1 || slot < 0 || slot >= n_slots)
-    return PFST_ERR_INVALID_ARG;
-  if (B == 0) return PFST_OK;
-  if (B > 0x7fffffffll / 4) return PFST_ERR_UNSUPPORTED;
-  return pfst::neigh_dots_impl(x, (const float*)nullptr, B, D, h, w, dilation, slot, n_slots, dots,
-                         static_cast<cudaStream_t>(stream));
-}
-
-int pfst_neigh_dots_slot_ft(const void* x, int32_t x_dtype, int64_t B, int32_t D, int32_t h, int32_t w,
-                            int32_t dilation, int32_t slot, int32_t n_slots, float* dots, void* stream) {
-  if (x_dtype == PFST_DT_F32)
-    return pfst_neigh_dots_slot(static_cast<const float*>(x), B, D, h, w, dilation, slot, n_slots, dots, stream);
-  if (x_dtype != PFST_DT_F16 && x_dtype != PFST_DT_BF16) return PFST_ERR_UNSUPPORTED;
-  if (!x || !dots || B < 0 || D < 1 || h < 1 || w < 1 || dilation < 1 || n_slots < 1 || slot < 0 || slot >= n_slots)
-    return PFST_ERR_INVALID_ARG;
-  if (B == 0) return PFST_OK;
-  if (B > 0x7fffffffll / 4) return PFST_ERR_UNSUPPORTED;
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  if (x_dtype == PFST_DT_F16)
-    return pfst::neigh_dots_impl(static_cast<const __half*>(x), (const __half*)nullptr, B, D, h, w, dilation, slot,
-                           n_slots, dots, s);
-  return pfst::neigh_dots_impl(static_cast<const __nv_bfloat16*>(x), (const __nv_bfloat16*)nullptr, B, D, h, w, dilation,
-                         slot, n_slots, dots, s);
+int pfst_neigh_dots_slot(const void* x, int32_t x_dtype, int64_t B, int32_t D, int32_t h, int32_t w,
+                         int32_t dilation, int32_t slot, int32_t n_slots, float* dots, void* stream) {
+  return pfst::with_float_dt(x_dtype, [&](auto t) {
+    using T = decltype(t);
+    if (!x || !dots || B < 0 || D < 1 || h < 1 || w < 1 || dilation < 1 || n_slots < 1 || slot < 0 ||
+        slot >= n_slots)
+      return PFST_ERR_INVALID_ARG;
+    if (B == 0) return PFST_OK;
+    if (B > 0x7fffffffll / 4) return PFST_ERR_UNSUPPORTED;
+    return pfst::neigh_dots_impl(static_cast<const T*>(x), (const T*)nullptr, B, D, h, w, dilation, slot, n_slots,
+                                 dots, static_cast<cudaStream_t>(stream));
+  });
 }
 
 int pfst_neigh_grad(const float* x, const float* coef, int64_t B, int32_t D, int32_t h, int32_t w,
@@ -901,8 +888,8 @@ static int neigh_grad_proto(const float* x, const float* coef, int64_t B, int32_
   // shapes the fused kernels do not cover: two passes over grad_x
   const int rc = pfst_neigh_grad(x, coef, B, D, h, w, dilation, grad_x, stream);
   if (rc != PFST_OK) return rc;
-  return pfst_proto_dist_bwd_lbl(x, B, D, h, w, labels, LabelDt<L>::value, lab_h, lab_w, mu, seen, C, dist, acc,
-                                 grad_loss, grad_x, 1, stream);
+  return pfst_proto_dist_bwd(x, B, D, h, w, labels, LabelDt<L>::value, lab_h, lab_w, mu, seen, C, dist, acc,
+                             grad_loss, grad_x, 1, stream);
 }
 
 }  // namespace pfst
@@ -910,24 +897,13 @@ static int neigh_grad_proto(const float* x, const float* coef, int64_t B, int32_
 extern "C" {
 
 int pfst_neigh_grad_proto(const float* x, const float* coef, int64_t B, int32_t D, int32_t h, int32_t w,
-                          int32_t dilation, const int64_t* labels, int32_t lab_h, int32_t lab_w,
-                          const float* mu, const uint8_t* seen, int32_t C, const float* dist,
-                          const double* acc, const float* grad_loss, float* grad_x, void* stream) {
-  return pfst::neigh_grad_proto(x, coef, B, D, h, w, dilation, labels, lab_h, lab_w, mu, seen, C, dist, acc,
-                                grad_loss, grad_x, stream);
-}
-
-int pfst_neigh_grad_proto_lbl(const float* x, const float* coef, int64_t B, int32_t D, int32_t h, int32_t w,
-                              int32_t dilation, const void* labels, int32_t label_dtype, int32_t lab_h,
-                              int32_t lab_w, const float* mu, const uint8_t* seen, int32_t C, const float* dist,
-                              const double* acc, const float* grad_loss, float* grad_x, void* stream) {
-  if (label_dtype == PFST_DT_I64)
-    return pfst::neigh_grad_proto(x, coef, B, D, h, w, dilation, static_cast<const int64_t*>(labels), lab_h, lab_w,
-                                  mu, seen, C, dist, acc, grad_loss, grad_x, stream);
-  if (label_dtype == PFST_DT_U8)
-    return pfst::neigh_grad_proto(x, coef, B, D, h, w, dilation, static_cast<const uint8_t*>(labels), lab_h, lab_w,
-                                  mu, seen, C, dist, acc, grad_loss, grad_x, stream);
-  return PFST_ERR_UNSUPPORTED;
+                          int32_t dilation, const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w,
+                          const float* mu, const uint8_t* seen, int32_t C, const float* dist, const double* acc,
+                          const float* grad_loss, float* grad_x, void* stream) {
+  return pfst::with_label_dt(label_dtype, [&](auto l) {
+    return pfst::neigh_grad_proto(x, coef, B, D, h, w, dilation, static_cast<const decltype(l)*>(labels), lab_h,
+                                  lab_w, mu, seen, C, dist, acc, grad_loss, grad_x, stream);
+  });
 }
 
 }  // extern "C"

@@ -687,7 +687,7 @@ pfgst_loss_unfold_grad_kernel(const LossParams P, float* __restrict__ grad_logit
   }
 }
 
-// bits of the `options` argument of the *_ex entry points
+// bits of the `options` argument of pfst_pfgst_loss_ws_bytes / _fwd / _bwd
 constexpr int kOptGauss = 1, kOptProbEma = 2, kOptUnfoldGrad = 4, kOptMargin = 8, kOptMargin2 = 16;
 
 static int fill_params(LossParams& P, const float* dots, int ksplit, int64_t B, int fh, int fw, int up,
@@ -753,7 +753,7 @@ static int apply_options(LossParams& P, int options, float sigma, const float* l
 
 extern "C" {
 
-int64_t pfst_pfgst_loss_ws_bytes_ex(int64_t B, int32_t C, int32_t fh, int32_t fw, int32_t up, int32_t options) {
+int64_t pfst_pfgst_loss_ws_bytes(int64_t B, int32_t C, int32_t fh, int32_t fw, int32_t up, int32_t options) {
   if (B < 0 || C < 1 || fh < 1 || fw < 1 || up < 1) return 0;
   const size_t gplane = (size_t)fh * fw * up * up;
   size_t extra = 0;
@@ -763,83 +763,56 @@ int64_t pfst_pfgst_loss_ws_bytes_ex(int64_t B, int32_t C, int32_t fh, int32_t fw
                    16 * sizeof(long long) + 16 + extra);
 }
 
-int64_t pfst_pfgst_loss_ws_bytes(int64_t B, int32_t C, int32_t fh, int32_t fw, int32_t up) {
-  return pfst_pfgst_loss_ws_bytes_ex(B, C, fh, fw, up, 0);
-}
-
-int pfst_pfgst_loss_fwd_lbl(const float* dots, int32_t ksplit, int64_t B, int32_t fh, int32_t fw, int32_t up,
-                            const float* logits, int32_t C, int32_t lh, int32_t lw, float lscale_h,
-                            float lscale_w, const void* gt, const void* mix, int32_t gt_h, int32_t gt_w,
-                            int32_t dilation, int32_t top_k, const float* weights6_host, void* workspace,
-                            double* stats, float* losses, float* density, uint8_t* eroded, int32_t options,
-                            float sigma, const float* logits_ema, const float* margin_host, int32_t label_dtype,
-                            void* stream) {
-  if (label_dtype != PFST_DT_I64 && label_dtype != PFST_DT_U8) return PFST_ERR_UNSUPPORTED;
-  pfst::LossParams P;
-  int rc = pfst::fill_params(P, dots, ksplit, B, fh, fw, up, logits, C, lh, lw, lscale_h, lscale_w, gt,
-                             mix, gt_h, gt_w, dilation, top_k, weights6_host, workspace);
-  if (rc != PFST_OK) return rc;
-  rc = pfst::apply_options(P, options, sigma, logits_ema, margin_host);
-  if (rc != PFST_OK) return rc;
-  if (!stats || !losses) return PFST_ERR_INVALID_ARG;
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  // (the prep kernel zeroes the integer accumulators: no memset node between the kernels)
-  const int64_t total = (int64_t)P.B * P.gh * P.gw;
-  if (total == 0) return PFST_OK;
-  {
-    const int64_t n_a = (int64_t)2 * P.B * 5 * fh * fw;
-    const int64_t blocks_a = (n_a + pfst::kPrepThreads - 1) / pfst::kPrepThreads;
-    const int64_t blocks_b = (total + pfst::kPrepThreads - 1) / pfst::kPrepThreads;
-    if (blocks_a + blocks_b > 0x7fffffffll) return PFST_ERR_UNSUPPORTED;
-    void (*prep)(const pfst::LossParams, int);
-    if (label_dtype == PFST_DT_U8)
-      prep = C <= 8 ? pfst::pfgst_loss_prep_kernel<8, uint8_t>
-                    : (C <= 40 ? pfst::pfgst_loss_prep_kernel<40, uint8_t> : pfst::pfgst_loss_prep_kernel<pfst::kMaxC, uint8_t>);
-    else
-      prep = C <= 8 ? pfst::pfgst_loss_prep_kernel<8, int64_t>
-                    : (C <= 40 ? pfst::pfgst_loss_prep_kernel<40, int64_t> : pfst::pfgst_loss_prep_kernel<pfst::kMaxC, int64_t>);
-    prep<<<(unsigned)(blocks_a + blocks_b), pfst::kPrepThreads, 0, s>>>(P, (int)blocks_a);
-    PFST_CHECK_LAUNCH("pfst_pfgst_loss_fwd/prep");
-  }
-  if (P.gh > 65535 || P.B > 65535) return PFST_ERR_UNSUPPORTED;
-  const dim3 grid((unsigned)((P.gw + pfst::kLpPix - 1) / pfst::kLpPix), (unsigned)P.gh, (unsigned)P.B);
-  pfst::pfgst_loss_fwd_kernel<<<grid, pfst::kLpThreads, 0, s>>>(
-      P, stats, losses, density, eroded);
-  PFST_CHECK_LAUNCH("pfst_pfgst_loss_fwd");
-  return PFST_OK;
-}
-
-int pfst_pfgst_loss_fwd_ex(const float* dots, int32_t ksplit, int64_t B, int32_t fh, int32_t fw, int32_t up,
-                           const float* logits, int32_t C, int32_t lh, int32_t lw, float lscale_h,
-                           float lscale_w, const int64_t* gt, const int64_t* mix, int32_t gt_h, int32_t gt_w,
-                           int32_t dilation, int32_t top_k, const float* weights6_host, void* workspace,
-                           double* stats, float* losses, float* density, uint8_t* eroded, int32_t options,
-                           float sigma, const float* logits_ema, const float* margin_host, void* stream) {
-  return pfst_pfgst_loss_fwd_lbl(dots, ksplit, B, fh, fw, up, logits, C, lh, lw, lscale_h, lscale_w, gt, mix, gt_h,
-                                 gt_w, dilation, top_k, weights6_host, workspace, stats, losses, density, eroded,
-                                 options, sigma, logits_ema, margin_host, PFST_DT_I64, stream);
-}
-
 int pfst_pfgst_loss_fwd(const float* dots, int32_t ksplit, int64_t B, int32_t fh, int32_t fw, int32_t up,
                         const float* logits, int32_t C, int32_t lh, int32_t lw, float lscale_h,
-                        float lscale_w, const int64_t* gt, const int64_t* mix, int32_t gt_h, int32_t gt_w,
+                        float lscale_w, const void* gt, const void* mix, int32_t gt_h, int32_t gt_w,
                         int32_t dilation, int32_t top_k, const float* weights6_host, void* workspace,
-                        double* stats, float* losses, float* density, uint8_t* eroded, void* stream) {
-  return pfst_pfgst_loss_fwd_ex(dots, ksplit, B, fh, fw, up, logits, C, lh, lw, lscale_h, lscale_w, gt, mix, gt_h,
-                                gt_w, dilation, top_k, weights6_host, workspace, stats, losses, density, eroded, 0,
-                                0.f, nullptr, nullptr, stream);
+                        double* stats, float* losses, float* density, uint8_t* eroded, int32_t options,
+                        float sigma, const float* logits_ema, const float* margin_host, int32_t label_dtype,
+                        void* stream) {
+  return pfst::with_label_dt(label_dtype, [&](auto l) {
+    using L = decltype(l);
+    pfst::LossParams P;
+    int rc = pfst::fill_params(P, dots, ksplit, B, fh, fw, up, logits, C, lh, lw, lscale_h, lscale_w, gt,
+                               mix, gt_h, gt_w, dilation, top_k, weights6_host, workspace);
+    if (rc != PFST_OK) return rc;
+    rc = pfst::apply_options(P, options, sigma, logits_ema, margin_host);
+    if (rc != PFST_OK) return rc;
+    if (!stats || !losses) return PFST_ERR_INVALID_ARG;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    // (the prep kernel zeroes the integer accumulators: no memset node between the kernels)
+    const int64_t total = (int64_t)P.B * P.gh * P.gw;
+    if (total == 0) return PFST_OK;
+    {
+      const int64_t n_a = (int64_t)2 * P.B * 5 * fh * fw;
+      const int64_t blocks_a = (n_a + pfst::kPrepThreads - 1) / pfst::kPrepThreads;
+      const int64_t blocks_b = (total + pfst::kPrepThreads - 1) / pfst::kPrepThreads;
+      if (blocks_a + blocks_b > 0x7fffffffll) return PFST_ERR_UNSUPPORTED;
+      auto prep = C <= 8 ? pfst::pfgst_loss_prep_kernel<8, L>
+                         : (C <= 40 ? pfst::pfgst_loss_prep_kernel<40, L> : pfst::pfgst_loss_prep_kernel<pfst::kMaxC, L>);
+      prep<<<(unsigned)(blocks_a + blocks_b), pfst::kPrepThreads, 0, s>>>(P, (int)blocks_a);
+      PFST_CHECK_LAUNCH("pfst_pfgst_loss_fwd/prep");
+    }
+    if (P.gh > 65535 || P.B > 65535) return PFST_ERR_UNSUPPORTED;
+    const dim3 grid((unsigned)((P.gw + pfst::kLpPix - 1) / pfst::kLpPix), (unsigned)P.gh, (unsigned)P.B);
+    pfst::pfgst_loss_fwd_kernel<<<grid, pfst::kLpThreads, 0, s>>>(
+        P, stats, losses, density, eroded);
+    PFST_CHECK_LAUNCH("pfst_pfgst_loss_fwd");
+    return PFST_OK;
+  });
 }
 
 // The backward reads the per-pixel label classes the forward's prep kernel left in the workspace, never gt
 // or mix themselves: the label dtype is only validated here.
-int pfst_pfgst_loss_bwd_lbl(const float* dots, int32_t ksplit, int64_t B, int32_t fh, int32_t fw, int32_t up,
-                            const float* logits, int32_t C, int32_t lh, int32_t lw, float lscale_h,
-                            float lscale_w, const void* gt, const void* mix, int32_t gt_h, int32_t gt_w,
-                            int32_t dilation, int32_t top_k, const float* weights6_host, const void* workspace,
-                            const double* stats, const float* grad_losses, float* coef, float* grad_logits,
-                            int32_t options, float sigma, const float* logits_ema, const float* margin_host,
-                            int32_t label_dtype, void* stream) {
-  if (label_dtype != PFST_DT_I64 && label_dtype != PFST_DT_U8) return PFST_ERR_UNSUPPORTED;
+int pfst_pfgst_loss_bwd(const float* dots, int32_t ksplit, int64_t B, int32_t fh, int32_t fw, int32_t up,
+                        const float* logits, int32_t C, int32_t lh, int32_t lw, float lscale_h,
+                        float lscale_w, const void* gt, const void* mix, int32_t gt_h, int32_t gt_w,
+                        int32_t dilation, int32_t top_k, const float* weights6_host, const void* workspace,
+                        const double* stats, const float* grad_losses, float* coef, float* grad_logits,
+                        int32_t options, float sigma, const float* logits_ema, const float* margin_host,
+                        int32_t label_dtype, void* stream) {
+  const int tag_rc = pfst::with_label_dt(label_dtype, [](auto) { return PFST_OK; });
+  if (tag_rc != PFST_OK) return tag_rc;
   pfst::LossParams P;
   int rc = pfst::fill_params(P, dots, ksplit, B, fh, fw, up, logits, C, lh, lw, lscale_h, lscale_w, gt,
                              mix, gt_h, gt_w, dilation, top_k, weights6_host, const_cast<void*>(workspace));
@@ -880,29 +853,6 @@ int pfst_pfgst_loss_bwd_lbl(const float* dots, int32_t ksplit, int64_t B, int32_
     PFST_CHECK_LAUNCH("pfst_pfgst_loss_bwd/unfold_grad");
   }
   return PFST_OK;
-}
-
-int pfst_pfgst_loss_bwd_ex(const float* dots, int32_t ksplit, int64_t B, int32_t fh, int32_t fw, int32_t up,
-                           const float* logits, int32_t C, int32_t lh, int32_t lw, float lscale_h,
-                           float lscale_w, const int64_t* gt, const int64_t* mix, int32_t gt_h, int32_t gt_w,
-                           int32_t dilation, int32_t top_k, const float* weights6_host, const void* workspace,
-                           const double* stats, const float* grad_losses, float* coef, float* grad_logits,
-                           int32_t options, float sigma, const float* logits_ema, const float* margin_host,
-                           void* stream) {
-  return pfst_pfgst_loss_bwd_lbl(dots, ksplit, B, fh, fw, up, logits, C, lh, lw, lscale_h, lscale_w, gt, mix, gt_h,
-                                 gt_w, dilation, top_k, weights6_host, workspace, stats, grad_losses, coef,
-                                 grad_logits, options, sigma, logits_ema, margin_host, PFST_DT_I64, stream);
-}
-
-int pfst_pfgst_loss_bwd(const float* dots, int32_t ksplit, int64_t B, int32_t fh, int32_t fw, int32_t up,
-                        const float* logits, int32_t C, int32_t lh, int32_t lw, float lscale_h,
-                        float lscale_w, const int64_t* gt, const int64_t* mix, int32_t gt_h, int32_t gt_w,
-                        int32_t dilation, int32_t top_k, const float* weights6_host, const void* workspace,
-                        const double* stats, const float* grad_losses, float* coef, float* grad_logits,
-                        void* stream) {
-  return pfst_pfgst_loss_bwd_ex(dots, ksplit, B, fh, fw, up, logits, C, lh, lw, lscale_h, lscale_w, gt, mix, gt_h,
-                                gt_w, dilation, top_k, weights6_host, workspace, stats, grad_losses, coef,
-                                grad_logits, 0, 0.f, nullptr, nullptr, stream);
 }
 
 }  // extern "C"

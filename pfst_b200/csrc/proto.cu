@@ -909,7 +909,7 @@ int pfst_proto_accum_is_masked(int32_t C, int32_t h, int32_t w) {
 
 namespace {
 
-template <class L, class T = float>
+template <class L, class T>
 int proto_accum(const T* feats, int64_t B, int32_t D, int32_t h, int32_t w, const L* labels, int32_t lab_h,
                 int32_t lab_w, const float* conf, float conf_thr, int32_t C, float* packed, void* stream) {
   if (sizeof(L) == 1 && (int64_t)lab_h * lab_w > 0x7fffffffll) return PFST_ERR_UNSUPPORTED;   // 32-bit gathers
@@ -958,62 +958,15 @@ int proto_accum(const T* feats, int64_t B, int32_t D, int32_t h, int32_t w, cons
 
 extern "C" {
 
-int pfst_proto_accum(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
-                     const int64_t* labels, int32_t lab_h, int32_t lab_w, const float* conf,
+int pfst_proto_accum(const void* feats, int32_t feat_dtype, int64_t B, int32_t D, int32_t h, int32_t w,
+                     const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w, const float* conf,
                      float conf_thr, int32_t C, float* packed, void* stream) {
-  return proto_accum(feats, B, D, h, w, labels, lab_h, lab_w, conf, conf_thr, C, packed, stream);
-}
-
-int pfst_proto_accum_lbl(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
-                         const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w,
-                         const float* conf, float conf_thr, int32_t C, float* packed, void* stream) {
-  if (label_dtype == PFST_DT_I64)
-    return proto_accum(feats, B, D, h, w, static_cast<const int64_t*>(labels), lab_h, lab_w, conf, conf_thr, C,
-                       packed, stream);
-  if (label_dtype == PFST_DT_U8)
-    return proto_accum(feats, B, D, h, w, static_cast<const uint8_t*>(labels), lab_h, lab_w, conf, conf_thr, C,
-                       packed, stream);
-  return PFST_ERR_UNSUPPORTED;
-}
-
-}  // extern "C"
-
-namespace {
-
-template <class T>
-int proto_accum_ft(const void* feats, int64_t B, int32_t D, int32_t h, int32_t w, const void* labels,
-                   int32_t label_dtype, int32_t lab_h, int32_t lab_w, const float* conf, float conf_thr, int32_t C,
-                   float* packed, void* stream) {
-  const T* f = static_cast<const T*>(feats);
-  if (label_dtype == PFST_DT_I64)
-    return proto_accum(f, B, D, h, w, static_cast<const int64_t*>(labels), lab_h, lab_w, conf, conf_thr, C, packed,
-                       stream);
-  if (label_dtype == PFST_DT_U8)
-    return proto_accum(f, B, D, h, w, static_cast<const uint8_t*>(labels), lab_h, lab_w, conf, conf_thr, C, packed,
-                       stream);
-  return PFST_ERR_UNSUPPORTED;
-}
-
-}  // namespace
-
-extern "C" {
-
-int pfst_proto_accum_ft(const void* feats, int32_t feat_dtype, int64_t B, int32_t D, int32_t h, int32_t w,
-                        const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w,
-                        const float* conf, float conf_thr, int32_t C, float* packed, void* stream) {
-  switch (feat_dtype) {
-    case PFST_DT_F32:
-      return proto_accum_ft<float>(feats, B, D, h, w, labels, label_dtype, lab_h, lab_w, conf, conf_thr, C, packed,
-                                   stream);
-    case PFST_DT_F16:
-      return proto_accum_ft<__half>(feats, B, D, h, w, labels, label_dtype, lab_h, lab_w, conf, conf_thr, C, packed,
-                                    stream);
-    case PFST_DT_BF16:
-      return proto_accum_ft<__nv_bfloat16>(feats, B, D, h, w, labels, label_dtype, lab_h, lab_w, conf, conf_thr, C,
-                                           packed, stream);
-    default:
-      return PFST_ERR_UNSUPPORTED;
-  }
+  return pfst::with_float_dt(feat_dtype, [&](auto t) {
+    return pfst::with_label_dt(label_dtype, [&](auto l) {
+      return proto_accum(static_cast<const decltype(t)*>(feats), B, D, h, w, static_cast<const decltype(l)*>(labels),
+                         lab_h, lab_w, conf, conf_thr, C, packed, stream);
+    });
+  });
 }
 
 int64_t pfst_proto_order_ws_bytes(int64_t B, int32_t h, int32_t w, int32_t C) {
@@ -1046,22 +999,13 @@ int proto_order(const L* labels, int64_t B, int32_t h, int32_t w, int32_t lab_h,
 
 extern "C" {
 
-int pfst_proto_order(const int64_t* labels, int64_t B, int32_t h, int32_t w, int32_t lab_h, int32_t lab_w,
-                     const float* conf, float conf_thr, int32_t C, float* counts, void* workspace,
+int pfst_proto_order(const void* labels, int32_t label_dtype, int64_t B, int32_t h, int32_t w, int32_t lab_h,
+                     int32_t lab_w, const float* conf, float conf_thr, int32_t C, float* counts, void* workspace,
                      void* stream) {
-  return proto_order(labels, B, h, w, lab_h, lab_w, conf, conf_thr, C, counts, workspace, stream);
-}
-
-int pfst_proto_order_lbl(const void* labels, int32_t label_dtype, int64_t B, int32_t h, int32_t w, int32_t lab_h,
-                         int32_t lab_w, const float* conf, float conf_thr, int32_t C, float* counts,
-                         void* workspace, void* stream) {
-  if (label_dtype == PFST_DT_I64)
-    return proto_order(static_cast<const int64_t*>(labels), B, h, w, lab_h, lab_w, conf, conf_thr, C, counts,
+  return pfst::with_label_dt(label_dtype, [&](auto l) {
+    return proto_order(static_cast<const decltype(l)*>(labels), B, h, w, lab_h, lab_w, conf, conf_thr, C, counts,
                        workspace, stream);
-  if (label_dtype == PFST_DT_U8)
-    return proto_order(static_cast<const uint8_t*>(labels), B, h, w, lab_h, lab_w, conf, conf_thr, C, counts,
-                       workspace, stream);
-  return PFST_ERR_UNSUPPORTED;
+  });
 }
 
 }  // extern "C"
@@ -1101,43 +1045,21 @@ int proto_accum_ordered(const T* feats, int64_t B, int32_t D, int32_t h, int32_t
 
 extern "C" {
 
-int pfst_proto_accum_ordered(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w, int32_t C,
-                             const void* workspace, float* packed, void* stream) {
-  return proto_accum_ordered(feats, B, D, h, w, C, workspace, packed, stream);
-}
-
-int pfst_proto_accum_ordered_ft(const void* feats, int32_t feat_dtype, int64_t B, int32_t D, int32_t h, int32_t w,
-                                int32_t C, const void* workspace, float* packed, void* stream) {
-  switch (feat_dtype) {
-    case PFST_DT_F32:
-      return proto_accum_ordered(static_cast<const float*>(feats), B, D, h, w, C, workspace, packed, stream);
-    case PFST_DT_F16:
-      return proto_accum_ordered(static_cast<const __half*>(feats), B, D, h, w, C, workspace, packed, stream);
-    case PFST_DT_BF16:
-      return proto_accum_ordered(static_cast<const __nv_bfloat16*>(feats), B, D, h, w, C, workspace, packed, stream);
-    default:
-      return PFST_ERR_UNSUPPORTED;
-  }
+int pfst_proto_accum_ordered(const void* feats, int32_t feat_dtype, int64_t B, int32_t D, int32_t h, int32_t w,
+                             int32_t C, const void* workspace, float* packed, void* stream) {
+  return pfst::with_float_dt(feat_dtype, [&](auto t) {
+    return proto_accum_ordered(static_cast<const decltype(t)*>(feats), B, D, h, w, C, workspace, packed, stream);
+  });
 }
 
 int pfst_proto_finalize(float* packed, int32_t C, int32_t D, const float* mu_prev,
-                        const uint8_t* seen_prev, float a32, float b32, float* mu_out, int64_t* cnt_out,
-                        uint8_t* seen_out, int32_t reset_packed, void* stream) {
-  if (!packed || !mu_out || C < 1 || D < 1) return PFST_ERR_INVALID_ARG;
-  pfst::proto_finalize_kernel<<<(unsigned)C, 128, 0, static_cast<cudaStream_t>(stream)>>>(
-      packed, C, D, mu_prev, seen_prev, a32, b32, 0.0, nullptr, mu_out, cnt_out, seen_out, reset_packed);
-  PFST_CHECK_LAUNCH("pfst_proto_finalize");
-  return PFST_OK;
-}
-
-int pfst_proto_finalize_dev(float* packed, int32_t C, int32_t D, const float* mu_prev,
-                            const uint8_t* seen_prev, double alpha, int64_t* iter_state, float* mu_out,
-                            int64_t* cnt_out, uint8_t* seen_out, int32_t reset_packed, void* stream) {
+                        const uint8_t* seen_prev, double alpha, int64_t* iter_state, float* mu_out,
+                        int64_t* cnt_out, uint8_t* seen_out, int32_t reset_packed, void* stream) {
   if (!packed || !mu_out || !iter_state || C < 1 || D < 1) return PFST_ERR_INVALID_ARG;
   pfst::proto_finalize_kernel<<<(unsigned)C, 128, 0, static_cast<cudaStream_t>(stream)>>>(
       packed, C, D, mu_prev, seen_prev, 0.f, 1.f, alpha, reinterpret_cast<long long*>(iter_state), mu_out, cnt_out,
       seen_out, reset_packed);
-  PFST_CHECK_LAUNCH("pfst_proto_finalize_dev");
+  PFST_CHECK_LAUNCH("pfst_proto_finalize");
   return PFST_OK;
 }
 
@@ -1186,46 +1108,24 @@ static int proto_dist_common(bool bwd, const float* feats, int64_t B, int32_t D,
 
 extern "C" {
 
-int pfst_proto_dist_fwd(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
-                        const int64_t* labels, int32_t lab_h, int32_t lab_w, const float* mu,
-                        const uint8_t* seen, int32_t C, float* dist, double* acc, float* loss, void* stream) {
-  return proto_dist_common(false, feats, B, D, h, w, labels, lab_h, lab_w, mu, seen, C, dist, acc, loss, nullptr,
-                           nullptr, 0, static_cast<cudaStream_t>(stream));
+int pfst_proto_dist_fwd(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w, const void* labels,
+                        int32_t label_dtype, int32_t lab_h, int32_t lab_w, const float* mu, const uint8_t* seen,
+                        int32_t C, float* dist, double* acc, float* loss, void* stream) {
+  return pfst::with_label_dt(label_dtype, [&](auto l) {
+    return proto_dist_common(false, feats, B, D, h, w, static_cast<const decltype(l)*>(labels), lab_h, lab_w, mu,
+                             seen, C, dist, acc, loss, nullptr, nullptr, 0, static_cast<cudaStream_t>(stream));
+  });
 }
 
-int pfst_proto_dist_bwd(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
-                        const int64_t* labels, int32_t lab_h, int32_t lab_w, const float* mu,
-                        const uint8_t* seen, int32_t C, const float* dist, const double* acc,
-                        const float* grad_loss, float* grad_feats, int32_t accumulate, void* stream) {
-  return proto_dist_common(true, feats, B, D, h, w, labels, lab_h, lab_w, mu, seen, C, const_cast<float*>(dist),
-                           const_cast<double*>(acc), nullptr, grad_loss, grad_feats, accumulate,
-                           static_cast<cudaStream_t>(stream));
-}
-
-int pfst_proto_dist_fwd_lbl(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
-                            const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w, const float* mu,
-                            const uint8_t* seen, int32_t C, float* dist, double* acc, float* loss, void* stream) {
-  if (label_dtype == PFST_DT_I64)
-    return pfst_proto_dist_fwd(feats, B, D, h, w, static_cast<const int64_t*>(labels), lab_h, lab_w, mu, seen, C,
-                               dist, acc, loss, stream);
-  if (label_dtype == PFST_DT_U8)
-    return proto_dist_common(false, feats, B, D, h, w, static_cast<const uint8_t*>(labels), lab_h, lab_w, mu, seen,
-                             C, dist, acc, loss, nullptr, nullptr, 0, static_cast<cudaStream_t>(stream));
-  return PFST_ERR_UNSUPPORTED;
-}
-
-int pfst_proto_dist_bwd_lbl(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w,
-                            const void* labels, int32_t label_dtype, int32_t lab_h, int32_t lab_w, const float* mu,
-                            const uint8_t* seen, int32_t C, const float* dist, const double* acc,
-                            const float* grad_loss, float* grad_feats, int32_t accumulate, void* stream) {
-  if (label_dtype == PFST_DT_I64)
-    return pfst_proto_dist_bwd(feats, B, D, h, w, static_cast<const int64_t*>(labels), lab_h, lab_w, mu, seen, C,
-                               dist, acc, grad_loss, grad_feats, accumulate, stream);
-  if (label_dtype == PFST_DT_U8)
-    return proto_dist_common(true, feats, B, D, h, w, static_cast<const uint8_t*>(labels), lab_h, lab_w, mu, seen,
-                             C, const_cast<float*>(dist), const_cast<double*>(acc), nullptr, grad_loss, grad_feats,
-                             accumulate, static_cast<cudaStream_t>(stream));
-  return PFST_ERR_UNSUPPORTED;
+int pfst_proto_dist_bwd(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w, const void* labels,
+                        int32_t label_dtype, int32_t lab_h, int32_t lab_w, const float* mu, const uint8_t* seen,
+                        int32_t C, const float* dist, const double* acc, const float* grad_loss, float* grad_feats,
+                        int32_t accumulate, void* stream) {
+  return pfst::with_label_dt(label_dtype, [&](auto l) {
+    return proto_dist_common(true, feats, B, D, h, w, static_cast<const decltype(l)*>(labels), lab_h, lab_w, mu,
+                             seen, C, const_cast<float*>(dist), const_cast<double*>(acc), nullptr, grad_loss,
+                             grad_feats, accumulate, static_cast<cudaStream_t>(stream));
+  });
 }
 
 int pfst_proto_dist_all(const float* feats, int64_t B, int32_t D, int32_t h, int32_t w, const float* mu,

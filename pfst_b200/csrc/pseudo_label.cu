@@ -358,15 +358,7 @@ static int launch_pl(const T* logits, int64_t B, int C, int64_t HW, float thr,
   return PFST_OK;
 }
 
-}  // namespace pfst
-
-extern "C" {
-
-}  // extern "C"
-
-namespace pfst {
-
-template <class L, class T = float>
+template <class L, class T>
 static int pseudo_label(const T* logits, int64_t B, int32_t C, int64_t HW, float thr,
                         const float* thr_per_class, int32_t mode, int64_t reject_label, L* label,
                         float* conf, float* weight_part, unsigned long long* count, void* stream) {
@@ -388,67 +380,16 @@ static int pseudo_label(const T* logits, int64_t B, int32_t C, int64_t HW, float
 
 extern "C" {
 
-int pfst_pseudo_label(const float* logits, int64_t B, int32_t C, int64_t HW, float thr,
-                      const float* thr_per_class, int32_t mode, int64_t reject_label,
-                      int64_t* label, float* conf, float* weight_part,
-                      unsigned long long* count, void* stream) {
-  return pfst::pseudo_label(logits, B, C, HW, thr, thr_per_class, mode, reject_label, label, conf,
-                            weight_part, count, stream);
-}
-
-int pfst_pseudo_label_lbl(const float* logits, int64_t B, int32_t C, int64_t HW, float thr,
-                          const float* thr_per_class, int32_t mode, int64_t reject_label,
-                          void* label, int32_t label_dtype, float* conf, float* weight_part,
-                          unsigned long long* count, void* stream) {
-  if (label_dtype == PFST_DT_I64)
-    return pfst::pseudo_label(logits, B, C, HW, thr, thr_per_class, mode, reject_label,
-                              static_cast<int64_t*>(label), conf, weight_part, count, stream);
-  if (label_dtype == PFST_DT_U8)
-    return pfst::pseudo_label(logits, B, C, HW, thr, thr_per_class, mode, reject_label,
-                              static_cast<uint8_t*>(label), conf, weight_part, count, stream);
-  return PFST_ERR_UNSUPPORTED;
-}
-
-}  // extern "C"
-
-namespace pfst {
-
-template <class T>
-static int pseudo_label_ft(const void* logits, int64_t B, int32_t C, int64_t HW, float thr,
-                           const float* thr_per_class, int32_t mode, int64_t reject_label, void* label,
-                           int32_t label_dtype, float* conf, float* weight_part, unsigned long long* count,
-                           void* stream) {
-  const T* x = static_cast<const T*>(logits);
-  if (label_dtype == PFST_DT_I64)
-    return pseudo_label(x, B, C, HW, thr, thr_per_class, mode, reject_label, static_cast<int64_t*>(label), conf,
-                        weight_part, count, stream);
-  if (label_dtype == PFST_DT_U8)
-    return pseudo_label(x, B, C, HW, thr, thr_per_class, mode, reject_label, static_cast<uint8_t*>(label), conf,
-                        weight_part, count, stream);
-  return PFST_ERR_UNSUPPORTED;
-}
-
-}  // namespace pfst
-
-extern "C" {
-
-int pfst_pseudo_label_ft(const void* logits, int32_t logit_dtype, int64_t B, int32_t C, int64_t HW, float thr,
-                         const float* thr_per_class, int32_t mode, int64_t reject_label, void* label,
-                         int32_t label_dtype, float* conf, float* weight_part, unsigned long long* count,
-                         void* stream) {
-  switch (logit_dtype) {
-    case PFST_DT_F32:
-      return pfst::pseudo_label_ft<float>(logits, B, C, HW, thr, thr_per_class, mode, reject_label, label,
-                                          label_dtype, conf, weight_part, count, stream);
-    case PFST_DT_F16:
-      return pfst::pseudo_label_ft<__half>(logits, B, C, HW, thr, thr_per_class, mode, reject_label, label,
-                                           label_dtype, conf, weight_part, count, stream);
-    case PFST_DT_BF16:
-      return pfst::pseudo_label_ft<__nv_bfloat16>(logits, B, C, HW, thr, thr_per_class, mode, reject_label, label,
-                                                  label_dtype, conf, weight_part, count, stream);
-    default:
-      return PFST_ERR_UNSUPPORTED;
-  }
+int pfst_pseudo_label(const void* logits, int32_t logit_dtype, int64_t B, int32_t C, int64_t HW, float thr,
+                      const float* thr_per_class, int32_t mode, int64_t reject_label, void* label,
+                      int32_t label_dtype, float* conf, float* weight_part, unsigned long long* count,
+                      void* stream) {
+  return pfst::with_float_dt(logit_dtype, [&](auto t) {
+    return pfst::with_label_dt(label_dtype, [&](auto l) {
+      return pfst::pseudo_label(static_cast<const decltype(t)*>(logits), B, C, HW, thr, thr_per_class, mode,
+                                reject_label, static_cast<decltype(l)*>(label), conf, weight_part, count, stream);
+    });
+  });
 }
 
 int pfst_selftest_exp(const float* x, int64_t n, unsigned long long* mismatches, void* stream) {

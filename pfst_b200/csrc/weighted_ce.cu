@@ -579,24 +579,14 @@ static int weighted_ce(const float* logits, const L* labels, const float* weight
 
 extern "C" {
 
-int pfst_weighted_ce(const float* logits, const int64_t* labels, const float* weight, const float* class_weight,
-                     int64_t B, int32_t C, int32_t lh, int32_t lw, int32_t H, int32_t W, int64_t ignore_index,
-                     float loss_weight, float* grad_logits, double* stats, float* out2, void* stream) {
-  return pfst::weighted_ce(logits, labels, weight, class_weight, B, C, lh, lw, H, W, ignore_index, loss_weight,
-                           grad_logits, stats, out2, stream);
-}
-
-int pfst_weighted_ce_lbl(const float* logits, const void* labels, int32_t label_dtype, const float* weight,
-                         const float* class_weight, int64_t B, int32_t C, int32_t lh, int32_t lw, int32_t H,
-                         int32_t W, int64_t ignore_index, float loss_weight, float* grad_logits, double* stats,
-                         float* out2, void* stream) {
-  if (label_dtype == PFST_DT_I64)
-    return pfst::weighted_ce(logits, static_cast<const int64_t*>(labels), weight, class_weight, B, C, lh, lw, H, W,
-                             ignore_index, loss_weight, grad_logits, stats, out2, stream);
-  if (label_dtype == PFST_DT_U8)
-    return pfst::weighted_ce(logits, static_cast<const uint8_t*>(labels), weight, class_weight, B, C, lh, lw, H, W,
-                             ignore_index, loss_weight, grad_logits, stats, out2, stream);
-  return PFST_ERR_UNSUPPORTED;
+int pfst_weighted_ce(const float* logits, const void* labels, int32_t label_dtype, const float* weight,
+                     const float* class_weight, int64_t B, int32_t C, int32_t lh, int32_t lw, int32_t H, int32_t W,
+                     int64_t ignore_index, float loss_weight, float* grad_logits, double* stats, float* out2,
+                     void* stream) {
+  return pfst::with_label_dt(label_dtype, [&](auto l) {
+    return pfst::weighted_ce(logits, static_cast<const decltype(l)*>(labels), weight, class_weight, B, C, lh, lw, H,
+                             W, ignore_index, loss_weight, grad_logits, stats, out2, stream);
+  });
 }
 
 }  // extern "C"

@@ -99,6 +99,7 @@ class PluginEngine:
         self._ev = [torch.cuda.Event() for _ in range(8)]
         self._bufs: dict = {}
         self._gout = torch.zeros(8, dtype=torch.float32, device=self.device)
+        self._gout_proto = self._gout[6:]   # the upstream gradient of the prototype distance
         self._token = 0
         self._fwd = None                  # state of the last aux_forward, consumed by aux_backward
         self.ema_blocks_per_sm = int(os.environ.get("PFST_PLUGIN_EMA_BLOCKS_PER_SM", "0"))
@@ -143,8 +144,8 @@ class PluginEngine:
         prototypes on features)."""
         if label_dtype not in ops.LABEL_DTYPES:
             raise TypeError(f"label maps must be torch.int64 or torch.uint8, got {label_dtype}")
-        B, Cc, H, W = ema_logits.shape
-        ldt = ops._teacher(ema_logits, "ema_logits")      # fp32, fp16 or bf16: the teacher pass's own dtype
+        B, _, H, W = ema_logits.shape
+        ops._teacher(ema_logits, "ema_logits")            # fp32, fp16 or bf16: the teacher pass's own dtype
         use_x = x_ema is not None and (self.loss_cfg is not None or self.proto_cfg is not None)
         if use_x:
             ops._teacher(x_ema, "x_ema")
@@ -172,10 +173,8 @@ class PluginEngine:
                 with torch.cuda.stream(self._side):
                     ops.neigh_dots_slot(x_ema, geo.dilation // geo.up, 0, b["dots"])
                     self._ev[3].record(self._side)
-            _lib.call("pfst_pseudo_label_ft", ema_logits.data_ptr(), ldt, B, Cc, H * W, float(thr),
-                      None if thr_vec is None else thr_vec.data_ptr(), 0, -1, b["label"].data_ptr(),
-                      ops._TORCH2DT[label_dtype], b["conf"].data_ptr(), None if b["wpart"] is None else b["wpart"].data_ptr(),
-                      b["count"].data_ptr(), main.cuda_stream)
+            ops.launch_pseudo_label(ema_logits, thr, thr_vec, 0, -1, b["label"], b["conf"], b["wpart"], b["count"],
+                                    main.cuda_stream)
             masked = bank is not None and bank.masked(x_ema.shape[2], x_ema.shape[3], x_ema)
             if dots_here and not masked:
                 main.wait_event(self._ev[3])             # the label sort never runs next to a TMA dots kernel (step.py)
@@ -219,9 +218,9 @@ class PluginEngine:
             raise PfstError("aux_forward without teacher_outputs(x_ema) in this iteration")
         for name, t, dt in (("logits_trg", logits_trg, torch.float32), ("x_src", x_src, torch.float32)):
             ops._dev(t, name, dt)
-        ldt = ops._labels(gt, "gt")                  # int64 or uint8; mix_masks shares gt's dtype
+        ops._labels(gt, "gt")                        # int64 or uint8; mix_masks shares gt's dtype
         ops._labels(mix_masks, "mix_masks", like=gt)
-        Bf, D, h, w = x_src.shape
+        Bf, _, h, w = x_src.shape
         if a["dots"].shape[2:] != (Bf, 5, h, w):
             raise PfstError("PFGSTLoss: x_ema / x_src shape mismatch")
         bank = self.bank if self.proto_cfg is not None else None
@@ -229,8 +228,8 @@ class PluginEngine:
         b = self._bufs.get(skey)
         if b is None:
             e = lambda shape, dt: torch.empty(shape, dtype=dt, device=self.device)  # noqa: E731
-            ws_bytes = int(_lib.load().pfst_pfgst_loss_ws_bytes(geo.B, geo.C, geo.fh, geo.fw, geo.up))
-            b = dict(ws=e((ws_bytes,), torch.uint8), stats=e((16,), torch.float64), losses=e((6,), torch.float32),
+            b = dict(ws=e((ops.pfgst_loss_ws_bytes(geo),), torch.uint8), stats=e((16,), torch.float64),
+                     losses=e((6,), torch.float32),
                      dist=e((Bf, h, w), torch.float32), acc=e((4,), torch.float64), ploss=e((1,), torch.float32),
                      ploss_w=e((1,), torch.float32),
                      density=e((geo.B, 1, geo.gh, geo.gw), torch.float32) if want_vis else None,
@@ -238,12 +237,9 @@ class PluginEngine:
             b["loss_views"] = [b["losses"][i] for i in range(6)]      # 0-dim views handed to the log ledger
             b["ploss_view"] = b["ploss_w"][0]
             self._bufs[skey] = b
-        H, W = gt.shape[-2], gt.shape[-1]
         dots, ks = a["dots"], a["ks"]
-        w6 = ops._w6(cfg["w6"])
-        common = (dots.data_ptr(), ks, geo.B, geo.fh, geo.fw, geo.up, logits_trg.data_ptr(), geo.C, geo.lh, geo.lw,
-                  geo.lscale, geo.lscale, gt.data_ptr(), mix_masks.data_ptr(), geo.gt_h, geo.gt_w, geo.dilation,
-                  int(cfg["top_k"]), w6, b["ws"].data_ptr(), b["stats"].data_ptr())
+        loss = ops.pfgst_loss_args(dots, ks, geo, logits_trg, gt, mix_masks, cfg["top_k"], cfg["w6"], b["ws"],
+                                   b["stats"])
         pw = (C.c_float * 1)(float(self.proto_cfg.get('weight', 0.1))) if bank is not None else None
         pp = (C.c_void_p * 1)(b["ploss"].data_ptr())
 
@@ -255,22 +251,18 @@ class PluginEngine:
                 ops.neigh_dots_slot(x_src, geo.dilation // geo.up, 1, dots)
                 self._ev[5].record(self._side)
                 if bank is not None:
-                    _lib.call("pfst_proto_dist_fwd_lbl", x_src.data_ptr(), Bf, D, h, w, gt.data_ptr(), ldt, H, W,
-                              bank.mu.data_ptr(), bank.seen.data_ptr(), self.C, b["dist"].data_ptr(),
-                              b["acc"].data_ptr(), b["ploss"].data_ptr(), self._side.cuda_stream)
+                    ops.launch_proto_dist_fwd(x_src, gt, bank.mu, bank.seen, b["dist"], b["acc"], b["ploss"],
+                                              self._side.cuda_stream)
                     _lib.call("pfst_pack_scalars", pp, pw, 1, b["ploss_w"].data_ptr(), self._side.cuda_stream)
                     self._ev[6].record(self._side)
             main.wait_event(self._ev[5])
-            _lib.call("pfst_pfgst_loss_fwd_lbl", *common, b["losses"].data_ptr(),
-                      None if b["density"] is None else b["density"].data_ptr(),
-                      None if b["eroded"] is None else b["eroded"].data_ptr(), *ops.SHIPPED_LOSS_ARGS, ldt, main.cuda_stream)
+            ops.launch_pfgst_loss_fwd(loss, b["losses"], b["density"], b["eroded"], main.cuda_stream)
             if bank is not None:
                 main.wait_event(self._ev[6])
 
         key = skey + (logits_trg.data_ptr(), x_src.data_ptr(), gt.data_ptr(), mix_masks.data_ptr(), dots.data_ptr(),
                       bank is not None)
-        return dict(key=key, launch=launch, common=common, w6=w6, b=b, geo=geo, bank=bank, keep=(pw, pp),
-                    shapes=(Bf, D, h, w, H, W), ldt=ldt)
+        return dict(key=key, launch=launch, loss=loss, b=b, geo=geo, bank=bank, keep=(pw, pp))
 
     def aux_run(self, plan: dict) -> None:
         self._gb.run(plan["key"], plan["launch"])
@@ -301,21 +293,19 @@ class PluginEngine:
         wts = (C.c_float * 7)(wa, wa, wa, wa, wa, wa,
                               wp * float(self.proto_cfg.get('weight', 0.1)) if bank is not None else 0.0)
         _lib.call("pfst_pack_scalars", ptrs, wts, 7, self._gout.data_ptr(), s)
-        Bf, D, h, w, H, W = f["shapes"]
+        Bf, _, h, w = x_src.shape
         coef = torch.empty((Bf, 9, h, w), dtype=torch.float32, device=self.device)
         glog = torch.empty_like(logits_trg) if need_logits else None
-        _lib.call("pfst_pfgst_loss_bwd_lbl", *f["common"], self._gout.data_ptr(), coef.data_ptr(),
-                  None if glog is None else glog.data_ptr(), *ops.SHIPPED_LOSS_ARGS, f["ldt"], s)
+        ops.launch_pfgst_loss_bwd(f["loss"], self._gout, coef, glog, s)
         gx = None
         if need_x:
             gx = torch.empty_like(x_src)
             d = geo.dilation // geo.up
             if bank is not None:
-                _lib.call("pfst_neigh_grad_proto_lbl", x_src.data_ptr(), coef.data_ptr(), Bf, D, h, w, d,
-                          gt.data_ptr(), f["ldt"], H, W, bank.mu.data_ptr(), bank.seen.data_ptr(), self.C, b["dist"].data_ptr(),
-                          b["acc"].data_ptr(), self._gout.data_ptr() + 24, gx.data_ptr(), s)
+                ops.launch_neigh_grad_proto(x_src, coef, d, gt, bank.mu, bank.seen, b["dist"], b["acc"],
+                                            self._gout_proto, gx, s)
             else:
-                _lib.call("pfst_neigh_grad", x_src.data_ptr(), coef.data_ptr(), Bf, D, h, w, d, gx.data_ptr(), s)
+                ops.launch_neigh_grad(x_src, coef, d, gx, s)
         return glog, gx
 
     def close(self) -> None:

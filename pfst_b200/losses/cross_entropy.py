@@ -33,7 +33,7 @@ class _UpsampleCE(torch.autograd.Function):
         grad = torch.empty_like(seg_logit) if need_grad else None
         stats = torch.empty(4, dtype=torch.float64, device=dev)
         out2 = torch.empty(2, dtype=torch.float32, device=dev)
-        _lib.call("pfst_weighted_ce_lbl", ops._dev(seg_logit, "seg_logit", torch.float32),
+        _lib.call("pfst_weighted_ce", ops._dev(seg_logit, "seg_logit", torch.float32),
                   labels.data_ptr(), ops._labels(labels, "seg_label"), ops._opt(seg_weight, "seg_weight", torch.float32),
                   ops._opt(class_weight, "class_weight", torch.float32), B, C, lh, lw, H, W, int(ignore_index),
                   float(loss_weight), None if grad is None else grad.data_ptr(), stats.data_ptr(), out2.data_ptr(),

@@ -33,6 +33,10 @@ def _opt(t: Optional[torch.Tensor], name: str, dtype=None) -> Optional[int]:
     return None if t is None else _dev(t, name, dtype)
 
 
+def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
+    return None if t is None else t.data_ptr()
+
+
 LABEL_DTYPES = (torch.int64, torch.uint8)
 
 
@@ -145,7 +149,7 @@ class EmaTable:
             return
         if stream is None:
             stream = torch.cuda.current_stream(self.device).cuda_stream
-        _lib.call("pfst_ema_update_multi_ex", *self._ptrs, self.n_chunks, self.CHUNK, a32, b32, mode,
+        _lib.call("pfst_ema_update_multi", *self._ptrs, self.n_chunks, self.CHUNK, a32, b32, mode,
                   int(blocks_per_sm), stream)
 
 
@@ -179,7 +183,7 @@ def pseudo_label(logits: torch.Tensor, thr: float = 0.0, thr_per_class: Optional
     if logits.dim() != 4:
         raise ValueError("logits must be (B,C,H,W)")
     B, Cc, H, W = logits.shape
-    fdt = _teacher(logits, "logits")
+    _teacher(logits, "logits")
     if label_dtype not in LABEL_DTYPES:
         raise TypeError(f"label_dtype must be torch.int64 or torch.uint8, got {label_dtype}")
     if label_dtype == torch.uint8 and (Cc > 255 or int(reject_label) > 255):
@@ -193,11 +197,18 @@ def pseudo_label(logits: torch.Tensor, thr: float = 0.0, thr_per_class: Optional
         if thr_per_class.numel() != Cc:
             raise ValueError("thr_per_class must have C entries")
         _dev(thr_per_class, "thr_per_class", torch.float32)
-    _lib.call("pfst_pseudo_label_ft", logits.data_ptr(), fdt, B, Cc, H * W, float(thr),
-              None if thr_per_class is None else thr_per_class.data_ptr(), mode, int(reject_label),
-              label.data_ptr(), _TORCH2DT[label_dtype], conf.data_ptr(), None if wpart is None else wpart.data_ptr(),
-              count.data_ptr(), _stream())
+    launch_pseudo_label(logits, thr, thr_per_class, mode, reject_label, label, conf, wpart, count, _stream())
     return label, conf, count, wpart
+
+
+# The launch functions below pass tensors their caller has already validated (and allocated) to one entry
+# point, in ABI order, on the raw stream `stream`: no checks, no allocation. The dtype tags, the loss
+# weights and the shipped PFGSTLoss options are formed here only.
+def launch_pseudo_label(logits, thr, thr_per_class, mode, reject_label, label, conf, wpart, count, stream) -> None:
+    B, Cc, H, W = logits.shape
+    _lib.call("pfst_pseudo_label", logits.data_ptr(), _FLOAT2DT[logits.dtype], B, Cc, H * W, float(thr),
+              _ptr(thr_per_class), int(mode), int(reject_label), label.data_ptr(), _TORCH2DT[label.dtype],
+              conf.data_ptr(), _ptr(wpart), count.data_ptr(), stream)
 
 
 def pseudo_weight_fill(shape, count: torch.Tensor, ps_size: int, ignore_top: int = 0,
@@ -215,7 +226,7 @@ def class_presence(gt: torch.Tensor, out: Optional[torch.Tensor] = None) -> torc
     dt = _labels(gt, "gt")
     if out is None:
         out = torch.empty(9, dtype=torch.int32, device=gt.device)
-    _lib.call("pfst_class_presence_lbl", gt.data_ptr(), dt, gt.numel(), _dev(out, "presence", torch.int32),
+    _lib.call("pfst_class_presence", gt.data_ptr(), dt, gt.numel(), _dev(out, "presence", torch.int32),
               _stream())
     return out
 
@@ -228,7 +239,7 @@ def class_mix(gt: torch.Tensor, chosen: torch.Tensor, img: Optional[torch.Tensor
     """Fused ClassMix. gt (B,1,H,W) int64 or uint8; chosen int32 (B,8) bitmasks. The pseudo label, the
     mixed label and the mask share gt's dtype.
     -> (mixed_img|None, mixed_lbl|None, mixed_weight|None, mix_mask|None)"""
-    dt = _labels(gt, "gt")
+    _labels(gt, "gt")
     B, H, W = gt.shape[0], gt.shape[-2], gt.shape[-1]
     if gt.numel() != B * H * W:
         raise ValueError("gt must be (B,1,H,W) or (B,H,W)")
@@ -236,14 +247,12 @@ def class_mix(gt: torch.Tensor, chosen: torch.Tensor, img: Optional[torch.Tensor
     if chosen.numel() != B * 8:
         raise ValueError("chosen must hold 8 words per image")
     dev = gt.device
-    channels = 0
     mixed_img = mixed_lbl = mixed_w = mask = None
     if img is not None:
         _dev(img, "img", torch.float32)
         _dev(trg_img, "trg_img", torch.float32)
         if img.shape != trg_img.shape or img.shape[0] != B or img.shape[-2:] != gt.shape[-2:]:
             raise ValueError("img/trg_img shape mismatch")
-        channels = img.shape[1]
         mixed_img = torch.empty_like(img)
     if pseudo_lbl is not None:
         _labels(pseudo_lbl, "pseudo_label", like=gt)
@@ -259,12 +268,18 @@ def class_mix(gt: torch.Tensor, chosen: torch.Tensor, img: Optional[torch.Tensor
         _dev(mixed_w, "weight_out", torch.float32)
     if want_mask:
         mask = torch.empty((B, 1, H, W), dtype=gt.dtype, device=dev)
-    p = lambda t: None if t is None else t.data_ptr()
-    _lib.call("pfst_class_mix_lbl", gt.data_ptr(), chosen.data_ptr(), p(img), p(trg_img), p(pseudo_lbl),
-              p(weight_in) if want_weight else None, p(count), int(ps_size), int(ignore_top),
-              int(ignore_bottom), B, channels, H, W, p(mixed_img), p(mixed_lbl), p(mixed_w), p(mask), dt,
-              _stream())
+    launch_class_mix(gt, chosen, img, trg_img, pseudo_lbl, weight_in if want_weight else None, count, ps_size,
+                     ignore_top, ignore_bottom, mixed_img, mixed_lbl, mixed_w, mask, _stream())
     return mixed_img, mixed_lbl, mixed_w, mask
+
+
+def launch_class_mix(gt, chosen, img, trg_img, pseudo_lbl, weight_in, count, ps_size, ignore_top, ignore_bottom,
+                     mixed_img, mixed_lbl, mixed_weight, mix_mask, stream) -> None:
+    B, H, W = gt.shape[0], gt.shape[-2], gt.shape[-1]
+    _lib.call("pfst_class_mix", gt.data_ptr(), chosen.data_ptr(), _ptr(img), _ptr(trg_img), _ptr(pseudo_lbl),
+              _ptr(weight_in), _ptr(count), int(ps_size), int(ignore_top), int(ignore_bottom), B,
+              0 if img is None else img.shape[1], H, W, _ptr(mixed_img), _ptr(mixed_lbl), _ptr(mixed_weight),
+              _ptr(mix_mask), _TORCH2DT[gt.dtype], stream)
 
 
 # ----------------------------------------------------------- V1/V4: confusion
@@ -477,7 +492,7 @@ def neigh_dots_slot(x: torch.Tensor, dilation: int, slot: int, dots: Optional[to
         dots = torch.empty((ks, n_slots, B, 5, h, w), dtype=torch.float32, device=x.device)
     elif dots.numel() != ks * n_slots * B * 5 * h * w:
         raise ValueError("dots buffer has the wrong size")
-    _lib.call("pfst_neigh_dots_slot_ft", x.data_ptr(), fdt, B, D, h, w, int(dilation), int(slot), int(n_slots),
+    _lib.call("pfst_neigh_dots_slot", x.data_ptr(), fdt, B, D, h, w, int(dilation), int(slot), int(n_slots),
               _dev(dots, "dots", torch.float32), _stream())
     return dots, ks
 
@@ -489,23 +504,45 @@ def neigh_grad(x: torch.Tensor, coef: torch.Tensor, dilation: int, out: Optional
     gradient is added in the same pass over x."""
     _dev(x, "x", torch.float32)
     _dev(coef, "coef", torch.float32)
-    B, D, h, w = x.shape
+    B, _, h, w = x.shape
     if tuple(coef.shape) != (B, 9, h, w):
         raise ValueError("coef must be (B,9,h,w)")
     grad = torch.empty_like(x) if out is None else out
     _dev(grad, "grad_x", torch.float32)
     if proto is None:
-        _lib.call("pfst_neigh_grad", x.data_ptr(), coef.data_ptr(), B, D, h, w, int(dilation), grad.data_ptr(),
-                  _stream())
+        launch_neigh_grad(x, coef, dilation, grad, _stream())
     else:
         lab, mu, seen = proto["labels"], proto["mu"], proto.get("seen")
-        dt = _labels(lab, "labels")
-        _lib.call("pfst_neigh_grad_proto_lbl", x.data_ptr(), coef.data_ptr(), B, D, h, w, int(dilation),
-                  lab.data_ptr(), dt, lab.shape[-2], lab.shape[-1], _dev(mu, "mu", torch.float32),
-                  _opt(seen, "seen", torch.uint8), mu.shape[0], _dev(proto["dist"], "dist", torch.float32),
-                  _dev(proto["acc"], "acc", torch.float64), _dev(proto["grad_loss"], "grad_loss", torch.float32),
-                  grad.data_ptr(), _stream())
+        _labels(lab, "labels")
+        _dev(mu, "mu", torch.float32)
+        _opt(seen, "seen", torch.uint8)
+        _dev(proto["dist"], "dist", torch.float32)
+        _dev(proto["acc"], "acc", torch.float64)
+        _dev(proto["grad_loss"], "grad_loss", torch.float32)
+        launch_neigh_grad_proto(x, coef, dilation, lab, mu, seen, proto["dist"], proto["acc"], proto["grad_loss"],
+                                grad, _stream())
     return grad
+
+
+def launch_neigh_grad(x, coef, dilation, grad_x, stream) -> None:
+    B, D, h, w = x.shape
+    _lib.call("pfst_neigh_grad", x.data_ptr(), coef.data_ptr(), B, D, h, w, int(dilation), grad_x.data_ptr(), stream)
+
+
+def launch_neigh_grad_proto(x, coef, dilation, labels, mu, seen, dist, acc, grad_loss, grad_x, stream) -> None:
+    """grad_loss: fp32 tensor whose first element is the upstream gradient of the prototype distance."""
+    B, D, h, w = x.shape
+    _lib.call("pfst_neigh_grad_proto", x.data_ptr(), coef.data_ptr(), B, D, h, w, int(dilation), labels.data_ptr(),
+              _TORCH2DT[labels.dtype], labels.shape[-2], labels.shape[-1], mu.data_ptr(), _ptr(seen), mu.shape[0],
+              dist.data_ptr(), acc.data_ptr(), grad_loss.data_ptr(), grad_x.data_ptr(), stream)
+
+
+def launch_proto_dist_fwd(feats, labels, mu, seen, dist, acc, loss, stream) -> None:
+    """mu: (C, D) prototypes; seen: uint8[C] or None."""
+    B, D, h, w = feats.shape
+    _lib.call("pfst_proto_dist_fwd", feats.data_ptr(), B, D, h, w, labels.data_ptr(), _TORCH2DT[labels.dtype],
+              labels.shape[-2], labels.shape[-1], mu.data_ptr(), _ptr(seen), mu.shape[0], dist.data_ptr(),
+              acc.data_ptr(), loss.data_ptr(), stream)
 
 
 class LossGeometry:
@@ -534,15 +571,7 @@ class LossGeometry:
         self.dilation = int(dilation)
 
 
-def _w6(weights6):
-    arr = (C.c_float * 6)(*[float(v) for v in weights6])
-    return arr
-
-
 LOSS_SIM_GAUSSIAN, LOSS_CROSS_PROB_EMA, LOSS_UNFOLD_GRAD, LOSS_SRC_MARGIN, LOSS_SRC_MARGIN2 = 1, 2, 4, 8, 16   # PFST_LOSS_*
-# the (options, sigma, logits_ema, margin) arguments of pfst_pfgst_loss_{fwd,bwd}_lbl for the shipped
-# configuration: options 0, so sigma, logits_ema and margin are not read
-SHIPPED_LOSS_ARGS = (0, 0.0, None, None)
 
 
 def _loss_options(options: int, logits_ema, geo: LossGeometry):
@@ -555,12 +584,8 @@ def _loss_options(options: int, logits_ema, geo: LossGeometry):
             # (pfgst_loss.py:175): any other shape fails there too
             raise PfstError(f"PFGSTLoss(cross_prob_type='ema'): logits_ema {tuple(logits_ema.shape)} must have the "
                             f"loss-grid shape {(geo.B, geo.C, geo.gh, geo.gw)} (the reference broadcasts p * q)")
-        return logits_ema.data_ptr()
+        return logits_ema
     return None
-
-
-def _margin(margin):
-    return None if margin is None else (C.c_float * 2)(float(margin[0]), float(margin[1]))
 
 
 def pfgst_loss_fwd(dots, ks, geo: LossGeometry, logits, gt, mix, top_k, weights6, want_vis=True,
@@ -570,20 +595,16 @@ def pfgst_loss_fwd(dots, ks, geo: LossGeometry, logits, gt, mix, top_k, weights6
     dev = logits.device
     _dev(dots, "dots", torch.float32)
     _dev(logits, "logits", torch.float32)
-    dt = _labels(gt, "gt")
+    _labels(gt, "gt")
     _labels(mix, "mix", like=gt)
-    q_ptr = _loss_options(options, logits_ema, geo)
+    logits_ema = _loss_options(options, logits_ema, geo)
     stats = torch.empty(16, dtype=torch.float64, device=dev)
-    ws_bytes = int(_lib.load().pfst_pfgst_loss_ws_bytes_ex(geo.B, geo.C, geo.fh, geo.fw, geo.up, int(options)))
-    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    ws = torch.empty(pfgst_loss_ws_bytes(geo, options), dtype=torch.uint8, device=dev)
     losses = torch.empty(6, dtype=torch.float32, device=dev)
     density = torch.empty((geo.B, 1, geo.gh, geo.gw), dtype=torch.float32, device=dev) if want_vis else None
     eroded = torch.empty((geo.B, 1, geo.gh, geo.gw), dtype=torch.uint8, device=dev) if want_vis else None
-    _lib.call("pfst_pfgst_loss_fwd_lbl", dots.data_ptr(), ks, geo.B, geo.fh, geo.fw, geo.up, logits.data_ptr(),
-              geo.C, geo.lh, geo.lw, geo.lscale, geo.lscale, gt.data_ptr(), mix.data_ptr(), geo.gt_h, geo.gt_w,
-              geo.dilation, int(top_k), _w6(weights6), ws.data_ptr(), stats.data_ptr(), losses.data_ptr(),
-              None if density is None else density.data_ptr(), None if eroded is None else eroded.data_ptr(),
-              int(options), float(sigma), q_ptr, _margin(margin), dt, _stream())
+    args = pfgst_loss_args(dots, ks, geo, logits, gt, mix, top_k, weights6, ws, stats)
+    launch_pfgst_loss_fwd(args, losses, density, eroded, _stream(), options, sigma, logits_ema, margin)
     return losses, (stats, ws), density, eroded
 
 
@@ -592,15 +613,45 @@ def pfgst_loss_bwd(dots, ks, geo: LossGeometry, logits, gt, mix, top_k, weights6
     """-> (coef (B,9,fh,fw), grad_logits|None)."""
     dev = logits.device
     _dev(grad_losses, "grad_losses", torch.float32)
-    dt = _labels(gt, "gt")
+    _labels(gt, "gt")
     _labels(mix, "mix", like=gt)
-    q_ptr = _loss_options(options, logits_ema, geo)
+    logits_ema = _loss_options(options, logits_ema, geo)
     stats, ws = stats
     coef = torch.empty((geo.B, 9, geo.fh, geo.fw), dtype=torch.float32, device=dev)
     glog = torch.empty_like(logits) if want_logits_grad else None
-    _lib.call("pfst_pfgst_loss_bwd_lbl", dots.data_ptr(), ks, geo.B, geo.fh, geo.fw, geo.up, logits.data_ptr(),
-              geo.C, geo.lh, geo.lw, geo.lscale, geo.lscale, gt.data_ptr(), mix.data_ptr(), geo.gt_h, geo.gt_w,
-              geo.dilation, int(top_k), _w6(weights6), ws.data_ptr(), stats.data_ptr(), grad_losses.data_ptr(),
-              coef.data_ptr(), None if glog is None else glog.data_ptr(), int(options), float(sigma), q_ptr,
-              _margin(margin), dt, _stream())
+    args = pfgst_loss_args(dots, ks, geo, logits, gt, mix, top_k, weights6, ws, stats)
+    launch_pfgst_loss_bwd(args, grad_losses, coef, glog, _stream(), options, sigma, logits_ema, margin)
     return coef, glog
+
+
+def pfgst_loss_ws_bytes(geo: LossGeometry, options: int = 0) -> int:
+    """Bytes of the workspace pfgst_loss_fwd leaves for pfgst_loss_bwd."""
+    return int(_lib.load().pfst_pfgst_loss_ws_bytes(geo.B, geo.C, geo.fh, geo.fw, geo.up, int(options)))
+
+
+def pfgst_loss_args(dots, ks, geo: LossGeometry, logits, gt, mix, top_k, weights6, ws, stats) -> tuple:
+    """The arguments pfst_pfgst_loss_fwd and _bwd share, marshalled once: addresses, not tensors, so that a
+    caller can keep them from the forward to the backward without keeping the inputs alive."""
+    w6 = (C.c_float * 6)(*[float(v) for v in weights6])
+    return ((dots.data_ptr(), ks, geo.B, geo.fh, geo.fw, geo.up, logits.data_ptr(), geo.C, geo.lh, geo.lw,
+             geo.lscale, geo.lscale, gt.data_ptr(), mix.data_ptr(), geo.gt_h, geo.gt_w, geo.dilation, int(top_k), w6,
+             ws.data_ptr(), stats.data_ptr()), _TORCH2DT[gt.dtype])
+
+
+def _margin(margin):
+    return None if margin is None else (C.c_float * 2)(float(margin[0]), float(margin[1]))
+
+
+# options = 0 is the shipped configuration: sigma, logits_ema and margin are then not read
+def launch_pfgst_loss_fwd(args, losses, density, eroded, stream, options: int = 0, sigma: float = 0.0,
+                          logits_ema=None, margin=None) -> None:
+    common, ldt = args
+    _lib.call("pfst_pfgst_loss_fwd", *common, losses.data_ptr(), _ptr(density), _ptr(eroded), int(options),
+              float(sigma), _ptr(logits_ema), _margin(margin), ldt, stream)
+
+
+def launch_pfgst_loss_bwd(args, grad_losses, coef, grad_logits, stream, options: int = 0, sigma: float = 0.0,
+                          logits_ema=None, margin=None) -> None:
+    common, ldt = args
+    _lib.call("pfst_pfgst_loss_bwd", *common, grad_losses.data_ptr(), _ptr(coef), _ptr(grad_logits), int(options),
+              float(sigma), _ptr(logits_ema), _margin(margin), ldt, stream)

@@ -144,7 +144,7 @@ class PrototypeBank:
                 raise PfstError(f"prototype accumulation does not support B={B}, h={h}, w={w}, C={self.C}")
             self._order_ws = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
             self._order_key = key
-        _lib.call("pfst_proto_order_lbl", labels.data_ptr(), ops._labels(labels, "labels"), B, h, w, labels.shape[-2],
+        _lib.call("pfst_proto_order", labels.data_ptr(), ops._labels(labels, "labels"), B, h, w, labels.shape[-2],
                   labels.shape[-1], ops._opt(conf, "conf", torch.float32), float(conf_thr), self.C,
                   self.packed.data_ptr() + 4 * self.C * self.D, self._order_ws.data_ptr(), ops._stream())
 
@@ -154,7 +154,7 @@ class PrototypeBank:
             raise ValueError("feature dim mismatch")
         if self._order_key != (B, h, w):
             raise PfstError("accumulate_ordered: call order() for this batch geometry first")
-        _lib.call("pfst_proto_accum_ordered_ft", feats.data_ptr(), ops._teacher(feats, "feats"), B, D, h, w, self.C,
+        _lib.call("pfst_proto_accum_ordered", feats.data_ptr(), ops._teacher(feats, "feats"), B, D, h, w, self.C,
                   self._order_ws.data_ptr(), self.packed.data_ptr(), ops._stream())
 
     def accumulate_single_launch(self, feats: torch.Tensor, labels: torch.Tensor,
@@ -164,7 +164,7 @@ class PrototypeBank:
         B, D, h, w = feats.shape
         if D != self.D:
             raise ValueError("feature dim mismatch")
-        _lib.call("pfst_proto_accum_ft", feats.data_ptr(), ops._teacher(feats, "feats"), B, D, h, w,
+        _lib.call("pfst_proto_accum", feats.data_ptr(), ops._teacher(feats, "feats"), B, D, h, w,
                   labels.data_ptr(), ops._labels(labels, "labels"), labels.shape[-2], labels.shape[-1],
                   ops._opt(conf, "conf", torch.float32), float(conf_thr), self.C, self.packed.data_ptr(),
                   ops._stream())
@@ -206,7 +206,7 @@ class PrototypeBank:
                       self.counts.data_ptr(), self.seen.data_ptr(), pb.boards.data_ptr(), pb.rank, pb.world,
                       pb.status.data_ptr(), pb.timeout_ns, stream)
             return
-        _lib.call("pfst_proto_finalize_dev", self.packed.data_ptr(), self.C, self.D, self.mu.data_ptr(),
+        _lib.call("pfst_proto_finalize", self.packed.data_ptr(), self.C, self.D, self.mu.data_ptr(),
                   self.seen.data_ptr(), float(self.alpha), self.iter_state.data_ptr(), self.mu.data_ptr(),
                   self.counts.data_ptr(), self.seen.data_ptr(), 1, stream)
 
@@ -219,16 +219,16 @@ class _ProtoDistFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, feats, labels, mu, seen):
         feats = feats.contiguous()
-        B, D, h, w = feats.shape
-        C = mu.shape[0]
+        B, _, h, w = feats.shape
         dev = feats.device
         dist = torch.empty((B, h, w), dtype=torch.float32, device=dev)
         acc = torch.empty(4, dtype=torch.float64, device=dev)
         loss = torch.empty(1, dtype=torch.float32, device=dev)
-        _lib.call("pfst_proto_dist_fwd_lbl", ops._dev(feats, "feats", torch.float32), B, D, h, w,
-                  labels.data_ptr(), ops._labels(labels, "labels"), labels.shape[-2], labels.shape[-1],
-                  ops._dev(mu, "mu", torch.float32), ops._opt(seen, "seen", torch.uint8), C, dist.data_ptr(),
-                  acc.data_ptr(), loss.data_ptr(), ops._stream())
+        ops._dev(feats, "feats", torch.float32)
+        ops._labels(labels, "labels")
+        ops._dev(mu, "mu", torch.float32)
+        ops._opt(seen, "seen", torch.uint8)
+        ops.launch_proto_dist_fwd(feats, labels, mu, seen, dist, acc, loss, ops._stream())
         ctx.save_for_backward(feats, labels, mu, seen, dist, acc)
         return loss[0]
 
@@ -238,7 +238,7 @@ class _ProtoDistFn(torch.autograd.Function):
         B, D, h, w = feats.shape
         grad = torch.empty_like(feats)
         g = grad_out.reshape(1).contiguous().float()
-        _lib.call("pfst_proto_dist_bwd_lbl", feats.data_ptr(), B, D, h, w, labels.data_ptr(),
+        _lib.call("pfst_proto_dist_bwd", feats.data_ptr(), B, D, h, w, labels.data_ptr(),
                   ops._labels(labels, "labels"), labels.shape[-2],
                   labels.shape[-1], mu.data_ptr(), None if seen is None else seen.data_ptr(), mu.shape[0],
                   dist.data_ptr(), acc.data_ptr(), g.data_ptr(), grad.data_ptr(), 0, ops._stream())

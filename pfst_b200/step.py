@@ -44,7 +44,7 @@ from typing import Optional
 import numpy as np
 import torch
 
-from . import _lib, ops
+from . import ops
 from .prototypes import PrototypeBank
 from .utils.dacs_transforms import ClassMixPlan
 
@@ -59,15 +59,13 @@ class _Buffers:
         f32, i64 = torch.float32, torch.int64
         e = lambda shape, dt: torch.empty(shape, dtype=dt, device=dev)  # noqa: E731
         # the label maps follow gt's dtype (int64 or uint8)
-        self.ldt = ops._TORCH2DT[label_dtype]
         self.label, self.conf, self.count = e((B, H, W), label_dtype), e((B, H, W), f32), e((1,), i64)
         self.mixed_img, self.mixed_lbl = e(img_shape, f32), e((B, 1, H, W), label_dtype)
         self.weight, self.mix_mask = e((B, H, W), f32), e((B, 1, H, W), label_dtype)
         Bf, D, h, w = feat_shape
         self.ks = ops.neigh_dots_splits(Bf, D, h, w)
         self.dots = e((self.ks, 2, Bf, 5, h, w), f32)
-        ws_bytes = int(_lib.load().pfst_pfgst_loss_ws_bytes(geo.B, geo.C, geo.fh, geo.fw, geo.up))
-        self.ws = e((ws_bytes,), torch.uint8)
+        self.ws = e((ops.pfgst_loss_ws_bytes(geo),), torch.uint8)
         self.stats, self.losses = e((16,), torch.float64), e((6,), f32)
         self.dist, self.acc, self.ploss = e((Bf, h, w), f32), e((4,), torch.float64), e((1,), f32)
         self.coef, self.grad_logits, self.grad_x = e((Bf, 9, h, w), f32), e(logits_shape, f32), e(feat_shape, f32)
@@ -135,7 +133,6 @@ class SelfTrainingStep:
 
     # ------------------------------------------------------------------ segments
     def _segment_a(self, b: _Buffers, ema_logits, x_ema, geo):
-        B, C, H, W = ema_logits.shape
         main = torch.cuda.current_stream()
         fork, join = self._ev[0], self._ev[1]
         fork.record(main)
@@ -143,9 +140,7 @@ class SelfTrainingStep:
         with torch.cuda.stream(self._side):                       # branch 2: L2 on x_ema
             ops.neigh_dots_slot(x_ema, geo.dilation // geo.up, 0, b.dots)
             join.record(self._side)
-        _lib.call("pfst_pseudo_label_ft", ema_logits.data_ptr(), ops._FLOAT2DT[ema_logits.dtype], B, C, H * W,
-                  float(self.thr), None, 0, -1, b.label.data_ptr(), b.ldt, b.conf.data_ptr(), None, b.count.data_ptr(),
-                  ops._stream())
+        ops.launch_pseudo_label(ema_logits, self.thr, None, 0, -1, b.label, b.conf, None, b.count, ops._stream())
         if self.bank.masked(x_ema.shape[2], x_ema.shape[3], x_ema):
             self.bank.accumulate(x_ema, b.label)                  # one masked launch next to dots(x_ema)
             main.wait_event(join)
@@ -160,15 +155,11 @@ class SelfTrainingStep:
         all-reduce is in flight), then proto_finalize, then 'b2' = distance forward + fused backward."""
         main = torch.cuda.current_stream()
         s = main.cuda_stream
-        B, H, W = gt.shape[0], gt.shape[-2], gt.shape[-1]
-        Bf, D, h, w = x_src.shape
         bank = self.bank
         fork, dots_done, join = self._ev[2], self._ev[3], self._ev[4]
 
         def dist_fwd():
-            _lib.call("pfst_proto_dist_fwd_lbl", x_src.data_ptr(), Bf, D, h, w, gt.data_ptr(), b.ldt, H, W,
-                      bank.mu.data_ptr(), bank.seen.data_ptr(), self.C, b.dist.data_ptr(), b.acc.data_ptr(),
-                      b.ploss.data_ptr(), ops._stream())
+            ops.launch_proto_dist_fwd(x_src, gt, bank.mu, bank.seen, b.dist, b.acc, b.ploss, ops._stream())
 
         if part in ("all", "b1"):
             fork.record(main)
@@ -181,27 +172,23 @@ class SelfTrainingStep:
                         self._side.wait_event(mu_ready)
                     dist_fwd()
                     join.record(self._side)
-            _lib.call("pfst_class_mix_lbl", gt.data_ptr(), chosen.data_ptr(), img.data_ptr(), trg_img.data_ptr(),
-                      b.label.data_ptr(), None, b.count.data_ptr(), b.label.numel(), 0, 0, B, img.shape[1], H, W,
-                      b.mixed_img.data_ptr(), b.mixed_lbl.data_ptr(), b.weight.data_ptr(), b.mix_mask.data_ptr(),
-                      b.ldt, s)
+            ops.launch_class_mix(gt, chosen, img, trg_img, b.label, None, b.count, b.label.numel(), 0, 0,
+                                 b.mixed_img, b.mixed_lbl, b.weight, b.mix_mask, s)
             main.wait_event(dots_done)
-            w6 = ops._w6(self.w6)
-            common = (b.dots.data_ptr(), b.ks, geo.B, geo.fh, geo.fw, geo.up, logits_trg.data_ptr(), geo.C,
-                      geo.lh, geo.lw, geo.lscale, geo.lscale, gt.data_ptr(), b.mix_mask.data_ptr(), geo.gt_h,
-                      geo.gt_w, geo.dilation, int(self.top_k), w6, b.ws.data_ptr(), b.stats.data_ptr())
-            _lib.call("pfst_pfgst_loss_fwd_lbl", *common, b.losses.data_ptr(), None, None, *ops.SHIPPED_LOSS_ARGS, b.ldt, s)
+            loss = self._loss_args(b, gt, logits_trg, geo)
+            ops.launch_pfgst_loss_fwd(loss, b.losses, None, None, s)
             # backward of (sum of the six losses + proto_weight * proto loss)
-            _lib.call("pfst_pfgst_loss_bwd_lbl", *common, self.gout.data_ptr(), b.coef.data_ptr(),
-                      b.grad_logits.data_ptr(), *ops.SHIPPED_LOSS_ARGS, b.ldt, s)
+            ops.launch_pfgst_loss_bwd(loss, self.gout, b.coef, b.grad_logits, s)
             if part == "all":
                 main.wait_event(join)
         if part == "b2":
             dist_fwd()
         if part in ("all", "b2"):
-            _lib.call("pfst_neigh_grad_proto_lbl", x_src.data_ptr(), b.coef.data_ptr(), Bf, D, h, w,
-                      geo.dilation // geo.up, gt.data_ptr(), b.ldt, H, W, bank.mu.data_ptr(), bank.seen.data_ptr(),
-                      self.C, b.dist.data_ptr(), b.acc.data_ptr(), self.gproto.data_ptr(), b.grad_x.data_ptr(), s)
+            ops.launch_neigh_grad_proto(x_src, b.coef, geo.dilation // geo.up, gt, bank.mu, bank.seen, b.dist, b.acc,
+                                        self.gproto, b.grad_x, s)
+
+    def _loss_args(self, b: _Buffers, gt, logits_trg, geo):
+        return ops.pfgst_loss_args(b.dots, b.ks, geo, logits_trg, gt, b.mix_mask, self.top_k, self.w6, b.ws, b.stats)
 
     def _multi_rank(self) -> bool:
         if self._world is None:
@@ -236,8 +223,7 @@ class SelfTrainingStep:
         dots(x_ema) and dots(x_src) waits for it; tests/test_gpu_step_fused.py checks every replay."""
         ema_logits, x_ema, geo = args_a
         img, trg_img, gt, chosen, logits_trg, x_src, _ = args_b
-        B, C, H, W = ema_logits.shape
-        Bf, D, h, w = x_src.shape
+        Bf, _, h, w = x_src.shape
         bank = self.bank
         cur = torch.cuda.current_stream()
         main = cur
@@ -251,9 +237,7 @@ class SelfTrainingStep:
         with torch.cuda.stream(self._side):
             ops.neigh_dots_slot(x_ema, geo.dilation // geo.up, 0, b.dots)
             dots_ema.record(self._side)
-        _lib.call("pfst_pseudo_label_ft", ema_logits.data_ptr(), ops._FLOAT2DT[ema_logits.dtype], B, C, H * W,
-                  float(self.thr), None, 0, -1, b.label.data_ptr(), b.ldt, b.conf.data_ptr(), None, b.count.data_ptr(),
-                  s)
+        ops.launch_pseudo_label(ema_logits, self.thr, None, 0, -1, b.label, b.conf, None, b.count, s)
         pl_done.record(main)
         unsafe = os.environ.get("PFST_DAG_UNSAFE") == "1"           # reproduces DESIGN.md 3.2 (tools/dots_replay_check.py)
         masked = bank.masked(h, w, x_ema)      # few classes: no sort kernel -> nothing to keep away from the TMA kernels
@@ -279,37 +263,26 @@ class SelfTrainingStep:
                 dist.all_reduce(bank.packed, op=dist.ReduceOp.SUM, group=bank.group)
             bank.finalize_captured(self._comm.cuda_stream, local_only=not reduce)
             self._comm.wait_event(dots_src)
-            _lib.call("pfst_proto_dist_fwd_lbl", x_src.data_ptr(), Bf, D, h, w, gt.data_ptr(), b.ldt, H, W,
-                      bank.mu.data_ptr(), bank.seen.data_ptr(), self.C, b.dist.data_ptr(), b.acc.data_ptr(),
-                      b.ploss.data_ptr(), self._comm.cuda_stream)
+            ops.launch_proto_dist_fwd(x_src, gt, bank.mu, bank.seen, b.dist, b.acc, b.ploss, self._comm.cuda_stream)
             proto_done.record(self._comm)
-        _lib.call("pfst_class_mix_lbl", gt.data_ptr(), chosen.data_ptr(), img.data_ptr(), trg_img.data_ptr(),
-                  b.label.data_ptr(), None, b.count.data_ptr(), b.label.numel(), 0, 0, B, img.shape[1], H, W,
-                  b.mixed_img.data_ptr(), b.mixed_lbl.data_ptr(), b.weight.data_ptr(), b.mix_mask.data_ptr(),
-                  b.ldt, s)
+        ops.launch_class_mix(gt, chosen, img, trg_img, b.label, None, b.count, b.label.numel(), 0, 0, b.mixed_img,
+                             b.mixed_lbl, b.weight, b.mix_mask, s)
         main.wait_event(dots_src)
-        w6 = ops._w6(self.w6)
-        common = (b.dots.data_ptr(), b.ks, geo.B, geo.fh, geo.fw, geo.up, logits_trg.data_ptr(), geo.C,
-                  geo.lh, geo.lw, geo.lscale, geo.lscale, gt.data_ptr(), b.mix_mask.data_ptr(), geo.gt_h,
-                  geo.gt_w, geo.dilation, int(self.top_k), w6, b.ws.data_ptr(), b.stats.data_ptr())
-        _lib.call("pfst_pfgst_loss_fwd_lbl", *common, b.losses.data_ptr(), None, None, *ops.SHIPPED_LOSS_ARGS, b.ldt, s)
+        loss = self._loss_args(b, gt, logits_trg, geo)
+        ops.launch_pfgst_loss_fwd(loss, b.losses, None, None, s)
         if self.split_bwd:
             # the x_src gradient pass only needs the coefficient maps: grad_logits on the idle side stream
             stats_done, logits_done = self._ev[9], self._ev[0]
             stats_done.record(main)
             self._side.wait_event(stats_done)
-            _lib.call("pfst_pfgst_loss_bwd_lbl", *common, self.gout.data_ptr(), None, b.grad_logits.data_ptr(),
-                      *ops.SHIPPED_LOSS_ARGS, b.ldt, self._side.cuda_stream)
+            ops.launch_pfgst_loss_bwd(loss, self.gout, None, b.grad_logits, self._side.cuda_stream)
             logits_done.record(self._side)
-            _lib.call("pfst_pfgst_loss_bwd_lbl", *common, self.gout.data_ptr(), b.coef.data_ptr(), None,
-                      *ops.SHIPPED_LOSS_ARGS, b.ldt, s)
+            ops.launch_pfgst_loss_bwd(loss, self.gout, b.coef, None, s)
         else:
-            _lib.call("pfst_pfgst_loss_bwd_lbl", *common, self.gout.data_ptr(), b.coef.data_ptr(),
-                      b.grad_logits.data_ptr(), *ops.SHIPPED_LOSS_ARGS, b.ldt, s)
+            ops.launch_pfgst_loss_bwd(loss, self.gout, b.coef, b.grad_logits, s)
         main.wait_event(proto_done)
-        _lib.call("pfst_neigh_grad_proto_lbl", x_src.data_ptr(), b.coef.data_ptr(), Bf, D, h, w,
-                  geo.dilation // geo.up, gt.data_ptr(), b.ldt, H, W, bank.mu.data_ptr(), bank.seen.data_ptr(),
-                  self.C, b.dist.data_ptr(), b.acc.data_ptr(), self.gproto.data_ptr(), b.grad_x.data_ptr(), s)
+        ops.launch_neigh_grad_proto(x_src, b.coef, geo.dilation // geo.up, gt, bank.mu, bank.seen, b.dist, b.acc,
+                                    self.gproto, b.grad_x, s)
         if self.split_bwd:
             main.wait_event(logits_done)
         if main is not cur:

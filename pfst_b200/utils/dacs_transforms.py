@@ -143,7 +143,7 @@ class ClassMixPlan:
         self._batches[slot] = batch
         if stream is None:
             stream = torch.cuda.current_stream()
-        _lib.call("pfst_class_presence_lbl", gt.data_ptr(), dt, gt.numel(), self._presence.data_ptr(),
+        _lib.call("pfst_class_presence", gt.data_ptr(), dt, gt.numel(), self._presence.data_ptr(),
                   stream.cuda_stream)
         _lib.call("pfst_copy_async", self._presence_host.data_ptr() + 36 * slot, self._presence.data_ptr(), 36,
                   stream.cuda_stream)

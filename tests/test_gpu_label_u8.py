@@ -182,7 +182,7 @@ def test_proto_bank_u8_equals_i64(cuda, monkeypatch, C, feat, lab, force):
     assert _close(lb_, la) and _close(gb, ga)
 
 
-def test_neigh_grad_proto_u8_equals_i64(cuda):
+def test_neigh_grad_proto_tagged_u8_equals_i64(cuda):
     B, D, h, w, C = 2, 32, 32, 32, 6
     g = torch.Generator().manual_seed(2)
     x = torch.randn((B, D, h, w), generator=g).to(cuda)
@@ -196,7 +196,7 @@ def test_neigh_grad_proto_u8_equals_i64(cuda):
         dist = torch.empty((B, h, w), device=cuda)
         acc = torch.empty(4, dtype=torch.float64, device=cuda)
         loss = torch.empty(1, device=cuda)
-        _lib.call("pfst_proto_dist_fwd_lbl", x.data_ptr(), B, D, h, w, lb.data_ptr(), ops._labels(lb, "l"), 128, 128,
+        _lib.call("pfst_proto_dist_fwd", x.data_ptr(), B, D, h, w, lb.data_ptr(), ops._labels(lb, "l"), 128, 128,
                   mu.data_ptr(), seen.data_ptr(), C, dist.data_ptr(), acc.data_ptr(), loss.data_ptr(), ops._stream())
         proto = dict(labels=lb, mu=mu, seen=seen, dist=dist, acc=acc, grad_loss=torch.full((1,), 0.1, device=cuda))
         gx = ops.neigh_grad(x, coef, 2, proto=proto)

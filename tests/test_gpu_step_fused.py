@@ -29,7 +29,7 @@ def test_dots_slot_matches_pair_launch(cuda, B, D, h, w, dil):
 
 @pytest.mark.parametrize("B,D,h,w,dil,C,H,W", [(2, 64, 64, 64, 2, 6, 512, 512), (2, 48, 32, 32, 1, 33, 64, 64),
                                                 (3, 16, 15, 15, 2, 33, 120, 120), (1, 520, 16, 32, 2, 4, 64, 128)])
-def test_grad_proto_is_bit_identical_to_two_passes(cuda, B, D, h, w, dil, C, H, W):
+def test_fused_grad_proto_is_bit_identical_to_two_tagged_passes(cuda, B, D, h, w, dil, C, H, W):
     g = torch.Generator().manual_seed(2)
     x = torch.relu(torch.randn((B, D, h, w), generator=g)).to(cuda)
     coef = torch.randn((B, 9, h, w), generator=g).to(cuda)
@@ -41,11 +41,11 @@ def test_grad_proto_is_bit_identical_to_two_passes(cuda, B, D, h, w, dil, C, H, 
     dist = torch.empty((B, h, w), dtype=torch.float32, device=cuda)
     acc = torch.empty(4, dtype=torch.float64, device=cuda)
     loss = torch.empty(1, dtype=torch.float32, device=cuda)
-    _lib.call("pfst_proto_dist_fwd", x.data_ptr(), B, D, h, w, labels.data_ptr(), H, W, mu.data_ptr(),
+    _lib.call("pfst_proto_dist_fwd", x.data_ptr(), B, D, h, w, labels.data_ptr(), _lib.DT_I64, H, W, mu.data_ptr(),
               seen.data_ptr(), C, dist.data_ptr(), acc.data_ptr(), loss.data_ptr(), ops._stream())
     gl = torch.full((1,), 0.37, dtype=torch.float32, device=cuda)
     two = ops.neigh_grad(x, coef, dil)
-    _lib.call("pfst_proto_dist_bwd", x.data_ptr(), B, D, h, w, labels.data_ptr(), H, W, mu.data_ptr(),
+    _lib.call("pfst_proto_dist_bwd", x.data_ptr(), B, D, h, w, labels.data_ptr(), _lib.DT_I64, H, W, mu.data_ptr(),
               seen.data_ptr(), C, dist.data_ptr(), acc.data_ptr(), gl.data_ptr(), two.data_ptr(), 1, ops._stream())
     one = ops.neigh_grad(x, coef, dil, proto=dict(labels=labels, mu=mu, seen=seen, dist=dist, acc=acc, grad_loss=gl))
     assert torch.equal(one, two)

@@ -217,7 +217,7 @@ def test_teacher_dtype_errors_raise_before_launch(cuda):
 
 
 @pytest.mark.gpu
-def test_ft_entry_points_refuse_unknown_tags(cuda):
+def test_teacher_entry_points_refuse_unknown_tags(cuda):
     B, C, D, h, w = 2, 6, 16, 16, 16
     x = torch.randn((B, C, h, w), device=cuda)
     lab = torch.empty((B, h, w), dtype=torch.int64, device=cuda)
@@ -230,16 +230,16 @@ def test_ft_entry_points_refuse_unknown_tags(cuda):
     L = _lib.load()
     s = ops._stream()
     for tag in (0, 1, 2, 15, 19, -1):                        # label tags and neighbours are not float tags
-        assert L.pfst_pseudo_label_ft(x.data_ptr(), tag, B, C, h * w, 0.5, None, 0, -1, lab.data_ptr(),
-                                      _lib.DT_I64, conf.data_ptr(), None, count.data_ptr(), s) == -2
-        assert L.pfst_neigh_dots_slot_ft(feats.data_ptr(), tag, B, D, h, w, 1, 0, 2, dots.data_ptr(), s) == -2
-        assert L.pfst_proto_accum_ft(feats.data_ptr(), tag, B, D, h, w, lab.data_ptr(), _lib.DT_I64, h, w, None,
-                                     0.0, C, packed.data_ptr(), s) == -2
-        assert L.pfst_proto_accum_ordered_ft(feats.data_ptr(), tag, B, D, h, w, C, ws.data_ptr(),
-                                             packed.data_ptr(), s) == -2
+        assert L.pfst_pseudo_label(x.data_ptr(), tag, B, C, h * w, 0.5, None, 0, -1, lab.data_ptr(),
+                                   _lib.DT_I64, conf.data_ptr(), None, count.data_ptr(), s) == -2
+        assert L.pfst_neigh_dots_slot(feats.data_ptr(), tag, B, D, h, w, 1, 0, 2, dots.data_ptr(), s) == -2
+        assert L.pfst_proto_accum(feats.data_ptr(), tag, B, D, h, w, lab.data_ptr(), _lib.DT_I64, h, w, None,
+                                  0.0, C, packed.data_ptr(), s) == -2
+        assert L.pfst_proto_accum_ordered(feats.data_ptr(), tag, B, D, h, w, C, ws.data_ptr(),
+                                          packed.data_ptr(), s) == -2
     # an unknown label tag is refused as well
-    assert L.pfst_pseudo_label_ft(x.bfloat16().data_ptr(), _lib.DT_BF16, B, C, h * w, 0.5, None, 0, -1,
-                                  lab.data_ptr(), 7, conf.data_ptr(), None, count.data_ptr(), s) == -2
+    assert L.pfst_pseudo_label(x.bfloat16().data_ptr(), _lib.DT_BF16, B, C, h * w, 0.5, None, 0, -1,
+                               lab.data_ptr(), 7, conf.data_ptr(), None, count.data_ptr(), s) == -2
     torch.cuda.synchronize()
     assert int(packed.abs().sum()) == 0
 

@@ -156,8 +156,9 @@ def main():
         ploss = torch.empty(1, dtype=torch.float32, device=dev)
 
         def dist_fwd(i):
-            _lib.call("pfst_proto_dist_fwd", xs[i].data_ptr(), B, D, h, w, lab3.data_ptr(), H, W, mu.data_ptr(),
-                      bank.seen.data_ptr(), C, dist.data_ptr(), acc.data_ptr(), ploss.data_ptr(), ops._stream())
+            _lib.call("pfst_proto_dist_fwd", xs[i].data_ptr(), B, D, h, w, lab3.data_ptr(), _lib.DT_I64, H, W,
+                      mu.data_ptr(), bank.seen.data_ptr(), C, dist.data_ptr(), acc.data_ptr(), ploss.data_ptr(),
+                      ops._stream())
         report("proto_dist_fwd", 4 * D * p, dist_fwd)
         logits = inp["logits_trg"].to(dev)
         mix = (torch.rand((B, 1, H, W), generator=g) < 0.5).long().to(dev)
@@ -180,8 +181,8 @@ def main():
         report("neigh_grad_proto", 8 * D * p, lambda i: ops.neigh_grad(xs[i], coef, fd, out=grads[i], proto=pr))
 
         def dist_bwd(i):
-            _lib.call("pfst_proto_dist_bwd", xs[i].data_ptr(), B, D, h, w, lab3.data_ptr(), H, W, mu.data_ptr(),
-                      bank.seen.data_ptr(), C, dist.data_ptr(), acc.data_ptr(), gl.data_ptr(),
+            _lib.call("pfst_proto_dist_bwd", xs[i].data_ptr(), B, D, h, w, lab3.data_ptr(), _lib.DT_I64, H, W,
+                      mu.data_ptr(), bank.seen.data_ptr(), C, dist.data_ptr(), acc.data_ptr(), gl.data_ptr(),
                       grads[i].data_ptr(), 0, ops._stream())
         report("proto_dist_bwd", 8 * D * p, dist_bwd)
         del xs, grads
