@@ -446,7 +446,9 @@ int pfst_proto_dist_all(const float* feats, int64_t B, int32_t D, int32_t h, int
  *   grad_logits (nullable, (B,C,lh,lw), zeroed here) = d out2[0] / d logits
  * in ONE pass: the up-sampled logits are never materialised. Integer up-sampling factors
  * only (H = s*lh, W = s*lw). stats: device double[4] workspace (zeroed here).
- * labels: (B,H,W) of label_dtype (PFST_DT_I64 or PFST_DT_U8, else PFST_ERR_UNSUPPORTED).  */
+ * labels: (B,H,W) of label_dtype (PFST_DT_I64 or PFST_DT_U8, else PFST_ERR_UNSUPPORTED).
+ * labels and weight may start at any element alignment. B = 0 reads nothing (logits and
+ * labels may be null) and writes out2 = {NaN, 0}, the reference's mean and accuracy.       */
 int pfst_weighted_ce(const float* logits, const void* labels, int32_t label_dtype,
                      const float* weight, const float* class_weight, int64_t B, int32_t C,
                      int32_t lh, int32_t lw, int32_t H, int32_t W, int64_t ignore_index,

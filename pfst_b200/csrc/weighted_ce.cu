@@ -517,17 +517,24 @@ template <class L>
 static int weighted_ce(const float* logits, const L* labels, const float* weight, const float* class_weight,
                        int64_t B, int32_t C, int32_t lh, int32_t lw, int32_t H, int32_t W, int64_t ignore_index,
                        float loss_weight, float* grad_logits, double* stats, float* out2, void* stream) {
-  if (!logits || !labels || !stats || !out2 || B < 0 || C < 1 || lh < 1 || lw < 1 || H < 1 || W < 1)
+  // an empty batch reads nothing, so its (empty) tensors may have null data pointers
+  if ((B > 0 && (!logits || !labels)) || !stats || !out2 || B < 0 || C < 1 || lh < 1 || lw < 1 || H < 1 || W < 1)
     return PFST_ERR_INVALID_ARG;
   if (C > pfst::kCeMaxC || B > 65535) return PFST_ERR_UNSUPPORTED;
   // the fused kernel covers integer up-sampling factors (H/4 logits -> H in every shipped config)
   if (H % lh != 0 || W % lw != 0 || H / lh != W / lw) return PFST_ERR_UNSUPPORTED;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   PFST_CUDA_TRY(cudaMemsetAsync(stats, 0, 4 * sizeof(double), s), "pfst_weighted_ce/memset");
+  if (B == 0) {
+    // the reference's mean over no pixels is NaN (all-ones bytes are a NaN) and accuracy.py returns 0
+    // for an empty batch
+    PFST_CUDA_TRY(cudaMemsetAsync(out2, 0xff, sizeof(float), s), "pfst_weighted_ce/empty-loss");
+    PFST_CUDA_TRY(cudaMemsetAsync(out2 + 1, 0, sizeof(float), s), "pfst_weighted_ce/empty-acc");
+    return PFST_OK;
+  }
   if (grad_logits)
     PFST_CUDA_TRY(cudaMemsetAsync(grad_logits, 0, sizeof(float) * (size_t)B * C * lh * lw, s),
                   "pfst_weighted_ce/memset-grad");
-  if (B == 0) return PFST_OK;
   pfst::CeParams P{logits, labels, weight, class_weight, (int)B, C, lh, lw, H, W, H / lh,
                    ignore_index, loss_weight, grad_logits, stats, out2};
   // factor-4 up-sampling with few classes (every shipped config): cell-per-thread register kernel.
@@ -537,7 +544,11 @@ static int weighted_ce(const float* logits, const L* labels, const float* weight
   static const bool force_v1 = getenv("PFST_CE_V1") != nullptr;
   static const bool fast = getenv("PFST_CE_EXACT") == nullptr;
   static const int ty = getenv("PFST_CE_TY") ? atoi(getenv("PFST_CE_TY")) : 8;
-  const bool rows_ok = sizeof(L) == 8 || (reinterpret_cast<uintptr_t>(labels) & 1u) == 0;
+  // the factor-4 kernel reads a cell row of labels as two 16-byte (int64) or 2-byte (uint8) halves and
+  // its weights as float2 (every row offset is even), so it needs maps aligned to that; other views,
+  // such as a contiguous view at an odd storage offset, take the general kernel's scalar loads
+  const bool rows_ok = reinterpret_cast<uintptr_t>(labels) % (sizeof(L) == 8 ? 16 : 2) == 0 &&
+                       reinterpret_cast<uintptr_t>(weight) % 8 == 0;
   if (!force_v1 && C <= 8 && H == 4 * lh && W == 4 * lw && rows_ok) {
     const int TY = ty == 16 ? 16 : 8;
     const dim3 grid4((unsigned)((lw + pfst::kCeTile - 1) / pfst::kCeTile), (unsigned)((lh + TY - 1) / TY), (unsigned)B);

@@ -137,7 +137,6 @@ def test_weighted_ce_u8_equals_i64(cuda, C, factor, weighted, offset):
     lab = _labels(B, H, W, C, 4, cuda)[:, 0]
     w = torch.rand((B, H, W), generator=g).to(cuda) if weighted else None
     res = []
-    # the int64 rows stay 16-byte aligned: the int64 kernel's 16-byte row loads assume it
     for lab_ in (lab, _u8(lab, offset)):
         x = logits.clone().requires_grad_(True)
         loss, acc = upsample_cross_entropy(x, lab_, w)
