@@ -455,6 +455,29 @@ int pfst_weighted_ce(const float* logits, const void* labels, int32_t label_dtyp
                      float loss_weight, float* grad_logits, double* stats, float* out2,
                      void* stream);
 
+/* pfst_weighted_ce for logits of logit_dtype: PFST_DT_F32, or PFST_DT_F16 / PFST_DT_BF16 (a decode
+ * head run under autocast); any other tag returns PFST_ERR_UNSUPPORTED before any other argument
+ * check. pfst_weighted_ce(...) is pfst_weighted_ce_dt with PFST_DT_F32. The result is what mmseg's
+ * @force_fp32 losses compute on logits.float(): each logit is converted to fp32 once, on load
+ * (exact), so out2 and grad_logits equal the fp32 call's on the upcast logits (up to the order of
+ * the float atomics). grad_logits stays an fp32 buffer: pfst_scale_cast turns it into the logits'
+ * dtype. A 16-bit view may start at any element; it takes the same kernel as its fp32 upcast.
+ *
+ * pfst_scale_cast: dst[i] = (dst_dtype)(src[i] * *scale) for i < n, an IEEE fp32 product rounded
+ * ONCE to dst_dtype (PFST_DT_F32, PFST_DT_F16 or PFST_DT_BF16, round to nearest even; any other tag
+ * returns PFST_ERR_UNSUPPORTED before any other argument check). This is the backward of
+ * `loss(logits.float())`: the fp32 gradient times the upstream gradient, then the cast's backward.
+ * Rounding the gradient to 16 bits first and multiplying after would round twice. scale: device
+ * float[1] (the upstream gradient; read on the device, nothing synchronises). src, scale: 4-byte
+ * aligned; dst: aligned to its element. n = 0 reads and writes nothing (pointers may be null). */
+int pfst_weighted_ce_dt(const void* logits, int32_t logit_dtype, const void* labels,
+                        int32_t label_dtype, const float* weight, const float* class_weight,
+                        int64_t B, int32_t C, int32_t lh, int32_t lw, int32_t H, int32_t W,
+                        int64_t ignore_index, float loss_weight, float* grad_logits,
+                        double* stats, float* out2, void* stream);
+int pfst_scale_cast(const float* src, const float* scale, int64_t n, void* dst, int32_t dst_dtype,
+                    void* stream);
+
 /* ---- next row (SURVEY.md §8f rank 4): offline class-wise thresholds -------------------
  * Replaces PseudoLabelingHookV4._cal_threshold
  * (rsiseg/core/hook/pseudo_labeling_hookv4.py:173-205): for the n sampled pixels idx[] (row

@@ -16,9 +16,15 @@
 // per-class gradients privately; only the low-res tile (17*17*C values) goes to global
 // memory with atomics.
 // HBM-bound in principle: (8 + 4 [+4]) B per high-res pixel.
+// The logits may be fp32, fp16 or bf16 (a student run under autocast): every value is converted to
+// fp32 once, as the low-resolution tile is staged (exact), and all arithmetic after that is the fp32
+// code. The gradient is always accumulated and written in fp32; scale_cast_kernel turns it into the
+// logits' dtype in the backward.
 #include <float.h>
 #include <math.h>
 #include <stdlib.h>
+
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -30,8 +36,18 @@ constexpr int kCeThreads = kCeTile * kCeTile;
 constexpr int kCeMaxC = 64;
 constexpr int kCeRegC = 8;                       // up to this many classes the up-sampled logits stay in registers
 
+// The kernels' last template argument LT names the input types: a label type L (int64 or uint8) for fp32
+// logits, Lp<L, T> for logits of type T = __half or __nv_bfloat16. Both families are one templated
+// __global__ body each; the fp32 instantiations keep their names (weighted_ce_s4_kernel<6, ..., long>) and
+// the 16-bit ones are their twins (weighted_ce_s4_kernel<6, ..., pfst::Lp<long, __half>>).
+template <class L, class T> struct Lp {};
+template <class LT> struct CeTypes { using label = LT; using logit = float; };
+template <class L, class T> struct CeTypes<Lp<L, T>> { using label = L; using logit = T; };
+template <class L, class T>
+using CeIn = typename std::conditional<std::is_same<T, float>::value, L, Lp<L, T>>::type;
+
 struct CeParams {
-  const float* logits;       // (B, C, lh, lw)
+  const void* logits;        // (B, C, lh, lw), of the kernels' logits type T
   const void* labels;        // (B, H, W), int64 or uint8 (the kernels' L)
   const float* weight;       // (B, H, W) or null
   const float* class_weight; // (C) or null
@@ -58,9 +74,11 @@ __device__ __forceinline__ void ce_src(int dst, float scale, int in, int& i0, in
 // corners, so their per-class gradients are summed in a private shared-memory accumulator
 // ([class][corner][thread]: conflict-free, no atomics) and only four shared atomics per class and
 // thread fold them into the block's low-res tile; the tile goes to global memory once.
-template <bool REGC, bool PRIV, class L>
+template <bool REGC, bool PRIV, class LT>
 __global__ void __launch_bounds__(kCeThreads)
 weighted_ce_kernel(const CeParams P) {
+  using L = typename CeTypes<LT>::label;
+  using T = typename CeTypes<LT>::logit;
   extern __shared__ __align__(16) float ce_smem[];
   float* z_s = ce_smem;                                       // [C][kCeHalo*kCeHalo] low-res logits
   float* g_s = z_s + (size_t)P.C * kCeHalo * kCeHalo;           // same shape: gradient tile
@@ -69,11 +87,11 @@ weighted_ce_kernel(const CeParams P) {
   const int b = blockIdx.z;
   const int ly0 = blockIdx.y * kCeTile, lx0 = blockIdx.x * kCeTile;   // first cell of the tile
   const int64_t lplane = (int64_t)P.lh * P.lw;
-  const float* zb = P.logits + (int64_t)b * P.C * lplane;
+  const T* zb = static_cast<const T*>(P.logits) + (int64_t)b * P.C * lplane;
   for (int i = threadIdx.x; i < P.C * kCeHalo * kCeHalo; i += kCeThreads) {
     const int c = i / (kCeHalo * kCeHalo), r = i - c * (kCeHalo * kCeHalo);
     const int ly = ly0 + r / kCeHalo, lx = lx0 + r % kCeHalo;
-    z_s[i] = (ly < P.lh && lx < P.lw) ? zb[c * lplane + (int64_t)ly * P.lw + lx] : 0.f;
+    z_s[i] = (ly < P.lh && lx < P.lw) ? to_f32(zb[c * lplane + (int64_t)ly * P.lw + lx]) : 0.f;
     g_s[i] = 0.f;
   }
   if (P.grad && PRIV)
@@ -251,9 +269,11 @@ __device__ __forceinline__ float ex2_approx(float x) {
 
 // L = uint8: a cell row of 4 labels starts 2 pixels into a 4-pixel group (xb = 4 kx + 2), so it is
 // read as two 16-bit halves, as the int64 kernel reads two 16-byte halves (2-byte aligned rows).
-template <int CMAX, bool EXACT, bool FAST, bool GRAD, int TY, class L>
+template <int CMAX, bool EXACT, bool FAST, bool GRAD, int TY, class LT>
 __global__ void __launch_bounds__(kCeTile * TY, 512 / (kCeTile * TY))
 weighted_ce_s4_kernel(const CeParams P) {
+  using L = typename CeTypes<LT>::label;
+  using T = typename CeTypes<LT>::logit;
   extern __shared__ __align__(16) float ce_smem[];
   constexpr int NT = kCeTile * TY;                    // threads = cells of the tile (16 wide, TY tall)
   constexpr int HH = kCeHalo * (TY + 1);              // low-res points under the tile
@@ -264,7 +284,7 @@ weighted_ce_s4_kernel(const CeParams P) {
   const int b = blockIdx.z;
   const int ly0 = blockIdx.y * TY, lx0 = blockIdx.x * kCeTile;
   const int64_t lplane = (int64_t)P.lh * P.lw;
-  const float* zb = P.logits + (int64_t)b * C * lplane;
+  const T* zb = static_cast<const T*>(P.logits) + (int64_t)b * C * lplane;
   const int cy = threadIdx.x / kCeTile, cx = threadIdx.x % kCeTile;
   const int ky = ly0 + cy, kx = lx0 + cx;
   const bool active = ky < P.lh && kx < P.lw;
@@ -314,8 +334,8 @@ weighted_ce_s4_kernel(const CeParams P) {
     float t0[CMAX], t1[CMAX];
 #pragma unroll
     for (int c = 0; c < CMAX; ++c) {
-      t0[c] = c < C ? zb[c * lpl + o0] : 0.f;
-      t1[c] = (c < C && two) ? zb[c * lpl + o1] : 0.f;
+      t0[c] = c < C ? to_f32(zb[c * lpl + o0]) : 0.f;
+      t1[c] = (c < C && two) ? to_f32(zb[c * lpl + o1]) : 0.f;
     }
 #pragma unroll
     for (int c = 0; c < CMAX; ++c) {
@@ -513,8 +533,8 @@ weighted_ce_s4_kernel(const CeParams P) {
   }
 }
 
-template <class L>
-static int weighted_ce(const float* logits, const L* labels, const float* weight, const float* class_weight,
+template <class L, class T>
+static int weighted_ce(const T* logits, const L* labels, const float* weight, const float* class_weight,
                        int64_t B, int32_t C, int32_t lh, int32_t lw, int32_t H, int32_t W, int64_t ignore_index,
                        float loss_weight, float* grad_logits, double* stats, float* out2, void* stream) {
   // an empty batch reads nothing, so its (empty) tensors may have null data pointers
@@ -555,8 +575,9 @@ static int weighted_ce(const float* logits, const L* labels, const float* weight
     if (grid4.y > 65535) return PFST_ERR_UNSUPPORTED;
     const size_t smem4 = ((size_t)C * pfst::kCeHalo * (TY + 1) + (size_t)C * 4 * pfst::kCeTile * TY) * sizeof(float);
     void (*k4)(const pfst::CeParams);
+    using LT = pfst::CeIn<L, T>;
     const bool gr = grad_logits != nullptr;
-#define PFST_CE_PICK2(CM, EX, F, G) (TY == 16 ? pfst::weighted_ce_s4_kernel<CM, EX, F, G, 16, L> : pfst::weighted_ce_s4_kernel<CM, EX, F, G, 8, L>)
+#define PFST_CE_PICK2(CM, EX, F, G) (TY == 16 ? pfst::weighted_ce_s4_kernel<CM, EX, F, G, 16, LT> : pfst::weighted_ce_s4_kernel<CM, EX, F, G, 8, LT>)
 #define PFST_CE_PICK(CM, EX)                                                       \
   (fast ? (gr ? PFST_CE_PICK2(CM, EX, true, true) : PFST_CE_PICK2(CM, EX, true, false)) \
         : (gr ? PFST_CE_PICK2(CM, EX, false, true) : PFST_CE_PICK2(CM, EX, false, false)))
@@ -578,11 +599,64 @@ static int weighted_ce(const float* logits, const L* labels, const float* weight
   const bool use_priv = tile + priv <= 100 * 1024;          // keeps two blocks per SM
   const size_t smem = tile + (use_priv ? priv : 0);
   if (smem > 200 * 1024) return PFST_ERR_UNSUPPORTED;
-  auto k = C <= pfst::kCeRegC ? pfst::weighted_ce_kernel<true, true, L>
-                              : (use_priv ? pfst::weighted_ce_kernel<false, true, L> : pfst::weighted_ce_kernel<false, false, L>);
+  using LT = pfst::CeIn<L, T>;
+  auto k = C <= pfst::kCeRegC ? pfst::weighted_ce_kernel<true, true, LT>
+                              : (use_priv ? pfst::weighted_ce_kernel<false, true, LT> : pfst::weighted_ce_kernel<false, false, LT>);
   PFST_CUDA_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "pfst_weighted_ce/attr");
   k<<<grid, pfst::kCeThreads, smem, s>>>(P);
   PFST_CHECK_LAUNCH("pfst_weighted_ce");
+  return PFST_OK;
+}
+
+// ---- backward: the fp32 logits gradient times the upstream gradient, rounded once to the logits' dtype ----
+// dst[i] = (T)(src[i] * *scale), an IEEE fp32 product (__fmul_rn: never fused into anything) and a
+// round-to-nearest-even conversion: what autograd computes for `.float()` logits, where the upstream
+// gradient multiplies the fp32 gradient and the cast's backward rounds the product. For T = float it
+// is torch's `grad * grad_loss` bit for bit. `scale` stays on the device, so nothing waits for it.
+__device__ __forceinline__ float from_f32(float v, float) { return v; }
+__device__ __forceinline__ __half from_f32(float v, __half) { return __float2half_rn(v); }
+__device__ __forceinline__ __nv_bfloat16 from_f32(float v, __nv_bfloat16) { return __float2bfloat16_rn(v); }
+
+constexpr int kCastThreads = 256;
+
+// VEC: src 16-byte and dst 4-element aligned, four elements per thread and step; the elements past the
+// last whole group of four (and every element of an unaligned call) take the scalar loop
+template <class T, bool VEC>
+__global__ void __launch_bounds__(kCastThreads) scale_cast_kernel(const float* __restrict__ src,
+                                                                  const float* __restrict__ scale, int64_t n,
+                                                                  T* __restrict__ dst) {
+  const float k = *scale;
+  const int64_t stride = (int64_t)gridDim.x * kCastThreads;
+  const int64_t t0 = (int64_t)blockIdx.x * kCastThreads + threadIdx.x;
+  int64_t done = 0;
+  if (VEC) {
+    const int64_t n4 = n / 4;
+    for (int64_t i = t0; i < n4; i += stride) {
+      const float4 v = ldg_stream_f4(src + 4 * i);
+      using V = typename std::conditional<sizeof(T) == 4, float4, uint2>::type;   // four elements of T
+      alignas(sizeof(V)) const T r[4] = {from_f32(__fmul_rn(v.x, k), T{}), from_f32(__fmul_rn(v.y, k), T{}),
+                                         from_f32(__fmul_rn(v.z, k), T{}), from_f32(__fmul_rn(v.w, k), T{})};
+      *reinterpret_cast<V*>(dst + 4 * i) = *reinterpret_cast<const V*>(r);
+    }
+    done = 4 * n4;
+  }
+  for (int64_t i = done + t0; i < n; i += stride) dst[i] = from_f32(__fmul_rn(src[i], k), T{});
+}
+
+template <class T>
+static int scale_cast(const float* src, const float* scale, int64_t n, T* dst, void* stream) {
+  if (n < 0) return PFST_ERR_INVALID_ARG;
+  if (n == 0) return PFST_OK;                     // an empty gradient: nothing is read, pointers may be null
+  if (!src || !scale || !dst || !aligned4(src) || !aligned4(scale) ||
+      reinterpret_cast<uintptr_t>(dst) % sizeof(T) != 0)
+    return PFST_ERR_INVALID_ARG;
+  const bool vec = aligned16(src) && reinterpret_cast<uintptr_t>(dst) % (4 * sizeof(T)) == 0;
+  const int64_t work = vec ? (n + 3) / 4 : n;
+  const unsigned blocks = (unsigned)std::min<int64_t>((work + kCastThreads - 1) / kCastThreads, 16 * kNumSMs);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (vec) scale_cast_kernel<T, true><<<blocks, kCastThreads, 0, s>>>(src, scale, n, dst);
+  else scale_cast_kernel<T, false><<<blocks, kCastThreads, 0, s>>>(src, scale, n, dst);
+  PFST_CHECK_LAUNCH("pfst_scale_cast");
   return PFST_OK;
 }
 
@@ -590,13 +664,30 @@ static int weighted_ce(const float* logits, const L* labels, const float* weight
 
 extern "C" {
 
+int pfst_weighted_ce_dt(const void* logits, int32_t logit_dtype, const void* labels, int32_t label_dtype,
+                        const float* weight, const float* class_weight, int64_t B, int32_t C, int32_t lh, int32_t lw,
+                        int32_t H, int32_t W, int64_t ignore_index, float loss_weight, float* grad_logits,
+                        double* stats, float* out2, void* stream) {
+  return pfst::with_float_dt(logit_dtype, [&](auto t) {
+    return pfst::with_label_dt(label_dtype, [&](auto l) {
+      return pfst::weighted_ce(static_cast<const decltype(t)*>(logits), static_cast<const decltype(l)*>(labels),
+                               weight, class_weight, B, C, lh, lw, H, W, ignore_index, loss_weight, grad_logits,
+                               stats, out2, stream);
+    });
+  });
+}
+
 int pfst_weighted_ce(const float* logits, const void* labels, int32_t label_dtype, const float* weight,
                      const float* class_weight, int64_t B, int32_t C, int32_t lh, int32_t lw, int32_t H, int32_t W,
                      int64_t ignore_index, float loss_weight, float* grad_logits, double* stats, float* out2,
                      void* stream) {
-  return pfst::with_label_dt(label_dtype, [&](auto l) {
-    return pfst::weighted_ce(logits, static_cast<const decltype(l)*>(labels), weight, class_weight, B, C, lh, lw, H,
-                             W, ignore_index, loss_weight, grad_logits, stats, out2, stream);
+  return pfst_weighted_ce_dt(logits, PFST_DT_F32, labels, label_dtype, weight, class_weight, B, C, lh, lw, H, W,
+                             ignore_index, loss_weight, grad_logits, stats, out2, stream);
+}
+
+int pfst_scale_cast(const float* src, const float* scale, int64_t n, void* dst, int32_t dst_dtype, void* stream) {
+  return pfst::with_float_dt(dst_dtype, [&](auto t) {
+    return pfst::scale_cast(src, scale, n, static_cast<decltype(t)*>(dst), stream);
   });
 }
 

@@ -6,9 +6,15 @@
 The reference up-samples the (B,C,H/4,W/4) logits to (B,C,H,W), takes a log-softmax, gathers,
 multiplies by the pixel weights, averages over all pixels and computes the top-1 accuracy —
 about ten ATen kernels moving the 50 MB up-sampled tensor several times, forward and backward.
-`pfst_weighted_ce` (csrc/weighted_ce.cu) does all of it in one pass over the low-resolution
+`pfst_weighted_ce_dt` (csrc/weighted_ce.cu) does all of it in one pass over the low-resolution
 logits, labels and weights, and also leaves d loss / d logits behind, so the backward is a scalar
 multiply.
+
+The logits may be fp32, fp16 or bf16 (a decode head run under autocast). The result is what mmseg's
+`@force_fp32(apply_to=('seg_logit',))` losses compute on `seg_logit.float()`: the loss and the accuracy
+are fp32 and equal the fp32 path's on the upcast logits, and the logits' gradient has their dtype and
+equals the fp32 gradient times the upstream gradient, rounded once (`pfst_scale_cast`). There is no
+`.float()` copy in the forward and no multiply-and-cast pair in the backward.
 """
 from __future__ import annotations
 
@@ -18,6 +24,9 @@ import torch
 
 from .. import _lib, ops
 from .._lib import PfstError
+
+
+LOGIT_DTYPES = (torch.float32, torch.float16, torch.bfloat16)
 
 
 class _UpsampleCE(torch.autograd.Function):
@@ -30,15 +39,19 @@ class _UpsampleCE(torch.autograd.Function):
                             "up-sampling factor (unsupported resampling)")
         dev = seg_logit.device
         need_grad = seg_logit.requires_grad
-        grad = torch.empty_like(seg_logit) if need_grad else None
+        # the gradient is accumulated in fp32 whatever the logits' dtype; the backward rounds it once
+        grad = torch.empty_like(seg_logit, dtype=torch.float32) if need_grad else None
         stats = torch.empty(4, dtype=torch.float64, device=dev)
         out2 = torch.empty(2, dtype=torch.float32, device=dev)
-        _lib.call("pfst_weighted_ce", ops._dev(seg_logit, "seg_logit", torch.float32),
+        tag = ops._FLOAT2DT[seg_logit.dtype]
+        _lib.call("pfst_weighted_ce_dt", ops._dev(seg_logit, "seg_logit"), tag,
                   labels.data_ptr(), ops._labels(labels, "seg_label"), ops._opt(seg_weight, "seg_weight", torch.float32),
                   ops._opt(class_weight, "class_weight", torch.float32), B, C, lh, lw, H, W, int(ignore_index),
                   float(loss_weight), None if grad is None else grad.data_ptr(), stats.data_ptr(), out2.data_ptr(),
                   ops._stream())
         ctx.save_for_backward(grad)
+        ctx.logit_dtype = seg_logit.dtype
+        ctx.set_materialize_grads(False)            # acc_seg has no gradient: no zero tensor is filled for it
         loss, acc = out2[0], out2[1:2]
         ctx.mark_non_differentiable(acc)
         return loss, acc
@@ -46,14 +59,27 @@ class _UpsampleCE(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_loss, _grad_acc):
         (grad,) = ctx.saved_tensors
-        return (None if grad is None else grad * grad_loss), None, None, None, None, None
+        if grad is None or grad_loss is None:
+            return None, None, None, None, None, None
+        if ctx.logit_dtype == torch.float32:        # the same bits as pfst_scale_cast, less host time per call
+            return grad * grad_loss, None, None, None, None, None
+        # 16-bit logits: (fp32 gradient * upstream) rounded once to their dtype, in one launch
+        scale = grad_loss.float()
+        out = torch.empty(grad.shape, dtype=ctx.logit_dtype, device=grad.device)
+        _lib.call("pfst_scale_cast", grad.data_ptr(), scale.data_ptr(), grad.numel(), out.data_ptr(),
+                  ops._FLOAT2DT[ctx.logit_dtype], ops._stream())
+        return out, None, None, None, None, None
 
 
 def upsample_cross_entropy(seg_logit: torch.Tensor, seg_label: torch.Tensor, seg_weight: Optional[torch.Tensor] = None,
                            class_weight: Optional[torch.Tensor] = None, ignore_index: int = 255,
                            loss_weight: float = 1.0):
-    """-> (loss 0-dim, acc_seg (1,)). seg_logit (B,C,lh,lw) fp32; seg_label (B,1,H,W) or (B,H,W) int64 or uint8;
-    seg_weight (B,H,W) fp32 or None; class_weight (C,) fp32 or None."""
+    """-> (loss 0-dim fp32, acc_seg (1,) fp32). seg_logit (B,C,lh,lw) fp32, fp16 or bf16 (its gradient has its
+    dtype); seg_label (B,1,H,W) or (B,H,W) int64 or uint8; seg_weight (B,H,W) fp32 or None; class_weight (C,)
+    fp32 or None."""
+    if isinstance(seg_logit, torch.Tensor) and seg_logit.dtype not in LOGIT_DTYPES:
+        raise TypeError(f"seg_logit: decode-head logits must be torch.float32, torch.float16 or torch.bfloat16, "
+                        f"got {seg_logit.dtype}")
     if seg_label.dim() == 4:
         seg_label = seg_label[:, 0]
     seg_logit = seg_logit.contiguous()

@@ -52,8 +52,9 @@ def _labels(t: torch.Tensor, name: str, like: Optional[torch.Tensor] = None) -> 
 
 
 # The EMA teacher's outputs (pseudo-label logits, features) may come from a pass run under autocast; the
-# kernels that read them take fp32, fp16 or bf16 (converted to fp32 on load, exactly). Everything that
-# carries a gradient (the student's logits and features) stays fp32.
+# kernels that read them take fp32, fp16 or bf16 (converted to fp32 on load, exactly). The student's logits
+# and features given to the self-training step and PFGSTLoss stay fp32; only the decode-head loss
+# (losses/cross_entropy.py) also takes 16-bit student logits.
 TEACHER_DTYPES = (torch.float32, torch.float16, torch.bfloat16)
 _FLOAT2DT = {torch.float32: _lib.DT_F32, torch.float16: _lib.DT_F16, torch.bfloat16: _lib.DT_BF16}
 
