@@ -478,6 +478,34 @@ int pfst_weighted_ce_dt(const void* logits, int32_t logit_dtype, const void* lab
 int pfst_scale_cast(const float* src, const float* scale, int64_t n, void* dst, int32_t dst_dtype,
                     void* stream);
 
+/* ---- OHEM pixel sampler of the decode-head loss ------------------------------------------
+ * mmseg 0.x OHEMPixelSampler.sample(seg_logit, seg_label), whose map replaces seg_weight in
+ * BaseDecodeHead.losses (decode_head.py:249-283), with seg_logit the bilinear (align_corners=False)
+ * up-sampling of logits (B,C,lh,lw) to the labels' (H,W) by an integer factor s >= 1 (H = s*lh,
+ * W = s*lw; s = 1 is the sampler on already up-sampled logits). valid = label != ignore_index (and in
+ * [0, C)), n = #valid, batch_kept = min_kept * B:
+ *   thresh not NaN: key = softmax(up)[label] (fp32); kth = k-th smallest valid key, k = min(batch_kept,
+ *                   n - 1) (0 when n == 0); weight = valid & (key < max(kth, thresh)), where thresh wins
+ *                   only if it is larger (Python's max(min_threshold, thresh));
+ *   thresh NaN:     key = loss_weight * class_weight[label] * CE(up, label) (0 at ignored pixels); kth =
+ *                   the batch_kept-th largest valid key (the smallest when batch_kept >= n); the
+ *                   min(batch_kept, n) valid pixels with the largest keys get weight 1, and at a tie on
+ *                   kth the lower flat index goes first (a stable descending sort).
+ * Keys order as torch.sort orders them: NaN after every number. The up-sampled logits are never
+ * materialised and nothing synchronises the host: the order statistic is an exact radix select whose
+ * rank is read from the device count. logits: logit_dtype PFST_DT_F32 / F16 / BF16; labels (B,H,W):
+ * label_dtype PFST_DT_I64 / PFST_DT_U8 (an unknown tag returns PFST_ERR_UNSUPPORTED before any other
+ * check). class_weight: (C) fp32 or NULL. min_kept >= 2 (mmseg asserts min_kept > 1).
+ * workspace: pfst_ohem_ws_bytes(B, H, W) bytes, 16-byte aligned. Outputs: weight_out (B,H,W) fp32 0/1;
+ * keys_out (B,H,W) fp32 or NULL (ignored pixels: softmax(up)[0] with a thresh, 0 without); kth_out
+ * device float[1] or NULL. B = 0 reads nothing, writes kth_out = 0 (logits, labels, weight_out may be
+ * NULL); no valid pixel gives a zero map. B*H*W and C*lh*lw must be below 2^31. */
+int64_t pfst_ohem_ws_bytes(int64_t B, int32_t H, int32_t W);
+int pfst_ohem_weight(const void* logits, int32_t logit_dtype, const void* labels, int32_t label_dtype,
+                     const float* class_weight, int64_t B, int32_t C, int32_t lh, int32_t lw, int32_t H,
+                     int32_t W, int64_t ignore_index, float loss_weight, float thresh, int64_t min_kept,
+                     void* workspace, float* keys_out, float* kth_out, float* weight_out, void* stream);
+
 /* ---- next row (SURVEY.md §8f rank 4): offline class-wise thresholds -------------------
  * Replaces PseudoLabelingHookV4._cal_threshold
  * (rsiseg/core/hook/pseudo_labeling_hookv4.py:173-205): for the n sampled pixels idx[] (row

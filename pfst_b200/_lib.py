@@ -69,6 +69,9 @@ SIGNATURES: dict[str, tuple] = {
     "pfst_weighted_ce_dt": (C.c_int, [_vp, _i32, _vp, _i32, _vp, _vp, _i64, _i32, _i32, _i32, _i32, _i32, _i64,
                                       _f32, _vp, _vp, _vp, _vp]),
     "pfst_scale_cast": (C.c_int, [_vp, _vp, _i64, _vp, _i32, _vp]),
+    "pfst_ohem_ws_bytes": (_i64, [_i64, _i32, _i32]),
+    "pfst_ohem_weight": (C.c_int, [_vp, _i32, _vp, _i32, _vp, _i64, _i32, _i32, _i32, _i32, _i32, _i64, _f32, _f32,
+                                   _i64, _vp, _vp, _vp, _vp, _vp]),
     "pfst_proto_accum_is_masked": (C.c_int, [_i32, _i32, _i32]),
     "pfst_proto_accum": (C.c_int, [_vp, _i32, _i64, _i32, _i32, _i32, _vp, _i32, _i32, _i32, _vp, _f32, _i32, _vp,
                                    _vp]),

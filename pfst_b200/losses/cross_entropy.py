@@ -96,11 +96,16 @@ def upsample_cross_entropy(seg_logit: torch.Tensor, seg_label: torch.Tensor, seg
 
 
 def decode_head_losses(seg_logit, seg_label, seg_weight=None, *, ignore_index: int = 255, loss_weight: float = 1.0,
-                       class_weight=None, align_corners: bool = False, loss_name: str = "loss_ce") -> dict:
-    """Body of BaseDecodeHead.losses (decode_head.py:249-283) for the shipped configuration
-    (one CrossEntropyLoss, no OHEM sampler): {loss_name: loss, 'acc_seg': accuracy}."""
+                       class_weight=None, align_corners: bool = False, loss_name: str = "loss_ce",
+                       sampler=None) -> dict:
+    """Body of BaseDecodeHead.losses (decode_head.py:249-283) with one CrossEntropyLoss:
+    {loss_name: loss, 'acc_seg': accuracy}. sampler: the head's pixel sampler (an OHEMPixelSampler) or None;
+    as in the reference its map replaces seg_weight. It is computed from the low-resolution seg_logit on the
+    device (pfst_ohem_weight) and fed to the fused loss."""
     if align_corners:
         raise PfstError("decode_head_losses: align_corners=True is not covered by the fused kernel "
                         "(every shipped config uses align_corners=False)")
+    if sampler is not None:
+        seg_weight = sampler.weight_map(seg_logit, seg_label)
     loss, acc = upsample_cross_entropy(seg_logit, seg_label, seg_weight, class_weight, ignore_index, loss_weight)
     return {loss_name: loss, "acc_seg": acc}

@@ -455,6 +455,61 @@ def gaussian_blur(data: torch.Tensor, sigmas: Sequence[float], kernel_size: Opti
     return out
 
 
+# ------------------------------------------------------- OHEM pixel sampler
+def ohem_weight(seg_logit: torch.Tensor, seg_label: torch.Tensor, *, thresh: Optional[float] = None,
+                min_kept: int = 100000, ignore_index: int = 255, class_weight: Optional[torch.Tensor] = None,
+                loss_weight: float = 1.0, want_keys: bool = False):
+    """mmseg OHEMPixelSampler.sample on the bilinear (align_corners=False) up-sampling of seg_logit (B,C,lh,lw;
+    fp32, fp16 or bf16) to the size of seg_label ((B,1,H,W) or (B,H,W), int64 or uint8), an integer factor
+    H/lh = W/lw >= 1. thresh None: the min_kept * B valid pixels of largest loss_weight * class_weight[label] *
+    CE (ties at the boundary: lower flat index first); otherwise the valid pixels whose soft-max probability of
+    their label is below max(k-th smallest of those, thresh). -> (weight (B,H,W) fp32 0/1, kth (1,) fp32 on the
+    device: the order statistic the threshold came from, keys (B,H,W) fp32 or None)."""
+    if int(min_kept) <= 1:
+        raise ValueError(f"min_kept must be > 1 (mmseg OHEMPixelSampler), got {min_kept}")
+    if isinstance(seg_logit, torch.Tensor) and seg_logit.dtype not in _FLOAT2DT:
+        raise TypeError(f"seg_logit: logits must be torch.float32, torch.float16 or torch.bfloat16, "
+                        f"got {seg_logit.dtype}")
+    _dev(seg_logit, "seg_logit")
+    if seg_logit.dim() != 4:
+        raise ValueError("seg_logit must be (B,C,lh,lw)")
+    if seg_label.dim() == 4:
+        if seg_label.shape[1] != 1:
+            raise ValueError("seg_label must be (B,1,H,W) or (B,H,W)")
+        seg_label = seg_label[:, 0]
+    _labels(seg_label, "seg_label")
+    B, Cn, lh, lw = seg_logit.shape
+    if seg_label.dim() != 3 or seg_label.shape[0] != B:
+        raise ValueError("seg_label must hold one (H,W) map per image of seg_logit")
+    H, W = seg_label.shape[-2:]
+    if lh < 1 or lw < 1 or H % lh or W % lw or H // lh != W // lw:
+        raise PfstError(f"ohem_weight: {lh}x{lw} logits -> {H}x{W} labels is not an integer up-sampling factor "
+                        "(unsupported resampling)")
+    if class_weight is not None:
+        _dev(class_weight, "class_weight", torch.float32)
+        if class_weight.numel() != Cn:
+            raise ValueError("class_weight must have one entry per class")
+    dev = seg_logit.device
+    weight = torch.empty((B, H, W), dtype=torch.float32, device=dev)
+    kth = torch.empty(1, dtype=torch.float32, device=dev)
+    keys = torch.empty((B, H, W), dtype=torch.float32, device=dev) if want_keys else None
+    ws = torch.empty(max(int(_lib.load().pfst_ohem_ws_bytes(B, H, W)), 16), dtype=torch.uint8, device=dev)
+    launch_ohem_weight(seg_logit, seg_label, class_weight, ignore_index, loss_weight, thresh, min_kept, ws, keys, kth,
+                       weight, _stream())
+    return weight, kth, keys
+
+
+def launch_ohem_weight(seg_logit, seg_label, class_weight, ignore_index, loss_weight, thresh, min_kept, ws, keys, kth,
+                       weight, stream) -> None:
+    """seg_label (B,H,W); thresh None selects the top-k mode (a NaN thresh in the C ABI)."""
+    B, Cn, lh, lw = seg_logit.shape
+    H, W = seg_label.shape[-2:]
+    _lib.call("pfst_ohem_weight", seg_logit.data_ptr(), _FLOAT2DT[seg_logit.dtype], seg_label.data_ptr(),
+              _TORCH2DT[seg_label.dtype], _ptr(class_weight), B, Cn, lh, lw, H, W, int(ignore_index),
+              float(loss_weight), float("nan") if thresh is None else float(thresh), int(min_kept), ws.data_ptr(),
+              _ptr(keys), _ptr(kth), weight.data_ptr(), stream)
+
+
 # ------------------------------------------------------------ L1-L6: PFGST loss
 def neigh_dots(x_a: torch.Tensor, x_b: Optional[torch.Tensor], dilation: int):
     """-> (dots float32 (splits, T, B, 5, h, w), splits). x_a / x_b: fp32, fp16 or bf16. Two fp32 tensors

@@ -46,10 +46,16 @@ UDA = MODELS
 LOSSES = MODELS
 SEGMENTORS = MODELS
 PIPELINES = Registry("pipeline")       # rsiseg/datasets/builder.py: PIPELINES = Registry('pipeline')
+PIXEL_SAMPLERS = Registry("pixel sampler")   # mmseg/core/builder.py: PIXEL_SAMPLERS = Registry('pixel sampler')
 
 
 def build_loss(cfg):
     return LOSSES.build(cfg)
+
+
+def build_pixel_sampler(cfg, **default_args):
+    """mmseg's builder: a decode head calls build_pixel_sampler(self.sampler_cfg, context=self)."""
+    return PIXEL_SAMPLERS.build(cfg, **default_args)
 
 
 def build_segmentor(cfg, train_cfg=None, test_cfg=None):
